@@ -2,6 +2,7 @@
 """bench.py -- haplotype bp/s (one-hot) of the B200-native path, with roofline, CPU baseline, API and e2e legs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg3|cfg2|cfg1|cfg4|...]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over ONE batch of synthetic (region, sample) pairs: device-side batch prep,
@@ -18,6 +19,7 @@ Printed JSON line (rank 0): the driver's contract + `roofline`, `cpu_baseline`, 
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -129,6 +131,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100",
                                        "-i", str(self.idx)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)  # a run that fails before stop() does not leave the sampler behind
         except Exception:
             self.p = None
 
@@ -179,6 +182,43 @@ def alg_bytes(w, nvar: float, mode: str = "onehot", n_batches: int = 1) -> float
 def track_bytes(w, n_tracks: int) -> float:
     """4 B per realigned value written (SURVEY.md 8d; the intervals read add 12 B each, not counted)."""
     return 4.0 * n_tracks * w["pairs"] * 2 * w["window"]
+
+
+DUMP_BYTES = 64_000_000  # all files of one --dump-outputs, .npy headers included
+NPY_HEADER_BYTES = 256
+
+
+def dump_outputs(out_dir: Path, result, mode: str, budget: int = DUMP_BYTES, seed: int = 0) -> dict:
+    """Write one batch as a caller of the pipeline receives it (`FixedPipeline` / `Dataset.to_dataloader`) to
+    `out_dir/<name>.npy`: `haplotypes` (or `haps`, `var_idxs`, `ref_coords` when annotated) and `tracks` when realigned
+    tracks are on.  uint8 and float32 outputs are written as float32, int32 ones as float64 (exact).  When the files would
+    take more than `budget` bytes, every array keeps the same seeded sample of window positions (sorted), all other axes whole.
+    Returns {name: written shape}."""
+    import torch
+
+    seq, tracks = result if isinstance(result, tuple) else (result, None)
+    if mode == "annotated":
+        arrays = {"haps": (seq.haps, -1), "var_idxs": (seq.var_idxs, -1), "ref_coords": (seq.ref_coords, -1)}
+    else:
+        arrays = {"haplotypes": (seq, -2 if mode == "onehot" else -1)}
+    if tracks is not None:
+        arrays["tracks"] = (tracks, -1)
+    dtypes = {k: np.float64 if t.dtype in (torch.int32, torch.int64) else np.float32 for k, (t, _) in arrays.items()}
+    L = {t.shape[ax] for t, ax in arrays.values()}.pop()
+    per_pos = sum(t.numel() // L * np.dtype(dtypes[k]).itemsize for k, (t, _) in arrays.items())
+    keep = max(1, min(L, (budget - NPY_HEADER_BYTES * len(arrays)) // per_pos))
+    pos = None
+    if keep < L:
+        pos = np.sort(np.random.default_rng(seed).choice(L, keep, replace=False))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    shapes = {}
+    for k, (t, ax) in arrays.items():
+        if pos is not None:
+            t = t.index_select(ax % t.dim(), torch.from_numpy(pos).to(t.device))
+        a = t.cpu().numpy().astype(dtypes[k])
+        np.save(out_dir / f"{k}.npy", a)
+        shapes[k] = a.shape
+    return shapes
 
 
 # ----------------------------------------------------------------------------------------------
@@ -385,29 +425,41 @@ def run_b200(args):
         torch.cuda.synchronize()
         return e0.elapsed_time(e1)  # ms
 
-    def measure(pl, min_ms=60.0, max_rep=400):
-        for _ in range(max(1, -(-max(args.warmup, 3) // args.steps))):
-            timed_block(pl)
-        first = timed_block(pl)
-        reps = int(min(max_rep, max(5, np.ceil(min_ms / max(first, 1e-3))))) if first * 1 < min_ms else 1
-        if dist is not None:  # same repeat count on every rank (the blocks contain barriers)
-            t = torch.tensor([reps], device=dev)
+    def measure(pl, warm_ms=60.0, max_warm=400):
+        """Warm-up blocks (at least `--warmup` steps, and about `warm_ms` of device time so that clocks and caches are in
+        steady state), then ONE timed block: exactly `--steps` steps.  The timed block starts from the first resident index
+        set whatever the warm-up did, so its inputs, and what its last step computes, are the same from run to run."""
+        n_warm = max(1, -(-max(args.warmup, 3) // args.steps))
+        last = 0.0
+        for _ in range(n_warm):
+            last = timed_block(pl)
+        more = max(0, int(min(max_warm, np.ceil(warm_ms / max(last, 1e-3)))) - n_warm)
+        if dist is not None:  # same block count on every rank (the blocks contain barriers)
+            t = torch.tensor([more], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            reps = int(t.item())
-        times = [first] + [timed_block(pl) for _ in range(reps - 1)]
-        if dist is not None:  # max over ranks, block by block
-            t = torch.tensor(times, device=dev, dtype=torch.float64)
+            more = int(t.item())
+        for _ in range(more):
+            timed_block(pl)
+        set_i[0] = 0
+        ms = timed_block(pl)
+        if dist is not None:  # the slowest rank
+            t = torch.tensor([ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             per_rank = [torch.zeros(1, device=dev, dtype=torch.float64) for _ in range(world)]
-            dist.all_gather(per_rank, torch.tensor([float(np.median(times))], device=dev, dtype=torch.float64))
-            return [float(x) for x in t.tolist()], [float(x.item()) for x in per_rank]
-        return times, [float(np.median(times))]
+            dist.all_gather(per_rank, torch.tensor([ms], device=dev, dtype=torch.float64))
+            return float(t.item()), [float(x.item()) for x in per_rank], n_warm + more
+        return ms, [ms], n_warm + more
+
+    def last_step(pl):
+        """What the last step of the timed block returned to its caller: batch `ring - 1` of the last device call."""
+        return pl.halves[(n_sub - 1) % pl.n_halves].out.result((ring - 1) * pairs, pairs)
 
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    times, per_rank_ms = measure(pipe)
-    ms = float(np.median(times))
+    ms, per_rank_ms, warm_blocks = measure(pipe)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_step(pipe), mode)
     value = world * args.steps * bp_per_step / (ms * 1e-3)
     launches = pipe.launches_per_ring * n_sub
 
@@ -461,8 +513,7 @@ def run_b200(args):
                       r * 2 * bp_per_step * (4 + 4 * nt) <= args.ring_gib * (1 << 30)), default=1)
         if ring_t == ring:
             pipe_t = FixedPipeline(dst, pairs, ring=ring_t)
-            t_times, _ = measure(pipe_t, min_ms=40.0, max_rep=100)
-            t_ms = float(np.median(t_times))
+            t_ms, _, _ = measure(pipe_t, warm_ms=40.0, max_warm=100)
             tb = alg_bytes(w, nvar_per_step, mode) + track_bytes(w, nt)
             tracks_line = {"n_tracks": nt, "value": world * args.steps * bp_per_step / (t_ms * 1e-3), "unit": "bp/s",
                            "ms_per_step": t_ms / args.steps, "track_values_per_s": world * args.steps * nt * bp_per_step / (t_ms * 1e-3),
@@ -615,7 +666,7 @@ def run_b200(args):
     # `config` is identical in both arms (the driver compares them); how THIS arm runs the workload goes to `pipeline`
     cfg = workload_config(args.workload, w, host_batches(d, w, 1, args.seed + 1)[0]["nvar"], mode, n_tracks_main)
     pipeline = {"batches_per_device_call": ring, "device_calls_per_timed_block": n_sub, "halves": pipe.n_halves,
-                "cuda_graph": pipe.use_graph, "repeats": len(times), "launches_per_device_call": pipe.launches_per_ring,
+                "cuda_graph": pipe.use_graph, "warmup_blocks": warm_blocks, "launches_per_device_call": pipe.launches_per_ring,
                 "l2": f"{n_sets} resident index sets over {d.n_regions} regions of a {w['contig_len'] / 1e6:.0f} Mb contig (packed reference "
                       f"{w['contig_len'] / 2e6:.0f} MB); every device call writes {ring * out_bytes_step >> 20} MiB into its half "
                       "(> 126 MB L2 per call)",
@@ -624,9 +675,7 @@ def run_b200(args):
         "metric": "haplotype bp/s (%s)" % {"onehot": "one-hot", "u8": "uint8 bytes", "annotated": "annotated"}[mode],
         "value": value, "unit": "bp/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8",
-        "data": "synthetic", "config": cfg, "pipeline": pipeline, "repeats": len(times),
-        "timed_block_ms": {"median": ms, "min": float(np.min(times)), "max": float(np.max(times))},
-        "per_rank_ms": per_rank_ms,
+        "data": "synthetic", "config": cfg, "pipeline": pipeline, "timed_block_ms": ms, "per_rank_ms": per_rank_ms,
         "output_GBps": value * {"onehot": 4, "u8": 1, "annotated": 9}[mode] / 1e9, "algorithmic_GBps": step_achieved * world,
         "whole_step_frac": step_achieved / peak,
         "roofline": {"bound": "hbm", "kernel": kernel_name, "achieved": achieved, "peak": peak, "unit": "GB/s",
@@ -656,6 +705,7 @@ def run_b200(args):
 
 
 def main():
+    sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree (it may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=640)
@@ -670,7 +720,12 @@ def main():
     ap.add_argument("--ring-gib", type=float, default=12.0, help="output memory of the two ring halves, at most")
     ap.add_argument("--no-tracks", action="store_true", help="skip the cfg3t extra leg")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", type=Path, metavar="DIR",
+                    help="write the last timed step's batch to DIR/<name>.npy (float32 / float64, at most 64 MB: a fixed "
+                         "seeded sample of window positions when larger); the same arguments give the same arrays")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -38,11 +38,11 @@ _LIB = _HERE / f"libgvl_oracle_{_cpu_tag()}.so"
 _CFLAGS = ["-O3", "-march=native", "-ffp-contract=off", "-fPIC", "-shared", "-pthread"]
 
 
-def build(force: bool = False) -> Path:
+def build(force: bool = False, out: Path = _LIB) -> Path:
     """Compile the C restatement (gcc only; no reference sources involved)."""
-    if force or not _LIB.exists() or _LIB.stat().st_mtime < _SRC.stat().st_mtime:
-        subprocess.check_call(["gcc", *_CFLAGS, "-o", str(_LIB), str(_SRC)])
-    return _LIB
+    if force or not out.exists() or out.stat().st_mtime < _SRC.stat().st_mtime:
+        subprocess.check_call(["gcc", *_CFLAGS, "-o", str(out), str(_SRC)])
+    return out
 
 
 _lib = None
@@ -51,12 +51,19 @@ _lib = None
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        try:
-            build()
-        except Exception:
-            if not _LIB.exists():
-                raise
-        _lib = C.CDLL(str(_LIB))
+        path = _LIB
+        if not _LIB.exists() and not os.access(_HERE, os.W_OK):
+            # read-only source tree and no library for this CPU yet: compile into a temporary directory
+            import tempfile
+
+            path = build(out=Path(tempfile.mkdtemp(prefix="gvl_oracle_")) / _LIB.name)
+        else:
+            try:
+                build()
+            except Exception:
+                if not _LIB.exists():
+                    raise
+        _lib = C.CDLL(str(path))
         _lib.gvl_oracle_xorshift64.restype = C.c_uint64
         _lib.gvl_oracle_xorshift64.argtypes = [C.c_uint64]
         _lib.gvl_oracle_hash4.restype = C.c_uint64

@@ -1,8 +1,8 @@
 """Golden vectors for the `variants` cores produced by EXECUTING the reference's own pure-numpy twins.
 
-Run in the BUILD container only (needs /root/reference):
+Needs a checkout of the original GenVarLoader project:
 
-    python tests/golden/make_pyref_variants_golden.py
+    python tests/golden/make_pyref_variants_golden.py <genvarloader checkout>
 
 The reference keeps dtype-preserving numpy fallbacks next to its Rust cores (python/genvarloader/_dataset/_flat_variants.py:
 `_gather_rows_numpy` :545, `_compact_keep_numpy` :567, `_fill_empty_scalar_numpy` :624, `_fill_empty_seq_numpy` :660,
@@ -21,7 +21,9 @@ from pathlib import Path
 
 import numpy as np
 
-REF = Path("/root/reference/python/genvarloader/_dataset")
+REF_SUBDIR = Path("python/genvarloader/_dataset")
+# no fixture file may exceed 1 MB: `fill_empty_seq` keeps only the cases of at most this many bytes (71 of 80)
+MAX_CASE_BYTES = {"fill_empty_seq": 100_000}
 DST = Path(__file__).parent
 
 
@@ -35,6 +37,9 @@ def _lift(path: Path, names: set) -> dict:
 
 
 def _save(name: str, cases: list) -> None:
+    cap = MAX_CASE_BYTES.get(name)
+    if cap is not None:
+        cases = [c for c in cases if sum(np.asarray(a).nbytes for a in (*c[0], *c[1])) <= cap]
     out = {"n_cases": np.array(len(cases), np.int64), "n_args": np.array(len(cases[0][0]), np.int64),
            "n_gold": np.array(len(cases[0][1]), np.int64)}
     for ci, (args, gold) in enumerate(cases):
@@ -56,10 +61,10 @@ def _offsets(rng, n, max_len, empty_frac):
     return np.concatenate([[0], np.cumsum(ln)]).astype(np.int64)
 
 
-def main() -> None:
-    fv = _lift(REF / "_flat_variants.py", {"_gather_rows_numpy", "_compact_keep_numpy", "_fill_empty_scalar_numpy",
+def main(ref: Path) -> None:
+    fv = _lift(ref / "_flat_variants.py", {"_gather_rows_numpy", "_compact_keep_numpy", "_fill_empty_scalar_numpy",
                                            "_fill_empty_seq_numpy", "_fill_empty_fixed_numpy"})
-    ff = _lift(REF / "_flat_flanks.py", {"build_token_lut", "_slice_flanks", "_assemble_alt_windows"})
+    ff = _lift(ref / "_flat_flanks.py", {"build_token_lut", "_slice_flanks", "_assemble_alt_windows"})
     rng = np.random.default_rng(20260)
     gather, compact, fscalar, fseq, ffixed, alt_win = [], [], [], [], [], []
     for ci in range(40):
@@ -108,6 +113,7 @@ def main() -> None:
 
 
 if __name__ == "__main__":
-    if not REF.is_dir():
-        sys.exit("needs /root/reference (build container only)")
-    main()
+    ref = Path(sys.argv[1]) / REF_SUBDIR if len(sys.argv) > 1 else None
+    if ref is None or not ref.is_dir():
+        sys.exit("usage: make_pyref_variants_golden.py <genvarloader checkout>")
+    main(ref)
