@@ -172,6 +172,8 @@ class FixedPipeline:
     """See the module docstring.  `batch_size` = queries per logical batch, `ring` = batches per device call (0: eager
     single batches only), `halves` = ring buffers produced alternately."""
 
+    fused = True  # a device call of a ring half is one graph on one stream (bench.py reads this)
+
     def __init__(self, ds, batch_size: int, ring: int = 0, halves: int = 2, graph: bool = True):
         why = supports(ds)
         if why is not None:
@@ -184,7 +186,6 @@ class FixedPipeline:
         self.ref_slot = self.eng.empty_slot if (sp.is_ref or not sp.want_seqs) else -1
         self.ring, self.n_halves = int(ring), int(halves)
         self.use_graph = bool(graph) and os.environ.get("GVL_PIPE_GRAPH", "1") != "0"  # (0: eager launches, for tool runs)
-        self.fused = os.environ.get("GVL_PIPE_SPLIT", "0") != "1"
         b, dev = self.b, self.dev
         with torch.cuda.device(dev):
             # eager path (Dataset.__getitem__): one scratch set, one pinned index buffer
@@ -233,8 +234,8 @@ class FixedPipeline:
 
     # ------------------------------------------------------------------ one device call over n queries
     # Stage P ("plan"): batch prep + variant plan (+ track plan / tile prep).  Stage E ("execute"): the bandwidth-bound
-    # kernels.  The eager path runs both on the current stream (gvl_dev_fixed_run); rings run P on a plan stream and E
-    # on an execute stream, so the plan of ring k+1 (latency-bound, few CTAs) overlaps the execute launch of ring k.
+    # kernels.  The eager path runs both on the current stream (gvl_dev_fixed_run); a ring half runs both on its own stream
+    # (_stages_fused), so the plan of one half's call (latency-bound, few CTAs) overlaps the execute of the other's.
     def _stage_plan(self, eng: Engine, scr: _Scratch, idx_dev, jit_dev, n: int, sub_batch: int = 0):
         check(lib.gvl_dev_fixed_plan(eng.ctx.handle, C.addressof(scr.job), idx_dev.data_ptr(),
                                      jit_dev.data_ptr() if jit_dev is not None else None, n, sub_batch, _stream()))
@@ -284,7 +285,7 @@ class FixedPipeline:
         sp, b, dev, K = self.spec, self.b, self.dev, self.ring
         n = K * b
         with torch.cuda.device(dev):
-            self.s_plan, self.s_exec = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
+            self.s_plan, self.s_exec = torch.cuda.Stream(dev), torch.cuda.Stream(dev)  # the streams of even / odd halves
             for h in range(self.n_halves):
                 H = type("Half", (), {})()
                 H.eng = self.eng.fork()
@@ -295,9 +296,9 @@ class FixedPipeline:
                 H.pin_jit = H.pin.array[n:].view(np.int32)
                 H.idx = torch.zeros(n + (n + 1) // 2, dtype=torch.int64, device=dev)
                 H.jit = H.idx[n:].view(torch.int32)
-                H.planned, H.done, H.uploaded = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
+                H.done, H.uploaded = torch.cuda.Event(), torch.cuda.Event()
                 H.free = None
-                H.g_plan = H.g_exec = None
+                H.g_plan = None
                 self.halves.append(H)
             jit = (lambda H: H.jit if sp.jitter else None)
             # warm once outside capture: workspace growth allocates
@@ -310,25 +311,16 @@ class FixedPipeline:
             torch.cuda.synchronize(dev)
             for H in self.halves:
                 H.eng.check()
-            # Fused mode (default): ONE graph per half -- prep -> plan -> execute -- replayed on the half's own stream, so a
-            # device call is one graph launch and the plan of the next call (other half, other stream) still overlaps this
-            # call's execute.  Split mode (GVL_PIPE_SPLIT=1, the first round-2 design): stage P on a plan stream and stage E
-            # on an execute stream, two graphs and one cross-stream event per call.
+            # ONE graph per half -- prep -> plan -> execute -- replayed on the half's own stream, so a device call is one graph
+            # launch and the plan of the next call (other half, other stream) still overlaps this call's execute.
             for i, H in enumerate(self.halves):
-                H.stream = (self.s_plan, self.s_exec)[i % 2] if self.fused else None
-                H.side = torch.cuda.Stream(dev, priority=-1) if self.fused else None  # (its small kernels go first when SM slots free up)
+                H.stream = (self.s_plan, self.s_exec)[i % 2]
+                H.side = torch.cuda.Stream(dev, priority=-1)  # (its small kernels go first when SM slots free up)
             if self.use_graph:
                 for H in self.halves:
-                    if self.fused:
-                        H.g_plan = torch.cuda.CUDAGraph()
-                        with torch.cuda.graph(H.g_plan, stream=H.stream):
-                            self._stages_fused(H, jit(H), n, b)
-                        continue
-                    H.g_plan, H.g_exec = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(H.g_plan, stream=self.s_plan):
-                        self._stage_plan(H.eng, H.scr, H.idx, jit(H), n, sub_batch=b)
-                    with torch.cuda.graph(H.g_exec, stream=self.s_exec):
-                        self._stage_exec(H.eng, H.scr, H.out, n, sub_batch=b)
+                    H.g_plan = torch.cuda.CUDAGraph()
+                    with torch.cuda.graph(H.g_plan, stream=H.stream):
+                        self._stages_fused(H, jit(H), n, b)
 
     def _stages_fused(self, H, jit_dev, n: int, b: int):
         """One device call of half H on the current stream (= H.stream).  With realigned tracks the call forks: the track
@@ -369,10 +361,8 @@ class FixedPipeline:
         H = self.halves[h]
         n = self.ring * self.b
         sp = self.spec
-        s_in = H.stream if self.fused else self.s_plan  # the stream the indices arrive on and the plan runs on
+        s_in = H.stream  # the stream the indices arrive on and the device call runs on
         with torch.cuda.device(self.dev):
-            if not self.fused:
-                self.s_plan.wait_event(H.done)  # this half's previous execute has finished with the plan workspace / scratch
             if isinstance(ds_idx, np.ndarray):
                 H.uploaded.synchronize()  # the previous copy out of the pinned buffer has finished
                 H.pin.array[:n] = ds_idx
@@ -389,31 +379,14 @@ class FixedPipeline:
                         H.idx[:n].copy_(ds_idx, non_blocking=True)
                         if jitter is not None:
                             H.jit[:n].copy_(jitter, non_blocking=True)
-            if self.fused:
-                if H.free is not None:
-                    s_in.wait_event(H.free)  # the consumer has let go of this half's output buffers
-                with torch.cuda.stream(s_in):
-                    if H.g_plan is not None:
-                        H.g_plan.replay()
-                    else:
-                        self._stages_fused(H, H.jit if sp.jitter else None, n, self.b)
-                H.done.record(s_in)
-                return
-            with torch.cuda.stream(self.s_plan):
+            if H.free is not None:
+                s_in.wait_event(H.free)  # the consumer has let go of this half's output buffers
+            with torch.cuda.stream(s_in):
                 if H.g_plan is not None:
                     H.g_plan.replay()
                 else:
-                    self._stage_plan(H.eng, H.scr, H.idx, H.jit if sp.jitter else None, n, sub_batch=self.b)
-            H.planned.record(self.s_plan)
-            self.s_exec.wait_event(H.planned)
-            if H.free is not None:
-                self.s_exec.wait_event(H.free)  # the consumer has let go of this half's output buffers
-            with torch.cuda.stream(self.s_exec):
-                if H.g_exec is not None:
-                    H.g_exec.replay()
-                else:
-                    self._stage_exec(H.eng, H.scr, H.out, n, sub_batch=self.b)
-            H.done.record(self.s_exec)
+                    self._stages_fused(H, H.jit if sp.jitter else None, n, self.b)
+            H.done.record(s_in)
 
     def acquire(self, h: int) -> _Out:
         """Make the current stream wait for half `h`; returns its `_Out` (batch i = queries [i*b, (i+1)*b))."""

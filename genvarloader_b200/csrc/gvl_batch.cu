@@ -183,17 +183,6 @@ int gvl_dev_upload(gvl_ctx *ctx, void *dev, const void *host, int64_t bytes, gvl
 }
 
 // ---- one fixed-length batch, end to end (the C side of Dataset.__getitem__ / the loader's device calls) ----
-static int fixed_plan_prepared(gvl_ctx *ctx, const gvl_fixed_job *J, int64_t n, int64_t sub_batch, gvl_stream stream, int what);
-
-int gvl_dev_fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
-                       int64_t sub_batch, gvl_stream stream) {
-    if (!ctx || !J || !J->view || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: NULL argument");
-    if (J->realign && (J->mode < 0 || J->ref_slot >= 0 || !J->diffs || !J->track_lengths))
-        return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: realigned tracks need haplotypes, diffs and track_lengths scratch");
-    int rc = launch_batch_prep(ctx, J->view, ds_idx, jitter, false, n, sub_batch, J->ref_slot, J->n_tracks, J->annot_mask, &J->args, stream);
-    if (rc) return rc;
-    return fixed_plan_prepared(ctx, J, n, sub_batch, stream, 3);
-}
 
 // everything of gvl_dev_fixed_plan after the batch prep: the haplotype plan (what = 1), the track plan (what = 2) or both
 static int fixed_plan_prepared(gvl_ctx *ctx, const gvl_fixed_job *J, int64_t n, int64_t sub_batch, gvl_stream stream, int what) {
@@ -235,18 +224,32 @@ static int fixed_plan_prepared(gvl_ctx *ctx, const gvl_fixed_job *J, int64_t n, 
     return GVL_OK;
 }
 
+// batch prep + the plans `what` selects (as in fixed_plan_prepared); ds_idx / jitter as in launch_batch_prep
+static int fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_idx, const int32_t *jitter, bool inline_host,
+                      int64_t n, int64_t sub_batch, int what, gvl_stream stream) {
+    if (!ctx || !J || !J->view || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: NULL argument");
+    if (J->realign && (J->mode < 0 || J->ref_slot >= 0 || !J->diffs || !J->track_lengths))
+        return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: realigned tracks need haplotypes, diffs and track_lengths scratch");
+    int rc = launch_batch_prep(ctx, J->view, ds_idx, jitter, inline_host, n, sub_batch, J->ref_slot, J->n_tracks, J->annot_mask,
+                               &J->args, stream);
+    if (rc) return rc;
+    return fixed_plan_prepared(ctx, J, n, sub_batch, stream, what);
+}
+
+int gvl_dev_fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
+                       int64_t sub_batch, gvl_stream stream) {
+    return fixed_plan(ctx, J, ds_idx, jitter, false, n, sub_batch, 3, stream);
+}
+
 // One stage of a fixed-length batch, for callers that spread a device call over two streams (the track plan -- a chain of
 // small latency-bound kernels -- next to the bandwidth-bound haplotype execute): GVL_STAGE_HAP_PLAN = batch prep +
 // haplotype plan, GVL_STAGE_TRK_PLAN (needs the diffs of HAP_PLAN), GVL_STAGE_HAP_EXEC, GVL_STAGE_TRK_EXEC (needs TRK_PLAN).
 int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *J, int stage, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
                         int64_t sub_batch, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, float *trk, gvl_stream stream) {
-    if (!ctx || !J || !J->view || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: NULL argument");
-    int rc;
+    if (!ctx || !J || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: NULL argument");
     switch (stage) {
         case GVL_STAGE_HAP_PLAN:
-            rc = launch_batch_prep(ctx, J->view, ds_idx, jitter, false, n, sub_batch, J->ref_slot, J->n_tracks, J->annot_mask, &J->args, stream);
-            if (rc) return rc;
-            return fixed_plan_prepared(ctx, J, n, sub_batch, stream, 1);
+            return fixed_plan(ctx, J, ds_idx, jitter, false, n, sub_batch, 1, stream);
         case GVL_STAGE_TRK_PLAN:
             return fixed_plan_prepared(ctx, J, n, sub_batch, stream, 2);
         case GVL_STAGE_HAP_EXEC:
@@ -265,23 +268,9 @@ int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *J, int stage, const i
 
 int gvl_dev_fixed_exec(gvl_ctx *ctx, const gvl_fixed_job *J, int64_t n, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos,
                        float *trk, gvl_stream stream) {
-    if (!ctx || !J || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_exec: NULL argument");
-    int rc;
-    if (J->mode >= 0) {
-        if (!seq) return fail(GVL_ERR_ARG, "gvl_dev_fixed_exec: sequence output missing");
-        rc = gvl_dev_hap_exec(ctx, J->tab, J->mode, J->pad_char, seq, annot_v, annot_pos, stream);
-        if (rc) return rc;
-    }
-    if (J->n_tracks > 0) {
-        if (!trk) return fail(GVL_ERR_ARG, "gvl_dev_fixed_exec: track output missing");
-        if (J->realign)
-            rc = gvl_dev_realign_tracks_exec(ctx, trk, stream);
-        else
-            rc = gvl_dev_paint_tracks(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
-                                      n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, trk, stream);
-        if (rc) return rc;
-    }
-    return GVL_OK;
+    int rc = gvl_dev_fixed_stage(ctx, J, GVL_STAGE_HAP_EXEC, NULL, NULL, n, 0, seq, annot_v, annot_pos, trk, stream);
+    if (rc) return rc;
+    return gvl_dev_fixed_stage(ctx, J, GVL_STAGE_TRK_EXEC, NULL, NULL, n, 0, seq, annot_v, annot_pos, trk, stream);
 }
 
 int gvl_dev_fixed_run(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
@@ -293,12 +282,7 @@ int gvl_dev_fixed_run(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_id
     GVL_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (n <= INLINE_MAX) {  // small batch: the indices travel with the prep launch
-        if (!J->view || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_run: NULL argument");
-        if (J->realign && (J->mode < 0 || J->ref_slot >= 0 || !J->diffs || !J->track_lengths))
-            return fail(GVL_ERR_ARG, "gvl_dev_fixed_run: realigned tracks need haplotypes, diffs and track_lengths scratch");
-        int rc = launch_batch_prep(ctx, J->view, ds_idx, jitter, true, n, 0, J->ref_slot, J->n_tracks, J->annot_mask, &J->args, stream);
-        if (rc) return rc;
-        rc = fixed_plan_prepared(ctx, J, n, 0, stream, 3);
+        int rc = fixed_plan(ctx, J, ds_idx, jitter, true, n, 0, 3, stream);
         if (rc) return rc;
         return gvl_dev_fixed_exec(ctx, J, n, seq, annot_v, annot_pos, trk, stream);
     }

@@ -71,10 +71,7 @@ constexpr int EXEC_MIN_CTAS = 12;        // resident CTAs per SM the execute ker
 constexpr int EXEC_UNIT = EXEC_THREADS * 4;  // positions covered by one CTA-wide step (4 per thread)
 constexpr int TILE = 4096;       // haplotype positions per execute CTA for ragged plans (fixed plans pick theirs)
 constexpr int REC_CAP = 128;     // records staged in shared memory per pass
-#ifndef GVL_EXEC_MAX_UNITS
-#define GVL_EXEC_MAX_UNITS 16
-#endif
-constexpr int EXEC_MAX_UNITS = GVL_EXEC_MAX_UNITS;  // haplotype positions per CTA of the byte kernel, in units of 512
+constexpr int EXEC_MAX_UNITS = 16;  // haplotype positions per CTA of the byte kernel, in units of 512
 constexpr int DIR_Q = 1024;      // haplotype positions per directory entry (execute tiles are multiples of it)
 constexpr int64_t ALT_PAD = INT64_MIN;  // RecArrays.src sentinel: "ALT piece" is padding (leading pad)
 

@@ -18,13 +18,7 @@
 //           bytes with two aligned 32-bit loads + funnel shift, ALT/pad bytes patched in,
 //           reverse-complement and the encoding fused, one 16-byte store (one-hot) per step.
 //           Every output byte is written exactly once; no intermediate haplotype in HBM.
-#include <cstdlib>
-
 #include "gvl_internal.cuh"
-
-#ifndef GVL_LUT_ASM
-#define GVL_LUT_ASM 1     // 1: hand-written shared-memory addressing for the one-hot table (+2 %, profiles/)
-#endif
 
 namespace gvl {
 
@@ -83,8 +77,8 @@ __device__ __forceinline__ void write_dir(const HapPlanParams &P, int64_t k, int
 }
 
 // Serial (lock-step) plan of one row by ONE warp: the reference's loop, one variant per step.
-// Exact for any input order; used for rows whose variant list is not position-sorted and by the
-// GVL_PLAN=serial debugging switch.  The scan-based kernel below handles everything else.
+// Exact for any input order; the scan-based kernel (gvl_plan_par.cuh) calls it for rows whose
+// variant list is not position-sorted and handles everything else itself.
 __device__ void plan_row_serial(const HapPlanParams &P, const int64_t k, const int64_t rec_off_in = -1) {
     const int lane = lane_id();
     const int64_t query = k / P.ploidy;
@@ -254,25 +248,13 @@ __device__ void plan_row_serial(const HapPlanParams &P, const int64_t k, const i
     write_dir<32>(P, k, rec_off, overflow ? 0 : n_emit, lane);
 }
 
-__global__ void __launch_bounds__(PLAN_WARPS * 32) hap_plan_serial_kernel(HapPlanParams P) {
-    const int64_t k = (int64_t)blockIdx.x * PLAN_WARPS + (threadIdx.x >> 5);
-    if (k >= P.n_work) return;
-    plan_row_serial(P, k);
-    if (lane_id() == 0) plan_row_done(P.words, P.n_work);
-}
-
 #include "gvl_trk_plan.cuh"
 #include "gvl_plan_par.cuh"
 
 // Threads per (query, hap) row of the parallel plan kernel, from the mean list-length bound: one warp for short lists; one
 // 256-thread CTA up to ~4,000 variants (cfg3's ~600-variant rows: 52 us per 640 rows against 63 us with 512 threads -- a
-// half-empty second chunk costs more than a third pass; cfg2d's ~1,300-variant rows: 125 vs 144 us); 512 beyond.  GVL_PLAN_NT=32|256|512 forces a width (A/B runs).
+// half-empty second chunk costs more than a third pass; cfg2d's ~1,300-variant rows: 125 vs 144 us); 512 beyond.
 static int plan_width(int64_t max_records, int64_t n_work) {
-    static const int force_nt = [] {
-        const char *e = getenv("GVL_PLAN_NT");
-        return e ? atoi(e) : 0;
-    }();
-    if (force_nt == 32 || force_nt == 256 || force_nt == 512) return force_nt;
     if (max_records <= 40 * n_work) return 32;
     return max_records <= 4096 * n_work ? 256 : 512;
 }
@@ -485,19 +467,12 @@ __global__ void __launch_bounds__(EXEC_THREADS, EXEC_MIN_CTAS) hap_exec_kernel(H
     auto emit_ref4 = [&](int32_t j, uint32_t v, int32_t r0) {
         if (OH) {
             uint4 o;
-#if GVL_LUT_ASM
-            // table offset of base i = (byte_i * 4) | half: one shift + one 3-input logic op each
+            // table offset of base i = (byte_i * 4) | half: one shift + one 3-input logic op each (hand-written
+            // shared-memory addressing: +2 % over indexing the table, profiles/)
             o.x = lds_u32(lut_a + (((v << 2) & 0x3fcu) | lut_rc));
             o.y = lds_u32(lut_a + (((v >> 6) & 0x3fcu) | lut_rc));
             o.z = lds_u32(lut_a + (((v >> 14) & 0x3fcu) | lut_rc));
             o.w = lds_u32(lut_a + (((v >> 22) & 0x3fcu) | lut_rc));
-#else
-            const uint32_t *lut = s_lut + (rc ? 256 : 0);
-            o.x = lut[v & 0xffu];
-            o.y = lut[(v >> 8) & 0xffu];
-            o.z = lut[(v >> 16) & 0xffu];
-            o.w = lut[v >> 24];
-#endif
             if (MODE == GVL_MODE_ONEHOT) {
                 *reinterpret_cast<uint4 *>(out_row + 4 * (int64_t)j) = o;
             } else {
@@ -880,15 +855,8 @@ static int hap_plan_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_s
         P.dir = ctx->hap.dir;
         P.dir_stride = ctx->dir_stride = stride;
     }
-    static const bool force_serial = [] {
-        const char *e = getenv("GVL_PLAN");
-        return e && e[0] == 's';
-    }();
     const int nt = plan_width(max_records, n_work);
-    if (force_serial) {
-        const unsigned grid = (unsigned)((n_work + PLAN_WARPS - 1) / PLAN_WARPS);
-        hap_plan_serial_kernel<<<grid, PLAN_WARPS * 32, 0, st>>>(P);
-    } else if (nt == 32) {  // short lists: one warp per row, 4 rows per CTA
+    if (nt == 32) {  // short lists: one warp per row, 4 rows per CTA
         hap_plan_par_kernel<32, false><<<(unsigned)((n_work + 3) / 4), 128, 0, st>>>(P);
     } else if (nt == 256) {  // one 256-thread CTA per row
         hap_plan_par_kernel<256, false><<<(unsigned)n_work, 256, 0, st>>>(P);
@@ -1008,24 +976,15 @@ int gvl_dev_hap_exec(gvl_ctx *ctx, const gvl_sparse_tables *tab, int mode, uint8
     P.annot_v = annot_v;
     P.annot_pos = annot_pos;
     P.pad_char = pad_char;
-    // one-hot over the packed reference (gvl_hap_oh.cuh) when the caller supplied it; GVL_EXEC=bytes forces the
-    // byte-oriented kernel (A/B measurements, parity tests of both)
-    static const bool force_bytes = [] {
-        const char *e = getenv("GVL_EXEC");
-        return e && e[0] == 'b';
-    }();
-    const bool packed = mode == GVL_MODE_ONEHOT && tab->ref_packed && tab->alt_packed && !force_bytes &&
+    // one-hot over the packed reference (gvl_hap_oh.cuh) when the caller supplied it
+    const bool packed = mode == GVL_MODE_ONEHOT && tab->ref_packed && tab->alt_packed &&
                         !((uintptr_t)out & 31) && !((uintptr_t)tab->ref_packed & 15) && !((uintptr_t)tab->alt_packed & 15);
     int64_t grid;
     if (ctx->fixed_len >= 0 && packed) {
         // Tiles as long as they can be (<= OH_MAX_TILE) while the batch still gives every SM ~3 CTAs: a CTA's fixed
         // cost (two dependent round trips before its first store) is amortised over more positions, and a launch
         // that leaves CTA slots free lets the next batch's launch (another stream) overlap its latency phases
-        // with this one's store stream (measured: profiles/r1_packed.md).  GVL_OH_TILE overrides (A/B runs).
-        static const int64_t tile_env = [] {
-            const char *e = getenv("GVL_OH_TILE");
-            return e ? (int64_t)atoll(e) : (int64_t)0;
-        }();
+        // with this one's store stream (measured: profiles/r1_packed.md).
         const int64_t q = imax64((OH_THREADS / 32) * OH_GROUP, DIR_Q);  // whole groups per warp, whole directory quanta
         static const int sms = [] {
             int n = 148, dev = 0;
@@ -1042,7 +1001,6 @@ int gvl_dev_hap_exec(gvl_ctx *ctx, const gvl_sparse_tables *tab, int mode, uint8
             tl = 16384;
         // lists so dense that a 16,384-position tile needs a second staging pass (REC_CAP = 128): 8,192 (cfg2d: 304 -> 285 us)
         if (tl > 8192 && ctx->fixed_len > 0 && ctx->rec_bound_per_row * (int64_t)16384 > (int64_t)REC_CAP * ctx->fixed_len) tl = 8192;
-        if (tile_env > 0) tl = tile_env;
         tl = imax64(q, imin64(tl / q * q, OH_MAX_TILE));
         P.tile_len = (int32_t)tl;
         P.tiles_per_row = (ctx->fixed_len + P.tile_len - 1) / P.tile_len;
@@ -1103,15 +1061,6 @@ int gvl_dev_hap_exec(gvl_ctx *ctx, const gvl_sparse_tables *tab, int mode, uint8
 }
 
 int gvl_debug_last_exec_kernel(gvl_ctx *ctx) { return ctx ? ctx->last_exec_kernel : -1; }
-
-#if GVL_TRACE
-// trace builds only (profiles/trace_exec.py): device buffer u64[n_ctas * 6] the next execute launches log into
-__attribute__((visibility("default"))) int gvl_debug_set_trace(void *dev_buf) {
-    unsigned long long *p = (unsigned long long *)dev_buf;
-    GVL_CUDA(cudaMemcpyToSymbol(g_trace, &p, sizeof(p)));
-    return GVL_OK;
-}
-#endif
 
 int64_t gvl_packed_reference_words(int64_t n_bases) { return (imax64(n_bases, 0) + 7) / 8 + 4; }  // + zeroed slack
 

@@ -24,28 +24,15 @@ constexpr int OH_GROUP = 256;                                  // positions per 
 // (round 1 capped tiles at 16,384: its launches were single batches.  A ring launch has thousands of CTAs, and a CTA's fixed
 //  cost -- ~3.3 us of dependent round trips and barriers before its first store -- is worth amortising over twice the positions:
 //  cfg3 execute 272 -> 259 us per 20 batches.  The launch code shortens tiles again when variants are dense.)
-#ifndef GVL_OH_MAX_TILE
-#define GVL_OH_MAX_TILE 32768
-#endif
-constexpr int OH_MAX_TILE_WANTED = GVL_OH_MAX_TILE;            // haplotype positions per CTA, at most
+constexpr int OH_MAX_TILE_WANTED = 32768;                      // haplotype positions per CTA, at most
 
-#ifndef GVL_OH_THREADS
-#define GVL_OH_THREADS 128
-#endif
-#ifndef GVL_OH_MIN_CTAS
-#define GVL_OH_MIN_CTAS 8
-#endif
-constexpr int OH_THREADS = GVL_OH_THREADS;                     // threads per CTA of the packed kernel
-constexpr int OH_MIN_CTAS = GVL_OH_MIN_CTAS;
+constexpr int OH_THREADS = 128;                                // threads per CTA of the packed kernel
+constexpr int OH_MIN_CTAS = 8;
 // one thread per group builds the group table: a pass may not touch more groups than the CTA has threads
 constexpr int OH_MAX_TILE = OH_MAX_TILE_WANTED < (OH_THREADS - 2) * OH_GROUP ? OH_MAX_TILE_WANTED : (OH_THREADS - 2) * OH_GROUP / 1024 * 1024;
 constexpr int OH_MAX_GROUPS = OH_MAX_TILE / OH_GROUP + 2;      // groups a pass can touch (+ misaligned edges)
 static_assert(OH_MAX_GROUPS <= OH_THREADS && OH_MAX_TILE >= 1024, "group table: one thread per group");
-constexpr int OH_EDGE_ROUNDS = (2 * REC_CAP + 2 + GVL_OH_THREADS - 1) / GVL_OH_THREADS;  // edge slots per thread and pass
-#ifndef GVL_OH_UNROLL
-#define GVL_OH_UNROLL 4
-#endif
-constexpr int OH_UNROLL_LONG = GVL_OH_UNROLL;                              // groups per warp whose loads are issued together (long sparse rows)
+constexpr int OH_UNROLL_LONG = 4;                              // groups per warp whose loads are issued together (long sparse rows)
 
 struct OhRecs {
     int32_t a[REC_CAP + 2];   // ALT start (haplotype coordinate); a[m], a[m+1] sentinels
@@ -86,13 +73,7 @@ __device__ __forceinline__ uint2 lds_u64(uint32_t addr) {
     return v;
 }
 
-#ifndef GVL_EXP
-#define GVL_EXP 0  // timing experiments only (results are WRONG): 1 no stores, 2 every group plain, 4 no table lookups
-#endif
 __device__ __forceinline__ void stg_256(void *p, const uint2 &o0, const uint2 &o1, const uint2 &o2, const uint2 &o3) {
-#if GVL_EXP & 1
-    if (o0.x != 0x12345678u) return;
-#endif
     asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(o0.x), "r"(o0.y), "r"(o1.x),
                  "r"(o1.y), "r"(o2.x), "r"(o2.y), "r"(o3.x), "r"(o3.y)
                  : "memory");
@@ -195,37 +176,6 @@ __device__ __forceinline__ int oh_classify(const OhRecs &S, int il, int32_t p_lo
     return U_PATCH;
 }
 
-#ifndef GVL_TRACE
-#define GVL_TRACE 0  // 1: every CTA of hap_exec_oh_kernel logs 4 timestamps (profiles/trace_exec.py); never the shipped build
-#endif
-#if GVL_TRACE
-__device__ unsigned long long *g_trace = nullptr;  // [n_ctas][6]: smid, t0..t3 (globaltimer ns), clock64 at t0
-__device__ __forceinline__ unsigned long long gtime() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-#define GVL_TR(slot)                                                                                       \
-    do {                                                                                                   \
-        if (GVL_TRACE == 1 && g_trace && threadIdx.x == 0) g_trace[tr_cta * 6 + (slot)] = gtime();          \
-    } while (0)
-#else
-#define GVL_TR(slot) do { } while (0)
-#endif
-// GVL_TRACE == 2: cycles thread 0 of every CTA spends in each phase, summed over the passes of its tile (profiles/trace_dense.py):
-// g_trace[cta * 8 + i], i = 0 prologue, 1 record staging, 2 group table, 3 edge slots part 1, 4 group loop, 5 edge slots part 2,
-// 6 = passes, 7 = smid
-#if GVL_TRACE == 2
-#define GVL_TC(i)                       \
-    do {                                \
-        const long long now_ = clock64(); \
-        tc_acc[i] += now_ - tc_last;    \
-        tc_last = now_;                 \
-    } while (0)
-#else
-#define GVL_TC(i) do { } while (0)
-#endif
-
 // OH_UNROLL = groups per warp whose loads are issued together: 4 for long sparse rows (cfg3: 259 us per 20 batches against 270
 // with 2), 2 where most groups take the mixed path or a warp has only a handful of groups (cfg2d: 358 -> 304 us, cfg4: 613 ->
 // 551 us) -- the launch code picks (profiles/r2_plan.md).
@@ -234,16 +184,6 @@ __device__ __forceinline__ unsigned long long gtime() {
 template <int OH_UNROLL, int NT>
 __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_kernel(HapExecParams P) {
     constexpr int EDGE_ROUNDS = (2 * REC_CAP + 2 + NT - 1) / NT;  // edge slots per thread and pass
-#if GVL_TRACE
-    const unsigned long long tr_cta = blockIdx.x + (unsigned long long)gridDim.x * (blockIdx.y + (unsigned long long)gridDim.y * blockIdx.z);
-    if (GVL_TRACE == 1 && g_trace && threadIdx.x == 0) {
-        unsigned smid;
-        asm volatile("mov.u32 %0, %smid;" : "=r"(smid));
-        g_trace[tr_cta * 6 + 0] = smid;
-        g_trace[tr_cta * 6 + 5] = clock64();
-    }
-    GVL_TR(1);
-#endif
     __shared__ OhRecs S;
     __shared__ __align__(16) uint2 s_lut[256];         // byte (2 codes) -> 8 one-hot bytes
     __shared__ __align__(8) uint2 s_grp[OH_MAX_GROUPS];  // per group: {reference delta, idx | cnt << 8 | plain << 31}
@@ -251,10 +191,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
     __shared__ uint32_t s_edge[EDGE_ROUNDS][8][NT];
     __shared__ int64_t s_lo, s_hi;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-#if GVL_TRACE == 2
-    long long tc_acc[7] = {0, 0, 0, 0, 0, 0, 0};
-    long long tc_last = clock64();
-#endif
 
     // ---- tile -> (row, tile-in-row) ----
     int64_t row, tile;
@@ -340,8 +276,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
         s_hi = rp.n_rec ? d_hi : 0;
     }
     __syncthreads();
-    GVL_TR(2);
-    GVL_TC(0);
     const int64_t r_hi = s_hi;
     int64_t r = s_lo;
     int32_t cur = h0;
@@ -354,10 +288,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
 
     // common epilogue of a full unit: 8 codes (output order) -> 32 one-hot bytes, one 256-bit store
     auto emit8 = [&](uint8_t *dst, uint32_t v) {
-#if GVL_EXP & 4
-        stg_256(dst, make_uint2(v, v >> 1), make_uint2(v >> 2, v >> 3), make_uint2(v >> 4, v >> 5), make_uint2(v >> 6, v >> 7));
-        return;
-#endif
         const char *lut = reinterpret_cast<const char *>(s_lut);  // (a link-time constant: folds into the LDS offset)
         const uint2 o0 = *reinterpret_cast<const uint2 *>(lut + ((v << 3) & 0x7f8u));
         const uint2 o1 = *reinterpret_cast<const uint2 *>(lut + ((v >> 5) & 0x7f8u));
@@ -396,7 +326,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
         }
         if (tid == 0) S.a[m] = S.a[m + 1] = INT32_MAX;
         __syncthreads();
-        GVL_TC(1);
 
         // ---- output range of the pass in units of 8 positions aligned on the GLOBAL flat index (32-byte
         //      aligned stores); a group is 32 units (one per lane), warp w owns groups w, w+4, ... ----
@@ -429,9 +358,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
             s_grp[tid] = make_uint2((uint32_t)dl, (uint32_t)idx | ((uint32_t)cnt << 8) | (plain ? 0x80000000u : 0u));
         }
         __syncthreads();
-        GVL_TC(2);
 
-        GVL_TR(3);
         uint8_t *const out_lane = out_row + 4 * ((int64_t)j0 + 8 * lane);
         const int32_t pg0 = rc ? (L - OH_GROUP - j0) : j0;  // lowest haplotype position of group 0
         const int32_t pg_step = rc ? -OH_GROUP : OH_GROUP;
@@ -508,7 +435,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
         };
         for (int s_ = tid, rd = 0; s_ < n_slots; s_ += NT, rd++) edge_begin(s_, rd);  // (one round unless variants are dense)
         cp_async_commit();
-        GVL_TC(3);
 
         // ---- the group loop: every lane streams the units that are a single run ----
         for (int gb = warp; gb < n_groups; gb += OH_UNROLL * (NT / 32)) {
@@ -524,7 +450,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
                 unsigned nv = 15;
                 if (g < n_groups) {
                     const uint2 meta = s_grp[g];
-                    if ((GVL_EXP & 2) || (meta.y & 0x80000000u)) {  // plain: one delta for the whole group
+                    if (meta.y & 0x80000000u) {  // plain: one delta for the whole group
                         nv = 8;
                         const int64_t x = nb2 + (int32_t)(pg0 + pg_step * g + (int32_t)meta.x);
                         const uint32_t *w = reinterpret_cast<const uint32_t *>((uintptr_t)(x >> 1) & ~(uintptr_t)3);
@@ -580,7 +506,6 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
             }
         }
 
-        GVL_TC(4);
         // ---- edge slots, part 2: blend (the copies were started before the group loop) + store ----
         cp_async_wait<0>();
 #pragma unroll 1
@@ -629,25 +554,9 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
                 }
             }
         }
-        GVL_TC(5);
-#if GVL_TRACE == 2
-        tc_acc[6] += 1;
-#endif
         cur = seg_end;
         r += m_new;
     }
-#if GVL_TRACE == 2
-    if (g_trace && threadIdx.x == 0) {
-        for (int i = 0; i < 7; i++) g_trace[tr_cta * 8 + i] = (unsigned long long)tc_acc[i];
-        unsigned smid2;
-        asm volatile("mov.u32 %0, %smid;" : "=r"(smid2));
-        g_trace[tr_cta * 8 + 7] = smid2;
-    }
-#endif
-#if GVL_TRACE == 1
-    __syncthreads();
-    GVL_TR(4);
-#endif
 }
 
 }  // namespace gvl

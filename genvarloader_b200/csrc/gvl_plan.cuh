@@ -4,7 +4,7 @@
 // (src/reconstruct/mod.rs:39-256 for bytes, src/tracks/mod.rs:224-406 for tracks,
 // src/genotypes/mod.rs:15-125 for the length diff).  Here the same state machines are
 // expressed as `init / step / finish` functions over plain integers so that the serial device
-// plan routines (rows with unsorted lists, GVL_PLAN=s) can drive them in lock-step across a warp,
+// plan routines (rows with unsorted lists) can drive them in lock-step across a warp,
 // one variant per step with operands broadcast by shuffles, emitting a compact segment table
 // instead of copying bytes.  (The scan-based kernel of gvl_plan_par.cuh restates the same rules
 // as block-wide scans.)

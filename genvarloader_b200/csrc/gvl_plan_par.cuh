@@ -134,11 +134,11 @@ struct PlanSmem {
 // variant is max(ilen, 0) + 1 (:282), SNPs take part in the shift bookkeeping only and otherwise change nothing
 // (:310-314), and there is no leading-pad clause (the source window is query-relative, positions left of it just read 0).
 // Records go out as 32-byte TRec (output range, resume point, anchor, fill length, ilen) in window-relative coordinates.
-#ifndef GVL_PLAN_OCC
-#define GVL_PLAN_OCC 1024  // resident threads per SM the register allocation aims for (A/B: -DGVL_PLAN_OCC=1536)
-#endif
+// PLAN_OCC = resident threads per SM the register allocation aims for (1,280 or 1,536 spill and gain nothing:
+// profiles/r2_plan.md)
+constexpr int PLAN_OCC = 1024;
 template <int NT, bool TRK>
-__global__ void __launch_bounds__(NT == 32 ? 128 : NT, GVL_PLAN_OCC / (NT == 32 ? 128 : NT)) hap_plan_par_kernel(HapPlanParams P) {
+__global__ void __launch_bounds__(NT == 32 ? 128 : NT, PLAN_OCC / (NT == 32 ? 128 : NT)) hap_plan_par_kernel(HapPlanParams P) {
     constexpr int ROWS_PER_CTA = (NT == 32) ? 4 : 1;
     __shared__ PlanSmem<NT> s_all[ROWS_PER_CTA];
     PlanSmem<NT> &S = s_all[(NT == 32) ? (threadIdx.x >> 5) : 0];

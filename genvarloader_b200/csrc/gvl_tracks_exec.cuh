@@ -633,10 +633,8 @@ static_assert(sizeof(TileCtx) <= 128, "TileCtx must fit T3Smem::big_ctx");
 
 // 5 CTAs per SM (48 registers, 80 bytes of spills; shared memory allows no more): the kernel is bound by the latency chain of a
 // tile, so the fifth tile in flight pays (tracks step of a 20-batch ring 63.7 -> 60.3 us) although a single 134 MB call gains little
-#ifndef GVL_T3_MINB
-#define GVL_T3_MINB 5
-#endif
-__global__ void __launch_bounds__(T2_THREADS, GVL_T3_MINB) trk_exec3_kernel(TrkExecParams P, const TileDesc *__restrict__ tdesc) {
+constexpr int T3_MIN_CTAS = 5;
+__global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkExecParams P, const TileDesc *__restrict__ tdesc) {
     __shared__ __align__(16) T3Smem S;
     const unsigned track = blockIdx.y;
     const TileDesc *dp = tdesc + ((size_t)track * (size_t)P.grid_per_track + blockIdx.x);
