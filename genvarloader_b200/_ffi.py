@@ -89,6 +89,7 @@ def _load() -> C.CDLL:
     lib.gvl_launch_count.argtypes = [C.c_int]
     lib.gvl_packed_reference_words.restype = c_i64
     lib.gvl_packed_reference_words.argtypes = [c_i64]
+    lib.gvl_debug_last_launch.argtypes = [c_vp, c_vp, C.c_int]
     # the per-batch entries of the fixed-length path take plain ints (no per-call ctypes objects)
     lib.gvl_dev_fixed_plan.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp]
     lib.gvl_dev_fixed_exec.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
@@ -107,6 +108,22 @@ def check(code: int) -> None:
 
 def launch_count(reset: bool = False) -> int:
     return int(lib.gvl_launch_count(1 if reset else 0))
+
+
+# gvl_debug_last_launch: field names in the order of GVL_LAUNCH_* (include/gvl_b200.h), kernel names in the order of GVL_EXEC_*
+LAUNCH_FIELDS = ("plan_threads", "plan_static", "exec_kernel", "tile_len", "tiles_per_row", "rec_bound", "trk_plan_threads",
+                 "trk_plan_static")
+EXEC_KERNELS = ("bytes", "packed_2warp", "packed_unroll4", "packed_unroll2")
+
+
+def last_launch(handle) -> dict:
+    """The launch configuration the last plans and execute of a context chose (gvl_debug_last_launch), by field name;
+    `exec_kernel` is given by name."""
+    out = (C.c_int64 * len(LAUNCH_FIELDS))()
+    check(lib.gvl_debug_last_launch(handle, out, len(LAUNCH_FIELDS)))
+    d = dict(zip(LAUNCH_FIELDS, (int(x) for x in out)))
+    d["exec_kernel"] = EXEC_KERNELS[d["exec_kernel"]]
+    return d
 
 
 def ptr(x) -> C.c_void_p:

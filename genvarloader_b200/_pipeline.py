@@ -22,6 +22,7 @@ double-buffered mode: valid until the ring is refilled); `copy=True` hands out c
 from __future__ import annotations
 
 import ctypes as C
+import gc
 import os
 
 import numpy as np
@@ -317,10 +318,20 @@ class FixedPipeline:
                 H.stream = (self.s_plan, self.s_exec)[i % 2]
                 H.side = torch.cuda.Stream(dev, priority=-1)  # (its small kernels go first when SM slots free up)
             if self.use_graph:
-                for H in self.halves:
-                    H.g_plan = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(H.g_plan, stream=H.stream):
-                        self._stages_fused(H, jit(H), n, b)
+                # No garbage collection while a graph is being captured: collecting a dead context or pinned buffer of
+                # an earlier dataset frees device / host memory, which a capture does not permit (the capture fails).
+                # Collect first, then keep the collector off until the captures are done.
+                gc.collect()
+                gc_was_on = gc.isenabled()
+                gc.disable()
+                try:
+                    for H in self.halves:
+                        H.g_plan = torch.cuda.CUDAGraph()
+                        with torch.cuda.graph(H.g_plan, stream=H.stream):
+                            self._stages_fused(H, jit(H), n, b)
+                finally:
+                    if gc_was_on:
+                        gc.enable()
 
     def _stages_fused(self, H, jit_dev, n: int, b: int):
         """One device call of half H on the current stream (= H.stream).  With realigned tracks the call forks: the track

@@ -125,6 +125,7 @@ struct gvl_ctx {
     int64_t total;      // -1 = unknown (ragged before sync)
     int64_t *plan_out_offsets;  // device pointer supplied at plan time
     int last_exec_kernel;       // 0 byte-oriented, 1 packed one-hot (gvl_debug_last_exec_kernel)
+    int64_t last_launch[GVL_LAUNCH_FIELDS] = {};  // launch choices of the last plans / execute (gvl_debug_last_launch)
     void *trk_params;           // parameters of the pending track execute launch (gvl_tracks.cu)
     bool trk_plan_valid;
     // gvl_dev_fixed_run: rotating pinned staging slots for the per-call index upload (gvl_batch.cu)

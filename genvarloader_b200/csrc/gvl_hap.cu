@@ -856,6 +856,8 @@ static int hap_plan_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_s
         P.dir_stride = ctx->dir_stride = stride;
     }
     const int nt = plan_width(max_records, n_work);
+    ctx->last_launch[GVL_LAUNCH_PLAN_THREADS] = nt;
+    ctx->last_launch[GVL_LAUNCH_PLAN_STATIC] = P.row_stride > 0;
     if (nt == 32) {  // short lists: one warp per row, 4 rows per CTA
         hap_plan_par_kernel<32, false><<<(unsigned)((n_work + 3) / 4), 128, 0, st>>>(P);
     } else if (nt == 256) {  // one 256-thread CTA per row
@@ -908,6 +910,8 @@ int gvl_trk_plan_launch(gvl_ctx *ctx, const gvl_sparse_tables *tab, const Merged
     P.trecs = (TRec *)ctx->trk.trecs;
     P.track_lengths = track_lengths;
     const int nt = plan_width(max_records, n_work);
+    ctx->last_launch[GVL_LAUNCH_TRK_PLAN_THREADS] = nt;
+    ctx->last_launch[GVL_LAUNCH_TRK_PLAN_STATIC] = P.row_stride > 0;
     if (nt == 32) hap_plan_par_kernel<32, true><<<(unsigned)((n_work + 3) / 4), 128, 0, st>>>(P);
     else if (nt == 256) hap_plan_par_kernel<256, true><<<(unsigned)n_work, 256, 0, st>>>(P);
     else hap_plan_par_kernel<512, true><<<(unsigned)n_work, 512, 0, st>>>(P);
@@ -1034,6 +1038,7 @@ int gvl_dev_hap_exec(gvl_ctx *ctx, const gvl_sparse_tables *tab, int mode, uint8
     }
     if (mode == GVL_MODE_ONEHOT_CF && (ctx->fixed_len & 3))
         return fail(GVL_ERR_ARG, "gvl_dev_hap_exec: channels-first one-hot needs output_length %% 4 == 0");
+    int64_t kind = GVL_EXEC_BYTES;
     switch (mode) {
         case GVL_MODE_U8: hap_exec_kernel<GVL_MODE_U8><<<grid3, EXEC_THREADS, 0, st>>>(P); break;
         case GVL_MODE_ONEHOT:
@@ -1043,11 +1048,16 @@ int gvl_dev_hap_exec(gvl_ctx *ctx, const gvl_sparse_tables *tab, int mode, uint8
                 const bool sparse = ctx->fixed_len > 0 && ctx->rec_bound_per_row > 0 &&
                                     ctx->rec_bound_per_row * (int64_t)OH_MAX_TILE <= 100 * ctx->fixed_len;
                 const int64_t groups_per_warp = (imin64(P.tile_len, ctx->fixed_len) / OH_GROUP) / (OH_THREADS / 32);
-                if (imin64(P.tile_len, ctx->fixed_len) <= 8192 && P.tiles_per_row == 1)  // short rows: one tile per row, 2-warp CTAs
+                if (imin64(P.tile_len, ctx->fixed_len) <= 8192 && P.tiles_per_row == 1) {  // short rows: one tile per row, 2-warp CTAs
                     hap_exec_oh_kernel<2, 64><<<grid3, 64, 0, st>>>(P);
-                else if (ctx->fixed_len < 0 || (sparse && groups_per_warp >= 8))  // (ragged plans: as in round 1)
+                    kind = GVL_EXEC_PACKED_2WARP;
+                } else if (ctx->fixed_len < 0 || (sparse && groups_per_warp >= 8)) {  // (ragged plans: as in round 1)
                     hap_exec_oh_kernel<OH_UNROLL_LONG, OH_THREADS><<<grid3, OH_THREADS, 0, st>>>(P);
-                else hap_exec_oh_kernel<2, OH_THREADS><<<grid3, OH_THREADS, 0, st>>>(P);
+                    kind = GVL_EXEC_PACKED_UNROLL4;
+                } else {
+                    hap_exec_oh_kernel<2, OH_THREADS><<<grid3, OH_THREADS, 0, st>>>(P);
+                    kind = GVL_EXEC_PACKED_UNROLL2;
+                }
             }
             else hap_exec_kernel<GVL_MODE_ONEHOT><<<grid3, EXEC_THREADS, 0, st>>>(P);
             break;
@@ -1057,10 +1067,20 @@ int gvl_dev_hap_exec(gvl_ctx *ctx, const gvl_sparse_tables *tab, int mode, uint8
     }
     GVL_LAUNCH_CHECK();
     ctx->last_exec_kernel = packed ? 1 : 0;
+    ctx->last_launch[GVL_LAUNCH_EXEC_KERNEL] = kind;
+    ctx->last_launch[GVL_LAUNCH_TILE_LEN] = P.tile_len;
+    ctx->last_launch[GVL_LAUNCH_TILES_PER_ROW] = P.tiles_per_row;
+    ctx->last_launch[GVL_LAUNCH_REC_BOUND] = ctx->rec_bound_per_row;
     return GVL_OK;
 }
 
 int gvl_debug_last_exec_kernel(gvl_ctx *ctx) { return ctx ? ctx->last_exec_kernel : -1; }
+
+int gvl_debug_last_launch(gvl_ctx *ctx, int64_t *out, int n) {
+    if (!ctx || (!out && n > 0) || n < 0) return fail(GVL_ERR_ARG, "gvl_debug_last_launch: bad argument");
+    for (int i = 0; i < n && i < GVL_LAUNCH_FIELDS; i++) out[i] = ctx->last_launch[i];
+    return GVL_OK;
+}
 
 int64_t gvl_packed_reference_words(int64_t n_bases) { return (imax64(n_bases, 0) + 7) / 8 + 4; }  // + zeroed slack
 

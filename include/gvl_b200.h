@@ -561,6 +561,34 @@ int gvl_debug_xorshift64(gvl_ctx *ctx, uint64_t x, uint64_t *out);
  * (tests assert that the intended kernel ran). */
 int gvl_debug_last_exec_kernel(gvl_ctx *ctx);
 
+/* The launch configuration the last plans and execute of this context chose, recorded on the host when each choice is
+ * made (so also while a CUDA graph is being captured).  Fills out[0 .. min(n, GVL_LAUNCH_FIELDS)), in this order:
+ *   GVL_LAUNCH_PLAN_THREADS      threads per row of the last haplotype plan (32, 256 or 512)
+ *   GVL_LAUNCH_PLAN_STATIC       1 if that plan used static record slices (a bounded list length per row), else 0
+ *   GVL_LAUNCH_EXEC_KERNEL       the last gvl_dev_hap_exec's kernel: one of GVL_EXEC_*
+ *   GVL_LAUNCH_TILE_LEN          its output positions per tile
+ *   GVL_LAUNCH_TILES_PER_ROW     its tiles per row (0 for ragged plans)
+ *   GVL_LAUNCH_REC_BOUND         the record bound per row it chose from (after the typical-slot-length clamp)
+ *   GVL_LAUNCH_TRK_PLAN_THREADS  threads per row of the last track plan (32, 256 or 512)
+ *   GVL_LAUNCH_TRK_PLAN_STATIC   1 if that track plan used static record slices, else 0
+ * Values of a step that has not run yet on this context are 0.  A gvl_dev_hap_exec that has nothing to launch (no rows,
+ * no output positions, no tiles) returns before the choice and leaves the previous call's values in place.  Tests use it
+ * to assert which configuration they reach. */
+#define GVL_LAUNCH_PLAN_THREADS 0
+#define GVL_LAUNCH_PLAN_STATIC 1
+#define GVL_LAUNCH_EXEC_KERNEL 2
+#define GVL_LAUNCH_TILE_LEN 3
+#define GVL_LAUNCH_TILES_PER_ROW 4
+#define GVL_LAUNCH_REC_BOUND 5
+#define GVL_LAUNCH_TRK_PLAN_THREADS 6
+#define GVL_LAUNCH_TRK_PLAN_STATIC 7
+#define GVL_LAUNCH_FIELDS 8
+#define GVL_EXEC_BYTES 0          /* byte-oriented kernel (bytes, annotated, channels-first, one-hot without a packed reference) */
+#define GVL_EXEC_PACKED_2WARP 1   /* packed one-hot, 2-warp CTAs: one tile of <= 8,192 positions per row                  */
+#define GVL_EXEC_PACKED_UNROLL4 2 /* packed one-hot, 4 groups per warp in flight: long sparse rows, ragged plans          */
+#define GVL_EXEC_PACKED_UNROLL2 3 /* packed one-hot, 2 groups per warp in flight: everything else                         */
+int gvl_debug_last_launch(gvl_ctx *ctx, int64_t *out, int n);
+
 /* ====================================================================================
  * `variants` / `variant-windows` outputs (SURVEY.md section 8 f4): the variants of every (region, sample, ploid) row
  * themselves -- indices, positions, indel lengths, allele byte strings, flank / window tokens -- instead of the
