@@ -10,7 +10,7 @@ Mirrors (names, argument meaning, error behaviour, return shapes):
 
 Host work per call is O(batch) numpy (index maths, RNG draws in the reference's order); everything
 sample-scale lives on the GPU inside `Engine`.  Results are torch CUDA tensors.
-Not supported (outside the hot-path scope, raise): splicing, `variants` / `variant-windows`, AF filters.
+Not supported (outside the hot-path scope, raise): fixed-length or jittered spliced output, spliced `variants`.
 """
 from __future__ import annotations
 
@@ -626,15 +626,25 @@ class Dataset:
         return self.splice_rows is not None
 
     def _getitem_spliced(self, idx):
-        """One ragged haplotype per (splice row, sample, ploid): the row's elements are reconstructed as separate
-        kernel rows, laid out in (row, sample, ploid, element) order (the reference's permuted write,
-        _splice.py:56-160 / _haps.py:872-919), so the concatenation is free and the group offsets are the kernel's
-        row offsets sampled at cell boundaries.  Negative-strand elements are reverse-complemented one by one
-        (_query.py:269-288); jitter and fixed lengths do not apply to spliced output."""
-        if self.sequence_type not in ("haplotypes", "annotated"):
-            raise NotImplementedError("spliced output is implemented for 'haplotypes' and 'annotated' sequences")
+        """One ragged sequence per (splice row, sample[, ploid]) and, with tracks active, one ragged track per (splice row,
+        sample, track[, ploid]): a spliced cell is the concatenation, in splice-row order, of its elements' unspliced
+        outputs (jitter 0, ragged length).
+
+        Sequences: the row's elements are reconstructed as separate kernel rows, laid out in (row, sample, ploid, element)
+        order (the reference's permuted write, _splice.py:56-160 / _haps.py:872-919), so the concatenation is free and the
+        group offsets are the kernel's row offsets sampled at cell boundaries.  Negative-strand elements are
+        reverse-complemented one by one (_query.py:269-288).  "reference" sequences are the zero-variant case (no ploidy axis).
+
+        Tracks: the element batch E lists every (element region, sample) of the selected pairs in output order.  One track
+        call covers all of E and all active tracks -- realigned to the element haplotypes (rows (e, ploid)) or painted over
+        the element regions (rows e) -- and writes every row straight into its place in the concatenated output through a
+        per-row destination table (gvl_dev_realign_tracks_plan_rows / gvl_dev_paint_tracks_rows).  The values are those of
+        one unspliced call over E: the same fill seed (of E's dataset indices), FlankSample rows and track lengths."""
         if self.jitter or isinstance(self.output_length, (int, np.integer)):
             raise ValueError("spliced datasets return ragged haplotypes: use with_len('ragged') and jitter=0")
+        seq = self.sequence_type
+        if seq is not None and self.encoding == "onehot_cf":
+            raise ValueError("channels-first one-hot needs a fixed output length; spliced output is ragged")
         rows_all = self.splice_rows
         n_rows_all, n_s_all = len(rows_all), len(self._s_idx)
         if not isinstance(idx, tuple):
@@ -652,46 +662,128 @@ class Dataset:
             pairs = [(r, s_) for r in ri.ravel().tolist() for s_ in si.ravel().tolist()]
             outer = (ri.size, si.size)
         eng, dev, p, S = self.engine, self.engine.device, self.ploidy, len(self.sample_names)
-        q_reg, q_goi, cell_len = [], [], []
-        for r, s_ in pairs:
-            elems = rows_all[r]
-            for e in range(p):
-                q_reg.append(elems)
-                q_goi.append((elems * S + s_) * p + e)
-                cell_len.append(len(elems))
-        q_reg = np.concatenate(q_reg)
-        goi = np.concatenate(q_goi)[:, None].astype(np.int64)
-        regions = self.full_regions[q_reg]
-        to_rc = (regions[:, 3] == -1) if self.rc_neg else None
+        is_ref = seq == "reference"
+        rows_p = 1 if is_ref else p  # sequence rows per element
+        names = list(self.active_tracks)
+        t = len(names)
+        realign = t > 0 and seq in ("haplotypes", "annotated") and self.realign_tracks
+
+        # ---- the element batch E: (pair, element) in output order
+        elems = [rows_all[r] for r, _ in pairs]
+        n_pairs = len(pairs)
+        n_el = np.array([len(e) for e in elems], np.int64)               # K_c
+        e_first = np.concatenate([[0], np.cumsum(n_el)]).astype(np.int64)  # first element of pair c in E
+        e_reg = np.concatenate(elems).astype(np.int64)
+        e_pair = np.repeat(np.arange(n_pairs, dtype=np.int64), n_el)
+        e_k = np.arange(e_reg.size, dtype=np.int64) - e_first[e_pair]
+        ds_idx_e = e_reg * S + np.repeat(np.array([s_ for _, s_ in pairs], np.int64), n_el)
+        regions = self.full_regions[e_reg]
+        to_rc_e = (regions[:, 3] == -1) if self.rc_neg else None
+        e_len = (regions[:, 2] - regions[:, 1]).astype(np.int64)
+        n_e = e_reg.size
+
+        # sequence row of (e, h): pair c holds rows rows_p * e_first[c] ..., ploid-major, element-minor
+        q = ((rows_p * e_first[e_pair])[:, None] + np.arange(rows_p, dtype=np.int64)[None, :] * n_el[e_pair][:, None]
+             + e_k[:, None])
+        goi_e = ds_idx_e[:, None] * p + np.arange(p, dtype=np.int64)[None, :]
         pk = _Packer(dev)
-        i_reg, i_goi = pk.add(regions[:, :3], np.int32), pk.add(goi, np.int64)
-        i_sh = pk.add(np.zeros((len(goi), 1), np.int32), np.int32)
-        i_rc = pk.add(to_rc, np.uint8) if to_rc is not None else None
-        cell_starts = np.concatenate([[0], np.cumsum(cell_len)]).astype(np.int64)
-        i_cs = pk.add(cell_starts, np.int64)
+        if seq is not None:
+            inv = np.empty(n_e * rows_p, np.int64)  # element of every sequence row
+            inv[q.ravel()] = np.repeat(np.arange(n_e, dtype=np.int64), rows_p)
+            if is_ref:
+                s_goi = np.full((n_e, 1), eng.empty_slot, np.int64)
+            else:
+                s_goi = np.empty((n_e * p, 1), np.int64)
+                s_goi[q.ravel(), 0] = goi_e.ravel()
+            i_sreg = pk.add(regions[inv, :3], np.int32)
+            i_sgoi = pk.add(s_goi, np.int64)
+            i_ssh = pk.add(np.zeros((len(s_goi), 1), np.int32), np.int32)
+            i_src = pk.add(to_rc_e[inv], np.uint8) if to_rc_e is not None else None
+            cell_starts = (rows_p * e_first[:-1, None] + np.arange(rows_p, dtype=np.int64)[None, :] * n_el[:, None]).ravel()
+            i_cs = pk.add(np.append(cell_starts, rows_p * e_first[-1]), np.int64)
+        if t:
+            oi = np.stack([ds_idx_e if self.track_kinds[n] == "sample" else e_reg for n in names])
+            i_oi = pk.add(oi, np.int64)
+            if realign:
+                i_reg = pk.add(regions[:, :3], np.int32)
+                i_len = pk.add(e_len, np.int64)
+                i_goi_e = pk.add(goi_e, np.int64)
+                i_sh_e = pk.add(np.zeros((n_e, p), np.int32), np.int32)
+                i_rc_e = pk.add(np.repeat(to_rc_e, p), np.uint8) if to_rc_e is not None else None
+                i_q = pk.add(q, np.int64)
+                i_pf = pk.add(rows_p * e_first[e_pair], np.int64)       # first sequence row of the element's pair
+                i_pn = pk.add(rows_p * e_first[e_pair + 1], np.int64)   # ... and of the next pair
+            else:
+                # painted: lengths are the element region lengths, known here -- the whole table is built on the host
+                off_e = np.concatenate([[0], np.cumsum(e_len)]).astype(np.int64)
+                base_c = off_e[e_first]                                   # B_c (and the end of E at [n_pairs])
+                len_c = base_c[1:] - base_c[:-1]                          # L_c
+                i_off_e = pk.add(off_e, np.int64)
+                i_dst = pk.add(t * base_c[e_pair] + (off_e[:-1] - base_c[e_pair]), np.int64)
+                i_ts = pk.add(len_c[e_pair], np.int64)
+                i_rc_q = pk.add(to_rc_e, np.uint8) if to_rc_e is not None else None
+                i_st = pk.add(regions[:, 1], np.int32)
+                i_toff = pk.add(np.concatenate([[0], np.cumsum(np.repeat(len_c, t))]), np.int64)
         pk.upload()
-        keep = keep_off = None
-        if self.var_filter == "exonic":
-            keep, keep_off = self._exonic_keep(pk.get(i_goi), pk.get(i_reg), goi)
-        oo = eng.plan(pk.get(i_reg), pk.get(i_sh), pk.get(i_goi), -1, eng.max_records(goi), keep, keep_off,
-                      pk.get(i_rc) if i_rc is not None else None)
-        total = eng.total()
-        group_offsets = oo[pk.get(i_cs)]
-        shape = (*outer, p, None)
-        if self.sequence_type == "annotated":
-            h, av, ap = eng.execute("annotated")
-            out = RaggedAnnotatedHaps(Ragged(h, group_offsets, shape), Ragged(av, group_offsets, shape), Ragged(ap, group_offsets, shape))
-        elif self.encoding == "onehot":
-            out = Ragged(eng.execute("onehot").view(total, 4), group_offsets, shape)
-        elif self.encoding == "bytes":
-            out = Ragged(eng.execute("haplotypes"), group_offsets, shape)
-        else:
-            raise ValueError("channels-first one-hot needs a fixed output length; spliced output is ragged")
+
+        results = []
+        max_rec = 0 if is_ref else eng.max_records(goi_e)
+        oo = group_offsets = total = None
+        if seq is not None:
+            keep = keep_off = None
+            if self.var_filter == "exonic" and not is_ref:
+                keep, keep_off = self._exonic_keep(pk.get(i_sgoi), pk.get(i_sreg), s_goi)
+            diffs = torch.empty((len(s_goi), 1), dtype=torch.int32, device=dev) if realign else None
+            oo = eng.plan(pk.get(i_sreg), pk.get(i_ssh), pk.get(i_sgoi), -1, max_rec, keep, keep_off,
+                          pk.get(i_src) if i_src is not None else None, diffs=diffs, use_svar2=not is_ref)
+            total = eng.total()
+            group_offsets = oo[pk.get(i_cs)]
+            shape = (*outer, None) if is_ref else (*outer, p, None)
+            if seq == "annotated":
+                hh, av, ap = eng.execute("annotated")
+                results.append(RaggedAnnotatedHaps(Ragged(hh, group_offsets, shape), Ragged(av, group_offsets, shape),
+                                                   Ragged(ap, group_offsets, shape)))
+            elif self.encoding == "onehot":
+                results.append(Ragged(eng.execute("onehot").view(total, 4), group_offsets, shape))
+            else:
+                results.append(Ragged(eng.execute("haplotypes"), group_offsets, shape))
+        if t and realign:
+            # rows (e, h) of E; their haplotypes are sequence rows q[e, h] of the plan above
+            t_q = pk.get(i_q)
+            diffs_e = diffs.view(-1)[t_q]
+            track_lengths = (pk.get(i_len) - diffs_e.clamp(max=0).min(1).values.to(torch.int64)).to(torch.int32)
+            row_len = (oo[1:] - oo[:-1])[t_q].reshape(-1)
+            out_offsets = torch.zeros(n_e * p + 1, dtype=torch.int64, device=dev)
+            torch.cumsum(row_len, 0, out=out_offsets[1:])
+            base = oo[pk.get(i_pf)][:, None]  # B_c of the element's pair: cell (c, track, h) starts at t * B_c + ...
+            row_dst = (t * base + oo[t_q] - base).reshape(-1)
+            row_tstride = (oo[pk.get(i_pn)] - base[:, 0]).repeat_interleave(p)  # (a materialised copy: the kernel reads it by index)
+            keep = keep_off = None
+            if self.var_filter == "exonic":
+                keep, keep_off = self._exonic_keep(pk.get(i_goi_e), pk.get(i_reg), goi_e)
+            ids, params = lower([self.insertion_fill.get(n, Repeat5p()) for n in names])
+            if self.deterministic:
+                base_seed = int(np.bitwise_xor.reduce(ds_idx_e.astype(np.uint64)))  # _reconstruct.py:215-218
+            else:
+                base_seed = int(self.rng.integers(0, np.iinfo(np.uint64).max, dtype=np.uint64))  # :219-222
+            out = eng.realign_tracks(names, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), track_lengths,
+                                     out_offsets, total, ids, params, base_seed, max_rec, keep, keep_off,
+                                     pk.get(i_rc_e) if i_rc_e is not None else None, layout="rows", row_dst=row_dst,
+                                     row_tstride=row_tstride)
+            lens = (group_offsets[1:] - group_offsets[:-1]).view(n_pairs, 1, p).expand(n_pairs, t, p).reshape(-1)
+            offsets = torch.zeros(n_pairs * t * p + 1, dtype=torch.int64, device=dev)
+            torch.cumsum(lens, 0, out=offsets[1:])
+            results.append(Ragged(out, offsets, (*outer, t, p, None)))
+        elif t:
+            out = eng.paint_tracks(names, pk.get(i_oi), pk.get(i_st), pk.get(i_off_e), int(off_e[-1]),
+                                   pk.get(i_rc_q) if i_rc_q is not None else None, layout="rows", row_dst=pk.get(i_dst),
+                                   row_tstride=pk.get(i_ts))
+            results.append(Ragged(out, pk.get(i_toff), (*outer, t, None)))
         if self.output_length == "variable" and self.output_format != "flat":  # pad like the unspliced path (_query.py:94-127)
-            out = self._shape_output(out, None, False)
+            results = [self._shape_output(o, None, False) for o in results]
         if is_int(r_sel) and is_int(s_sel):
-            out = out.squeeze(0).squeeze(0) if hasattr(out, "squeeze") else out
-        return out
+            results = [o.squeeze(0).squeeze(0) for o in results]
+        return results[0] if len(results) == 1 else tuple(results)
 
     # ------------------------------------------------------------------ iteration (reference: to_dataloader, _impl.py:1963-2072)
     def to_dataloader(self, batch_size: int = 1, shuffle: bool = False, sampler=None, num_workers: int = 0, collate_fn=None,

@@ -516,20 +516,22 @@ class Engine:
     def realign_tracks(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                        total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
                        keep_offsets=None, to_rc=None, query_seed=None, out=None, layout="tbp", base_seed_dev=None,
-                       batch=None, sub_batch: int = 0):
+                       batch=None, sub_batch: int = 0, row_dst=None, row_tstride=None):
         """gvl_dev_realign_tracks: all `names` in one plan + one execute launch.
         offset_idxs: int64 (n_tracks, batch) device; out: float32 (n_tracks * total_per_track,), track-major
-        (layout="tbp", the reference's flat buffer) or with every query's tracks adjacent (layout="btp",
-        gvl_dev_realign_tracks_btp: the order the reference's (b, t, p, ~l) offsets describe)."""
+        (layout="tbp", the reference's flat buffer), with every query's tracks adjacent (layout="btp",
+        gvl_dev_realign_tracks_btp: the order the reference's (b, t, p, ~l) offsets describe) or wherever the
+        per-row table puts each row (layout="rows": row k of track t starts at row_dst[k] + t * row_tstride[k],
+        device int64 (batch * ploidy,) each; gvl_dev_realign_tracks_plan_rows)."""
         b_cap, ploidy = geno_offset_idx.shape
         batch = b_cap if batch is None else int(batch)  # (a prefix of preallocated buffers)
         n_tracks = len(names)
         if out is None:
             out = torch.empty(n_tracks * total_per_track, dtype=torch.float32, device=self.device)
-        if self.svar2 is not None:
+        if self.svar2 is not None or layout == "rows":
             self.realign_tracks_plan(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                                      total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
-                                     query_seed, layout, base_seed_dev, batch, sub_batch)
+                                     query_seed, layout, base_seed_dev, batch, sub_batch, row_dst, row_tstride)
             return self.realign_tracks_exec(out)
         itv = (Intervals * n_tracks)(*[self.tracks[n][4] for n in names])
         sid = (c_i32 * n_tracks)(*[int(s) for s in strategy_ids])
@@ -545,9 +547,10 @@ class Engine:
     def realign_tracks_plan(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                             total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
                             keep_offsets=None, to_rc=None, query_seed=None, layout="tbp", base_seed_dev=None, batch=None,
-                            sub_batch: int = 0):
-        """gvl_dev_realign_tracks_plan: everything of `realign_tracks` but the execute launch (variant plan, tile map,
-        per-tile searches); `realign_tracks_exec(out)` writes the values, possibly on another stream."""
+                            sub_batch: int = 0, row_dst=None, row_tstride=None):
+        """gvl_dev_realign_tracks_plan (layout="rows": gvl_dev_realign_tracks_plan_rows): everything of `realign_tracks`
+        but the execute launch (variant plan, tile map, per-tile searches); `realign_tracks_exec(out)` writes the values,
+        possibly on another stream."""
         b_cap, ploidy = geno_offset_idx.shape
         batch = b_cap if batch is None else int(batch)
         n_tracks = len(names)
@@ -555,6 +558,15 @@ class Engine:
         sid = (c_i32 * n_tracks)(*[int(s) for s in strategy_ids])
         par = (C.c_double * n_tracks)(*[float(p) for p in params])
         ch = self.svar2_channels(geno_offset_idx) if self.svar2 is not None else None
+        if layout == "rows":
+            if row_dst is None or row_tstride is None:
+                raise ValueError('layout="rows" needs row_dst and row_tstride')
+            check(lib.gvl_dev_realign_tracks_plan_rows(
+                self.ctx.handle, C.byref(self.tab), C.byref(ch) if ch is not None else None, ptr(regions), ptr(shifts),
+                ptr(geno_offset_idx), batch, ploidy, ptr(keep), ptr(keep_offsets), ptr(to_rc), n_tracks, itv, ptr(offset_idxs),
+                ptr(track_lengths), ptr(out_offsets), int(total_per_track), sid, par, int(base_seed), ptr(base_seed_dev),
+                int(sub_batch), ptr(query_seed), int(max_records), ptr(row_dst), ptr(row_tstride), _stream()))
+            return
         check(lib.gvl_dev_realign_tracks_plan(
             self.ctx.handle, C.byref(self.tab), C.byref(ch) if ch is not None else c_vp(0), ptr(regions), ptr(shifts),
             ptr(geno_offset_idx), c_i64(batch), c_i64(ploidy),
@@ -576,13 +588,21 @@ class Engine:
         return out
 
     def paint_tracks(self, names, offset_idxs, starts, out_offsets, total_per_track: int, to_rc=None, out=None,
-                     n_queries=None):
+                     n_queries=None, layout="btp", row_dst=None, row_tstride=None):
         """gvl_dev_paint_tracks: stored intervals of all `names` painted in one launch, (b, t, ~l) order,
-        masked rows reversed.  offset_idxs: int64 (n_tracks, batch) device."""
+        masked rows reversed.  offset_idxs: int64 (n_tracks, batch) device.  layout="rows"
+        (gvl_dev_paint_tracks_rows): query q of track t starts at row_dst[q] + t * row_tstride[q] instead."""
         n_tracks, n_q = len(names), int(starts.numel() if n_queries is None else n_queries)
         itv = (Intervals * n_tracks)(*[self.tracks[n][4] for n in names])
         if out is None:
             out = torch.empty(n_tracks * int(total_per_track), dtype=torch.float32, device=self.device)
+        if layout == "rows":
+            if row_dst is None or row_tstride is None:
+                raise ValueError('layout="rows" needs row_dst and row_tstride')
+            check(lib.gvl_dev_paint_tracks_rows(self.ctx.handle, n_tracks, itv, ptr(offset_idxs), ptr(starts), n_q,
+                                                ptr(out_offsets), int(total_per_track), ptr(to_rc), ptr(row_dst),
+                                                ptr(row_tstride), ptr(out), _stream()))
+            return out
         check(lib.gvl_dev_paint_tracks(self.ctx.handle, c_i64(n_tracks), itv, ptr(offset_idxs), ptr(starts), c_i64(n_q),
                                        ptr(out_offsets), c_i64(int(total_per_track)), ptr(to_rc), ptr(out), _stream()))
         return out

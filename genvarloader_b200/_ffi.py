@@ -95,6 +95,11 @@ def _load() -> C.CDLL:
     lib.gvl_dev_fixed_exec.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
     lib.gvl_dev_fixed_stage.argtypes = [c_vp, c_vp, C.c_int, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
     lib.gvl_dev_fixed_run.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
+    # track entries with an explicit destination per row (spliced output)
+    lib.gvl_dev_realign_tracks_plan_rows.argtypes = [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_i64,
+                                                     c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_u64, c_vp, c_i64, c_vp, c_i64,
+                                                     c_vp, c_vp, c_vp]
+    lib.gvl_dev_paint_tracks_rows.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
     return lib
 
 

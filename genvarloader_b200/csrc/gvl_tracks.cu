@@ -142,7 +142,8 @@ static int trk_execute(gvl_ctx *ctx, float *out, cudaStream_t st) {
 static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t n_queries, int64_t n_tracks,
                            const TrkDesc *host_desc, const int64_t *offset_idxs, int64_t total_per_track,
                            const int64_t *query_seed, uint64_t base_seed, float *out, int layout_btp, cudaStream_t st,
-                           const uint64_t *base_seed_dev = nullptr, int64_t sub_batch = 0) {
+                           const uint64_t *base_seed_dev = nullptr, int64_t sub_batch = 0, const int64_t *row_dst = nullptr,
+                           const int64_t *row_tstride = nullptr) {
     if (n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "at most %d tracks per call", MAX_TRACKS);
     static_assert(sizeof(TrkDesc) * MAX_TRACKS <= GVL_TRK_DESC_BYTES, "descriptor buffer too small");
     TrkDesc *d_desc = nullptr;
@@ -177,7 +178,7 @@ static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t
     int rc;
     if ((rc = ensure_tdesc(ctx, ctx->trk, grid))) return rc;
     TileDesc *tdesc = (TileDesc *)ctx->trk.tdesc;
-    trk_tile_prep_kernel<<<(unsigned)((grid + 3) / 4), 128, 0, st>>>(P, tdesc);  // one warp per tile
+    trk_tile_prep_kernel<<<(unsigned)((grid + 3) / 4), 128, 0, st>>>(P, row_dst, row_tstride, tdesc);  // one warp per tile
     GVL_LAUNCH_CHECK();
     // the execute launch may follow later, on another stream (gvl_dev_realign_tracks_exec): keep its parameters
     if (!ctx->trk_params) ctx->trk_params = malloc(sizeof(TrkExecParams));
@@ -209,7 +210,7 @@ static int realign_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_sv
                         const int32_t *strategy_ids, const double *params, uint64_t base_seed,
                         const int64_t *query_seed, int64_t max_records, float *out, gvl_stream stream,
                         int layout_btp = 0, const uint64_t *base_seed_dev = nullptr, int64_t sub_batch = 0,
-                        bool plan_only = false) {
+                        bool plan_only = false, const int64_t *row_dst = nullptr, const int64_t *row_tstride = nullptr) {
     if (!ctx || !tab || !regions || !shifts || !(geno_offset_idx || svar2) || !(itv || dense) || !(offset_idxs || dense) ||
         !track_lengths || !out_offsets || !strategy_ids || !params)
         return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks: NULL argument");
@@ -253,7 +254,7 @@ static int realign_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_sv
         desc[t].param = params[t];
     }
     return launch_trk_exec(ctx, n_work, ploidy, batch, n_tracks, desc, offset_idxs, total_per_track, query_seed,
-                           base_seed, out, layout_btp, st, base_seed_dev, sub_batch);
+                           base_seed, out, layout_btp, st, base_seed_dev, sub_batch, row_dst, row_tstride);
 }
 
 int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
@@ -298,6 +299,23 @@ int gvl_dev_realign_tracks_plan(gvl_ctx *ctx, const gvl_sparse_tables *tab, cons
                         itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets, total_per_track, strategy_ids,
                         params, base_seed, query_seed, max_records, nullptr, stream, layout_btp ? 1 : 0, base_seed_dev, sub_batch,
                         true);
+}
+
+int gvl_dev_realign_tracks_plan_rows(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                                     const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
+                                     int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
+                                     int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                                     const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
+                                     const int32_t *strategy_ids, const double *params, uint64_t base_seed,
+                                     const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
+                                     int64_t max_records, const int64_t *row_dst, const int64_t *row_tstride, gvl_stream stream) {
+    if (!itv || !offset_idxs || !row_dst || !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_plan_rows: NULL argument");
+    if (svar2 && (!svar2->vk_off || !svar2->dense_range || !svar2->dense_present_off))
+        return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_plan_rows: NULL channel");
+    return realign_impl(ctx, tab, svar2, regions, shifts, geno_offset_idx, batch, ploidy, keep, keep_offsets, to_rc, n_tracks,
+                        itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets, total_per_track, strategy_ids,
+                        params, base_seed, query_seed, max_records, nullptr, stream, 0, base_seed_dev, sub_batch, true, row_dst,
+                        row_tstride);
 }
 
 int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream) {
@@ -362,16 +380,16 @@ int gvl_dev_intervals_to_tracks(gvl_ctx *ctx, const gvl_intervals *itv, const in
     return launch_trk_exec(ctx, n_queries, 1, n_queries, 1, &desc, offset_idxs, total, nullptr, 0, out, 0, st);
 }
 
-int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                         const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                         const uint8_t *to_rc, float *out, gvl_stream stream) {
-    if (!ctx || !itv || !offset_idxs || !starts || !out_offsets)
-        return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks: NULL argument");
-    if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks: 0..%d tracks per call", MAX_TRACKS);
+static int paint_impl(const char *who, gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                      const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                      const uint8_t *to_rc, float *out, gvl_stream stream, const int64_t *row_dst = nullptr,
+                      const int64_t *row_tstride = nullptr) {
+    if (!ctx || !itv || !offset_idxs || !starts || !out_offsets) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
+    if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "%s: 0..%d tracks per call", who, MAX_TRACKS);
     cudaStream_t st = (cudaStream_t)stream;
     GVL_CUDA(cudaSetDevice(ctx->device));
     if (n_queries == 0 || n_tracks == 0 || total_per_track == 0) return GVL_OK;
-    if (!out || ((uintptr_t)out & 15)) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks: out must be 16-byte aligned");
+    if (!out || ((uintptr_t)out & 15)) return fail(GVL_ERR_ARG, "%s: out must be 16-byte aligned", who);
     int rc;
     if ((rc = ensure_rows(ctx, ctx->trk, n_queries))) return rc;
     if ((rc = ensure_trecs(ctx, ctx->trk, 1))) return rc;
@@ -389,7 +407,24 @@ int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *it
         desc[t].strategy = GVL_FILL_REPEAT_5P;
         desc[t].param = 0.0;
     }
-    return launch_trk_exec(ctx, n_queries, 1, n_queries, n_tracks, desc, offset_idxs, total_per_track, nullptr, 0, out, 1, st);
+    return launch_trk_exec(ctx, n_queries, 1, n_queries, n_tracks, desc, offset_idxs, total_per_track, nullptr, 0, out, 1, st,
+                           nullptr, 0, row_dst, row_tstride);
+}
+
+int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                         const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                         const uint8_t *to_rc, float *out, gvl_stream stream) {
+    return paint_impl("gvl_dev_paint_tracks", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets, total_per_track,
+                      to_rc, out, stream);
+}
+
+int gvl_dev_paint_tracks_rows(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                              const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                              const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, float *out,
+                              gvl_stream stream) {
+    if (!row_dst || !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks_rows: NULL argument");
+    return paint_impl("gvl_dev_paint_tracks_rows", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
+                      total_per_track, to_rc, out, stream, row_dst, row_tstride);
 }
 
 static int run_prng(gvl_ctx *ctx, uint64_t a, uint64_t b, uint64_t c, uint64_t d, int which, uint64_t *out) {

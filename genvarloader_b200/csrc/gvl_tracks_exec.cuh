@@ -245,7 +245,11 @@ __device__ __forceinline__ void t2_set_bit(uint32_t *mk, uint32_t *mk2, int u) {
 // =====================================================================================
 // tile preparation: one thread per (track, tile)
 // =====================================================================================
-__global__ void __launch_bounds__(128) trk_tile_prep_kernel(TrkExecParams P, TileDesc *__restrict__ tdesc) {
+// row_dst / row_tstride (gvl_dev_*_rows): explicit destination of every row, out_base = row_dst[row] + track *
+// row_tstride[row]; NULL row_dst = the fixed layout of P.layout_btp.  (Kernel arguments of their own, not members of
+// TrkExecParams: the execute kernel takes the same struct, and a larger struct would move its tdesc argument.)
+__global__ void __launch_bounds__(128) trk_tile_prep_kernel(TrkExecParams P, const int64_t *__restrict__ row_dst,
+                                                            const int64_t *__restrict__ row_tstride, TileDesc *__restrict__ tdesc) {
     // one WARP per (track, tile): the searches are 32-ary (a probe per lane), the record counts one strided pass
     const int lane = threadIdx.x & 31;
     const int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -289,7 +293,9 @@ __global__ void __launch_bounds__(128) trk_tile_prep_kernel(TrkExecParams P, Til
             D.m = 1;
             D.cnt = 0;
             int64_t row_base = track * P.total_per_track + rp.out_off;  // flat index of the row's first value
-            if (P.layout_btp) {  // all tracks of a query adjacent: block of the query, then track, then the row inside the block
+            if (row_dst) {
+                row_base = row_dst[row] + track * row_tstride[row];
+            } else if (P.layout_btp) {  // all tracks of a query adjacent: block of the query, then track, then the row inside the block
                 const int64_t k0 = query * P.ploidy;
                 const int64_t blk0 = P.rows[k0].out_off;
                 const int64_t blk_len = P.rows[k0 + P.ploidy - 1].out_off + P.rows[k0 + P.ploidy - 1].length - blk0;

@@ -248,6 +248,24 @@ int gvl_dev_realign_tracks_plan(gvl_ctx *ctx, const gvl_sparse_tables *tab, cons
                                 int64_t max_records, int layout_btp, gvl_stream stream);
 int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream);
 
+/* gvl_dev_realign_tracks_plan with an explicit destination for every row in place of a fixed layout (`layout_btp` is
+ * replaced by the table); followed by gvl_dev_realign_tracks_exec like the plan it extends.
+ *   row_dst      device i64[b*p]: flat index in `out` of value 0 of row k = q*p + h for track 0
+ *   row_tstride  device i64[b*p]: distance from track t to track t+1 of row k
+ * Row k of track t goes to out[row_dst[k] + t*row_tstride[k] ...], out_offsets[k+1]-out_offsets[k] values, reversed on
+ * masked rows as in the other layouts.  The caller guarantees that the ranges of all (row, track) pairs are disjoint and
+ * lie inside [0, n_tracks*total_per_track): every value is then written exactly once when they cover the buffer.
+ * out_offsets still gives each row's length and must be gap-free.  Used for spliced output: the elements of a splice row
+ * are separate rows written straight into their place in the concatenation. */
+int gvl_dev_realign_tracks_plan_rows(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                                     const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
+                                     int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
+                                     int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                                     const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
+                                     const int32_t *strategy_ids, const double *params, uint64_t base_seed,
+                                     const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
+                                     int64_t max_records, const int64_t *row_dst, const int64_t *row_tstride, gvl_stream stream);
+
 /* shift_and_realign_tracks_sparse on device (src/ffi/mod.rs:2439-2458): ONE track whose source is
  * a dense f32 window per query (`tracks` ragged by `track_offsets` i64[b+1]) instead of intervals.
  * track_lengths[q] = track_offsets[q+1]-track_offsets[q] as device i32[b]. */
@@ -283,6 +301,14 @@ int gvl_dev_intervals_to_tracks(gvl_ctx *ctx, const gvl_intervals *itv, const in
 int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
                          const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
                          const uint8_t *to_rc, float *out, gvl_stream stream);
+
+/* gvl_dev_paint_tracks with an explicit destination for every query (row_dst / row_tstride: device i64[n_queries], the
+ * same table and the same caller guarantee as gvl_dev_realign_tracks_plan_rows): row (q, t) starts at
+ * out[row_dst[q] + t*row_tstride[q]]. */
+int gvl_dev_paint_tracks_rows(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                              const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                              const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, float *out,
+                              gvl_stream stream);
 
 /* ---- device layer: the small entries either side of reconstruction ------------------ */
 /* choose_exonic_variants, src/ffi/mod.rs:229-238 -> src/genotypes/mod.rs:132-176: for every (query, hap) row,
