@@ -98,16 +98,7 @@ class Dataset:
         eng = Engine(device, reference, ref_offsets, v_starts, ilens, alt_alleles, alt_offsets, geno_v_idxs, geno_offsets)
         if ref_alleles is not None or variant_info or dosages is not None:
             eng.set_variant_fields(ref_alleles, variant_info, dosages)
-        kinds = {}
-        for name, t in (tracks or {}).items():
-            eng.add_track(name, *t)
-            kinds[name] = (track_kinds or {}).get(name, "sample")
-        regions = np.ascontiguousarray(regions, np.int32)
-        if regions.shape[1] == 3:
-            regions = np.concatenate([regions, np.ones((len(regions), 1), np.int32)], 1)
-        names = tuple(sample_names) if sample_names is not None else tuple(f"s{i}" for i in range(n_samples))
-        return cls(engine=eng, full_regions=regions, sample_names=names, ploidy=int(ploidy), max_jitter=int(max_jitter),
-                   track_kinds=kinds, active_tracks=tuple(kinds), rng=np.random.default_rng(rng))
+        return cls._from_engine(eng, regions, n_samples, ploidy, max_jitter, tracks, track_kinds, sample_names, rng)
 
     @classmethod
     def from_synth(cls, device, d, rng=None, svar2=None) -> "Dataset":
@@ -128,17 +119,8 @@ class Dataset:
         (python/genvarloader/_dataset/_svar2_haps.py:183): per-(region, sample, ploid) var_key ranges, per-region dense
         windows and presence bits (docs/source/format.md:88-96) stay in HBM, every read merges the two channels on the
         device (src/svar2/mod.rs:45-66).  `sv`: see `synth.to_svar2_dataset` for the arrays."""
-        regions = np.ascontiguousarray(regions, np.int32)
         eng = Engine.from_svar2(device, reference, ref_offsets, sv, len(regions) * int(n_samples) * int(ploidy))
-        kinds = {}
-        for name, t in (tracks or {}).items():
-            eng.add_track(name, *t)
-            kinds[name] = (track_kinds or {}).get(name, "sample")
-        if regions.shape[1] == 3:
-            regions = np.concatenate([regions, np.ones((len(regions), 1), np.int32)], 1)
-        names = tuple(sample_names) if sample_names is not None else tuple(f"s{i}" for i in range(n_samples))
-        return cls(engine=eng, full_regions=regions, sample_names=names, ploidy=int(ploidy), max_jitter=int(max_jitter),
-                   track_kinds=kinds, active_tracks=tuple(kinds), rng=np.random.default_rng(rng))
+        return cls._from_engine(eng, regions, n_samples, ploidy, max_jitter, tracks, track_kinds, sample_names, rng)
 
     @classmethod
     def open(cls, path, reference=None, device="cuda", jitter: int = 0, rng=None, deterministic: bool = True,
@@ -170,13 +152,26 @@ class Dataset:
                          pad_char=ref.pad_char)
         if has_geno and (a.get("ref_alleles") is not None or a.get("variant_info")):
             eng.set_variant_fields(a.get("ref_alleles"), a.get("variant_info"))  # "variants" output: REF strings, INFO columns
-        for name, t in a["tracks"].items():
-            eng.add_track(name, *t)
-        ds = cls(engine=eng, full_regions=a["full_regions"], sample_names=tuple(samples), ploidy=ploidy,
-                 max_jitter=a["max_jitter"], track_kinds=dict(a["track_kinds"]), active_tracks=tuple(a["track_kinds"]),
-                 sequence_type="haplotypes" if has_geno else None, rng=np.random.default_rng(rng),
-                 region_map=np.ascontiguousarray(a["region_map"], np.int64), bed_columns=a.get("bed_columns"))
+        ds = cls._from_engine(eng, a["full_regions"], len(samples), ploidy, a["max_jitter"], a["tracks"], a["track_kinds"],
+                              samples, rng, sequence_type="haplotypes" if has_geno else None,
+                              region_map=np.ascontiguousarray(a["region_map"], np.int64), bed_columns=a.get("bed_columns"))
         return ds.with_settings(jitter=jitter, deterministic=deterministic, rc_neg=rc_neg)
+
+    @classmethod
+    def _from_engine(cls, eng, regions, n_samples: int, ploidy: int, max_jitter: int, tracks, track_kinds, sample_names, rng,
+                     **settings) -> "Dataset":
+        """The common tail of the constructors: register `tracks` on `eng` (kind "sample" unless `track_kinds` says
+        otherwise), give 3-column regions a + strand, name the samples s0, s1, ... unless named."""
+        kinds = {}
+        for name, t in (tracks or {}).items():
+            eng.add_track(name, *t)
+            kinds[name] = (track_kinds or {}).get(name, "sample")
+        regions = np.ascontiguousarray(regions, np.int32)
+        if regions.shape[1] == 3:
+            regions = np.concatenate([regions, np.ones((len(regions), 1), np.int32)], 1)
+        names = tuple(sample_names) if sample_names is not None else tuple(f"s{i}" for i in range(n_samples))
+        return cls(engine=eng, full_regions=regions, sample_names=names, ploidy=int(ploidy), max_jitter=int(max_jitter),
+                   track_kinds=kinds, active_tracks=tuple(kinds), rng=np.random.default_rng(rng), **settings)
 
     # ------------------------------------------------------------------ properties (reference: _impl.py:954-1110)
     @property
@@ -664,9 +659,8 @@ class Dataset:
         eng, dev, p, S = self.engine, self.engine.device, self.ploidy, len(self.sample_names)
         is_ref = seq == "reference"
         rows_p = 1 if is_ref else p  # sequence rows per element
-        names = list(self.active_tracks)
-        t = len(names)
-        realign = t > 0 and seq in ("haplotypes", "annotated") and self.realign_tracks
+        t = len(self.active_tracks)
+        realign = self._realigns
 
         # ---- the element batch E: (pair, element) in output order
         elems = [rows_all[r] for r, _ in pairs]
@@ -702,7 +696,7 @@ class Dataset:
             cell_starts = (rows_p * e_first[:-1, None] + np.arange(rows_p, dtype=np.int64)[None, :] * n_el[:, None]).ravel()
             i_cs = pk.add(np.append(cell_starts, rows_p * e_first[-1]), np.int64)
         if t:
-            oi = np.stack([ds_idx_e if self.track_kinds[n] == "sample" else e_reg for n in names])
+            oi = np.stack([ds_idx_e if self.track_kinds[n] == "sample" else e_reg for n in self.active_tracks])
             i_oi = pk.add(oi, np.int64)
             if realign:
                 i_reg = pk.add(regions[:, :3], np.int32)
@@ -733,25 +727,13 @@ class Dataset:
             keep = keep_off = None
             if self.var_filter == "exonic" and not is_ref:
                 keep, keep_off = self._exonic_keep(pk.get(i_sgoi), pk.get(i_sreg), s_goi)
-            diffs = torch.empty((len(s_goi), 1), dtype=torch.int32, device=dev) if realign else None
-            oo = eng.plan(pk.get(i_sreg), pk.get(i_ssh), pk.get(i_sgoi), -1, max_rec, keep, keep_off,
-                          pk.get(i_src) if i_src is not None else None, diffs=diffs, use_svar2=not is_ref)
-            total = eng.total()
+            oo, total, diffs = self._plan_seqs(pk.get(i_sreg), pk.get(i_ssh), pk.get(i_sgoi), -1, max_rec, keep, keep_off,
+                                               pk.get(i_src) if i_src is not None else None)
             group_offsets = oo[pk.get(i_cs)]
-            shape = (*outer, None) if is_ref else (*outer, p, None)
-            if seq == "annotated":
-                hh, av, ap = eng.execute("annotated")
-                results.append(RaggedAnnotatedHaps(Ragged(hh, group_offsets, shape), Ragged(av, group_offsets, shape),
-                                                   Ragged(ap, group_offsets, shape)))
-            elif self.encoding == "onehot":
-                results.append(Ragged(eng.execute("onehot").view(total, 4), group_offsets, shape))
-            else:
-                results.append(Ragged(eng.execute("haplotypes"), group_offsets, shape))
+            results.append(self._execute_seqs(group_offsets, (*outer, None) if is_ref else (*outer, p, None), total))
         if t and realign:
             # rows (e, h) of E; their haplotypes are sequence rows q[e, h] of the plan above
             t_q = pk.get(i_q)
-            diffs_e = diffs.view(-1)[t_q]
-            track_lengths = (pk.get(i_len) - diffs_e.clamp(max=0).min(1).values.to(torch.int64)).to(torch.int32)
             row_len = (oo[1:] - oo[:-1])[t_q].reshape(-1)
             out_offsets = torch.zeros(n_e * p + 1, dtype=torch.int64, device=dev)
             torch.cumsum(row_len, 0, out=out_offsets[1:])
@@ -761,24 +743,14 @@ class Dataset:
             keep = keep_off = None
             if self.var_filter == "exonic":
                 keep, keep_off = self._exonic_keep(pk.get(i_goi_e), pk.get(i_reg), goi_e)
-            ids, params = lower([self.insertion_fill.get(n, Repeat5p()) for n in names])
-            if self.deterministic:
-                base_seed = int(np.bitwise_xor.reduce(ds_idx_e.astype(np.uint64)))  # _reconstruct.py:215-218
-            else:
-                base_seed = int(self.rng.integers(0, np.iinfo(np.uint64).max, dtype=np.uint64))  # :219-222
-            out = eng.realign_tracks(names, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), track_lengths,
-                                     out_offsets, total, ids, params, base_seed, max_rec, keep, keep_off,
-                                     pk.get(i_rc_e) if i_rc_e is not None else None, layout="rows", row_dst=row_dst,
-                                     row_tstride=row_tstride)
-            lens = (group_offsets[1:] - group_offsets[:-1]).view(n_pairs, 1, p).expand(n_pairs, t, p).reshape(-1)
-            offsets = torch.zeros(n_pairs * t * p + 1, dtype=torch.int64, device=dev)
-            torch.cumsum(lens, 0, out=offsets[1:])
-            results.append(Ragged(out, offsets, (*outer, t, p, None)))
+            results.append(self._realigned_tracks(
+                ds_idx_e, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), pk.get(i_len), diffs.view(-1)[t_q],
+                out_offsets, total, max_rec, keep, keep_off, pk.get(i_rc_e) if i_rc_e is not None else None, group_offsets,
+                (*outer, t, p, None), row_dst=row_dst, row_tstride=row_tstride))
         elif t:
-            out = eng.paint_tracks(names, pk.get(i_oi), pk.get(i_st), pk.get(i_off_e), int(off_e[-1]),
-                                   pk.get(i_rc_q) if i_rc_q is not None else None, layout="rows", row_dst=pk.get(i_dst),
-                                   row_tstride=pk.get(i_ts))
-            results.append(Ragged(out, pk.get(i_toff), (*outer, t, None)))
+            results.append(self._painted_tracks(pk.get(i_oi), pk.get(i_st), pk.get(i_off_e), int(off_e[-1]),
+                                                pk.get(i_rc_q) if i_rc_q is not None else None, pk.get(i_toff),
+                                                (*outer, t, None), row_dst=pk.get(i_dst), row_tstride=pk.get(i_ts)))
         if self.output_length == "variable" and self.output_format != "flat":  # pad like the unspliced path (_query.py:94-127)
             results = [self._shape_output(o, None, False) for o in results]
         if is_int(r_sel) and is_int(s_sel):
@@ -876,8 +848,6 @@ class Dataset:
         want_seqs = self.sequence_type is not None
         want_tracks = len(self.active_tracks) > 0
         is_ref = self.sequence_type == "reference"
-        realign = (want_tracks and want_seqs and not is_ref and self.realign_tracks
-                   and self.sequence_type not in ("variants", "variant-windows"))
         to_rc_q = (self.full_regions[r_idx, 3] == -1) if self.rc_neg else None
         lengths = (regions[:, 2] - regions[:, 1]).astype(np.int64)
 
@@ -925,57 +895,85 @@ class Dataset:
                                    max_records=max_rec).cpu().numpy()
                 max_shift = dd.clip(min=0) + (lengths - out_len).clip(min=0)[:, None]
                 t_shifts = torch.from_numpy(self.rng.integers(0, max_shift + 1, dtype=np.int32)).to(dev)
-            if realign:
-                diffs = torch.empty((b, rows_p), dtype=torch.int32, device=dev)
-            oo = eng.plan(t_reg, t_shifts, t_goi, out_len, max_rec, keep, keep_off, t_rc, diffs=diffs, use_svar2=not is_ref)
-            total = eng.total()
-            shape = (b, None) if is_ref else (b, p, None)  # Ref has no ploidy axis (_dataset/_ref.py)
-            if self.sequence_type == "annotated":
-                h, av, ap = eng.execute("annotated")
-                results.append(RaggedAnnotatedHaps(Ragged(h, oo, shape), Ragged(av, oo, shape), Ragged(ap, oo, shape)))
-            elif self.encoding == "bytes":
-                results.append(Ragged(eng.execute("haplotypes"), oo, shape))
-            elif self.encoding == "onehot":
-                results.append(Ragged(eng.execute("onehot").view(total, 4), oo, shape))
-            else:
-                cf = eng.execute("onehot_cf")
-                results.append(cf.view(b, 4, out_len) if is_ref else cf.view(b, p, 4, out_len))
+            oo, total, diffs = self._plan_seqs(t_reg, t_shifts, t_goi, out_len, max_rec, keep, keep_off, t_rc)
+            # Ref has no ploidy axis (_dataset/_ref.py)
+            results.append(self._execute_seqs(oo, (b, None) if is_ref else (b, p, None), total))
         if want_tracks:
-            names = list(self.active_tracks)
-            t = len(names)
-            if realign:
-                # HapsTracks.__call__, _reconstruct.py:182-300
-                lengths_d = torch.from_numpy(lengths).to(dev)
-                track_lengths = (lengths_d - diffs.clamp(max=0).min(1).values.to(torch.int64)).to(torch.int32)
-                ids, params = lower([self.insertion_fill.get(n, Repeat5p()) for n in names])
-                if self.deterministic:
-                    base_seed = int(np.bitwise_xor.reduce(ds_idx.astype(np.uint64)))  # :215-218
-                else:
-                    base_seed = int(self.rng.integers(0, np.iinfo(np.uint64).max, dtype=np.uint64))  # :219-222
-                # the reference's flat buffer is track-major (_reconstruct.py:238) while its offsets describe
-                # (b, t, p, ~l) (:292-300); the kernel writes the latter directly so data and offsets agree for t > 1
-                out = eng.realign_tracks(names, t_reg, t_shifts, t_goi, pk.get(i_tr), track_lengths, oo, total, ids, params,
-                                         base_seed, max_rec, keep, keep_off, t_rc, layout="btp")
-                lens_bp = (oo[1:] - oo[:-1]).view(b, p)
-                lens = lens_bp.view(b, 1, p).expand(b, t, p).reshape(-1)
-                offsets = torch.zeros(b * t * p + 1, dtype=torch.int64, device=dev)
-                torch.cumsum(lens, 0, out=offsets[1:])
-                results.append(Ragged(out, offsets, (b, t, p, None)))
+            t = len(self.active_tracks)
+            if self._realigns:
+                results.append(self._realigned_tracks(ds_idx, t_reg, t_shifts, t_goi, pk.get(i_tr), torch.from_numpy(lengths).to(dev),
+                                                      diffs, oo, total, max_rec, keep, keep_off, t_rc, oo, (b, t, p, None)))
             else:
-                # Tracks alone / un-realigned: paint the stored intervals (Tracks._call_float32, _tracks.py:370-420)
                 out_len_q = np.full(b, int(self.output_length), np.int64) if fixed else lengths
                 offs = np.concatenate([[0], np.cumsum(out_len_q)]).astype(np.int64)
                 d_off = torch.from_numpy(offs).to(dev)
-                starts = t_reg[:, 1].contiguous()
-                per = int(offs[-1])
-                # all tracks in one launch, written in (b, t, ~l) order, negative-strand rows reversed
-                out = eng.paint_tracks(names, pk.get(i_tr), starts, d_off, per, pk.get(i_trc) if i_trc is not None else None)
-                lens_q = d_off[1:] - d_off[:-1]
-                lens = lens_q.view(b, 1).expand(b, t).reshape(-1)
-                offsets = torch.zeros(b * t + 1, dtype=torch.int64, device=dev)
-                torch.cumsum(lens, 0, out=offsets[1:])
-                results.append(Ragged(out, offsets, (b, t, None)))
+                results.append(self._painted_tracks(pk.get(i_tr), t_reg[:, 1].contiguous(), d_off, int(offs[-1]),
+                                                    pk.get(i_trc) if i_trc is not None else None, _cell_offsets(d_off, t),
+                                                    (b, t, None)))
         return tuple(results)
+
+    # ---- read steps shared by the unspliced (_reconstruct) and spliced (_getitem_spliced) reads
+    @property
+    def _realigns(self) -> bool:
+        """Tracks are realigned to the haplotypes; otherwise their stored intervals are painted over the regions."""
+        return bool(self.active_tracks) and self.sequence_type in ("haplotypes", "annotated") and self.realign_tracks
+
+    def _fills(self, names) -> tuple:
+        """(strategy ids, parameters) of the insertion fills of the tracks `names` (Repeat5p unless set)."""
+        return lower([self.insertion_fill.get(n, Repeat5p()) for n in names])
+
+    def _fill_seed(self, ds_idx) -> int:
+        """Base seed of a realignment call over the dataset indices `ds_idx`."""
+        if self.deterministic:
+            return int(np.bitwise_xor.reduce(ds_idx.astype(np.uint64)))  # _reconstruct.py:215-218
+        return int(self.rng.integers(0, np.iinfo(np.uint64).max, dtype=np.uint64))  # :219-222
+
+    def _plan_seqs(self, t_reg, t_shifts, t_goi, out_len: int, max_rec: int, keep, keep_off, t_rc):
+        """Plan one sequence row per entry of `t_goi`: (row offsets, total length, per-row diffs for realigned tracks or
+        None)."""
+        eng = self.engine
+        diffs = torch.empty(tuple(t_goi.shape), dtype=torch.int32, device=eng.device) if self._realigns else None
+        oo = eng.plan(t_reg, t_shifts, t_goi, out_len, max_rec, keep, keep_off, t_rc, diffs=diffs,
+                      use_svar2=self.sequence_type != "reference")
+        return oo, eng.total(), diffs
+
+    def _execute_seqs(self, offsets, shape, total: int):
+        """Execute the planned rows in this dataset's sequence output: ragged over `offsets` with `shape`, or dense
+        (`shape` without its ragged axis) for channels-first one-hot."""
+        eng = self.engine
+        if self.sequence_type == "annotated":
+            h, av, ap = eng.execute("annotated")
+            return RaggedAnnotatedHaps(Ragged(h, offsets, shape), Ragged(av, offsets, shape), Ragged(ap, offsets, shape))
+        if self.encoding == "bytes":
+            return Ragged(eng.execute("haplotypes"), offsets, shape)
+        if self.encoding == "onehot":
+            return Ragged(eng.execute("onehot").view(total, 4), offsets, shape)
+        return eng.execute("onehot_cf").view(*shape[:-1], 4, int(self.output_length))
+
+    def _realigned_tracks(self, ds_idx, t_reg, t_shifts, t_goi, t_oi, lengths, diffs, row_offsets, total: int, max_rec: int,
+                          keep, keep_off, t_rc, seq_offsets, shape, **rows) -> Ragged:
+        """All active tracks realigned to planned haplotype rows in one call (HapsTracks.__call__, _reconstruct.py:182-300).
+        One query per row of `t_goi` (dataset indices `ds_idx`, region `lengths`, planned `diffs`); its values go to
+        `row_offsets` in (query, track, ploid) order or, given `row_dst` / `row_tstride`, where that table puts them.
+        The (cell, track, ploid) rows take the lengths of the sequence rows at `seq_offsets`."""
+        names = list(self.active_tracks)
+        ids, params = self._fills(names)
+        # a query's track window is its region less its longest net deletion (_reconstruct.py:191-196)
+        track_lengths = (lengths - diffs.clamp(max=0).min(1).values.to(torch.int64)).to(torch.int32)
+        # the reference's flat buffer is track-major (_reconstruct.py:238) while its offsets describe (b, t, p, ~l)
+        # (:292-300); the kernel writes the latter directly so data and offsets agree for t > 1
+        out = self.engine.realign_tracks(names, t_reg, t_shifts, t_goi, t_oi, track_lengths, row_offsets, total, ids, params,
+                                         self._fill_seed(ds_idx), max_rec, keep, keep_off, t_rc,
+                                         layout="rows" if rows else "btp", **rows)
+        return Ragged(out, _cell_offsets(seq_offsets, len(names), self.ploidy), shape)
+
+    def _painted_tracks(self, t_oi, starts, row_offsets, total: int, t_rc, offsets, shape, **rows) -> Ragged:
+        """The stored intervals of all active tracks painted in one launch (Tracks._call_float32, _tracks.py:370-420),
+        negative-strand rows reversed, in (query, track) order or, given `row_dst` / `row_tstride`, where that table puts
+        each row.  `offsets`: of the output cells."""
+        out = self.engine.paint_tracks(list(self.active_tracks), t_oi, starts, row_offsets, total, t_rc,
+                                       layout="rows" if rows else "btp", **rows)
+        return Ragged(out, offsets, shape)
 
     def _get_variants(self, t_goi, t_rc, b: int, regions, n_variants: int) -> RaggedVariants:
         p, eng = self.ploidy, self.engine
@@ -1037,6 +1035,15 @@ class Dataset:
         return res
 
 
+def _cell_offsets(row_offsets: torch.Tensor, t: int, p: int = 1) -> torch.Tensor:
+    """Offsets of track cells (n, t, p) whose lengths are those of the sequence rows (n, p) at `row_offsets`."""
+    n = (row_offsets.numel() - 1) // p
+    lens = (row_offsets[1:] - row_offsets[:-1]).view(n, 1, p).expand(n, t, p).reshape(-1)
+    offsets = torch.zeros(n * t * p + 1, dtype=torch.int64, device=row_offsets.device)
+    torch.cumsum(lens, 0, out=offsets[1:])
+    return offsets
+
+
 class _Packer:
     """All O(batch) host arrays of one call in ONE pinned buffer and ONE async H2D copy."""
 
@@ -1075,41 +1082,21 @@ class BatchLoader:
             raise ValueError("batch_size must be a positive integer")
         self.ds, self.batch_size, self.shuffle, self.sampler = ds, batch_size, shuffle, sampler
         self.drop_last, self.return_indices, self.transform = drop_last, return_indices, transform
-        if generator is None or isinstance(generator, (int, np.integer)):
-            self._rng = np.random.default_rng(generator)
-        elif isinstance(generator, np.random.Generator):
-            self._rng = generator
-        else:  # torch.Generator
-            self._rng = np.random.default_rng(int(generator.initial_seed()))
+        self._rng = _as_rng(generator)
 
     def __len__(self) -> int:
         n = len(self.sampler) if self.sampler is not None else len(self.ds)
         return n // self.batch_size if self.drop_last else -(-n // self.batch_size)
 
     def __iter__(self):
-        if self.sampler is not None:
-            order = (np.ascontiguousarray(self.sampler, np.int64).ravel() if isinstance(self.sampler, np.ndarray)
-                     else np.fromiter(iter(self.sampler), np.int64))
-        elif self.shuffle:
-            order = self._rng.permutation(len(self.ds))
-        else:
-            order = np.arange(len(self.ds), dtype=np.int64)
+        order = epoch_order(self.ds, self.sampler, self.shuffle, self._rng)
         n_s = self.ds.n_samples
         for lo in range(0, len(order), self.batch_size):
             idx = order[lo: lo + self.batch_size]
             if len(idx) < self.batch_size and self.drop_last:
                 return
             r, s_ = idx // n_s, idx % n_s  # np.unravel_index(idx, dataset.shape), _torch.py:293
-            batch = self.ds[r, s_]
-            if not isinstance(batch, tuple):
-                batch = (batch,)
-            if self.return_indices:  # the (region, sample) indices the dataset was indexed with, _torch.py:299-300
-                batch = (*batch, r, s_)
-            if self.transform is not None:
-                batch = self.transform(*batch)  # _torch.py:302-303
-            elif len(batch) == 1:
-                batch = batch[0]
-            yield batch
+            yield _batch_tail(self.ds[r, s_], (r, s_) if self.return_indices else None, self.transform)
 
 
 class _MapDataset:
@@ -1124,11 +1111,36 @@ class _MapDataset:
 
     def __getitem__(self, idx):
         r_idx, s_idx = np.unravel_index(idx, self.dataset.shape)
-        batch = self.dataset[r_idx, s_idx]
-        if not isinstance(batch, tuple):
-            batch = (batch,)
-        if self.include_indices:
-            batch = (*batch, r_idx, s_idx)
-        if self.transform is not None:
-            return self.transform(*batch)
-        return batch[0] if len(batch) == 1 else batch
+        return _batch_tail(self.dataset[r_idx, s_idx], (r_idx, s_idx) if self.include_indices else None, self.transform)
+
+
+def _as_rng(generator) -> np.random.Generator:
+    """The numpy generator of a loader's `generator` argument: None / a seed, a numpy Generator or a torch.Generator."""
+    if generator is None or isinstance(generator, (int, np.integer)):
+        return np.random.default_rng(generator)
+    if isinstance(generator, np.random.Generator):
+        return generator
+    return np.random.default_rng(int(generator.initial_seed()))  # torch.Generator
+
+
+def epoch_order(ds, sampler, shuffle, rng) -> np.ndarray:
+    """Flat (region, sample) indices of one epoch, in the order the loader reads them."""
+    if sampler is not None:
+        if isinstance(sampler, np.ndarray):  # (an index array is its own sampler: no per-element iteration)
+            return np.ascontiguousarray(sampler, np.int64).ravel()
+        return np.fromiter(iter(sampler), np.int64)
+    if shuffle:
+        return rng.permutation(len(ds)).astype(np.int64)
+    return np.arange(len(ds), dtype=np.int64)
+
+
+def _batch_tail(batch, indices, transform):
+    """What a loader yields for one batch: its outputs, then the (region, sample) `indices` it was read with unless None
+    (_torch.py:299-300), passed through `transform` (_torch.py:302-303); a lone output is returned bare."""
+    if not isinstance(batch, tuple):
+        batch = (batch,)
+    if indices is not None:
+        batch = (*batch, *indices)
+    if transform is not None:
+        return transform(*batch)
+    return batch[0] if len(batch) == 1 else batch

@@ -513,6 +513,27 @@ class Engine:
         return diffs
 
     # ------------------------------------------------------------------ tracks
+    def track_descs(self, names, strategy_ids=None, params=None):
+        """Descriptor arrays of a track call: the interval table of every track in `names` and, for realignment, its
+        insertion-fill id and parameter (None, None when painting)."""
+        n = len(names)
+        itv = (Intervals * n)(*[self.tracks[x][4] for x in names])
+        if strategy_ids is None:
+            return itv, None, None
+        return itv, (c_i32 * n)(*[int(s) for s in strategy_ids]), (C.c_double * n)(*[float(p) for p in params])
+
+    def _realign_args(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets, total_per_track,
+                      strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc, query_seed, base_seed_dev, batch,
+                      sub_batch):
+        """The arguments every gvl_dev_realign_tracks* entry takes after its variant source and before its layout."""
+        b_cap, ploidy = geno_offset_idx.shape
+        batch = b_cap if batch is None else int(batch)  # (a prefix of preallocated buffers)
+        itv, sid, par = self.track_descs(names, strategy_ids, params)
+        return (ptr(regions), ptr(shifts), ptr(geno_offset_idx), c_i64(batch), c_i64(ploidy), ptr(keep), ptr(keep_offsets),
+                ptr(to_rc), c_i64(len(names)), itv, ptr(offset_idxs), ptr(track_lengths), ptr(out_offsets),
+                c_i64(int(total_per_track)), sid, par, c_u64(int(base_seed)), ptr(base_seed_dev), c_i64(int(sub_batch)),
+                ptr(query_seed), c_i64(int(max_records)))
+
     def realign_tracks(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                        total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
                        keep_offsets=None, to_rc=None, query_seed=None, out=None, layout="tbp", base_seed_dev=None,
@@ -523,25 +544,18 @@ class Engine:
         gvl_dev_realign_tracks_btp: the order the reference's (b, t, p, ~l) offsets describe) or wherever the
         per-row table puts each row (layout="rows": row k of track t starts at row_dst[k] + t * row_tstride[k],
         device int64 (batch * ploidy,) each; gvl_dev_realign_tracks_plan_rows)."""
-        b_cap, ploidy = geno_offset_idx.shape
-        batch = b_cap if batch is None else int(batch)  # (a prefix of preallocated buffers)
-        n_tracks = len(names)
         if out is None:
-            out = torch.empty(n_tracks * total_per_track, dtype=torch.float32, device=self.device)
+            out = torch.empty(len(names) * total_per_track, dtype=torch.float32, device=self.device)
         if self.svar2 is not None or layout == "rows":
             self.realign_tracks_plan(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                                      total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
                                      query_seed, layout, base_seed_dev, batch, sub_batch, row_dst, row_tstride)
             return self.realign_tracks_exec(out)
-        itv = (Intervals * n_tracks)(*[self.tracks[n][4] for n in names])
-        sid = (c_i32 * n_tracks)(*[int(s) for s in strategy_ids])
-        par = (C.c_double * n_tracks)(*[float(p) for p in params])
+        args = self._realign_args(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
+                                  total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
+                                  query_seed, base_seed_dev, batch, sub_batch)
         fn = lib.gvl_dev_realign_tracks_btp if layout == "btp" else lib.gvl_dev_realign_tracks
-        check(fn(
-            self.ctx.handle, C.byref(self.tab), ptr(regions), ptr(shifts), ptr(geno_offset_idx), c_i64(batch),
-            c_i64(ploidy), ptr(keep), ptr(keep_offsets), ptr(to_rc), c_i64(n_tracks), itv, ptr(offset_idxs),
-            ptr(track_lengths), ptr(out_offsets), c_i64(int(total_per_track)), sid, par, c_u64(int(base_seed)),
-            ptr(base_seed_dev), c_i64(int(sub_batch)), ptr(query_seed), c_i64(int(max_records)), ptr(out), _stream()))
+        check(fn(self.ctx.handle, C.byref(self.tab), *args, ptr(out), _stream()))
         return out
 
     def realign_tracks_plan(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
@@ -551,28 +565,19 @@ class Engine:
         """gvl_dev_realign_tracks_plan (layout="rows": gvl_dev_realign_tracks_plan_rows): everything of `realign_tracks`
         but the execute launch (variant plan, tile map, per-tile searches); `realign_tracks_exec(out)` writes the values,
         possibly on another stream."""
-        b_cap, ploidy = geno_offset_idx.shape
-        batch = b_cap if batch is None else int(batch)
-        n_tracks = len(names)
-        itv = (Intervals * n_tracks)(*[self.tracks[n][4] for n in names])
-        sid = (c_i32 * n_tracks)(*[int(s) for s in strategy_ids])
-        par = (C.c_double * n_tracks)(*[float(p) for p in params])
+        if layout == "rows" and (row_dst is None or row_tstride is None):
+            raise ValueError('layout="rows" needs row_dst and row_tstride')
+        args = self._realign_args(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
+                                  total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
+                                  query_seed, base_seed_dev, batch, sub_batch)
         ch = self.svar2_channels(geno_offset_idx) if self.svar2 is not None else None
+        src = C.byref(ch) if ch is not None else c_vp(0)
         if layout == "rows":
-            if row_dst is None or row_tstride is None:
-                raise ValueError('layout="rows" needs row_dst and row_tstride')
-            check(lib.gvl_dev_realign_tracks_plan_rows(
-                self.ctx.handle, C.byref(self.tab), C.byref(ch) if ch is not None else None, ptr(regions), ptr(shifts),
-                ptr(geno_offset_idx), batch, ploidy, ptr(keep), ptr(keep_offsets), ptr(to_rc), n_tracks, itv, ptr(offset_idxs),
-                ptr(track_lengths), ptr(out_offsets), int(total_per_track), sid, par, int(base_seed), ptr(base_seed_dev),
-                int(sub_batch), ptr(query_seed), int(max_records), ptr(row_dst), ptr(row_tstride), _stream()))
-            return
-        check(lib.gvl_dev_realign_tracks_plan(
-            self.ctx.handle, C.byref(self.tab), C.byref(ch) if ch is not None else c_vp(0), ptr(regions), ptr(shifts),
-            ptr(geno_offset_idx), c_i64(batch), c_i64(ploidy),
-            ptr(keep), ptr(keep_offsets), ptr(to_rc), c_i64(n_tracks), itv, ptr(offset_idxs), ptr(track_lengths),
-            ptr(out_offsets), c_i64(int(total_per_track)), sid, par, c_u64(int(base_seed)), ptr(base_seed_dev),
-            c_i64(int(sub_batch)), ptr(query_seed), c_i64(int(max_records)), C.c_int(1 if layout == "btp" else 0), _stream()))
+            check(lib.gvl_dev_realign_tracks_plan_rows(self.ctx.handle, C.byref(self.tab), src, *args, ptr(row_dst),
+                                                       ptr(row_tstride), _stream()))
+        else:
+            check(lib.gvl_dev_realign_tracks_plan(self.ctx.handle, C.byref(self.tab), src, *args,
+                                                  C.c_int(1 if layout == "btp" else 0), _stream()))
 
     def realign_tracks_exec(self, out):
         check(lib.gvl_dev_realign_tracks_exec(self.ctx.handle, ptr(out), _stream()))
@@ -593,7 +598,7 @@ class Engine:
         masked rows reversed.  offset_idxs: int64 (n_tracks, batch) device.  layout="rows"
         (gvl_dev_paint_tracks_rows): query q of track t starts at row_dst[q] + t * row_tstride[q] instead."""
         n_tracks, n_q = len(names), int(starts.numel() if n_queries is None else n_queries)
-        itv = (Intervals * n_tracks)(*[self.tracks[n][4] for n in names])
+        itv = self.track_descs(names)[0]
         if out is None:
             out = torch.empty(n_tracks * int(total_per_track), dtype=torch.float32, device=self.device)
         if layout == "rows":

@@ -29,9 +29,9 @@ import numpy as np
 import torch
 
 from . import _ffi
+from ._dataset import _as_rng, _batch_tail, epoch_order
 from ._engine import MODES, Engine, _raw_stream, _stream
-from ._ffi import BatchArgs, DatasetView, FixedJob, Intervals, c_i32, c_i64, c_u8, c_u64, c_vp, check, lib, ptr
-from ._insertion_fill import Repeat5p, lower
+from ._ffi import BatchArgs, DatasetView, FixedJob, c_i64, c_u8, c_u64, c_vp, check, lib, ptr
 from ._types import AnnotatedHaps
 
 
@@ -69,7 +69,7 @@ class _Spec:
         self.annotated = ds.sequence_type == "annotated"
         self.names = list(ds.active_tracks)
         self.t = len(self.names)
-        self.realign = self.t > 0 and self.want_seqs and not self.is_ref and ds.realign_tracks
+        self.realign = ds._realigns
         self.rows_p = 1 if (self.is_ref or not self.want_seqs) else self.p
         self.rc_neg = bool(ds.rc_neg)
         self.jitter = int(ds.jitter)
@@ -83,7 +83,7 @@ class _Spec:
         for i, n in enumerate(self.names):
             if ds.track_kinds[n] == "annot":
                 self.annot_mask |= 1 << i
-        self.fill_ids, self.fill_params = lower([ds.insertion_fill.get(n, Repeat5p()) for n in self.names]) if self.t else ([], [])
+        self.fill_ids, self.fill_params = ds._fills(self.names)
 
 
 def supports(ds) -> str | None:
@@ -222,9 +222,7 @@ class FixedPipeline:
             keep.append(sv)
         itv = sid = par = None
         if sp.t:
-            itv = (Intervals * sp.t)(*[eng.tracks[n][4] for n in sp.names])
-            sid = (c_i32 * sp.t)(*[int(x) for x in sp.fill_ids])
-            par = (C.c_double * sp.t)(*[float(x) for x in sp.fill_params])
+            itv, sid, par = eng.track_descs(sp.names, sp.fill_ids, sp.fill_params)
             keep.extend([itv, sid, par])
         adr = lambda x: c_vp(C.addressof(x)) if x is not None else c_vp(0)
         mode = MODES[sp.mode] if sp.want_seqs else -1
@@ -491,24 +489,14 @@ class PipelinedLoader:
                     pipe.submit(h, flat, j)
                 continue
             for lo in range(0, len(chunk), b):
-                m = min(b, len(chunk) - lo)
-                batch = out.result(lo, m, clone=self.copy)
-                if not plain:
-                    batch = batch if isinstance(batch, tuple) else (batch,)
-                    if self.return_indices:  # the (region, sample) indices the dataset was indexed with, _torch.py:293-300
-                        c = chunk[lo: lo + m]
-                        batch = (*batch, c // n_s, c % n_s)
-                    if self.transform is not None:
-                        batch = self.transform(*batch)  # _torch.py:302-303
-                    elif len(batch) == 1:
-                        batch = batch[0]
-                yield batch
+                c = chunk[lo: lo + b]
+                yield _batch_tail(out.result(lo, len(c), clone=self.copy), (c // n_s, c % n_s) if self.return_indices else None,
+                                  self.transform)
             pipe.release(h)
             nxt = ring_i + pipe.n_halves
             if nxt < n_rings:
                 flat, j, chunks[nxt] = fill(nxt)
                 pipe.submit(h, flat, j)
-
 
     # ------------------------------------------------------------------ host delivery
     def _host_half(self, h: int):
@@ -545,37 +533,12 @@ class PipelinedLoader:
             ev.synchronize()  # the ring is in host memory
             chunk = chunks.pop(ring_i)
             for lo in range(0, len(chunk), b):
-                m = min(b, len(chunk) - lo)
-                batch = twin.result(lo, m, clone=self.copy)
+                c = chunk[lo: lo + b]
+                batch = twin.result(lo, len(c), clone=self.copy)
                 batch = tuple(x.numpy() if isinstance(x, torch.Tensor) else x for x in (batch if isinstance(batch, tuple) else (batch,)))
-                if self.return_indices:
-                    c = chunk[lo: lo + m]
-                    batch = (*batch, c // n_s, c % n_s)
-                if self.transform is not None:
-                    batch = self.transform(*batch)
-                elif len(batch) == 1:
-                    batch = batch[0]
-                yield batch
+                yield _batch_tail(batch, (c // n_s, c % n_s) if self.return_indices else None, self.transform)
             nxt = ring_i + pipe.n_halves
             if nxt < n_rings:  # (the consumer is past every batch of this half: its pinned twin may be overwritten)
                 flat, j, chunks[nxt] = fill(nxt)
                 pipe.submit(h, flat, j)
                 start_copy(h)
-
-
-def _as_rng(generator):
-    if generator is None or isinstance(generator, (int, np.integer)):
-        return np.random.default_rng(generator)
-    if isinstance(generator, np.random.Generator):
-        return generator
-    return np.random.default_rng(int(generator.initial_seed()))  # torch.Generator
-
-
-def epoch_order(ds, sampler, shuffle, rng) -> np.ndarray:
-    if sampler is not None:
-        if isinstance(sampler, np.ndarray):  # (an index array is its own sampler: no per-element iteration)
-            return np.ascontiguousarray(sampler, np.int64).ravel()
-        return np.fromiter(iter(sampler), np.int64)
-    if shuffle:
-        return rng.permutation(len(ds)).astype(np.int64)
-    return np.arange(len(ds), dtype=np.int64)
