@@ -10,7 +10,7 @@ Mirrors (names, argument meaning, error behaviour, return shapes):
 
 Host work per call is O(batch) numpy (index maths, RNG draws in the reference's order); everything
 sample-scale lives on the GPU inside `Engine`.  Results are torch CUDA tensors.
-Not supported (outside the hot-path scope, raise): fixed-length or jittered spliced output, spliced `variants`.
+Not supported (outside the hot-path scope, raise): fixed-length or jittered spliced output.
 """
 from __future__ import annotations
 
@@ -235,33 +235,50 @@ class Dataset:
             x = x.reshape(*out_reshape, x.shape[-1])
         return x
 
+    def _counts(self, regions, samples, per_index) -> np.ndarray:
+        """Counts of the selected (region, sample) pairs shaped like `ds[regions, samples]`: `per_index(ds_idx)` gives int32
+        (n, k) per dataset index.  A spliced (splice row, sample) sums the counts of its elements."""
+        idx = (slice(None) if regions is None else regions, slice(None) if samples is None else samples)
+        if self.splice_rows is None:
+            ds_idx, squeeze, out_reshape = self._parse_idx(idx)
+            return self._shape_counts(per_index(ds_idx), squeeze, out_reshape)
+        _, ds_idx_e, _, e_first, outer, squeeze = self._spliced_batch(idx)
+        n = per_index(ds_idx_e)
+        x = np.add.reduceat(n, e_first[:-1], axis=0).astype(np.int32).reshape(*outer, n.shape[1])
+        return x.reshape(n.shape[1]) if squeeze else x
+
     def n_variants(self, regions=None, samples=None) -> np.ndarray:
-        """`Dataset.n_variants`, _impl.py:1293-1340: variants per (region, sample, ploid) -> int32 (..., ploidy)."""
-        ds_idx, squeeze, out_reshape = self._parse_idx((slice(None) if regions is None else regions,
-                                                        slice(None) if samples is None else samples))
-        p = self.ploidy
-        goi = ds_idx[:, None] * p + np.arange(p, dtype=np.int64)[None, :]
+        """`Dataset.n_variants`, _impl.py:1293-1340: variants per (region, sample, ploid) -> int32 (..., ploidy).  Spliced:
+        per (splice row, sample, ploid), the sum over the row's elements."""
         if self.engine.svar2 is not None:
             raise NotImplementedError("n_variants of an svar2-backed dataset needs the presence-bit popcounts (not kept on the host)")
-        go = self.engine.geno_offsets_host
-        n = np.maximum(go[1, goi] - go[0, goi], 0).astype(np.int32)
-        return self._shape_counts(n, squeeze, out_reshape)
+        p, go = self.ploidy, self.engine.geno_offsets_host
+
+        def per_index(ds_idx):
+            goi = ds_idx[:, None] * p + np.arange(p, dtype=np.int64)[None, :]
+            return np.maximum(go[1, goi] - go[0, goi], 0).astype(np.int32)
+
+        return self._counts(regions, samples, per_index)
 
     def n_intervals(self, regions=None, samples=None) -> np.ndarray:
-        """`Dataset.n_intervals`, _impl.py:1848-1895: stored intervals per (region, sample) and ACTIVE track -> int32 (..., tracks)."""
-        ds_idx, squeeze, out_reshape = self._parse_idx((slice(None) if regions is None else regions,
-                                                        slice(None) if samples is None else samples))
-        if not self.active_tracks:
-            return self._shape_counts(np.zeros((len(ds_idx), 0), np.int32), squeeze, out_reshape)
-        r_idx = ds_idx // len(self.sample_names)
-        cols = []
+        """`Dataset.n_intervals`, _impl.py:1848-1895: stored intervals per (region, sample) and ACTIVE track -> int32 (..., tracks).
+        Spliced: per (splice row, sample, track), the sum over the row's elements (annotation tracks read the element's slot)."""
+        offs = []
         for name in self.active_tracks:
             off = self._cache.get(("itv_off", name))
             if off is None:
                 off = self._cache[("itv_off", name)] = self.engine.tracks[name][3].cpu().numpy()
-            slot = r_idx if self.track_kinds[name] == "annot" else ds_idx
-            cols.append((off[slot + 1] - off[slot]).astype(np.int32))
-        return self._shape_counts(np.stack(cols, -1), squeeze, out_reshape)
+            offs.append((off, self.track_kinds[name] == "annot"))
+
+        def per_index(ds_idx):
+            r_idx = ds_idx // len(self.sample_names)
+            cols = []
+            for off, annot in offs:
+                slot = r_idx if annot else ds_idx
+                cols.append((off[slot + 1] - off[slot]).astype(np.int32))
+            return np.stack(cols, -1) if cols else np.zeros((len(ds_idx), 0), np.int32)
+
+        return self._counts(regions, samples, per_index)
 
     def haplotype_lengths(self, regions=None, samples=None):
         """`Dataset.haplotype_lengths`, _impl.py:1234-1291: lengths of the JITTER-EXTENDED haplotypes -> int32 (..., ploidy);
@@ -620,6 +637,32 @@ class Dataset:
     def is_spliced(self) -> bool:
         return self.splice_rows is not None
 
+    def _spliced_batch(self, idx):
+        """The element batch E of a spliced selection `idx` (the index forms of `ds[...]`): every (element region, sample)
+        of the selected (splice row, sample) pairs, pairs in output order and a pair's elements in splice-row order ->
+        (e_reg, ds_idx_e, n_el, e_first, outer, squeeze).  Two paired arrays select pairs, `outer = (pairs,)`; any other
+        form selects the outer product, `outer = (rows, samples)`, squeezed away by an int/int index."""
+        if not isinstance(idx, tuple):
+            idx = (idx, slice(None))
+        r_sel, s_sel = idx
+        rows_all = self.splice_rows
+        ri = np.atleast_1d(_idx_to_array(r_sel, len(rows_all)))
+        si = np.atleast_1d(self._s_idx[_idx_to_array(s_sel, len(self._s_idx))])
+        is_int = lambda x: isinstance(x, (int, np.integer))
+        is_basic = lambda x: isinstance(x, (int, np.integer, slice))
+        if not is_basic(r_sel) and not is_basic(s_sel):  # paired
+            ri, si = (a.ravel() for a in np.broadcast_arrays(ri, si))
+            outer = (ri.size,)
+        else:
+            outer = (ri.size, si.size)
+            ri, si = np.repeat(ri.ravel(), si.size), np.tile(si.ravel(), ri.size)
+        elems = [rows_all[r] for r in ri.tolist()]
+        n_el = np.array([len(e) for e in elems], np.int64)                # K_c
+        e_first = np.concatenate([[0], np.cumsum(n_el)]).astype(np.int64)  # first element of pair c in E
+        e_reg = np.concatenate(elems).astype(np.int64)
+        ds_idx_e = e_reg * len(self.sample_names) + np.repeat(si, n_el)
+        return e_reg, ds_idx_e, n_el, e_first, outer, is_int(r_sel) and is_int(s_sel)
+
     def _getitem_spliced(self, idx):
         """One ragged sequence per (splice row, sample[, ploid]) and, with tracks active, one ragged track per (splice row,
         sample, track[, ploid]): a spliced cell is the concatenation, in splice-row order, of its elements' unspliced
@@ -634,43 +677,30 @@ class Dataset:
         call covers all of E and all active tracks -- realigned to the element haplotypes (rows (e, ploid)) or painted over
         the element regions (rows e) -- and writes every row straight into its place in the concatenated output through a
         per-row destination table (gvl_dev_realign_tracks_plan_rows / gvl_dev_paint_tracks_rows).  The values are those of
-        one unspliced call over E: the same fill seed (of E's dataset indices), FlankSample rows and track lengths."""
+        one unspliced call over E: the same fill seed (of E's dataset indices), FlankSample rows and track lengths.
+
+        Variants: the genotype rows of E are gathered in cell order -- (pair, ploid, element), or (pair, element, ploid)
+        under `unphased_union` so that the p rows folded into one belong to one element -- with every element's own strand
+        and contig, so each element row is its unspliced variants row (AF filter, dummy variant, strand, tokens) and a cell
+        is a contiguous run of rows: its offsets are the gathered row offsets sampled at cell boundaries."""
         if self.jitter or isinstance(self.output_length, (int, np.integer)):
             raise ValueError("spliced datasets return ragged haplotypes: use with_len('ragged') and jitter=0")
         seq = self.sequence_type
         if seq is not None and self.encoding == "onehot_cf":
             raise ValueError("channels-first one-hot needs a fixed output length; spliced output is ragged")
-        rows_all = self.splice_rows
-        n_rows_all, n_s_all = len(rows_all), len(self._s_idx)
-        if not isinstance(idx, tuple):
-            idx = (idx, slice(None))
-        r_sel, s_sel = idx
-        ri = np.atleast_1d(_idx_to_array(r_sel, n_rows_all))
-        si = np.atleast_1d(self._s_idx[_idx_to_array(s_sel, n_s_all)])
-        is_int = lambda x: isinstance(x, (int, np.integer))
-        is_basic = lambda x: isinstance(x, (int, np.integer, slice))
-        if not is_basic(r_sel) and not is_basic(s_sel):  # paired
-            ri, si = np.broadcast_arrays(ri, si)
-            pairs = list(zip(ri.ravel().tolist(), si.ravel().tolist()))
-            outer = (len(pairs),)
-        else:
-            pairs = [(r, s_) for r in ri.ravel().tolist() for s_ in si.ravel().tolist()]
-            outer = (ri.size, si.size)
-        eng, dev, p, S = self.engine, self.engine.device, self.ploidy, len(self.sample_names)
+        e_reg, ds_idx_e, n_el, e_first, outer, squeeze = self._spliced_batch(idx)
+        eng, dev, p = self.engine, self.engine.device, self.ploidy
         is_ref = seq == "reference"
+        is_var = seq in ("variants", "variant-windows")
+        fold = is_var and self.unphased_union
         rows_p = 1 if is_ref else p  # sequence rows per element
         t = len(self.active_tracks)
         realign = self._realigns
 
         # ---- the element batch E: (pair, element) in output order
-        elems = [rows_all[r] for r, _ in pairs]
-        n_pairs = len(pairs)
-        n_el = np.array([len(e) for e in elems], np.int64)               # K_c
-        e_first = np.concatenate([[0], np.cumsum(n_el)]).astype(np.int64)  # first element of pair c in E
-        e_reg = np.concatenate(elems).astype(np.int64)
+        n_pairs = n_el.size
         e_pair = np.repeat(np.arange(n_pairs, dtype=np.int64), n_el)
         e_k = np.arange(e_reg.size, dtype=np.int64) - e_first[e_pair]
-        ds_idx_e = e_reg * S + np.repeat(np.array([s_ for _, s_ in pairs], np.int64), n_el)
         regions = self.full_regions[e_reg]
         to_rc_e = (regions[:, 3] == -1) if self.rc_neg else None
         e_len = (regions[:, 2] - regions[:, 1]).astype(np.int64)
@@ -682,19 +712,26 @@ class Dataset:
         goi_e = ds_idx_e[:, None] * p + np.arange(p, dtype=np.int64)[None, :]
         pk = _Packer(dev)
         if seq is not None:
-            inv = np.empty(n_e * rows_p, np.int64)  # element of every sequence row
-            inv[q.ravel()] = np.repeat(np.arange(n_e, dtype=np.int64), rows_p)
-            if is_ref:
-                s_goi = np.full((n_e, 1), eng.empty_slot, np.int64)
+            if fold:  # variant rows (pair, element, ploid), folded to one per element: cell c = elements of pair c
+                inv = np.repeat(np.arange(n_e, dtype=np.int64), p)
+                s_goi = goi_e.reshape(-1, 1)
+                cell_starts = e_first
             else:
-                s_goi = np.empty((n_e * p, 1), np.int64)
-                s_goi[q.ravel(), 0] = goi_e.ravel()
-            i_sreg = pk.add(regions[inv, :3], np.int32)
+                inv = np.empty(n_e * rows_p, np.int64)  # element of every sequence row
+                inv[q.ravel()] = np.repeat(np.arange(n_e, dtype=np.int64), rows_p)
+                if is_ref:
+                    s_goi = np.full((n_e, 1), eng.empty_slot, np.int64)
+                else:
+                    s_goi = np.empty((n_e * p, 1), np.int64)
+                    s_goi[q.ravel(), 0] = goi_e.ravel()
+                cell_starts = (rows_p * e_first[:-1, None] + np.arange(rows_p, dtype=np.int64)[None, :] * n_el[:, None]).ravel()
+                cell_starts = np.append(cell_starts, rows_p * e_first[-1])
             i_sgoi = pk.add(s_goi, np.int64)
-            i_ssh = pk.add(np.zeros((len(s_goi), 1), np.int32), np.int32)
             i_src = pk.add(to_rc_e[inv], np.uint8) if to_rc_e is not None else None
-            cell_starts = (rows_p * e_first[:-1, None] + np.arange(rows_p, dtype=np.int64)[None, :] * n_el[:, None]).ravel()
-            i_cs = pk.add(np.append(cell_starts, rows_p * e_first[-1]), np.int64)
+            i_cs = pk.add(cell_starts, np.int64)
+            if not is_var:
+                i_sreg = pk.add(regions[inv, :3], np.int32)
+                i_ssh = pk.add(np.zeros((len(s_goi), 1), np.int32), np.int32)
         if t:
             oi = np.stack([ds_idx_e if self.track_kinds[n] == "sample" else e_reg for n in self.active_tracks])
             i_oi = pk.add(oi, np.int64)
@@ -723,7 +760,10 @@ class Dataset:
         results = []
         max_rec = 0 if is_ref else eng.max_records(goi_e)
         oo = group_offsets = total = None
-        if seq is not None:
+        if is_var:
+            results.append(self._get_variants(pk.get(i_sgoi), pk.get(i_src) if i_src is not None else None, regions[inv, 0],
+                                              max_rec, (*outer, 1 if fold else p, None), cells=pk.get(i_cs)))
+        elif seq is not None:
             keep = keep_off = None
             if self.var_filter == "exonic" and not is_ref:
                 keep, keep_off = self._exonic_keep(pk.get(i_sgoi), pk.get(i_sreg), s_goi)
@@ -753,7 +793,7 @@ class Dataset:
                                                 (*outer, t, None), row_dst=pk.get(i_dst), row_tstride=pk.get(i_ts)))
         if self.output_length == "variable" and self.output_format != "flat":  # pad like the unspliced path (_query.py:94-127)
             results = [self._shape_output(o, None, False) for o in results]
-        if is_int(r_sel) and is_int(s_sel):
+        if squeeze:
             results = [o.squeeze(0).squeeze(0) for o in results]
         return results[0] if len(results) == 1 else tuple(results)
 
@@ -795,8 +835,6 @@ class Dataset:
         if self.sequence_type is None and not self.active_tracks:
             raise ValueError("Dataset has neither sequences nor tracks active.")
         if self.splice_rows is not None:
-            if self.sequence_type in ("variants", "variant-windows"):
-                raise NotImplementedError("spliced 'variants' output is not built")
             return self._getitem_spliced(idx)
         ds_idx, squeeze, out_reshape = self._parse_idx(idx)
         pipe = self._eager_pipeline(len(ds_idx))
@@ -884,7 +922,8 @@ class Dataset:
         oo = total = diffs = None
         if self.sequence_type in ("variants", "variant-windows"):
             # Haps._get_variants -> get_variants_flat (_haps.py:602-609, _flat_variants.py:869-1112), on the device
-            results.append(self._get_variants(t_goi, t_rc, b, regions, max_rec))
+            results.append(self._get_variants(t_goi, t_rc, np.repeat(regions[:, 0], p), max_rec,
+                                              (b, 1 if self.unphased_union else p, None)))
             want_seqs = False
         if want_seqs:
             out_len = int(self.output_length) if fixed else -1
@@ -975,7 +1014,11 @@ class Dataset:
                                        layout="rows" if rows else "btp", **rows)
         return Ragged(out, offsets, shape)
 
-    def _get_variants(self, t_goi, t_rc, b: int, regions, n_variants: int) -> RaggedVariants:
+    def _get_variants(self, t_goi, t_rc, contigs, n_variants: int, shape, cells=None) -> RaggedVariants:
+        """The variants of the genotype rows `t_goi` (device strand flags `t_rc`, host `contigs` of every row) as a
+        RaggedVariants of `shape`.  `n_variants` = the sum of the rows' genotype slice lengths, known from the host copy of
+        the offsets (no sync for it).  `cells`: device indices into the gathered row offsets (rows folded under
+        `unphased_union`) at which the output cells start, the last one = the end; None = one cell per row."""
         p, eng = self.ploidy, self.engine
         fold = p if self.unphased_union else 1
         windows = self.sequence_type == "variant-windows"
@@ -988,13 +1031,11 @@ class Dataset:
         elif self.flank_length and self.token_alphabet is not None:
             lut, _ = build_token_lut(self.token_alphabet, self.unknown_token)
             tokens = dict(lut=lut, unk=self.unknown_token, L=self.flank_length, flank=True)
-        if tokens is not None:  # contig of every (b*p) row (_flat_variants.py:985-989)
-            row_contigs = torch.from_numpy(np.repeat(regions[:, 0].astype(np.int32), p)).to(eng.device)
-        # (n_variants = sum of the rows' genotype slice lengths, known from the host copy of the offsets: no sync for it)
+        if tokens is not None:  # contig of every row (_flat_variants.py:985-989)
+            row_contigs = torch.from_numpy(np.ascontiguousarray(contigs, np.int32)).to(eng.device)
         g = eng.gather_variants(t_goi, t_rc, self.var_fields, self.dummy_variant, self.min_af, self.max_af, fold, tokens, row_contigs,
                                 n_hint=n_variants)
-        shape = (b, 1 if self.unphased_union else p, None)
-        off = g["row_offsets"]
+        off = g["row_offsets"] if cells is None else g["row_offsets"][cells]
         fields = {}
         names = [n for n in self.var_fields if not (windows and n in ("alt", "ref"))]
         names += [n for n in ("ref_window", "alt_window", "ref", "alt") if windows and n in g]  # token buffers of the windows tail
