@@ -90,6 +90,7 @@ def _load() -> C.CDLL:
     lib.gvl_packed_reference_words.restype = c_i64
     lib.gvl_packed_reference_words.argtypes = [c_i64]
     lib.gvl_debug_last_launch.argtypes = [c_vp, c_vp, C.c_int]
+    lib.gvl_debug_track_tiles.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp]
     # the per-batch entries of the fixed-length path take plain ints (no per-call ctypes objects)
     lib.gvl_dev_fixed_plan.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp]
     lib.gvl_dev_fixed_exec.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
@@ -129,6 +130,24 @@ def last_launch(handle) -> dict:
     d = dict(zip(LAUNCH_FIELDS, (int(x) for x in out)))
     d["exec_kernel"] = EXEC_KERNELS[d["exec_kernel"]]
     return d
+
+
+# gvl_debug_track_tiles: fields of one tile entry, flag bits (GVL_TILE_* in include/gvl_b200.h)
+TILE_FIELDS = ("track", "row", "h0", "h1", "flags", "m", "cnt")
+TILE_RC, TILE_GENERIC, TILE_BIG = 1, 2, 4
+
+
+def track_tiles(handle):
+    """Tile descriptors of the last track execute a context prepared (gvl_debug_track_tiles): ``(tiles, n_tiles,
+    tdesc_bytes)`` with ``tiles`` an int32 array (tiles that exist, in grid order) x TILE_FIELDS, ``n_tiles`` the
+    descriptors of the call's grid and ``tdesc_bytes`` the bytes allocated for them.  Synchronizes the device."""
+    import numpy as np
+
+    n, nb = c_i64(0), c_i64(0)
+    check(lib.gvl_debug_track_tiles(handle, None, 0, C.byref(n), C.byref(nb)))
+    out = np.empty((max(n.value, 1), len(TILE_FIELDS)), np.int32)
+    check(lib.gvl_debug_track_tiles(handle, out.ctypes.data, n.value, C.byref(n), C.byref(nb)))
+    return out[: n.value][out[: n.value, 1] >= 0], int(n.value), int(nb.value)
 
 
 def ptr(x) -> C.c_void_p:

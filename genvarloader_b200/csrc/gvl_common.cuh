@@ -78,6 +78,8 @@ constexpr int64_t ALT_PAD = INT64_MIN;  // RecArrays.src sentinel: "ALT piece" i
 }  // namespace gvl
 
 #define GVL_TRK_DESC_BYTES 4096
+// bytes of one tile descriptor of the track execute (gvl_tracks_exec.cuh: TileDesc, which static_asserts this size)
+#define GVL_TILE_DESC_BYTES 112
 
 struct gvl_static_entry {
     void *dev;
@@ -104,8 +106,9 @@ struct gvl_workspace {
     // track plans: 32-byte AoS records (gvl_tracks.cu: TrkRec)
     void *trecs;
     int64_t trec_cap;
-    void *tdesc;        // per (track, tile) descriptors of the track execute kernel (96 bytes each)
-    int64_t tdesc_cap;
+    void *tdesc;        // per (track, tile) descriptors of the track execute kernel (GVL_TILE_DESC_BYTES each)
+    int64_t tdesc_cap;  // descriptors it holds
+    int64_t tdesc_bytes;  // bytes allocated (checked against every tile-prep launch)
 };
 
 struct gvl_ctx {

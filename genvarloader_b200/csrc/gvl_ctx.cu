@@ -103,8 +103,10 @@ int ensure_tdesc(gvl_ctx *ctx, gvl_workspace &ws, int64_t n) {
     int64_t cap = n + n / 2 + 256;
     if (ws.tdesc) GVL_CUDA(cudaFree(ws.tdesc));
     ws.tdesc = nullptr;
-    GVL_CUDA(cudaMalloc(&ws.tdesc, 96 * (size_t)cap));
+    ws.tdesc_cap = ws.tdesc_bytes = 0;
+    GVL_CUDA(cudaMalloc(&ws.tdesc, GVL_TILE_DESC_BYTES * (size_t)cap));
     ws.tdesc_cap = cap;
+    ws.tdesc_bytes = GVL_TILE_DESC_BYTES * cap;
     return GVL_OK;
 }
 

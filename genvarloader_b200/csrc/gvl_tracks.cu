@@ -6,14 +6,15 @@
 // (src/tracks/mod.rs:224-406, 495-667) -> reverse_flat_rows_inplace (src/reverse.rs:25-38), called
 // once per track from a Python loop (_dataset/_reconstruct.py:228-290).
 //
-// Here: ONE plan launch per batch (the variant state machine does not depend on the track) and ONE
-// execute launch for all tracks.  Each execute CTA owns a tile of one (track, row): it paints the
-// stored intervals that cover the tile's source window into shared memory (no dense scratch in
-// HBM), then every thread produces 4 consecutive output values per step (source span copies,
-// deletion/insertion fills, trailing zeros, reversal for negative strands) and writes them with one
-// 16-byte store.
+// Here: ONE plan launch per batch (the variant state machine does not depend on the track), one tile-preparation
+// launch and ONE execute launch for all tracks.  Each execute CTA owns a tile of TRK_TILE output values of one
+// (track, row): it turns the tile's records and the stored intervals that reach into it into value markers in output
+// coordinates (no dense scratch in HBM), then every thread writes chunks of 16 consecutive output values with two
+// 32-byte stores (source span copies, deletion/insertion fills, trailing zeros, reversal for negative strands).  Unsorted
+// variant lists and dense sources resolve every value on its own.  gvl_tracks_exec.cuh has the details.
 #include <cstdlib>
 #include <cstring>
+#include <vector>
 
 #include "gvl_internal.cuh"
 
@@ -177,6 +178,9 @@ static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t
     if (grid > INT32_MAX) return fail(GVL_ERR_ARG, "too many track tiles");
     int rc;
     if ((rc = ensure_tdesc(ctx, ctx->trk, grid))) return rc;
+    if (grid * (int64_t)sizeof(TileDesc) > ctx->trk.tdesc_bytes)  // tile prep writes one descriptor per CTA of the grid
+        return fail(GVL_ERR_STATE, "track tile descriptors: %lld bytes needed, %lld allocated", (long long)(grid * (int64_t)sizeof(TileDesc)),
+                    (long long)ctx->trk.tdesc_bytes);
     TileDesc *tdesc = (TileDesc *)ctx->trk.tdesc;
     trk_tile_prep_kernel<<<(unsigned)((grid + 3) / 4), 128, 0, st>>>(P, row_dst, row_tstride, tdesc);  // one warp per tile
     GVL_LAUNCH_CHECK();
@@ -443,5 +447,33 @@ int gvl_debug_hash4(gvl_ctx *ctx, uint64_t a, uint64_t b, uint64_t c, uint64_t d
 }
 
 int gvl_debug_xorshift64(gvl_ctx *ctx, uint64_t x, uint64_t *out) { return run_prng(ctx, x, 0, 0, 0, 0, out); }
+
+int gvl_debug_track_tiles(gvl_ctx *ctx, int32_t *out, int64_t n_max, int64_t *n_tiles, int64_t *tdesc_bytes) {
+    if (!ctx || !n_tiles || !tdesc_bytes || n_max < 0 || (!out && n_max > 0))
+        return fail(GVL_ERR_ARG, "gvl_debug_track_tiles: bad argument");
+    GVL_CUDA(cudaSetDevice(ctx->device));
+    GVL_CUDA(cudaDeviceSynchronize());
+    *tdesc_bytes = ctx->trk.tdesc_bytes;
+    *n_tiles = 0;
+    if (!ctx->trk_params) return GVL_OK;
+    const TrkExecParams *P = (const TrkExecParams *)ctx->trk_params;
+    const int64_t grid = P->grid_per_track * P->n_tracks;
+    *n_tiles = grid;
+    if (n_max == 0) return GVL_OK;
+    if (grid * (int64_t)sizeof(TileDesc) > ctx->trk.tdesc_bytes)
+        return fail(GVL_ERR_STATE, "gvl_debug_track_tiles: %lld descriptors do not fit the buffer", (long long)grid);
+    std::vector<TileDesc> h((size_t)grid);
+    GVL_CUDA(cudaMemcpy(h.data(), ctx->trk.tdesc, sizeof(TileDesc) * (size_t)grid, cudaMemcpyDeviceToHost));
+    int64_t k = 0;
+    for (int64_t g = 0; g < grid && k < n_max; g++) {
+        const TileDesc &D = h[(size_t)g];
+        if (D.row < 0) continue;
+        int32_t *o = out + 7 * k++;
+        o[0] = (int32_t)(g / P->grid_per_track), o[1] = D.row, o[2] = D.h0, o[3] = D.h1, o[4] = D.flags, o[5] = D.m, o[6] = D.cnt;
+    }
+    for (; k < n_max; k++)
+        for (int f = 0; f < 7; f++) out[7 * k + f] = -1;
+    return GVL_OK;
+}
 
 }  // extern "C"

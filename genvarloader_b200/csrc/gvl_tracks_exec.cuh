@@ -7,9 +7,10 @@
 //
 // The output of one (track, row) is cut into TILES of T3_TILE values; every tile is independent:
 //
-//   trk_tile_prep_kernel   one THREAD per (track, tile): finds the tile's record cursor, the first stored interval that
-//                          reaches into it and the value in effect at its first position (binary searches, thousands
-//                          of them in parallel) and leaves a 112-byte descriptor.  All searching of the path lives here.
+//   trk_tile_prep_kernel   one WARP per (track, tile): finds the tile's record cursor, the first stored interval that
+//                          reaches into it and the value in effect at its first position (32-ary searches, a probe per
+//                          lane, thousands of them in parallel) and leaves a 112-byte descriptor.  All searching of the
+//                          path lives here.
 //   trk_exec3_kernel       one CTA per tile, no loop, two barriers.  It never materialises the source window: the stored
 //                          intervals are painted DIRECTLY IN OUTPUT COORDINATES as a run-length code --
 //       load     the descriptor (one broadcast load), then the tile's records and its slice of the interval SoA
@@ -35,6 +36,7 @@ constexpr int T3_ITV = 512;                 // stored intervals staged per sub-p
 constexpr int T3_REC = 96;                  // records staged per sub-pass (carry + new ones + sentinel)
 constexpr int T3_WORDS = T3_TILE / 32;
 constexpr int TD_RC = 1, TD_GENERIC = 2, TD_BIG = 4;  // TileDesc.flags
+static_assert(TD_RC == GVL_TILE_RC && TD_GENERIC == GVL_TILE_GENERIC && TD_BIG == GVL_TILE_BIG, "gvl_debug_track_tiles reports these flags");
 
 // What trk_tile_prep_kernel leaves for one (track, tile); row < 0 = no such tile.
 struct __align__(16) TileDesc {
@@ -51,7 +53,7 @@ struct __align__(16) TileDesc {
     int32_t m, cnt;     // records (carry included) / stored intervals the tile needs; TD_BIG when either exceeds the staging
     int32_t query;      // row / ploidy (hap = row - query * ploidy)
 };
-static_assert(sizeof(TileDesc) == 112, "TileDesc is 112 bytes");
+static_assert(sizeof(TileDesc) == GVL_TILE_DESC_BYTES, "TileDesc must be GVL_TILE_DESC_BYTES (ensure_tdesc sizes the buffer with it)");
 
 struct T3Smem {
     float val[T3_TILE];             // marker values by tile-relative haplotype position
@@ -243,7 +245,7 @@ __device__ __forceinline__ void t2_set_bit(uint32_t *mk, uint32_t *mk2, int u) {
 }
 
 // =====================================================================================
-// tile preparation: one thread per (track, tile)
+// tile preparation: one warp per (track, tile)
 // =====================================================================================
 // row_dst / row_tstride (gvl_dev_*_rows): explicit destination of every row, out_base = row_dst[row] + track *
 // row_tstride[row]; NULL row_dst = the fixed layout of P.layout_btp.  (Kernel arguments of their own, not members of

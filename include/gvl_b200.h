@@ -615,6 +615,18 @@ int gvl_debug_last_exec_kernel(gvl_ctx *ctx);
 #define GVL_EXEC_PACKED_UNROLL2 3 /* packed one-hot, 2 groups per warp in flight: everything else                         */
 int gvl_debug_last_launch(gvl_ctx *ctx, int64_t *out, int n);
 
+/* The tile descriptors of the last track execute this context prepared (every entry that realigns or paints tracks).
+ * Synchronizes the device, then copies the descriptors back.  *n_tiles = descriptors of that call's grid (tiles per
+ * track, an upper bound, times the tracks); *tdesc_bytes = bytes allocated for descriptors (at least *n_tiles times the
+ * descriptor size).  out: int32[7 * n_max]; entry k = (track, row, h0, h1, flags, m, cnt) of the k-th tile that exists,
+ * in grid order, where [h0, h1) is the tile in haplotype coordinates, flags a mask of GVL_TILE_*, m the records the tile
+ * stages (its carry included) and cnt the stored intervals it needs; entries past the last tile are -1.  n_max = 0 only
+ * reports the two counts.  Tests use it to assert which execute path every tile takes. */
+#define GVL_TILE_RC 1       /* the row is written reversed (negative strand)                                          */
+#define GVL_TILE_GENERIC 2  /* every value resolved on its own: unsorted variant list or dense source                  */
+#define GVL_TILE_BIG 4      /* more records or stored intervals than one pass stages: finished in sub-passes           */
+int gvl_debug_track_tiles(gvl_ctx *ctx, int32_t *out, int64_t n_max, int64_t *n_tiles, int64_t *tdesc_bytes);
+
 /* ====================================================================================
  * `variants` / `variant-windows` outputs (SURVEY.md section 8 f4): the variants of every (region, sample, ploid) row
  * themselves -- indices, positions, indel lengths, allele byte strings, flank / window tokens -- instead of the
