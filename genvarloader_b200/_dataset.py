@@ -20,7 +20,7 @@ from typing import Literal
 import numpy as np
 import torch
 
-from ._engine import Engine
+from ._engine import Engine, track_dtype_code
 from ._insertion_fill import InsertionFill, Repeat5p, lower
 from ._types import (AnnotatedHaps, DummyVariant, Ragged, RaggedAlleles, RaggedAnnotatedHaps, RaggedVariants, VarWindowOpt,
                      build_token_lut)
@@ -66,6 +66,7 @@ class Dataset:
     realign_tracks: bool = True
     output_format: str = "ragged"                     # "ragged" | "flat"  (with_output_format)
     encoding: str = "bytes"                           # "bytes" | "onehot" | "onehot_cf"  (this build's fused one-hot)
+    track_dtype: torch.dtype = torch.float32          # element type of track outputs (with_track_dtype, this build's extension)
     var_fields: tuple = ("alt", "ilen", "start")      # fields of the "variants" output (_haps.py:268)
     dummy_variant: object = None                      # DummyVariant for empty (region, sample, ploid) groups, or None
     unphased_union: bool = False                      # fold the ploidy rows of a (region, sample) into one (_flat_variants.py:925-938)
@@ -226,7 +227,7 @@ class Dataset:
     def __repr__(self) -> str:
         return (f"GVL dataset (B200-resident) with shape {self.shape}: sequences={self.sequence_type!r}, tracks={list(self.active_tracks)}, "
                 f"output_length={self.output_length!r}, jitter={self.jitter} (max {self.max_jitter}), deterministic={self.deterministic}, "
-                f"rc_neg={self.rc_neg}, is_subset={self.is_subset}, is_spliced={self.is_spliced}")
+                f"rc_neg={self.rc_neg}, is_subset={self.is_subset}, is_spliced={self.is_spliced}, track_dtype={self.track_dtype}")
 
     def _shape_counts(self, x: np.ndarray, squeeze: bool, out_reshape):
         if squeeze:
@@ -465,6 +466,17 @@ class Dataset:
         if encoding not in ("bytes", "onehot", "onehot_cf"):
             raise ValueError(f"Unknown encoding {encoding!r}")
         return self._evolve(encoding=encoding)
+
+    def with_track_dtype(self, dtype) -> "Dataset":
+        """Element type of the track outputs (this build's extension, like `with_encoding`): `torch.float32` (the default),
+        `torch.bfloat16` or `torch.float16`.  Values are computed in float32 as always and rounded to nearest even by the
+        track kernels' stores, so every read returns bit for bit `x.to(dtype)` of its float32 output `x` cast on the device
+        (float16 overflows to +-inf, subnormals are kept, NaN is the device's canonical NaN) -- without a second pass over
+        the batch, and with half the bytes written.  Shapes, offsets, padding and fills do not change."""
+        if not self.track_kinds:
+            raise ValueError("Dataset has no tracks; cannot set a track dtype.")
+        track_dtype_code(dtype)
+        return self._evolve(track_dtype=dtype)
 
     def with_tracks(self, tracks=None, kind=None) -> "Dataset":
         """Reference: `Dataset.with_tracks`, _impl.py:785-839.  `False`/`[]` disables tracks."""
@@ -814,7 +826,8 @@ class Dataset:
         contract: "only valid until the next batch is yielded"); `copy=True` (default) clones every batch.
         `to_host=True` (pipelined modes): batches are delivered as NUMPY arrays in pinned host memory -- every ring is copied
         device-to-host on a copy stream while the next one is produced, so a CPU consumer sees the PCIe copy rate instead of
-        copy + compute + launch latency per batch (`copy=False`: views valid until the half comes around again).
+        copy + compute + launch latency per batch (`copy=False`: views valid until the half comes around again).  float16
+        tracks arrive as numpy float16; bfloat16 tracks raise ValueError (numpy has no bfloat16).
         Datasets the pipeline cannot serve (ragged / variable lengths, random shifts, splicing, var_filter) fall back to
         `mode=None`."""
         if sampler is not None and shuffle:
@@ -1003,7 +1016,7 @@ class Dataset:
         # (:292-300); the kernel writes the latter directly so data and offsets agree for t > 1
         out = self.engine.realign_tracks(names, t_reg, t_shifts, t_goi, t_oi, track_lengths, row_offsets, total, ids, params,
                                          self._fill_seed(ds_idx), max_rec, keep, keep_off, t_rc,
-                                         layout="rows" if rows else "btp", **rows)
+                                         layout="rows" if rows else "btp", dtype=self.track_dtype, **rows)
         return Ragged(out, _cell_offsets(seq_offsets, len(names), self.ploidy), shape)
 
     def _painted_tracks(self, t_oi, starts, row_offsets, total: int, t_rc, offsets, shape, **rows) -> Ragged:
@@ -1011,7 +1024,7 @@ class Dataset:
         negative-strand rows reversed, in (query, track) order or, given `row_dst` / `row_tstride`, where that table puts
         each row.  `offsets`: of the output cells."""
         out = self.engine.paint_tracks(list(self.active_tracks), t_oi, starts, row_offsets, total, t_rc,
-                                       layout="rows" if rows else "btp", **rows)
+                                       layout="rows" if rows else "btp", dtype=self.track_dtype, **rows)
         return Ragged(out, offsets, shape)
 
     def _get_variants(self, t_goi, t_rc, contigs, n_variants: int, shape, cells=None) -> RaggedVariants:
@@ -1058,8 +1071,8 @@ class Dataset:
         elif self.output_length == "variable":
             if isinstance(o, RaggedAnnotatedHaps):
                 res = o.to_padded()
-            elif o.data.dtype == torch.float32:
-                res = o.to_padded(0.0)                               # tracks pad with 0 (_query.py:545-548)
+            elif o.data.is_floating_point():
+                res = o.to_padded(0.0)                               # tracks (any track dtype) pad with 0 (_query.py:545-548)
             else:
                 res = o.to_padded(0 if o.data.dim() > 1 else N_CHAR)  # bytes pad with N; one-hot with zeros
         else:

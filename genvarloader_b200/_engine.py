@@ -12,11 +12,21 @@ import numpy as np
 import torch
 
 from . import _ffi
-from ._ffi import (MODE_ANNOTATED, MODE_ONEHOT, MODE_ONEHOT_CF, MODE_U8, DatasetView, Intervals, SparseTables, Svar2Channels,
-                   c_i32, c_i64, c_u8, c_u64, c_vp, check, lib, ptr)
+from ._ffi import (MODE_ANNOTATED, MODE_ONEHOT, MODE_ONEHOT_CF, MODE_U8, TRACK_BF16, TRACK_F16, TRACK_F32, DatasetView, Intervals,
+                   SparseTables, Svar2Channels, c_i32, c_i64, c_u8, c_u64, c_vp, check, lib, ptr)
 
 MODES = {"haplotypes": MODE_U8, "u8": MODE_U8, "onehot": MODE_ONEHOT, "onehot_cf": MODE_ONEHOT_CF,
          "annotated": MODE_ANNOTATED}
+# element types of track outputs (GVL_TRACK_*): values are computed in float32 and narrowed at the kernel's store
+TRACK_DTYPES = {torch.float32: TRACK_F32, torch.bfloat16: TRACK_BF16, torch.float16: TRACK_F16}
+
+
+def track_dtype_code(dtype) -> int:
+    """GVL_TRACK_* code of a torch dtype; ValueError for anything but float32, bfloat16 and float16."""
+    code = TRACK_DTYPES.get(dtype) if isinstance(dtype, torch.dtype) else None
+    if code is None:
+        raise ValueError(f"track dtype must be torch.float32, torch.bfloat16 or torch.float16, got {dtype!r}")
+    return code
 
 
 _raw_stream = getattr(torch._C, "_cuda_getCurrentRawStream", None)  # ~1 us; torch.cuda.current_stream() costs ~15 us
@@ -537,16 +547,18 @@ class Engine:
     def realign_tracks(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                        total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
                        keep_offsets=None, to_rc=None, query_seed=None, out=None, layout="tbp", base_seed_dev=None,
-                       batch=None, sub_batch: int = 0, row_dst=None, row_tstride=None):
+                       batch=None, sub_batch: int = 0, row_dst=None, row_tstride=None, dtype=torch.float32):
         """gvl_dev_realign_tracks: all `names` in one plan + one execute launch.
-        offset_idxs: int64 (n_tracks, batch) device; out: float32 (n_tracks * total_per_track,), track-major
+        offset_idxs: int64 (n_tracks, batch) device; out: `dtype` (n_tracks * total_per_track,), track-major
         (layout="tbp", the reference's flat buffer), with every query's tracks adjacent (layout="btp",
         gvl_dev_realign_tracks_btp: the order the reference's (b, t, p, ~l) offsets describe) or wherever the
         per-row table puts each row (layout="rows": row k of track t starts at row_dst[k] + t * row_tstride[k],
-        device int64 (batch * ploidy,) each; gvl_dev_realign_tracks_plan_rows)."""
+        device int64 (batch * ploidy,) each; gvl_dev_realign_tracks_plan_rows).  `dtype` (of `out` when given): float32,
+        or bfloat16 / float16 -- the float32 values rounded to nearest even by the execute kernel's stores."""
         if out is None:
-            out = torch.empty(len(names) * total_per_track, dtype=torch.float32, device=self.device)
-        if self.svar2 is not None or layout == "rows":
+            track_dtype_code(dtype)
+            out = torch.empty(len(names) * total_per_track, dtype=dtype, device=self.device)
+        if self.svar2 is not None or layout == "rows" or out.dtype != torch.float32:
             self.realign_tracks_plan(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                                      total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
                                      query_seed, layout, base_seed_dev, batch, sub_batch, row_dst, row_tstride)
@@ -580,7 +592,9 @@ class Engine:
                                                   C.c_int(1 if layout == "btp" else 0), _stream()))
 
     def realign_tracks_exec(self, out):
-        check(lib.gvl_dev_realign_tracks_exec(self.ctx.handle, ptr(out), _stream()))
+        """gvl_dev_realign_tracks_exec_dtype: the planned call's values into `out`, in out's dtype (float32, bfloat16,
+        float16)."""
+        check(lib.gvl_dev_realign_tracks_exec_dtype(self.ctx.handle, ptr(out), track_dtype_code(out.dtype), _stream()))
         return out
 
     def intervals_to_tracks(self, name, offset_idxs, starts, out_offsets, total: int, out=None):
@@ -593,17 +607,26 @@ class Engine:
         return out
 
     def paint_tracks(self, names, offset_idxs, starts, out_offsets, total_per_track: int, to_rc=None, out=None,
-                     n_queries=None, layout="btp", row_dst=None, row_tstride=None):
+                     n_queries=None, layout="btp", row_dst=None, row_tstride=None, dtype=torch.float32):
         """gvl_dev_paint_tracks: stored intervals of all `names` painted in one launch, (b, t, ~l) order,
         masked rows reversed.  offset_idxs: int64 (n_tracks, batch) device.  layout="rows"
-        (gvl_dev_paint_tracks_rows): query q of track t starts at row_dst[q] + t * row_tstride[q] instead."""
+        (gvl_dev_paint_tracks_rows): query q of track t starts at row_dst[q] + t * row_tstride[q] instead.
+        `dtype` (of `out` when given): float32, bfloat16 or float16 (gvl_dev_paint_tracks_dtype)."""
         n_tracks, n_q = len(names), int(starts.numel() if n_queries is None else n_queries)
         itv = self.track_descs(names)[0]
         if out is None:
-            out = torch.empty(n_tracks * int(total_per_track), dtype=torch.float32, device=self.device)
+            track_dtype_code(dtype)
+            out = torch.empty(n_tracks * int(total_per_track), dtype=dtype, device=self.device)
+        if layout == "rows" and (row_dst is None or row_tstride is None):
+            raise ValueError('layout="rows" needs row_dst and row_tstride')
+        if out.dtype != torch.float32:
+            rows = layout == "rows"
+            check(lib.gvl_dev_paint_tracks_dtype(self.ctx.handle, n_tracks, itv, ptr(offset_idxs), ptr(starts), n_q,
+                                                 ptr(out_offsets), int(total_per_track), ptr(to_rc), ptr(row_dst if rows else None),
+                                                 ptr(row_tstride if rows else None), ptr(out), track_dtype_code(out.dtype),
+                                                 _stream()))
+            return out
         if layout == "rows":
-            if row_dst is None or row_tstride is None:
-                raise ValueError('layout="rows" needs row_dst and row_tstride')
             check(lib.gvl_dev_paint_tracks_rows(self.ctx.handle, n_tracks, itv, ptr(offset_idxs), ptr(starts), n_q,
                                                 ptr(out_offsets), int(total_per_track), ptr(to_rc), ptr(row_dst),
                                                 ptr(row_tstride), ptr(out), _stream()))

@@ -15,6 +15,7 @@ LIB_PATH = _PKG / "_lib" / os.environ.get("GVL_LIB_NAME", "libgvl_b200.so")  # (
 
 GVL_OK = 0
 MODE_U8, MODE_ONEHOT, MODE_ANNOTATED, MODE_ONEHOT_CF = 0, 1, 2, 3
+TRACK_F32, TRACK_BF16, TRACK_F16 = 0, 1, 2  # GVL_TRACK_*: element type of a track output
 
 c_i64, c_i32, c_u8, c_u64, c_vp = C.c_int64, C.c_int32, C.c_uint8, C.c_uint64, C.c_void_p
 
@@ -74,7 +75,7 @@ class FixedJob(C.Structure):
                 ("track_lengths", c_vp), ("paint_offsets", c_vp), ("itv", c_vp), ("strategy_ids", c_vp), ("params", c_vp),
                 ("ploidy", c_i64), ("rows_p", c_i64), ("output_length", c_i64), ("ref_slot", c_i64), ("n_tracks", c_i64),
                 ("max_slot_len", c_i64), ("typ_slot_len", c_i64), ("annot_mask", C.c_uint32), ("mode", c_i32), ("realign", c_i32), ("rc_neg", c_i32),
-                ("pad_char", c_u8)]
+                ("pad_char", c_u8), ("track_dtype", c_i32)]
 
 
 def _load() -> C.CDLL:
@@ -101,6 +102,10 @@ def _load() -> C.CDLL:
                                                      c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_u64, c_vp, c_i64, c_vp, c_i64,
                                                      c_vp, c_vp, c_vp]
     lib.gvl_dev_paint_tracks_rows.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
+    # track outputs of a chosen element type (GVL_TRACK_*)
+    lib.gvl_dev_realign_tracks_exec_dtype.argtypes = [c_vp, c_vp, c_i32, c_vp]
+    lib.gvl_dev_paint_tracks_dtype.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i32,
+                                               c_vp]
     return lib
 
 

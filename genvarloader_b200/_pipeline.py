@@ -30,7 +30,7 @@ import torch
 
 from . import _ffi
 from ._dataset import _as_rng, _batch_tail, epoch_order
-from ._engine import MODES, Engine, _raw_stream, _stream
+from ._engine import MODES, Engine, _raw_stream, _stream, track_dtype_code
 from ._ffi import BatchArgs, DatasetView, FixedJob, c_i64, c_u8, c_u64, c_vp, check, lib, ptr
 from ._types import AnnotatedHaps
 
@@ -84,6 +84,7 @@ class _Spec:
             if ds.track_kinds[n] == "annot":
                 self.annot_mask |= 1 << i
         self.fill_ids, self.fill_params = ds._fills(self.names)
+        self.track_dtype = ds.track_dtype
 
 
 def supports(ds) -> str | None:
@@ -139,7 +140,7 @@ class _Out:
                 self.av = torch.empty(b * rp * L, dtype=torch.int32, device=dev)
                 self.ap = torch.empty(b * rp * L, dtype=torch.int32, device=dev)
         if t:
-            self.trk = torch.empty(b * t * (p if spec.realign else 1) * L, dtype=torch.float32, device=dev)
+            self.trk = torch.empty(b * t * (p if spec.realign else 1) * L, dtype=spec.track_dtype, device=dev)
         self.spec, self.b = spec, b
 
     def result(self, lo: int = 0, n: int | None = None, clone: bool = False):
@@ -229,7 +230,7 @@ class FixedPipeline:
         return FixedJob(adr(self.view), adr(eng.tab), adr(sv), scr.args, ptr(scr.out_offsets), ptr(scr.diffs), ptr(scr.track_lengths),
                         ptr(self._paint_off) if (sp.t and not sp.realign) else c_vp(0), adr(itv), adr(sid), adr(par),
                         sp.p, sp.rows_p, sp.L, self.ref_slot, sp.t, max(eng.max_slot_len, 1), int(getattr(eng, "typ_slot_len", 0)), sp.annot_mask, mode,
-                        1 if sp.realign else 0, 1 if sp.rc_neg else 0, eng.pad_char)
+                        1 if sp.realign else 0, 1 if sp.rc_neg else 0, eng.pad_char, track_dtype_code(sp.track_dtype))
 
     # ------------------------------------------------------------------ one device call over n queries
     # Stage P ("plan"): batch prep + variant plan (+ track plan / tile prep).  Stage E ("execute"): the bandwidth-bound
@@ -420,6 +421,9 @@ class PipelinedLoader:
     """Re-iterable loader over a `Dataset` backed by a `FixedPipeline` (see `Dataset.to_dataloader(mode=...)`)."""
 
     def __init__(self, ds, batch_size, shuffle, sampler, drop_last, generator, return_indices, transform, copy, ring, to_host=False):
+        if to_host and ds.active_tracks and ds.track_dtype == torch.bfloat16:
+            raise ValueError("to_host=True delivers numpy arrays and numpy has no bfloat16: read bfloat16 tracks on the device, "
+                             "or use with_track_dtype(torch.float16) / torch.float32 for host delivery")
         self.ds, self.batch_size, self.shuffle, self.sampler = ds, int(batch_size), shuffle, sampler
         self.drop_last, self.return_indices, self.transform, self.copy = drop_last, return_indices, transform, copy
         self._rng = _as_rng(generator)

@@ -72,8 +72,11 @@ class Ragged:
         if n_rows and max_len:
             data, offsets = self.data.contiguous(), self.offsets.contiguous()
             itemsize = data.element_size() * int(np.prod(data.shape[1:], dtype=np.int64))  # one-hot rows: 4 bytes per position
-            np_dt = {torch.uint8: np.uint8, torch.int32: np.int32, torch.float32: np.float32, torch.int64: np.int64}[data.dtype]
-            pad_item = np.full(tuple(data.shape[1:]) or (1,), pad_value, np_dt).tobytes()
+            if data.dtype in (torch.bfloat16, torch.float16):  # 16-bit tracks (numpy has no bfloat16: torch gives the bits)
+                pad_item = torch.full(tuple(data.shape[1:]) or (1,), pad_value, dtype=data.dtype).view(torch.int16).numpy().tobytes()
+            else:
+                np_dt = {torch.uint8: np.uint8, torch.int32: np.int32, torch.float32: np.float32, torch.int64: np.int64}[data.dtype]
+                pad_item = np.full(tuple(data.shape[1:]) or (1,), pad_value, np_dt).tobytes()
             with torch.cuda.device(dev):
                 if len(pad_item) <= 8:
                     check(lib.gvl_dev_ragged_to_padded_fill(default_ctx(dev.index or 0).handle, ptr(data), ptr(offsets),

@@ -230,6 +230,8 @@ static int fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_id
     if (!ctx || !J || !J->view || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: NULL argument");
     if (J->realign && (J->mode < 0 || J->ref_slot >= 0 || !J->diffs || !J->track_lengths))
         return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: realigned tracks need haplotypes, diffs and track_lengths scratch");
+    if (J->track_dtype != GVL_TRACK_F32 && J->track_dtype != GVL_TRACK_BF16 && J->track_dtype != GVL_TRACK_F16)
+        return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: unknown track dtype %d", (int)J->track_dtype);
     int rc = launch_batch_prep(ctx, J->view, ds_idx, jitter, inline_host, n, sub_batch, J->ref_slot, J->n_tracks, J->annot_mask,
                                &J->args, stream);
     if (rc) return rc;
@@ -245,7 +247,7 @@ int gvl_dev_fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_i
 // small latency-bound kernels -- next to the bandwidth-bound haplotype execute): GVL_STAGE_HAP_PLAN = batch prep +
 // haplotype plan, GVL_STAGE_TRK_PLAN (needs the diffs of HAP_PLAN), GVL_STAGE_HAP_EXEC, GVL_STAGE_TRK_EXEC (needs TRK_PLAN).
 int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *J, int stage, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
-                        int64_t sub_batch, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, float *trk, gvl_stream stream) {
+                        int64_t sub_batch, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, void *trk, gvl_stream stream) {
     if (!ctx || !J || !J->tab) return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: NULL argument");
     switch (stage) {
         case GVL_STAGE_HAP_PLAN:
@@ -259,22 +261,23 @@ int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *J, int stage, const i
         case GVL_STAGE_TRK_EXEC:
             if (J->n_tracks <= 0) return GVL_OK;
             if (!trk) return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: track output missing");
-            if (J->realign) return gvl_dev_realign_tracks_exec(ctx, trk, stream);
-            return gvl_dev_paint_tracks(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
-                                        n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, trk, stream);
+            if (J->realign) return gvl_dev_realign_tracks_exec_dtype(ctx, trk, J->track_dtype, stream);
+            return gvl_dev_paint_tracks_dtype(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
+                                              n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, NULL, NULL, trk,
+                                              J->track_dtype, stream);
         default: return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: unknown stage %d", stage);
     }
 }
 
 int gvl_dev_fixed_exec(gvl_ctx *ctx, const gvl_fixed_job *J, int64_t n, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos,
-                       float *trk, gvl_stream stream) {
+                       void *trk, gvl_stream stream) {
     int rc = gvl_dev_fixed_stage(ctx, J, GVL_STAGE_HAP_EXEC, NULL, NULL, n, 0, seq, annot_v, annot_pos, trk, stream);
     if (rc) return rc;
     return gvl_dev_fixed_stage(ctx, J, GVL_STAGE_TRK_EXEC, NULL, NULL, n, 0, seq, annot_v, annot_pos, trk, stream);
 }
 
 int gvl_dev_fixed_run(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
-                      int64_t *idx_dev, int32_t *jitter_dev, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, float *trk,
+                      int64_t *idx_dev, int32_t *jitter_dev, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, void *trk,
                       gvl_stream stream) {
     if (!ctx || !J || n < 0 || (n > 0 && (!ds_idx || !idx_dev)) || (jitter && !jitter_dev))
         return fail(GVL_ERR_ARG, "gvl_dev_fixed_run: bad argument");

@@ -9,9 +9,14 @@
 // Here: ONE plan launch per batch (the variant state machine does not depend on the track), one tile-preparation
 // launch and ONE execute launch for all tracks.  Each execute CTA owns a tile of TRK_TILE output values of one
 // (track, row): it turns the tile's records and the stored intervals that reach into it into value markers in output
-// coordinates (no dense scratch in HBM), then every thread writes chunks of 16 consecutive output values with two
-// 32-byte stores (source span copies, deletion/insertion fills, trailing zeros, reversal for negative strands).  Unsorted
+// coordinates (no dense scratch in HBM), then every thread writes chunks of 16 consecutive output values with 32-byte
+// stores (source span copies, deletion/insertion fills, trailing zeros, reversal for negative strands).  Unsorted
 // variant lists and dense sources resolve every value on its own.  gvl_tracks_exec.cuh has the details.
+// The output is float32, bfloat16 or float16 (GVL_TRACK_*): one execute instantiation per type, values narrowed at the
+// store.
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -114,7 +119,7 @@ struct TrkExecParams {
     uint64_t base_seed;
     const uint64_t *base_seed_dev;  // optional: the seed(s) live in device memory (CUDA-graph replays with new batches)
     int64_t sub_batch;              // > 0: queries per logical batch (seed and FlankSample row index are per logical batch)
-    float *out;
+    void *out;                   // elements of the call's output type (trk_execute picks the instantiation)
     const TrkDesc *tracks;       // device array [n_tracks], or NULL: the descriptors travel in `inl`
     TrkDesc inl[8];              // (kernel parameters are captured by value: CUDA-graph safe)
 };
@@ -129,22 +134,31 @@ __global__ void prng_kernel(uint64_t a, uint64_t b, uint64_t c, uint64_t d, int 
 
 using namespace gvl;
 
-static int trk_execute(gvl_ctx *ctx, float *out, cudaStream_t st) {
+static bool track_dtype_ok(int32_t dtype) { return dtype == GVL_TRACK_F32 || dtype == GVL_TRACK_BF16 || dtype == GVL_TRACK_F16; }
+
+static int trk_execute(gvl_ctx *ctx, void *out, int32_t dtype, cudaStream_t st) {
     if (!ctx->trk_plan_valid || !ctx->trk_params) return fail(GVL_ERR_STATE, "track execute without a track plan");
-    if (!out || ((uintptr_t)out & 3)) return fail(GVL_ERR_ARG, "track output must be a float buffer");
+    if (!out || ((uintptr_t)out & 3)) return fail(GVL_ERR_ARG, "track output must be an aligned buffer");
     TrkExecParams P;
     memcpy(&P, ctx->trk_params, sizeof(P));
     P.out = out;
-    trk_exec3_kernel<<<dim3((unsigned)P.grid_per_track, (unsigned)P.n_tracks), T2_THREADS, 0, st>>>(P, (const TileDesc *)ctx->trk.tdesc);
+    const dim3 grid((unsigned)P.grid_per_track, (unsigned)P.n_tracks);
+    const TileDesc *tdesc = (const TileDesc *)ctx->trk.tdesc;
+    switch (dtype) {
+        case GVL_TRACK_F32: trk_exec3_kernel<float><<<grid, T2_THREADS, 0, st>>>(P, tdesc); break;
+        case GVL_TRACK_BF16: trk_exec3_kernel<__nv_bfloat16><<<grid, T2_THREADS, 0, st>>>(P, tdesc); break;
+        case GVL_TRACK_F16: trk_exec3_kernel<__half><<<grid, T2_THREADS, 0, st>>>(P, tdesc); break;
+        default: return fail(GVL_ERR_ARG, "unknown track dtype %d", (int)dtype);
+    }
     GVL_LAUNCH_CHECK();
     return GVL_OK;
 }
 
 static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t n_queries, int64_t n_tracks,
                            const TrkDesc *host_desc, const int64_t *offset_idxs, int64_t total_per_track,
-                           const int64_t *query_seed, uint64_t base_seed, float *out, int layout_btp, cudaStream_t st,
+                           const int64_t *query_seed, uint64_t base_seed, void *out, int layout_btp, cudaStream_t st,
                            const uint64_t *base_seed_dev = nullptr, int64_t sub_batch = 0, const int64_t *row_dst = nullptr,
-                           const int64_t *row_tstride = nullptr) {
+                           const int64_t *row_tstride = nullptr, int32_t dtype = GVL_TRACK_F32) {
     if (n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "at most %d tracks per call", MAX_TRACKS);
     static_assert(sizeof(TrkDesc) * MAX_TRACKS <= GVL_TRK_DESC_BYTES, "descriptor buffer too small");
     TrkDesc *d_desc = nullptr;
@@ -190,7 +204,7 @@ static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t
     memcpy(ctx->trk_params, &P, sizeof(P));
     ctx->trk_plan_valid = true;
     if (!out) return GVL_OK;  // plan only
-    return trk_execute(ctx, out, st);
+    return trk_execute(ctx, out, dtype, st);
 }
 
 // the scan-based plan kernel in track mode (gvl_hap.cu)
@@ -322,12 +336,17 @@ int gvl_dev_realign_tracks_plan_rows(gvl_ctx *ctx, const gvl_sparse_tables *tab,
                         row_tstride);
 }
 
-int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream) {
+int gvl_dev_realign_tracks_exec_dtype(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream) {
     if (!ctx) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: ctx is NULL");
+    if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: unknown track dtype %d", (int)dtype);
     GVL_CUDA(cudaSetDevice(ctx->device));
     if (!ctx->trk_plan_valid) return GVL_OK;  // (the plan was empty: nothing to write)
     if ((uintptr_t)out & 15) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: out must be 16-byte aligned");
-    return trk_execute(ctx, out, (cudaStream_t)stream);
+    return trk_execute(ctx, out, dtype, (cudaStream_t)stream);
+}
+
+int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream) {
+    return gvl_dev_realign_tracks_exec_dtype(ctx, out, GVL_TRACK_F32, stream);
 }
 
 int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
@@ -386,10 +405,11 @@ int gvl_dev_intervals_to_tracks(gvl_ctx *ctx, const gvl_intervals *itv, const in
 
 static int paint_impl(const char *who, gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
                       const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                      const uint8_t *to_rc, float *out, gvl_stream stream, const int64_t *row_dst = nullptr,
-                      const int64_t *row_tstride = nullptr) {
+                      const uint8_t *to_rc, void *out, gvl_stream stream, const int64_t *row_dst = nullptr,
+                      const int64_t *row_tstride = nullptr, int32_t dtype = GVL_TRACK_F32) {
     if (!ctx || !itv || !offset_idxs || !starts || !out_offsets) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
     if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "%s: 0..%d tracks per call", who, MAX_TRACKS);
+    if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "%s: unknown track dtype %d", who, (int)dtype);
     cudaStream_t st = (cudaStream_t)stream;
     GVL_CUDA(cudaSetDevice(ctx->device));
     if (n_queries == 0 || n_tracks == 0 || total_per_track == 0) return GVL_OK;
@@ -412,7 +432,7 @@ static int paint_impl(const char *who, gvl_ctx *ctx, int64_t n_tracks, const gvl
         desc[t].param = 0.0;
     }
     return launch_trk_exec(ctx, n_queries, 1, n_queries, n_tracks, desc, offset_idxs, total_per_track, nullptr, 0, out, 1, st,
-                           nullptr, 0, row_dst, row_tstride);
+                           nullptr, 0, row_dst, row_tstride, dtype);
 }
 
 int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
@@ -429,6 +449,15 @@ int gvl_dev_paint_tracks_rows(gvl_ctx *ctx, int64_t n_tracks, const gvl_interval
     if (!row_dst || !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks_rows: NULL argument");
     return paint_impl("gvl_dev_paint_tracks_rows", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
                       total_per_track, to_rc, out, stream, row_dst, row_tstride);
+}
+
+int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                               const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                               const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
+                               gvl_stream stream) {
+    if (!row_dst != !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks_dtype: row_dst and row_tstride go together");
+    return paint_impl("gvl_dev_paint_tracks_dtype", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
+                      total_per_track, to_rc, out, stream, row_dst, row_tstride, dtype);
 }
 
 static int run_prng(gvl_ctx *ctx, uint64_t a, uint64_t b, uint64_t c, uint64_t d, int which, uint64_t *out) {

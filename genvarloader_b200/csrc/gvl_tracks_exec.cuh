@@ -20,11 +20,14 @@
 //                in effect from there on -- into `val[]` plus a bit into a two-level bitmap; one thread per record
 //                drops the value in effect right after the variant; insertion fills other than Repeat5p are computed
 //                one value per thread and dropped as markers too;
-//       output   every lane owns chunks of 8 consecutive output values: it finds the last marker before its chunk with
-//                two bitmap probes (no block-wide scan), walks its 8 marker bits in registers, and writes the chunk
-//                with ONE 256-bit store (a warp instruction writes 1 KiB of contiguous output).
+//       output   every lane owns chunks of 16 consecutive output values: it finds the last marker before its chunk with
+//                two bitmap probes (no block-wide scan), walks its 16 marker bits in registers, and writes the chunk
+//                with 256-bit stores (float: two, lanes 64 bytes apart; bfloat16 / float16: one of packed pairs).
 //     The values themselves never travel through shared memory.  A tile whose source range holds more stored intervals
 //     (or records) than are staged at once is finished in further sub-passes (rare: intervals of a few bp).
+// The output element type T is float, __nv_bfloat16 or __half: every value is computed in float32 exactly as for float
+// output and narrowed at the store (cvt.rn, no .ftz: round to nearest even, overflow to inf, subnormals kept, NaN the
+// canonical one) -- bit for bit what a device-side cast of the float32 output gives.
 // Rows that need the reference's sequential semantics literally (variant lists that are not position-sorted leave
 // "jump" records) and dense f32 sources (shift_and_realign_tracks_sparse) take `t2_generic_segment`: every value
 // resolved on its own against the row's records and the source -- slow, exact for any input.
@@ -74,6 +77,30 @@ __device__ __forceinline__ void stg_f8(float *p, float a, float b, float c, floa
     asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d), "f"(e),
                  "f"(f), "f"(g), "f"(h)
                  : "memory");
+}
+
+// sixteen 16-bit values as eight packed pairs (lower address = lower half): one 256-bit store
+__device__ __forceinline__ void stg_b8(void *p, const uint32_t (&w)[8]) {
+    asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]),
+                 "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7])
+                 : "memory");
+}
+
+// a track value as output element T (the only place where the output type matters to the value)
+template <class T> __device__ __forceinline__ T to_out(float v);
+template <> __device__ __forceinline__ float to_out<float>(float v) { return v; }
+template <> __device__ __forceinline__ __nv_bfloat16 to_out<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half to_out<__half>(float v) { return __float2half_rn(v); }
+
+// two values as one packed pair of 16-bit elements, a in the lower half (cvt.rn.{bf16,f16}x2.f32: the rounding of to_out)
+template <class T> __device__ __forceinline__ uint32_t pack2(float a, float b);
+template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float a, float b) {
+    const __nv_bfloat162 x = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<const uint32_t *>(&x);
+}
+template <> __device__ __forceinline__ uint32_t pack2<__half>(float a, float b) {
+    const __half2 x = __floats2half2_rn(a, b);
+    return *reinterpret_cast<const uint32_t *>(&x);
 }
 
 // ---- sources ---------------------------------------------------------------------------------------------
@@ -207,13 +234,15 @@ __device__ float t2_generic_value(const TRec *__restrict__ recs, int32_t n_rec, 
     return tp < src.track_n ? src.at(tp) : 0.0f;  // :381-404 trailing zeros
 }
 
+template <class T>
 __device__ __noinline__ void t2_generic_segment(const TRec *__restrict__ recs, int32_t n_rec, int32_t ref0, SrcGlobal src,
-                                                int strategy, double param, float *__restrict__ out_row, int32_t L, bool rc, int32_t t0, int32_t t1,
+                                                int strategy, double param, T *__restrict__ out_row, int32_t L, bool rc, int32_t t0, int32_t t1,
                                    uint64_t base_seed, uint64_t qseed, uint64_t hap) {
     int32_t hint = -2;
     for (int32_t j = t0 + (int32_t)threadIdx.x; j < t1; j += T2_THREADS) {
         const int32_t p = rc ? (L - 1 - j) : j;
-        out_row[j] = t2_generic_value(recs, n_rec, ref0, src, strategy, param, p, base_seed, qseed, hap, hint);
+        // (one element per store: a 16-bit value never touches its neighbour)
+        out_row[j] = to_out<T>(t2_generic_value(recs, n_rec, ref0, src, strategy, param, p, base_seed, qseed, hap, hint));
     }
 }
 
@@ -366,17 +395,22 @@ __global__ void __launch_bounds__(128) trk_tile_prep_kernel(TrkExecParams P, con
 // execute: one CTA per tile
 // =====================================================================================
 // the output phase of a (sub-)pass: see the header comment
-template <bool RC>
-__device__ __forceinline__ void t3_write_chunks(const T3Smem &S, float *__restrict__ out_row, int32_t j0, int32_t n_chunks,
+template <bool RC, class T>
+__device__ __forceinline__ void t3_write_chunks(const T3Smem &S, T *__restrict__ out_row, int32_t j0, int32_t n_chunks,
                                                 int32_t jo_lo, int32_t jo_hi, int32_t L, int32_t cur) {
-    // Every thread owns 16 consecutive output values (64 bytes: two 256-bit stores; lanes 64 bytes apart still run at
-    // the full store rate on B200, 128 bytes per lane do not -- profiles/microbench/fill.py), so the search for the
+    // Every thread owns 16 consecutive output values (float: 64 bytes, two 256-bit stores; lanes 64 bytes apart still run
+    // at the full store rate on B200, 128 bytes per lane do not -- profiles/microbench/fill.py), so the search for the
     // value in effect before the chunk is paid once per 16 values and the walk carries it in a register.
+    // 16-bit output keeps the 16 values per thread: ONE 256-bit store of packed pairs, lanes 32 bytes apart (a warp
+    // instruction still writes 1 KiB of contiguous output).  32 values per thread would halve the chunk searches but
+    // double the marker walk each thread runs before its first store and halve the threads that store a tile; the
+    // kernel is bound by that per-tile latency chain, not by the searches, and one chunk geometry for every T keeps the
+    // walk, the bitmap reads and the tile-edge handling the same code.
     const uint32_t *mk = S.mk, *mk2 = S.mk2;
     const int tid = threadIdx.x;
     int32_t j = j0 + 16 * tid;                          // first output position of the thread's chunk
     int32_t u_lo = (RC ? (L - 16 - j) : j) - cur;       // its lowest tile-relative haplotype position
-    float *dst = out_row + j;
+    T *dst = out_row + j;
     for (int32_t c = tid; c < n_chunks; c += T2_THREADS, j += 16 * T2_THREADS, u_lo += RC ? -16 * T2_THREADS : 16 * T2_THREADS,
                  dst += 16 * T2_THREADS) {
         uint32_t bits;
@@ -401,22 +435,43 @@ __device__ __forceinline__ void t3_write_chunks(const T3Smem &S, float *__restri
             cv = S.val[32 * w + 31 - __clz(mm)];
         }
         const bool whole = j >= jo_lo && j + 16 <= jo_hi;
+        if constexpr (sizeof(T) == 2) {
+            float x[16];  // in OUTPUT order: haplotype position u_lo + i is output RC ? 15 - i : i of the chunk
 #pragma unroll
-        for (int h = 0; h < 2; h++) {  // two halves of 8 in HAPLOTYPE order; the reversed row stores them back to front
-            float x[8];                // in OUTPUT order: haplotype position u_lo + 8h + t is output RC ? 7 - t : t of its half
-#pragma unroll
-            for (int t = 0; t < 8; t++) {
-                if ((bits >> (8 * h + t)) & 1u) cv = S.val[u_lo + 8 * h + t];
-                x[RC ? 7 - t : t] = cv;
+            for (int i = 0; i < 16; i++) {
+                if ((bits >> i) & 1u) cv = S.val[u_lo + i];
+                x[RC ? 15 - i : i] = cv;
             }
-            const int off = RC ? 8 * (1 - h) : 8 * h;
             if (whole) {
-                stg_f8(dst + off, x[0], x[1], x[2], x[3], x[4], x[5], x[6], x[7]);
-            } else {  // chunk cut by the tile / row ends
+                uint32_t w[8];
+#pragma unroll
+                for (int k = 0; k < 8; k++) w[k] = pack2<T>(x[2 * k], x[2 * k + 1]);
+                stg_b8(dst, w);
+            } else {  // chunk cut by the tile / row ends: one 16-bit store per value of the range, nothing outside it
+#pragma unroll
+                for (int t = 0; t < 16; t++) {
+                    const int32_t jj = j + t;
+                    if (jj >= jo_lo && jj < jo_hi) dst[t] = to_out<T>(x[t]);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int h = 0; h < 2; h++) {  // two halves of 8 in HAPLOTYPE order; the reversed row stores them back to front
+                float x[8];                // in OUTPUT order: haplotype position u_lo + 8h + t is output RC ? 7 - t : t of its half
 #pragma unroll
                 for (int t = 0; t < 8; t++) {
-                    const int32_t jj = j + off + t;
-                    if (jj >= jo_lo && jj < jo_hi) dst[off + t] = x[t];
+                    if ((bits >> (8 * h + t)) & 1u) cv = S.val[u_lo + 8 * h + t];
+                    x[RC ? 7 - t : t] = cv;
+                }
+                const int off = RC ? 8 * (1 - h) : 8 * h;
+                if (whole) {
+                    stg_f8(reinterpret_cast<float *>(dst + off), x[0], x[1], x[2], x[3], x[4], x[5], x[6], x[7]);
+                } else {  // chunk cut by the tile / row ends
+#pragma unroll
+                    for (int t = 0; t < 8; t++) {
+                        const int32_t jj = j + off + t;
+                        if (jj >= jo_lo && jj < jo_hi) dst[off + t] = to_out<T>(x[t]);
+                    }
                 }
             }
         }
@@ -424,10 +479,11 @@ __device__ __forceinline__ void t3_write_chunks(const T3Smem &S, float *__restri
 }
 
 // what a tile needs beyond its descriptor (built once by the kernel; small enough to travel by value)
+template <class T>
 struct TileCtx {
     const TRec *recs;      // the row's records
-    float *out_row;        // the row's value 0
-    int64_t base_elems;    // its address in floats (32-byte alignment of the chunks)
+    T *out_row;            // the row's value 0
+    int64_t base_elems;    // its address in elements of T (alignment of the 16-value chunks: 64 bytes for float, 32 for 16-bit)
     SrcGlobal srcg;
     uint64_t base_seed, qseed, hap;
     double param;
@@ -436,8 +492,8 @@ struct TileCtx {
 
 // One tile.  BIG = false: everything the tile needs fits the staging (the descriptor says how much of it): one pass,
 // extents known.  BIG = true: sub-passes, each as long as the staged records / intervals reach.
-template <bool BIG>
-__device__ __forceinline__ void t3_tile(const TileCtx &X, const TileDesc &D, T3Smem &S) {
+template <bool BIG, class T>
+__device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, T3Smem &S) {
     const int tid = threadIdx.x;
     const int32_t L = D.L;
     const bool rc = (D.flags & TD_RC) != 0;
@@ -445,7 +501,7 @@ __device__ __forceinline__ void t3_tile(const TileCtx &X, const TileDesc &D, T3S
     const int64_t track_n = D.track_n, q_start = D.q_start;
     const TRec *__restrict__ recs = X.recs;
     const SrcGlobal &srcg = X.srcg;
-    float *__restrict__ out_row = X.out_row;
+    T *__restrict__ out_row = X.out_row;
     const int64_t base_elems = X.base_elems;
     const int32_t h1 = D.h1;
     int32_t cur = D.h0;
@@ -576,14 +632,14 @@ __device__ __forceinline__ void t3_tile(const TileCtx &X, const TileDesc &D, T3S
             __syncthreads();
         }
 
-        // ---- output: chunks of 16 values on 64-byte aligned addresses ----
+        // ---- output: chunks of 16 values on 16-element (float: 64-byte, 16-bit: 32-byte) aligned addresses ----
         const int32_t jo_lo = rc ? L - pass_end : cur;
         const int32_t jo_hi = rc ? L - cur : pass_end;
         const int32_t j0 = (int32_t)(((base_elems + jo_lo) & ~(int64_t)15) - base_elems);  // may be < jo_lo
         const int32_t n_chunks = (jo_hi - j0 + 15) >> 4;
         // (the two directions are separate instantiations: the walk then writes its registers in output order)
-        if (rc) t3_write_chunks<true>(S, out_row, j0, n_chunks, jo_lo, jo_hi, L, cur);
-        else t3_write_chunks<false>(S, out_row, j0, n_chunks, jo_lo, jo_hi, L, cur);
+        if (rc) t3_write_chunks<true, T>(S, out_row, j0, n_chunks, jo_lo, jo_hi, L, cur);
+        else t3_write_chunks<false, T>(S, out_row, j0, n_chunks, jo_lo, jo_hi, L, cur);
         if (!BIG || pass_end >= h1) break;
 
         // ---- (rare) the tile goes on: cursors of the next sub-pass ----
@@ -631,17 +687,19 @@ __device__ __forceinline__ void t3_tile(const TileCtx &X, const TileDesc &D, T3S
 // (the rare sub-pass variant is kept out of line: its register needs must not weigh on the common path)
 // (it takes its context from shared memory and re-reads the descriptor: structs passed by value or reference would
 //  make every thread of EVERY tile spill them to local memory before the branch)
+template <class T>
 __device__ __noinline__ void t3_tile_big(T3Smem *S, const TileDesc *__restrict__ dp) {
-    const TileCtx X = *reinterpret_cast<const TileCtx *>(S->big_ctx);
+    const TileCtx<T> X = *reinterpret_cast<const TileCtx<T> *>(S->big_ctx);
     const TileDesc D = *dp;
     __syncthreads();  // everyone holds its copy before shared memory is reused
-    t3_tile<true>(X, D, *S);
+    t3_tile<true, T>(X, D, *S);
 }
-static_assert(sizeof(TileCtx) <= 128, "TileCtx must fit T3Smem::big_ctx");
+static_assert(sizeof(TileCtx<float>) <= 128, "TileCtx must fit T3Smem::big_ctx");
 
 // 5 CTAs per SM (48 registers, 80 bytes of spills; shared memory allows no more): the kernel is bound by the latency chain of a
 // tile, so the fifth tile in flight pays (tracks step of a 20-batch ring 63.7 -> 60.3 us) although a single 134 MB call gains little
 constexpr int T3_MIN_CTAS = 5;
+template <class T>
 __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkExecParams P, const TileDesc *__restrict__ tdesc) {
     __shared__ __align__(16) T3Smem S;
     const unsigned track = blockIdx.y;
@@ -649,7 +707,7 @@ __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkE
     const TileDesc D = *dp;  // (same address in every thread: one broadcast load)
     if (D.row < 0) return;
     const TrkDesc *Tp = P.tracks ? P.tracks + track : nullptr;
-    TileCtx X;
+    TileCtx<T> X;
     {
         const int64_t query = D.query;
         // (queries and logical batch sizes are < 2^31: 32-bit division, the 64-bit one was 8 % of the kernel's instructions)
@@ -659,10 +717,10 @@ __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkE
         X.qseed = P.query_seed ? (uint64_t)P.query_seed[query] : (uint64_t)(sub ? (uint32_t)D.query - q_blk * sub : (uint32_t)D.query);
         X.base_seed = P.base_seed_dev ? P.base_seed_dev[q_blk] : P.base_seed;
         X.recs = P.trecs + D.rec_base;
-        X.out_row = P.out + D.out_base;
-        X.base_elems = (int64_t)(reinterpret_cast<uintptr_t>(P.out) >> 2) + D.out_base;
+        X.out_row = static_cast<T *>(P.out) + D.out_base;
+        X.base_elems = (int64_t)(reinterpret_cast<uintptr_t>(P.out) / sizeof(T)) + D.out_base;
         // (kernel parameters are indexed with a compile-time subscript: a run-time one would copy them to local memory)
-        const TrkDesc *T = Tp;
+        const TrkDesc *Td = Tp;
 #define GVL_TRK_PICK(i) case i: if (!Tp) { X.srcg.its = P.inl[i].itv_starts; X.srcg.ite = P.inl[i].itv_ends; X.srcg.itv = P.inl[i].itv_values; \
                                            X.srcg.dense = P.inl[i].dense; X.strategy = P.inl[i].strategy; X.param = P.inl[i].param; } break;
         switch (track) {
@@ -670,9 +728,9 @@ __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkE
             default: break;
         }
 #undef GVL_TRK_PICK
-        if (T) {
-            X.srcg.its = T->itv_starts, X.srcg.ite = T->itv_ends, X.srcg.itv = T->itv_values, X.srcg.dense = T->dense;
-            X.strategy = T->strategy, X.param = T->param;
+        if (Td) {
+            X.srcg.its = Td->itv_starts, X.srcg.ite = Td->itv_ends, X.srcg.itv = Td->itv_values, X.srcg.dense = Td->dense;
+            X.strategy = Td->strategy, X.param = Td->param;
         }
         X.srcg.itv_lo = D.it_lo, X.srcg.itv_hi = D.it_hi, X.srcg.q_start = D.q_start, X.srcg.track_n = D.track_n;
     }
@@ -684,10 +742,10 @@ __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkE
         return;
     }
     if (D.flags & TD_BIG) {
-        if (threadIdx.x == 0) *reinterpret_cast<TileCtx *>(S.big_ctx) = X;
+        if (threadIdx.x == 0) *reinterpret_cast<TileCtx<T> *>(S.big_ctx) = X;
         __syncthreads();
-        t3_tile_big(&S, dp);
+        t3_tile_big<T>(&S, dp);
     } else {
-        t3_tile<false>(X, D, S);
+        t3_tile<false, T>(X, D, S);
     }
 }

@@ -248,6 +248,18 @@ int gvl_dev_realign_tracks_plan(gvl_ctx *ctx, const gvl_sparse_tables *tab, cons
                                 int64_t max_records, int layout_btp, gvl_stream stream);
 int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream);
 
+/* Element type of a track output.  Values are computed in float32 as for GVL_TRACK_F32 and narrowed at the store with
+ * round-to-nearest-even (cvt.rn, no flush to zero: subnormals are kept, values beyond the float16 range become +-inf, NaN
+ * becomes the device's canonical NaN): bit for bit the float32 output cast to the type on the device.  Only the output
+ * changes: stored intervals stay float32. */
+#define GVL_TRACK_F32 0
+#define GVL_TRACK_BF16 1
+#define GVL_TRACK_F16 2
+/* gvl_dev_realign_tracks_exec writing elements of `dtype` (GVL_TRACK_*; any other value: GVL_ERR_ARG) into `out`
+ * (device, n_tracks * total_per_track elements, 16-byte aligned).  gvl_dev_realign_tracks_exec is its GVL_TRACK_F32 case.
+ * Serves every plan entry above (fixed layouts, per-row destinations, svar2 sources). */
+int gvl_dev_realign_tracks_exec_dtype(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream);
+
 /* gvl_dev_realign_tracks_plan with an explicit destination for every row in place of a fixed layout (`layout_btp` is
  * replaced by the table); followed by gvl_dev_realign_tracks_exec like the plan it extends.
  *   row_dst      device i64[b*p]: flat index in `out` of value 0 of row k = q*p + h for track 0
@@ -309,6 +321,14 @@ int gvl_dev_paint_tracks_rows(gvl_ctx *ctx, int64_t n_tracks, const gvl_interval
                               const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
                               const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, float *out,
                               gvl_stream stream);
+
+/* gvl_dev_paint_tracks_rows writing elements of `dtype` (GVL_TRACK_*, see gvl_dev_realign_tracks_exec_dtype) into `out`.
+ * row_dst and row_tstride both NULL: the (b, t, ~l) layout of gvl_dev_paint_tracks.  gvl_dev_paint_tracks and
+ * gvl_dev_paint_tracks_rows are its GVL_TRACK_F32 cases. */
+int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                               const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                               const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
+                               gvl_stream stream);
 
 /* ---- device layer: the small entries either side of reconstruction ------------------ */
 /* choose_exonic_variants, src/ffi/mod.rs:229-238 -> src/genotypes/mod.rs:132-176: for every (query, hap) row,
@@ -416,14 +436,16 @@ typedef struct gvl_fixed_job {
     int32_t realign;                  /* tracks are realigned to the haplotypes (needs mode >= 0 and ref_slot < 0) */
     int32_t rc_neg;                   /* reverse(-complement) rows of negative-strand regions */
     uint8_t pad_char;
+    int32_t track_dtype;              /* GVL_TRACK_* element type of `trk` (0 = float32) */
 } gvl_fixed_job;
 /* batch prep + variant plan (+ track plan and tile prep) of `n` queries; sub_batch as in gvl_dev_batch_prep. */
 int gvl_dev_fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *job, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
                        int64_t sub_batch, gvl_stream stream);
 /* the bandwidth-bound launches of the batch planned last on `ctx`: seq u8[n*rows_p*L (*4 one-hot)], annot_* i32[n*rows_p*L]
- * (GVL_MODE_ANNOTATED), trk f32[n*n_tracks*(ploidy|1)*L] in (b, t, p, L) / (b, t, L) order.  Unused outputs NULL. */
+ * (GVL_MODE_ANNOTATED), trk [n*n_tracks*(ploidy|1)*L] elements of job->track_dtype in (b, t, p, L) / (b, t, L) order.
+ * Unused outputs NULL. */
 int gvl_dev_fixed_exec(gvl_ctx *ctx, const gvl_fixed_job *job, int64_t n, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos,
-                       float *trk, gvl_stream stream);
+                       void *trk, gvl_stream stream);
 /* One stage of gvl_dev_fixed_plan / _exec, for callers that spread a device call over two streams: the track plan (a chain of
  * small latency-bound kernels) can run next to the bandwidth-bound haplotype execute.  Order: HAP_PLAN (batch prep +
  * haplotype plan) -> { HAP_EXEC, TRK_PLAN (reads the diffs of HAP_PLAN) } -> TRK_EXEC (after TRK_PLAN). */
@@ -432,14 +454,14 @@ int gvl_dev_fixed_exec(gvl_ctx *ctx, const gvl_fixed_job *job, int64_t n, uint8_
 #define GVL_STAGE_HAP_EXEC 3
 #define GVL_STAGE_TRK_EXEC 4
 int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *job, int stage, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
-                        int64_t sub_batch, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, float *trk, gvl_stream stream);
+                        int64_t sub_batch, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, void *trk, gvl_stream stream);
 /* The whole of a fixed-length `Dataset.__getitem__` in one call: ds_idx i64[n] / jitter i32[n] (optional) are HOST arrays
  * (pageable is fine, the caller may reuse them at once).  Up to 256 queries they travel BY VALUE with the batch-prep launch
  * (kernel parameter space: no copy, no event); larger batches are staged through a rotating pool of pinned slots owned by the
  * context into idx_dev / jitter_dev (device scratch, n entries), so the host never waits for earlier calls.  Indices are
  * range-checked against the view (GVL_ERR_ARG).  Then gvl_dev_fixed_plan + gvl_dev_fixed_exec on `stream`. */
 int gvl_dev_fixed_run(gvl_ctx *ctx, const gvl_fixed_job *job, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
-                      int64_t *idx_dev, int32_t *jitter_dev, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, float *trk,
+                      int64_t *idx_dev, int32_t *jitter_dev, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos, void *trk,
                       gvl_stream stream);
 
 /* ---- host layer: reference-shaped entries (host pointers in, host pointers out) ------ */
