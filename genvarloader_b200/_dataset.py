@@ -22,6 +22,7 @@ import torch
 
 from ._engine import Engine, track_dtype_code
 from ._insertion_fill import InsertionFill, Repeat5p, lower
+from ._variant_sizes import variant_buffer_sizes
 from ._types import (AnnotatedHaps, DummyVariant, Ragged, RaggedAlleles, RaggedAnnotatedHaps, RaggedVariants, VarWindowOpt,
                      build_token_lut)
 
@@ -828,8 +829,14 @@ class Dataset:
         device-to-host on a copy stream while the next one is produced, so a CPU consumer sees the PCIe copy rate instead of
         copy + compute + launch latency per batch (`copy=False`: views valid until the half comes around again).  float16
         tracks arrive as numpy float16; bfloat16 tracks raise ValueError (numpy has no bfloat16).
-        Datasets the pipeline cannot serve (ragged / variable lengths, random shifts, splicing, var_filter) fall back to
-        `mode=None`."""
+        `variants` / `variant-windows` (unspliced, no tracks, no var_filter, on the device): the same modes read `ring`
+        batches per device call (`_variants_loader.py`): one sizing pass over the ring's genotype rows and one wait, then
+        one variants tail over all of them, every batch a RaggedVariants with its own offsets starting at 0.  `ring=0`
+        targets about 2**20 variants per ring, estimated from the dataset's mean variants per genotype row (1 to 64 batches).
+        Rings alternate between two streams, so one is produced while the other is read; every ring gets fresh buffers, so
+        `copy=False` views stay valid for as long as they are held (at least until `ring` more batches have been drawn).
+        Other datasets the pipelines cannot serve (ragged / variable-length haplotypes, random shifts, splicing, var_filter)
+        fall back to `mode=None`."""
         if sampler is not None and shuffle:
             raise ValueError("sampler option is mutually exclusive with shuffle")
         if mode not in (None, "buffered", "double_buffered"):
@@ -840,6 +847,11 @@ class Dataset:
             if _pipeline.supports(self) is None:
                 return _pipeline.PipelinedLoader(self, int(batch_size), bool(shuffle), sampler, bool(drop_last), generator,
                                                  bool(return_indices), transform, bool(copy), ring, to_host=bool(to_host))
+            from . import _variants_loader
+
+            if not to_host and _variants_loader.supports(self) is None:
+                return _variants_loader.VariantsLoader(self, int(batch_size), bool(shuffle), sampler, bool(drop_last), generator,
+                                                       bool(return_indices), transform, bool(copy), ring)
         return BatchLoader(self, int(batch_size), bool(shuffle), sampler, bool(drop_last), generator, bool(return_indices), transform)
 
     # ------------------------------------------------------------------ the hot path
@@ -1030,33 +1042,54 @@ class Dataset:
     def _get_variants(self, t_goi, t_rc, contigs, n_variants: int, shape, cells=None) -> RaggedVariants:
         """The variants of the genotype rows `t_goi` (device strand flags `t_rc`, host `contigs` of every row) as a
         RaggedVariants of `shape`.  `n_variants` = the sum of the rows' genotype slice lengths, known from the host copy of
-        the offsets (no sync for it).  `cells`: device indices into the gathered row offsets (rows folded under
-        `unphased_union`) at which the output cells start, the last one = the end; None = one cell per row."""
-        p, eng = self.ploidy, self.engine
-        fold = p if self.unphased_union else 1
-        windows = self.sequence_type == "variant-windows"
-        tokens = row_contigs = None
-        if windows:
+        the offsets.  `cells`: device indices into the gathered row offsets (rows folded under `unphased_union`) at which
+        the output cells start, the last one = the end; None = one cell per row."""
+        row_contigs = None
+        if self._variant_tokens() is not None:  # contig of every row (_flat_variants.py:985-989)
+            row_contigs = torch.from_numpy(np.ascontiguousarray(contigs, np.int32)).to(self.engine.device)
+        g, _ = self._gather_variants(self.engine, t_goi, t_rc, row_contigs, n_variants)
+        off = g["row_offsets"] if cells is None else g["row_offsets"][cells]
+        return self._variants_result(g, off, shape)
+
+    def _variant_tokens(self):
+        """The token settings of the variants tail (Engine.gather_variants `tokens`), None without flank / window tokens."""
+        if self.sequence_type == "variant-windows":
             o = self.window_opt
             lut, _ = build_token_lut(o.token_alphabet, o.unknown_token)
-            tokens = dict(lut=lut, unk=o.unknown_token, L=o.flank_length, ref=1 if o.ref == "window" else 2,
-                          alt=1 if o.alt == "window" else 2)
-        elif self.flank_length and self.token_alphabet is not None:
+            return dict(lut=lut, unk=o.unknown_token, L=o.flank_length, ref=1 if o.ref == "window" else 2,
+                        alt=1 if o.alt == "window" else 2)
+        if self.flank_length and self.token_alphabet is not None:
             lut, _ = build_token_lut(self.token_alphabet, self.unknown_token)
-            tokens = dict(lut=lut, unk=self.unknown_token, L=self.flank_length, flank=True)
-        if tokens is not None:  # contig of every row (_flat_variants.py:985-989)
-            row_contigs = torch.from_numpy(np.ascontiguousarray(contigs, np.int32)).to(eng.device)
-        g = eng.gather_variants(t_goi, t_rc, self.var_fields, self.dummy_variant, self.min_af, self.max_af, fold, tokens, row_contigs,
-                                n_hint=n_variants)
-        off = g["row_offsets"] if cells is None else g["row_offsets"][cells]
-        fields = {}
+            return dict(lut=lut, unk=self.unknown_token, L=self.flank_length, flank=True)
+        return None
+
+    def _gather_variants(self, eng, t_goi, t_rc, row_contigs, n_variants: int):
+        """The variants tail over the genotype rows `t_goi` on `eng` (this dataset's engine or a fork of it) and the current
+        stream: the sizing pass and its one wait, then every buffer allocated at its final size -> (gather_variants dict,
+        VariantSizes with one cell per output row)."""
+        fold = self.ploidy if self.unphased_union else 1
+        tokens = self._variant_tokens()
+        sums = eng.variant_row_sizes(t_goi, self.min_af, self.max_af)
+        sizes = variant_buffer_sizes(sums, fold, self.dummy_variant, tokens["L"] if tokens is not None else 0)
+        g = eng.gather_variants(t_goi, t_rc, self.var_fields, sizes, n_variants, self.dummy_variant, self.min_af, self.max_af, fold,
+                                tokens, row_contigs)
+        return g, sizes
+
+    def _variant_field_names(self, g) -> list:
+        """The fields of a RaggedVariants in output order; `flank_tokens` last when present."""
+        windows = self.sequence_type == "variant-windows"
         names = [n for n in self.var_fields if not (windows and n in ("alt", "ref"))]
         names += [n for n in ("ref_window", "alt_window", "ref", "alt") if windows and n in g]  # token buffers of the windows tail
-        for name in names:
+        return names + (["flank_tokens"] if "flank_tokens" in g else [])
+
+    def _variants_result(self, g, off, shape) -> RaggedVariants:
+        fields = {}
+        for name in self._variant_field_names(g):
             v = g[name]
-            fields[name] = RaggedAlleles(v[0], v[1], off, shape) if isinstance(v, tuple) else Ragged(v, off, shape)
-        if "flank_tokens" in g:  # (b, p, ~v, 2 L): the trailing token axis stays on `data`
-            fields["flank_tokens"] = Ragged(g["flank_tokens"].view(-1, 2 * self.flank_length), off, shape)
+            if name == "flank_tokens":  # (b, p, ~v, 2 L): the trailing token axis stays on `data`
+                fields[name] = Ragged(v.view(-1, 2 * self.flank_length), off, shape)
+            else:
+                fields[name] = RaggedAlleles(v[0], v[1], off, shape) if isinstance(v, tuple) else Ragged(v, off, shape)
         return RaggedVariants(fields, off, shape)
 
     def _exonic_keep(self, t_goi, t_reg, goi):

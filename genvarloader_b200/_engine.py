@@ -15,6 +15,8 @@ from . import _ffi
 from ._ffi import (MODE_ANNOTATED, MODE_ONEHOT, MODE_ONEHOT_CF, MODE_U8, TRACK_BF16, TRACK_F16, TRACK_F32, DatasetView, Intervals,
                    SparseTables, Svar2Channels, c_i32, c_i64, c_u8, c_u64, c_vp, check, lib, ptr)
 
+_SVAR2_VARIANTS = ("`variants` output is built for the SVAR1 genotype CSR; the svar2 source decodes variants through its "
+                   "store (decode_variants_from_svar2_readbound, src/ffi/mod.rs:1692)")
 MODES = {"haplotypes": MODE_U8, "u8": MODE_U8, "onehot": MODE_ONEHOT, "onehot_cf": MODE_ONEHOT_CF,
          "annotated": MODE_ANNOTATED}
 # element types of track outputs (GVL_TRACK_*): values are computed in float32 and narrowed at the kernel's store
@@ -113,6 +115,7 @@ class Engine:
         self.var_info: dict[str, torch.Tensor] = {}   # 4-byte info columns on the device (output fields)
         self.var_info_host: dict[str, np.ndarray] = {}  # every info column (the AF filter is evaluated per variant on the host)
         self._af_tables: dict = {}
+        self._consts: dict = {}
         self.dosages = None
         self._n_work = 0
         self._fixed = -1
@@ -233,11 +236,49 @@ class Engine:
                 self._af_tables[key] = _dev(keep.astype(np.int32), np.int32, self.device)
         return self._af_tables[key]
 
-    def _scan_total(self, offsets: torch.Tensor) -> int:
-        return int(offsets[-1].item())  # the one synchronisation of a ragged output
+    def _const(self, a: np.ndarray) -> torch.Tensor:
+        """Device copy of a small constant array (token table, dummy allele), uploaded once: a pageable upload per read
+        would wait for the stream."""
+        key = (a.dtype.str, a.tobytes())
+        t = self._consts.get(key)
+        if t is None:
+            with torch.cuda.device(self.device):
+                t = self._consts[key] = _dev(a, a.dtype, self.device)
+        return t
 
-    def gather_variants(self, geno_offset_idx: torch.Tensor, to_rc_row, fields, dummy=None, min_af=None, max_af=None,
-                        fold: int = 1, tokens: dict | None = None, row_contigs=None, n_hint: int | None = None) -> dict:
+    def variant_row_sizes(self, geno_offset_idx: torch.Tensor, min_af=None, max_af=None) -> np.ndarray:
+        """gvl_dev_variant_row_sizes over the genotype rows `geno_offset_idx` (device i64) and one device-to-host copy: host
+        int64 (n_rows, 4) = (variants kept by the AF filter, sum of their ALT lengths, of their REF lengths -- 0 without
+        REF strings -- and of their reference spans).  The one wait of a variants read: it waits for the current stream."""
+        if self.svar2 is not None:
+            raise NotImplementedError(_SVAR2_VARIANTS)
+        goi = geno_offset_idx.reshape(-1)
+        n = goi.numel()
+        host = torch.empty((n, 4), dtype=torch.int64, pin_memory=True)
+        if n:
+            keep = self._af_keep_table(min_af, max_af) if (min_af is not None or max_af is not None) else None
+            ref_off = self.ref_alleles[1] if self.ref_alleles is not None else None
+            with torch.cuda.device(self.device):
+                out = torch.empty((n, 4), dtype=torch.int64, device=self.device)
+                check(lib.gvl_dev_variant_row_sizes(self.ctx.handle, C.byref(self.tab), ptr(goi), c_i64(n), ptr(keep), ptr(ref_off),
+                                                    ptr(out), _stream()))
+                host.copy_(out, non_blocking=True)
+                torch.cuda.current_stream(self.device).synchronize()
+        return host.numpy()
+
+    def rebase_offsets(self, offsets: torch.Tensor, n_batches: int, stride: int, bounds: torch.Tensor | None = None) -> torch.Tensor:
+        """gvl_dev_rebase_offsets: the offsets of `n_batches` consecutive batches read as one call, each batch's own offsets
+        starting at 0, back to back: batch i owns items [s_i, s_{i+1}) of `offsets` (n + 1 entries), s_i = min(i * stride, n),
+        or bounds[min(i * stride, len(bounds) - 1)] given device `bounds`.  Returns int64 (n + n_batches,)."""
+        n = offsets.numel() - 1
+        out = torch.empty(n + n_batches, dtype=torch.int64, device=self.device)
+        nb = bounds.numel() - 1 if bounds is not None else 0
+        check(lib.gvl_dev_rebase_offsets(self.ctx.handle, ptr(offsets), c_i64(n), ptr(bounds), c_i64(nb), c_i64(int(stride)),
+                                         c_i64(int(n_batches)), ptr(out), _stream()))
+        return out
+
+    def gather_variants(self, geno_offset_idx: torch.Tensor, to_rc_row, fields, sizes, n_gathered: int, dummy=None, min_af=None,
+                        max_af=None, fold: int = 1, tokens: dict | None = None, row_contigs=None) -> dict:
         """The tail of `get_variants_flat` (python/genvarloader/_dataset/_flat_variants.py:869-1112) on the device: per
         (b*p) row the variant indices of its genotype slice (gather_rows, src/variants/mod.rs:6-49), optional AF
         compaction (:112-153), positions / indel lengths / info columns (`table[v_idxs]`), ALT / REF allele strings
@@ -248,12 +289,13 @@ class Engine:
         "alt": likewise, "flank": bool} adds the token buffers of `assemble_variant_buffers` (src/variants/windows.rs:162-296):
         `flank_tokens` for the variants tail, `ref_window` / `alt_window` / tokenised `ref` / `alt` for the windows tail
         (then `alt` / `ref` in `fields` are skipped and nothing is reverse-complemented: windows are reference-oriented);
-        `row_contigs`: device i32, contig of every (b*p) row.  `n_hint`: the number of gathered variants when the caller
-        already knows it (the host holds the genotype offsets: `max_records`), which saves the first synchronisation.
+        `row_contigs`: device i32, contig of every (b*p) row.  `sizes`: the `VariantSizes` of these rows and settings
+        (`_variant_sizes.variant_buffer_sizes` over `variant_row_sizes`), `n_gathered`: the rows' summed genotype slice
+        lengths (`max_records`, from the host copy of the genotype offsets): every buffer is sized from them, so nothing
+        here waits for the device.
         Returns {"row_offsets": i64, "v_idxs": i32, name: tensor | (data, seq_offsets)}."""
         if self.svar2 is not None:
-            raise NotImplementedError("`variants` output is built for the SVAR1 genotype CSR; the svar2 source decodes variants "
-                                      "through its store (decode_variants_from_svar2_readbound, src/ffi/mod.rs:1692)")
+            raise NotImplementedError(_SVAR2_VARIANTS)
         h, dev, st = self.ctx.handle, self.device, _stream
         goi = geno_offset_idx.reshape(-1).contiguous()
         n_rows = goi.numel()
@@ -261,7 +303,7 @@ class Engine:
         with torch.cuda.device(dev):
             row_off = i64(n_rows + 1)
             check(lib.gvl_dev_gather_rows_offsets(h, ptr(goi), c_i64(n_rows), ptr(self.geno_starts), ptr(self.geno_stops), ptr(row_off), st()))
-            n = int(n_hint) if n_hint is not None else self._scan_total(row_off)
+            n = int(n_gathered)
             filtered = min_af is not None or max_af is not None
             v_idxs = torch.empty(n, dtype=torch.int32, device=dev)
             # positions and indel lengths ride along with the row gather (they are re-taken after an AF compaction)
@@ -285,7 +327,7 @@ class Engine:
                 keep = (take(self._af_keep_table(min_af, max_af)) != 0).view(torch.uint8)
                 pos, new_off = i64(n + 1), i64(n_rows + 1)
                 check(lib.gvl_dev_compact_keep_offsets(h, ptr(keep), c_i64(n), ptr(row_off), c_i64(n_rows), ptr(pos), ptr(new_off), st()))
-                n_keep = self._scan_total(pos)
+                n_keep = sizes.total("variants", filled=False)
                 kept = torch.empty(n_keep, dtype=torch.int32, device=dev)
                 check(lib.gvl_dev_compact_keep(h, ptr(v_idxs), ptr(keep), c_i64(n), ptr(pos), ptr(kept), st()))
                 if dosage is not None:  # compacted with the SAME mask (:923-926)
@@ -308,7 +350,7 @@ class Engine:
                 lut_np = np.ascontiguousarray(tokens["lut"])
                 tdt = torch.uint8 if lut_np.dtype == np.uint8 else torch.int32
                 tb = lut_np.dtype.itemsize
-                d_lut = torch.from_numpy(lut_np).to(dev)
+                d_lut = self._const(lut_np)
                 L = int(tokens["L"])
                 if fold > 1 and row_contigs is not None:
                     row_contigs = row_contigs[::fold].contiguous()
@@ -325,16 +367,16 @@ class Engine:
                         return data
                     w_off = i64(n + 1)
                     check(lib.gvl_dev_variant_windows_offsets(h, C.byref(self.tab), ptr(v_idxs), c_i64(n), c_i64(L), C.c_int(kind), ptr(w_off), st()))
-                    nt = self._scan_total(w_off)
+                    nt = sizes.total("alt_window" if kind == 1 else "ref_window", filled=False)
                     data = torch.empty(nt, dtype=tdt, device=dev)
                     check(lib.gvl_dev_variant_windows(h, C.byref(self.tab), ptr(v_idxs), ptr(v_contigs), c_i64(n), c_i64(L), C.c_int(kind),
                                                       c_u8(self.pad_char), ptr(d_lut), C.c_int(tb), ptr(w_off), c_i64(nt), ptr(data), st()))
                     return data, w_off
 
-                def tok_alleles(ab, ao):
+                def tok_alleles(name, ab, ao):
                     seq_off = i64(n + 1)
                     check(lib.gvl_dev_gather_alleles_offsets(h, ptr(v_idxs), c_i64(n), ptr(ao), ptr(seq_off), st()))
-                    nb = self._scan_total(seq_off)
+                    nb = sizes.total(name, filled=False)
                     data = torch.empty(nb, dtype=tdt, device=dev)
                     check(lib.gvl_dev_gather_alleles(h, ptr(v_idxs), c_i64(n), ptr(ab), ptr(ao), ptr(seq_off), c_i64(nb), ptr(d_lut),
                                                      C.c_int(tb), ptr(data), st()))
@@ -348,11 +390,11 @@ class Engine:
                     elif tokens.get("ref") == 2:
                         if self.ref_alleles is None:
                             raise ValueError("VarWindowOpt(ref='allele') needs the REF allele strings (ref_alleles=)")
-                        alleles["ref"], tok_dummy["ref"] = tok_alleles(*self.ref_alleles), d_ref
+                        alleles["ref"], tok_dummy["ref"] = tok_alleles("ref", *self.ref_alleles), d_ref
                     if tokens.get("alt") == 1:
                         alleles["alt_window"], tok_dummy["alt_window"] = window(1), 2 * L + d_alt
                     elif tokens.get("alt") == 2:
-                        alleles["alt"], tok_dummy["alt"] = tok_alleles(self.alt_alleles, self.alt_offsets), d_alt
+                        alleles["alt"], tok_dummy["alt"] = tok_alleles("alt", self.alt_alleles, self.alt_offsets), d_alt
                     to_rc_row = None
                 elif tokens.get("flank") and L > 0:
                     # 2 L tokens per variant; carried as a two-level ragged with constant strides so that the dummy fill
@@ -368,7 +410,7 @@ class Engine:
                     ab, ao = (self.alt_alleles, self.alt_offsets) if name == "alt" else self.ref_alleles
                     seq_off = i64(n + 1)
                     check(lib.gvl_dev_gather_alleles_offsets(h, ptr(v_idxs), c_i64(n), ptr(ao), ptr(seq_off), st()))
-                    nb = self._scan_total(seq_off)
+                    nb = sizes.total(name, filled=False)
                     data = torch.empty(nb, dtype=torch.uint8, device=dev)
                     check(lib.gvl_dev_gather_alleles(h, ptr(v_idxs), c_i64(n), ptr(ab), ptr(ao), ptr(seq_off), c_i64(nb), c_vp(0),
                                                      C.c_int(1), ptr(data), st()))
@@ -400,7 +442,7 @@ class Engine:
             # ---- one dummy variant per empty row (fill_empty_groups, _flat_variants.py:501-535) ----
             new_off = i64(n_rows + 1)
             check(lib.gvl_dev_fill_empty_offsets(h, ptr(row_off), c_i64(n_rows), ptr(new_off), st()))
-            n_new = self._scan_total(new_off)
+            n_new = sizes.total("variants")
             for name in list(out):
                 t = out[name]
                 np_dt = np.float32 if t.dtype == torch.float32 else np.int32
@@ -416,11 +458,11 @@ class Engine:
                     db = np.full(tok_dummy[name], tokens["unk"], np.uint8 if data.dtype == torch.uint8 else np.int32)
                 else:
                     db = np.frombuffer(dummy.alt if name == "alt" else dummy.ref, np.uint8)
-                d_dummy = torch.from_numpy(db.copy()).to(dev)
+                d_dummy = self._const(db)
                 new_seq = i64(n_new + 1)
                 check(lib.gvl_dev_fill_empty_seq_offsets(h, ptr(row_off), c_i64(n_rows), ptr(seq_off), c_i64(db.size), ptr(new_off),
                                                          c_i64(n_new), ptr(src_var), ptr(new_seq), st()))
-                nb = self._scan_total(new_seq)
+                nb = sizes.total(name)
                 filled = torch.empty(nb, dtype=data.dtype, device=dev)
                 check(lib.gvl_dev_fill_empty_seq(h, ptr(data), C.c_int(data.element_size()), ptr(seq_off), ptr(d_dummy), ptr(src_var),
                                                  ptr(new_seq), c_i64(n_new), c_i64(nb), ptr(filled), st()))

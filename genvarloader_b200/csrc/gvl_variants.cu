@@ -412,6 +412,64 @@ struct TakeU32 {
     __device__ void operator()(int64_t i) const { o[i] = __ldg(t + v[i]); }
 };
 
+// ---------------------------------------------------------------- sizing and ring offsets
+// One warp per genotype row: the lanes stride over the row's slice and reduce with a fixed shuffle tree, so a row of
+// thousands of variants costs its warp ~len / 32 steps and an empty row costs one.  Integer sums: exact and reproducible.
+constexpr int SIZE_T = 256;
+constexpr int SIZE_ROWS = SIZE_T / 32;  // rows per CTA
+
+__global__ void __launch_bounds__(SIZE_T)
+    variant_row_sizes_kernel(const int64_t *__restrict__ goi, int64_t n_rows, const int64_t *__restrict__ o_starts,
+                             const int64_t *__restrict__ o_stops, const int32_t *__restrict__ geno_v_idxs,
+                             const int32_t *__restrict__ keep, const int64_t *__restrict__ alt_off,
+                             const int64_t *__restrict__ ref_off, const int32_t *__restrict__ ilens, int64_t *__restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    for (int64_t r = (int64_t)blockIdx.x * SIZE_ROWS + (threadIdx.x >> 5); r < n_rows; r += (int64_t)gridDim.x * SIZE_ROWS) {
+        const int64_t g = goi[r], lo = o_starts[g], hi = o_stops[g];
+        int64_t n = 0, alt = 0, ref = 0, span = 0;
+        for (int64_t k = lo + lane; k < hi; k += 32) {
+            const int32_t v = __ldg(geno_v_idxs + k);
+            if (keep && !__ldg(keep + v)) continue;
+            n += 1;
+            alt += __ldg(alt_off + v + 1) - __ldg(alt_off + v);
+            if (ref_off) ref += __ldg(ref_off + v + 1) - __ldg(ref_off + v);
+            span += 1 - imin64((int64_t)__ldg(ilens + v), 0);
+        }
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            n += __shfl_xor_sync(0xffffffffu, n, d);
+            alt += __shfl_xor_sync(0xffffffffu, alt, d);
+            ref += __shfl_xor_sync(0xffffffffu, ref, d);
+            span += __shfl_xor_sync(0xffffffffu, span, d);
+        }
+        if (lane < 4) out[r * 4 + lane] = lane == 0 ? n : lane == 1 ? alt : lane == 2 ? ref : span;
+    }
+}
+
+// start of batch i of a ring: s_i = min(i * stride, n) over the items, or bounds[min(i * stride, n_bounds)]
+struct RingBounds {
+    const int64_t *bounds;
+    int64_t stride, n, n_bounds;
+    __device__ int64_t operator()(int64_t i) const {
+        if (!bounds) return imin64(i * stride, n);
+        return __ldg(bounds + imin64(i * stride, n_bounds));
+    }
+};
+
+// batch i owns out[s_i + i .. s_{i+1} + i]: the last batch i with s_i + i <= e (K is tens: a short binary search)
+__global__ void __launch_bounds__(256) rebase_offsets_kernel(const int64_t *__restrict__ off, RingBounds B, int64_t n_batches,
+                                                             int64_t n_out, int64_t *__restrict__ out) {
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n_out; e += (int64_t)gridDim.x * blockDim.x) {
+        int64_t lo = 0, hi = n_batches;
+        while (hi - lo > 1) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (B(mid) + mid <= e) lo = mid;
+            else hi = mid;
+        }
+        out[e] = __ldg(off + e - lo) - __ldg(off + B(lo));
+    }
+}
+
 inline cudaStream_t S(gvl_stream s) { return (cudaStream_t)s; }
 
 }  // namespace
@@ -614,6 +672,34 @@ int gvl_dev_take_u32(gvl_ctx *ctx, const void *table, const int32_t *v_idxs, int
     VARG(table && v_idxs && out, "gvl_dev_take_u32");
     GVL_CUDA(cudaSetDevice(ctx->device));
     return for_each(TakeU32{(const uint32_t *)table, v_idxs, (uint32_t *)out}, n, S(stream));
+}
+
+int gvl_dev_variant_row_sizes(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int64_t *geno_offset_idx, int64_t n_rows,
+                              const int32_t *keep_table, const int64_t *ref_offsets, int64_t *out_sizes, gvl_stream stream) {
+    VARG(ctx && tab && n_rows >= 0, "gvl_dev_variant_row_sizes");
+    if (n_rows == 0) return GVL_OK;
+    VARG(geno_offset_idx && out_sizes && tab->geno_starts && tab->geno_stops && tab->geno_v_idxs && tab->alt_offsets && tab->ilens,
+         "gvl_dev_variant_row_sizes");
+    GVL_CUDA(cudaSetDevice(ctx->device));
+    const int64_t blocks = imin64((n_rows + SIZE_ROWS - 1) / SIZE_ROWS, 148 * 16);
+    variant_row_sizes_kernel<<<(unsigned)blocks, SIZE_T, 0, S(stream)>>>(geno_offset_idx, n_rows, tab->geno_starts, tab->geno_stops,
+                                                                          tab->geno_v_idxs, keep_table, tab->alt_offsets,
+                                                                          ref_offsets, tab->ilens, out_sizes);
+    GVL_LAUNCH_CHECK();
+    return GVL_OK;
+}
+
+int gvl_dev_rebase_offsets(gvl_ctx *ctx, const int64_t *offsets, int64_t n, const int64_t *bounds, int64_t n_bounds,
+                           int64_t stride, int64_t n_batches, int64_t *out, gvl_stream stream) {
+    VARG(ctx && n >= 0 && n_batches >= 1 && stride >= 0 && (!bounds || n_bounds >= 0), "gvl_dev_rebase_offsets");
+    VARG(offsets && out, "gvl_dev_rebase_offsets");
+    GVL_CUDA(cudaSetDevice(ctx->device));
+    const int64_t n_out = n + n_batches;
+    const int64_t blocks = imin64((n_out + 255) / 256, 148 * 16);
+    rebase_offsets_kernel<<<(unsigned)blocks, 256, 0, S(stream)>>>(offsets, RingBounds{bounds, stride, n, n_bounds}, n_batches,
+                                                                   n_out, out);
+    GVL_LAUNCH_CHECK();
+    return GVL_OK;
 }
 
 }  // extern "C"

@@ -733,6 +733,21 @@ int gvl_dev_variant_windows(gvl_ctx *ctx, const gvl_sparse_tables *tab, const in
                             int64_t n, int64_t flank_len, int kind, uint8_t pad_char, const void *lut, int tok_bytes,
                             const int64_t *win_offsets, int64_t total, void *out, gvl_stream stream);
 
+/* Every buffer length of a variants read, from four sums per genotype row r (slot g = geno_offset_idx[r], the variants
+ * geno_v_idxs[geno_starts[g] .. geno_stops[g]) of the row, those with keep_table[v] == 0 left out; keep_table = per-variant
+ * int32 AF flags, NULL keeps every variant): out_sizes i64[n_rows * 4], row r = (variants kept, sum of their ALT lengths,
+ * sum of their REF lengths from ref_offsets (0 when NULL), sum of their reference spans 1 - min(ilen, 0)).  One warp per
+ * row, no atomics: reproducible, and safe to capture in a graph. */
+int gvl_dev_variant_row_sizes(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int64_t *geno_offset_idx, int64_t n_rows,
+                              const int32_t *keep_table, const int64_t *ref_offsets, int64_t *out_sizes, gvl_stream stream);
+/* Batch-local offsets of K consecutive batches read as one call.  offsets i64[n + 1] run over the items of the whole ring;
+ * batch i owns items [s_i, s_{i+1}) with s_i = min(i * stride, n) when bounds is NULL, else s_i = bounds[min(i * stride,
+ * n_bounds)] (bounds i64[n_bounds + 1], e.g. the ring's row offsets: a batch's rows turned into its variants).  s_0 must be
+ * 0 and s_K must be n.  Writes offsets[s_i .. s_{i+1}] - offsets[s_i] to out[s_i + i .. s_{i+1} + i]: out i64[n + K], every
+ * batch's offsets starting at 0, one launch for all K batches. */
+int gvl_dev_rebase_offsets(gvl_ctx *ctx, const int64_t *offsets, int64_t n, const int64_t *bounds, int64_t n_bounds,
+                           int64_t stride, int64_t n_batches, int64_t *out, gvl_stream stream);
+
 /* ---- host layer of the same entries: the reference's #[pyfunction] argument lists, host pointers in.  The reference
  * returns arrays it allocates; here a call leaves its results on the device, reports their sizes, and the caller copies
  * each one out with gvl_variants_fetch(which) into a buffer of exactly that size (results stay valid until the next
