@@ -4,7 +4,7 @@ from ._insertion_fill import Constant, FlankSample, InsertionFill, Interpolate, 
 
 __all__ = ["Dataset", "Engine", "AnnotatedHaps", "Ragged", "RaggedAnnotatedHaps", "InsertionFill", "Repeat5p",
            "Repeat5pNormalized", "Constant", "FlankSample", "Interpolate", "Reference", "DummyVariant", "RaggedAlleles",
-           "RaggedVariants", "VarWindowOpt"]
+           "RaggedVariants", "RaggedIntervals", "VarWindowOpt"]
 
 
 def __getattr__(name):  # torch + the CUDA library are loaded on first use
@@ -20,7 +20,8 @@ def __getattr__(name):  # torch + the CUDA library are loaded on first use
         from ._engine import Engine
 
         return Engine
-    if name in ("AnnotatedHaps", "Ragged", "RaggedAnnotatedHaps", "DummyVariant", "RaggedAlleles", "RaggedVariants", "VarWindowOpt"):
+    if name in ("AnnotatedHaps", "Ragged", "RaggedAnnotatedHaps", "DummyVariant", "RaggedAlleles", "RaggedVariants", "RaggedIntervals",
+                "VarWindowOpt"):
         from . import _types
 
         return getattr(_types, name)

@@ -23,8 +23,8 @@ import torch
 from ._engine import Engine, track_dtype_code
 from ._insertion_fill import InsertionFill, Repeat5p, lower
 from ._variant_sizes import variant_buffer_sizes
-from ._types import (AnnotatedHaps, DummyVariant, Ragged, RaggedAlleles, RaggedAnnotatedHaps, RaggedVariants, VarWindowOpt,
-                     build_token_lut)
+from ._types import (AnnotatedHaps, DummyVariant, Ragged, RaggedAlleles, RaggedAnnotatedHaps, RaggedIntervals, RaggedVariants,
+                     VarWindowOpt, build_token_lut)
 
 SeqKind = Literal["reference", "haplotypes", "annotated"]
 N_CHAR = ord("N")
@@ -59,6 +59,7 @@ class Dataset:
     output_length: object = "ragged"                  # "ragged" | "variable" | int
     sequence_type: object = "haplotypes"              # "reference" | "haplotypes" | "annotated" | None
     active_tracks: tuple = ()
+    track_output: str = "tracks"                      # with_tracks(kind=...): "tracks" (values) | "intervals"
     insertion_fill: dict = field(default_factory=dict)
     jitter: int = 0
     deterministic: bool = True
@@ -363,6 +364,9 @@ class Dataset:
                              "with_settings(unphased_union=False).")  # _impl.py:769-779
         if (self.min_af is not None or self.max_af is not None) and self.sequence_type not in ("variants", "variant-windows"):
             raise NotImplementedError("Filtering by AF is not supported for haplotype output yet.")  # _haps.py:695-698
+        if self.track_output == "intervals" and self._realigns:
+            raise ValueError("kind='intervals' returns the stored intervals, which are not realigned to haplotypes: set "
+                             "with_settings(realign_tracks=False), or use with_seqs('reference') or with_seqs(None).")
         if self.encoding != "bytes" and self.sequence_type not in ("haplotypes", "reference"):
             raise ValueError("one-hot encoding applies to 'haplotypes' / 'reference' sequences only")
         if self.encoding == "onehot_cf":
@@ -480,9 +484,12 @@ class Dataset:
         return self._evolve(track_dtype=dtype)
 
     def with_tracks(self, tracks=None, kind=None) -> "Dataset":
-        """Reference: `Dataset.with_tracks`, _impl.py:785-839.  `False`/`[]` disables tracks."""
-        if kind not in (None, "tracks"):
-            raise NotImplementedError("only kind='tracks' (base-pair resolution) is in the hot-path scope")
+        """Reference: `Dataset.with_tracks`, _impl.py:785-839.  `False`/`[]` disables tracks.  `kind`: None keeps the
+        current output kind; "tracks" returns base-pair values (painted or realigned), "intervals" the stored intervals
+        that overlap each read's window, clipped to it (`RaggedIntervals`, one cell per (..., track); DESIGN.md §7).
+        Intervals are not realigned: with haplotypes, set `with_settings(realign_tracks=False)` first."""
+        if kind not in (None, "tracks", "intervals"):
+            raise ValueError(f"Unknown track kind {kind!r}: 'tracks' or 'intervals'")
         if tracks is None:
             names = tuple(self.track_kinds)
         elif tracks is False:
@@ -492,12 +499,15 @@ class Dataset:
         missing = [t for t in names if t not in self.track_kinds]
         if missing:
             raise ValueError(f"Track(s) {missing} not found. Available tracks: {self.available_tracks}")
-        return self._evolve(active_tracks=names)
+        return self._evolve(active_tracks=names, track_output=self.track_output if kind is None else kind)
 
     def with_insertion_fill(self, strategy) -> "Dataset":
         """Reference: `Dataset.with_insertion_fill`, _impl.py:841-878 (one strategy for all tracks or a dict)."""
         if not self.track_kinds:
             raise ValueError("Dataset has no tracks; cannot configure insertion fill.")
+        if self.track_output == "intervals":
+            raise ValueError("with_insertion_fill has no effect on kind='intervals' (intervals are not realigned); use "
+                             "with_tracks(kind='tracks') first.")
         if self.sequence_type not in ("haplotypes", "annotated"):
             raise ValueError("with_insertion_fill is only meaningful for datasets with both haplotypes and tracks "
                              "(use with_seqs to activate haplotypes first).")
@@ -757,6 +767,14 @@ class Dataset:
                 i_q = pk.add(q, np.int64)
                 i_pf = pk.add(rows_p * e_first[e_pair], np.int64)       # first sequence row of the element's pair
                 i_pn = pk.add(rows_p * e_first[e_pair + 1], np.int64)   # ... and of the next pair
+            elif self.track_output == "intervals":
+                # rows (pair, track, element), each element over its own region: cell (pair, track) is a run of rows
+                tt = np.arange(t, dtype=np.int64)
+                row_of = (t * e_first[e_pair])[:, None] + tt[None, :] * n_el[e_pair][:, None] + e_k[:, None]
+                slot, tw = _interval_rows(oi, regions[:, 1], regions[:, 2], row_of)
+                i_islot, i_itw = pk.add(slot, np.int64), pk.add(tw, np.int32)
+                i_icells = pk.add(np.append((t * e_first[:-1, None] + tt[None, :] * n_el[:, None]).ravel(), t * e_first[-1]),
+                                  np.int64)
             else:
                 # painted: lengths are the element region lengths, known here -- the whole table is built on the host
                 off_e = np.concatenate([[0], np.cumsum(e_len)]).astype(np.int64)
@@ -800,6 +818,8 @@ class Dataset:
                 ds_idx_e, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), pk.get(i_len), diffs.view(-1)[t_q],
                 out_offsets, total, max_rec, keep, keep_off, pk.get(i_rc_e) if i_rc_e is not None else None, group_offsets,
                 (*outer, t, p, None), row_dst=row_dst, row_tstride=row_tstride))
+        elif t and self.track_output == "intervals":
+            results.append(self._track_intervals(pk.get(i_islot), pk.get(i_itw), (*outer, t, None), cells=pk.get(i_icells)))
         elif t:
             results.append(self._painted_tracks(pk.get(i_oi), pk.get(i_st), pk.get(i_off_e), int(off_e[-1]),
                                                 pk.get(i_rc_q) if i_rc_q is not None else None, pk.get(i_toff),
@@ -835,8 +855,8 @@ class Dataset:
         targets about 2**20 variants per ring, estimated from the dataset's mean variants per genotype row (1 to 64 batches).
         Rings alternate between two streams, so one is produced while the other is read; every ring gets fresh buffers, so
         `copy=False` views stay valid for as long as they are held (at least until `ring` more batches have been drawn).
-        Other datasets the pipelines cannot serve (ragged / variable-length haplotypes, random shifts, splicing, var_filter)
-        fall back to `mode=None`."""
+        Other datasets the pipelines cannot serve (ragged / variable-length haplotypes, random shifts, splicing, var_filter,
+        track intervals) fall back to `mode=None`."""
         if sampler is not None and shuffle:
             raise ValueError("sampler option is mutually exclusive with shuffle")
         if mode not in (None, "buffered", "double_buffered"):
@@ -917,6 +937,7 @@ class Dataset:
         # geno_offset_idx = ravel (region, sample, ploid), _haps.py:757-768.  "reference" rows use the engine's
         # empty CSR slot: the zero-variant case of the same kernels (get_reference, src/reference/mod.rs:56-120).
         rows_p = 1 if is_ref else p
+        out_len_q = np.full(b, int(self.output_length), np.int64) if fixed else lengths  # painted track / interval window
         if is_ref:
             goi = np.full((b, 1), eng.empty_slot, np.int64)
         else:
@@ -928,12 +949,16 @@ class Dataset:
         i_goi = pk.add(goi, np.int64)
         i_rc = pk.add(to_rc, np.uint8) if to_rc is not None else None
         i_sh = pk.add(np.zeros((b, rows_p), np.int32), np.int32)
-        i_tr = i_trc = None
+        i_tr = i_trc = i_islot = i_itw = None
         if want_tracks:
             oi = np.stack([ds_idx if self.track_kinds[n] == "sample" else r_idx for n in self.active_tracks])
-            i_tr = pk.add(oi, np.int64)
-            if to_rc_q is not None:
-                i_trc = pk.add(to_rc_q, np.uint8)
+            if self.track_output == "intervals":  # rows (q, track)
+                slot, tw = _interval_rows(oi, regions[:, 1], regions[:, 1] + out_len_q, np.arange(b * len(oi)).reshape(b, len(oi)))
+                i_islot, i_itw = pk.add(slot, np.int64), pk.add(tw, np.int32)
+            else:
+                i_tr = pk.add(oi, np.int64)
+                if to_rc_q is not None:
+                    i_trc = pk.add(to_rc_q, np.uint8)
         pk.upload()
         t_reg, t_goi, t_shifts = pk.get(i_reg), pk.get(i_goi), pk.get(i_sh)
         t_rc = pk.get(i_rc) if i_rc is not None else None
@@ -967,8 +992,9 @@ class Dataset:
             if self._realigns:
                 results.append(self._realigned_tracks(ds_idx, t_reg, t_shifts, t_goi, pk.get(i_tr), torch.from_numpy(lengths).to(dev),
                                                       diffs, oo, total, max_rec, keep, keep_off, t_rc, oo, (b, t, p, None)))
+            elif i_islot is not None:
+                results.append(self._track_intervals(pk.get(i_islot), pk.get(i_itw), (b, t, None)))
             else:
-                out_len_q = np.full(b, int(self.output_length), np.int64) if fixed else lengths
                 offs = np.concatenate([[0], np.cumsum(out_len_q)]).astype(np.int64)
                 d_off = torch.from_numpy(offs).to(dev)
                 results.append(self._painted_tracks(pk.get(i_tr), t_reg[:, 1].contiguous(), d_off, int(offs[-1]),
@@ -1039,6 +1065,17 @@ class Dataset:
                                        layout="rows" if rows else "btp", dtype=self.track_dtype, **rows)
         return Ragged(out, offsets, shape)
 
+    def _track_intervals(self, row_slot, row_tw, shape, cells=None) -> RaggedIntervals:
+        """The stored intervals of the active tracks over one window per row (gvl_dev_track_intervals): row k reads slot
+        `row_slot[k]` (device int64) of track `row_tw[0, k]` over [`row_tw[1, k]`, `row_tw[2, k]`) (device int32 (3, n),
+        `_interval_rows`), clipped to it.  Strand changes nothing: coordinates stay on the reference.  `cells`: device
+        indices into the row offsets at which the output cells start, the last one = the end; None = one cell per row."""
+        off, starts, ends, values = self.engine.track_intervals(list(self.active_tracks), row_slot, row_tw[0], row_tw[1],
+                                                                row_tw[2], dtype=self.track_dtype)
+        if cells is not None:
+            off = off[cells]
+        return RaggedIntervals(Ragged(starts, off, shape), Ragged(ends, off, shape), Ragged(values, off, shape))
+
     def _get_variants(self, t_goi, t_rc, contigs, n_variants: int, shape, cells=None) -> RaggedVariants:
         """The variants of the genotype rows `t_goi` (device strand flags `t_rc`, host `contigs` of every row) as a
         RaggedVariants of `shape`.  `n_variants` = the sum of the rows' genotype slice lengths, known from the host copy of
@@ -1099,8 +1136,11 @@ class Dataset:
 
     # ---- output shaping, _query.py:94-127 ----
     def _shape_output(self, o, out_reshape, squeeze):
-        if isinstance(o, (torch.Tensor, AnnotatedHaps, RaggedVariants)) or self.output_format == "flat" or self.output_length == "ragged":
-            res = o  # already dense (fixed-length pipeline, channels-first one-hot); "flat"/"ragged" hand the flat triple back
+        if (isinstance(o, (torch.Tensor, AnnotatedHaps, RaggedVariants, RaggedIntervals)) or self.output_format == "flat"
+                or self.output_length == "ragged"):
+            # already dense (fixed-length pipeline, channels-first one-hot), ragged by nature (variants, intervals: the
+            # ragged axis counts items, not positions); "flat"/"ragged" hand the flat triple back
+            res = o
         elif self.output_length == "variable":
             if isinstance(o, RaggedAnnotatedHaps):
                 res = o.to_padded()
@@ -1120,6 +1160,19 @@ class Dataset:
         if squeeze:
             res = res.squeeze(0)  # (1 [p] l) -> ([p] l), _query.py:120-122
         return res
+
+
+def _interval_rows(oi: np.ndarray, w0: np.ndarray, w1: np.ndarray, row_of: np.ndarray):
+    """Host rows of a `_track_intervals` read: (element e, track t) reads slot oi[t, e] over [w0[e], w1[e]) as row
+    row_of[e, t] -> (slots int64 (n,), int32 (3, n) of track, w0, w1)."""
+    n_e, t = row_of.shape
+    slot = np.empty(n_e * t, np.int64)
+    tw = np.empty((3, n_e * t), np.int32)
+    slot[row_of] = oi.T
+    tw[0, row_of] = np.arange(t, dtype=np.int32)[None, :]
+    tw[1, row_of] = np.asarray(w0)[:, None]
+    tw[2, row_of] = np.asarray(w1)[:, None]
+    return slot, tw
 
 
 def _cell_offsets(row_offsets: torch.Tensor, t: int, p: int = 1) -> torch.Tensor:

@@ -677,6 +677,27 @@ class Engine:
                                        ptr(out_offsets), c_i64(int(total_per_track)), ptr(to_rc), ptr(out), _stream()))
         return out
 
+    def track_intervals(self, names, row_slot, row_track, row_w0, row_w1, dtype=torch.float32):
+        """gvl_dev_track_intervals: row k = the stored intervals of slot row_slot[k] (device i64) of track
+        names[row_track[k]] (device i32) that overlap [row_w0[k], row_w1[k]) (device i32), clipped to it.  A sizing call,
+        ONE wait for the total, then the emit call into buffers of exactly that size.  Returns (offsets i64 (n + 1,),
+        starts i32, ends i32, values of `dtype`): float32, or bfloat16 / float16 narrowed at the kernel's store."""
+        code = track_dtype_code(dtype)
+        n = int(row_slot.numel())
+        itv = self.track_descs(names)[0]
+        dev = self.device
+        offsets = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        rows = (ptr(row_slot), ptr(row_track), ptr(row_w0), ptr(row_w1), c_i64(n), ptr(offsets))
+        check(lib.gvl_dev_track_intervals(self.ctx.handle, itv, len(names), *rows, 0, None, None, None, code, _stream()))
+        total = int(offsets[-1])  # the read's one wait
+        starts = torch.empty(total, dtype=torch.int32, device=dev)
+        ends = torch.empty(total, dtype=torch.int32, device=dev)
+        values = torch.empty(total, dtype=dtype, device=dev)
+        if total:
+            check(lib.gvl_dev_track_intervals(self.ctx.handle, itv, len(names), *rows, total, ptr(starts), ptr(ends), ptr(values),
+                                              code, _stream()))
+        return offsets, starts, ends, values
+
     def check(self) -> None:
         """Synchronise and surface device-side status flags (workspace overflow)."""
         self.ctx.check(torch.cuda.current_stream().cuda_stream)

@@ -106,6 +106,8 @@ def _load() -> C.CDLL:
     lib.gvl_dev_realign_tracks_exec_dtype.argtypes = [c_vp, c_vp, c_i32, c_vp]
     lib.gvl_dev_paint_tracks_dtype.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i32,
                                                c_vp]
+    lib.gvl_dev_track_intervals.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32,
+                                            c_vp]
     return lib
 
 

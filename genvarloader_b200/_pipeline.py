@@ -101,6 +101,8 @@ def supports(ds) -> str | None:
         return "random shifts (deterministic=False) are drawn on the host from the batch's diffs"
     if ds.sequence_type is None and not ds.active_tracks:
         return "nothing to read"
+    if ds.track_output == "intervals" and ds.active_tracks:
+        return "track intervals are ragged by nature"
     if len(ds.active_tracks) > 8:
         return "more than 8 tracks"
     return None

@@ -222,6 +222,41 @@ class RaggedVariants:
         return self.reshape(tuple(outer))
 
 
+@dataclass(frozen=True)
+class RaggedIntervals:
+    """The `with_tracks(kind="intervals")` output: per (..., track) cell, the stored intervals that overlap the read's
+    window, in ascending position, clipped to it, in absolute 0-based reference coordinates.  Three `Ragged` fields share
+    `offsets` (intervals per cell): `starts` and `ends` int32, `values` of the dataset's track dtype."""
+
+    starts: Ragged
+    ends: Ragged
+    values: Ragged
+
+    @property
+    def offsets(self) -> torch.Tensor:
+        return self.starts.offsets
+
+    @property
+    def shape(self) -> tuple:
+        return self.starts.shape
+
+    @property
+    def lengths(self) -> torch.Tensor:
+        return self.starts.lengths
+
+    def reshape(self, shape) -> "RaggedIntervals":
+        return RaggedIntervals(self.starts.reshape(shape), self.ends.reshape(shape), self.values.reshape(shape))
+
+    def squeeze(self, axis=None) -> "RaggedIntervals":
+        return RaggedIntervals(self.starts.squeeze(axis), self.ends.squeeze(axis), self.values.squeeze(axis))
+
+    def to_list(self) -> list:
+        """Host copy: one list of (start, end, value) per cell, cells in row-major order (tests, debugging)."""
+        s, e = self.starts.data.cpu().tolist(), self.ends.data.cpu().tolist()
+        v, o = self.values.data.float().cpu().tolist(), self.offsets.cpu().tolist()
+        return [list(zip(s[a:b], e[a:b], v[a:b])) for a, b in zip(o[:-1], o[1:])]
+
+
 def build_token_lut(alphabet, unknown_token: int):
     """256-entry byte -> token table (reference `build_token_lut`, _flat_flanks.py:23-40): byte i of the alphabet maps to
     token i, every other byte (N, padding outside the contig) to `unknown_token`; uint8 when every token fits, else int32."""

@@ -143,6 +143,8 @@ struct gvl_ctx {
     int64_t zeros_bytes;
     void *var_scratch = nullptr;    // block sums of the offset scans (gvl_variants.cu)
     int64_t var_scratch_bytes = 0;
+    int64_t *itv_counts = nullptr;  // per-row interval counts of gvl_dev_track_intervals (gvl_tracks.cu)
+    int64_t itv_counts_cap = 0;
     std::vector<std::pair<void *, int64_t>> var_results;  // device results of the last host-layer variants entry (gvl_variants_fetch)
     // host layer
     std::map<const void *, gvl_static_entry> statics;

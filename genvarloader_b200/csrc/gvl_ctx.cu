@@ -192,6 +192,7 @@ void gvl_ctx_destroy(gvl_ctx *ctx) {
     cudaFree(ctx->trk_desc);
     cudaFree(ctx->zeros);
     cudaFree(ctx->var_scratch);
+    cudaFree(ctx->itv_counts);
     free(ctx->trk_params);
     if (ctx->host_words) cudaFreeHost(ctx->host_words);
     for (auto &kv : ctx->statics) cudaFree(kv.second.dev);

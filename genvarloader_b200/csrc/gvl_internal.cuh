@@ -14,6 +14,9 @@ int ensure_trecs(gvl_ctx *ctx, gvl_workspace &ws, int64_t n);
 int ensure_tdesc(gvl_ctx *ctx, gvl_workspace &ws, int64_t n);
 int ensure_zeros(gvl_ctx *ctx, int64_t bytes, cudaStream_t st);
 int ensure_var_scratch(gvl_ctx *ctx, int64_t bytes);
+// off[0] = 0, off[i + 1] = lengths[0] + ... + lengths[i]: the offset scan of the variants tail (gvl_variants.cu) over a
+// device array of lengths
+int scan_lengths(gvl_ctx *ctx, const int64_t *lengths, int64_t n, int64_t *off, cudaStream_t st);
 
 #define GVL_CUDA(expr)                                                                                  \
     do {                                                                                                \

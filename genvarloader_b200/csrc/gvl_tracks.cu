@@ -14,6 +14,9 @@
 // variant lists and dense sources resolve every value on its own.  gvl_tracks_exec.cuh has the details.
 // The output is float32, bfloat16 or float16 (GVL_TRACK_*): one execute instantiation per type, values narrowed at the
 // store.
+//
+// gvl_dev_track_intervals returns the stored intervals themselves instead of painting them: a count kernel (one warp per
+// row, two 32-ary searches), the offset scan of the variants tail, and an emit kernel that copies each row's run.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -128,6 +131,73 @@ struct TrkExecParams {
 
 __global__ void prng_kernel(uint64_t a, uint64_t b, uint64_t c, uint64_t d, int which, uint64_t *out) {
     *out = which ? hash4(a, b, c, d) : xorshift64(a);
+}
+
+// =====================================================================================
+// intervals: a slot's stored intervals over one window per row, clipped (gvl_dev_track_intervals)
+// =====================================================================================
+constexpr int ITV_THREADS = 256;  // 8 warps per CTA, one warp per row
+
+struct ItvRows {
+    gvl_intervals tracks[MAX_TRACKS];  // (by value: 40 bytes each, the parameters stay under 4 KB)
+    int64_t n_tracks;
+    const int64_t *slot;
+    const int32_t *track, *w0, *w1;
+    int64_t n_rows;
+};
+
+// The intervals of row q that reach into its window [w0, w1): [lo, lo + n) of its track's arrays, or n = 0 (also for a
+// slot or track out of range).  A slot is sorted and free of overlaps, so its starts and its ends are both sorted: lo is
+// the first interval with end > w0 and lo + n the first with start >= w1.  `count` = false skips the second search.
+// Every lane of the warp calls it for the same row.
+__device__ __forceinline__ const gvl_intervals *itv_row(const ItvRows &R, int64_t q, bool count, int64_t &lo, int64_t &n) {
+    lo = n = 0;
+    const int32_t t = __ldg(R.track + q), w0 = __ldg(R.w0 + q), w1 = __ldg(R.w1 + q);
+    const int64_t slot = __ldg(R.slot + q);
+    if (t < 0 || t >= R.n_tracks || w1 <= w0) return nullptr;
+    const gvl_intervals *I = &R.tracks[t];
+    if (slot < 0 || slot >= I->n_slots) return nullptr;
+    const int64_t s1 = __ldg(I->itv_offsets + slot + 1);
+    lo = warp_upper_le(I->itv_ends, __ldg(I->itv_offsets + slot), s1, w0) + 1;
+    if (count) n = warp_upper_le(I->itv_starts, lo, s1, w1 - 1) + 1 - lo;
+    else n = s1 - lo;  // (an upper bound: the caller knows the count)
+    return I;
+}
+
+__global__ void __launch_bounds__(ITV_THREADS) itv_count_kernel(const __grid_constant__ ItvRows R, int64_t *__restrict__ counts) {
+    const int64_t n_warps = (int64_t)gridDim.x * (ITV_THREADS / 32);
+    for (int64_t q = ((int64_t)blockIdx.x * ITV_THREADS + threadIdx.x) / 32; q < R.n_rows; q += n_warps) {
+        int64_t lo, n;
+        itv_row(R, q, true, lo, n);
+        if (lane_id() == 0) counts[q] = n;
+    }
+}
+
+// Row q's intervals go to [off[q], off[q + 1]): lanes copy consecutive intervals (coalesced loads and stores), the first
+// and the last one clipped to the window, values narrowed to T at the store as in the track execute (to_out).  A row that
+// does not fit `cap` or its slot is left unwritten.
+template <class T>
+__global__ void __launch_bounds__(ITV_THREADS) itv_emit_kernel(const __grid_constant__ ItvRows R, const int64_t *__restrict__ off,
+                                                               int64_t cap, int32_t *__restrict__ o_starts,
+                                                               int32_t *__restrict__ o_ends, T *__restrict__ o_values) {
+    const int lane = lane_id();
+    const int64_t n_warps = (int64_t)gridDim.x * (ITV_THREADS / 32);
+    for (int64_t q = ((int64_t)blockIdx.x * ITV_THREADS + threadIdx.x) / 32; q < R.n_rows; q += n_warps) {
+        const int64_t o = __ldg(off + q), n = __ldg(off + q + 1) - o;
+        if (n <= 0 || o < 0 || o + n > cap) continue;
+        int64_t lo, avail;
+        const gvl_intervals *I = itv_row(R, q, false, lo, avail);
+        if (!I || n > avail) continue;
+        const int32_t w0 = __ldg(R.w0 + q), w1 = __ldg(R.w1 + q);
+        for (int64_t i = lane; i < n; i += 32) {
+            int32_t s = __ldg(I->itv_starts + lo + i), e = __ldg(I->itv_ends + lo + i);
+            if (i == 0) s = max(s, w0);
+            if (i == n - 1) e = min(e, w1);
+            o_starts[o + i] = s;
+            o_ends[o + i] = e;
+            o_values[o + i] = to_out<T>(__ldg(I->itv_values + lo + i));
+        }
+    }
 }
 
 }  // namespace gvl
@@ -458,6 +528,69 @@ int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_interva
     if (!row_dst != !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks_dtype: row_dst and row_tstride go together");
     return paint_impl("gvl_dev_paint_tracks_dtype", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
                       total_per_track, to_rc, out, stream, row_dst, row_tstride, dtype);
+}
+
+static int ensure_itv_counts(gvl_ctx *ctx, int64_t n) {
+    if (n <= ctx->itv_counts_cap) return GVL_OK;
+    GVL_CUDA(cudaDeviceSynchronize());
+    if (ctx->itv_counts) GVL_CUDA(cudaFree(ctx->itv_counts));
+    ctx->itv_counts = nullptr;
+    ctx->itv_counts_cap = 0;
+    const int64_t cap = imax64(2 * n, 4096);
+    GVL_CUDA(cudaMalloc(&ctx->itv_counts, sizeof(int64_t) * (size_t)cap));
+    ctx->itv_counts_cap = cap;
+    return GVL_OK;
+}
+
+int gvl_dev_track_intervals(gvl_ctx *ctx, const gvl_intervals *tracks, int64_t n_tracks, const int64_t *row_slot,
+                            const int32_t *row_track, const int32_t *row_w0, const int32_t *row_w1, int64_t n_rows,
+                            int64_t *out_offsets, int64_t cap, int32_t *out_starts, int32_t *out_ends, void *out_values,
+                            int32_t track_dtype, gvl_stream stream) {
+    const char *who = "gvl_dev_track_intervals";
+    if (!ctx || !out_offsets || n_rows < 0 || cap < 0) return fail(GVL_ERR_ARG, "%s: NULL argument or negative size", who);
+    if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "%s: 0..%d tracks per call", who, MAX_TRACKS);
+    if (!track_dtype_ok(track_dtype)) return fail(GVL_ERR_ARG, "%s: unknown track dtype %d", who, (int)track_dtype);
+    if (n_tracks && !tracks) return fail(GVL_ERR_ARG, "%s: NULL tracks", who);
+    for (int64_t t = 0; t < n_tracks; t++)
+        if (!tracks[t].itv_starts || !tracks[t].itv_ends || !tracks[t].itv_values || !tracks[t].itv_offsets || tracks[t].n_slots < 0)
+            return fail(GVL_ERR_ARG, "%s: track %lld has a NULL array", who, (long long)t);
+    if (n_rows && (!row_slot || !row_track || !row_w0 || !row_w1)) return fail(GVL_ERR_ARG, "%s: NULL row array", who);
+    if (cap && (!out_starts || !out_ends || !out_values)) return fail(GVL_ERR_ARG, "%s: NULL output with cap > 0", who);
+    cudaStream_t st = (cudaStream_t)stream;
+    GVL_CUDA(cudaSetDevice(ctx->device));
+    ItvRows R;
+    memset(&R, 0, sizeof(R));
+    for (int64_t t = 0; t < n_tracks; t++) R.tracks[t] = tracks[t];
+    R.n_tracks = n_tracks;
+    R.slot = row_slot;
+    R.track = row_track;
+    R.w0 = row_w0;
+    R.w1 = row_w1;
+    R.n_rows = n_rows;
+    const unsigned blocks = (unsigned)imin64(imax64((n_rows + ITV_THREADS / 32 - 1) / (ITV_THREADS / 32), 1), 148 * 32);
+    if (cap == 0) {  // sizing call: counts, then their offsets
+        int rc;
+        if (n_rows) {
+            if ((rc = ensure_itv_counts(ctx, n_rows))) return rc;
+            itv_count_kernel<<<blocks, ITV_THREADS, 0, st>>>(R, ctx->itv_counts);
+            GVL_LAUNCH_CHECK();
+        }
+        return scan_lengths(ctx, ctx->itv_counts, n_rows, out_offsets, st);
+    }
+    if (n_rows == 0) return GVL_OK;
+    switch (track_dtype) {
+        case GVL_TRACK_F32:
+            itv_emit_kernel<float><<<blocks, ITV_THREADS, 0, st>>>(R, out_offsets, cap, out_starts, out_ends, (float *)out_values);
+            break;
+        case GVL_TRACK_BF16:
+            itv_emit_kernel<__nv_bfloat16><<<blocks, ITV_THREADS, 0, st>>>(R, out_offsets, cap, out_starts, out_ends,
+                                                                           (__nv_bfloat16 *)out_values);
+            break;
+        default:
+            itv_emit_kernel<__half><<<blocks, ITV_THREADS, 0, st>>>(R, out_offsets, cap, out_starts, out_ends, (__half *)out_values);
+    }
+    GVL_LAUNCH_CHECK();
+    return GVL_OK;
 }
 
 static int run_prng(gvl_ctx *ctx, uint64_t a, uint64_t b, uint64_t c, uint64_t d, int which, uint64_t *out) {

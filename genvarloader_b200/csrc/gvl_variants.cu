@@ -161,6 +161,11 @@ int scan_offsets(gvl_ctx *ctx, F f, int64_t n, int64_t *off, cudaStream_t st) {
     return GVL_OK;
 }
 
+struct ArrayLen {
+    const int64_t *len;
+    __device__ int64_t operator()(int64_t i) const { return __ldg(len + i); }
+};
+
 // last segment s in [0, n_seg) with off[s] <= e (off[0] = 0 <= e always): empty segments are skipped
 __device__ __forceinline__ int64_t seg_of(const int64_t *__restrict__ off, int64_t n_seg, int64_t e) {
     int64_t lo = 0, hi = n_seg;
@@ -473,6 +478,14 @@ __global__ void __launch_bounds__(256) rebase_offsets_kernel(const int64_t *__re
 inline cudaStream_t S(gvl_stream s) { return (cudaStream_t)s; }
 
 }  // namespace
+
+namespace gvl {
+
+int scan_lengths(gvl_ctx *ctx, const int64_t *lengths, int64_t n, int64_t *off, cudaStream_t st) {
+    return scan_offsets(ctx, ArrayLen{lengths}, n, off, st);
+}
+
+}  // namespace gvl
 
 #define VARG(cond, name) \
     if (!(cond)) return fail(GVL_ERR_ARG, name ": NULL argument or bad size")

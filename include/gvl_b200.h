@@ -330,6 +330,21 @@ int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_interva
                                const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
                                gvl_stream stream);
 
+/* The stored intervals of one slot over one window per row (the "intervals" kind of Dataset.with_tracks).  tracks is a
+ * HOST array of n_tracks (<= 64) descriptors; row k (device arrays of n_rows entries) reads slot row_slot[k] of track
+ * row_track[k] over the window [row_w0[k], row_w1[k]): the intervals with end > w0 and start < w1, in stored order, the
+ * first one's start raised to w0 and the last one's end lowered to w1.  An empty window (w1 <= w0), or a slot or track
+ * out of range, gives no intervals.  Two calls over the same rows:
+ *   cap == 0: writes out_offsets (device i64[n_rows + 1], row k's intervals at [out_offsets[k], out_offsets[k + 1])) and
+ *             nothing else; the caller reads out_offsets[n_rows] to size the outputs;
+ *   cap > 0:  reads those out_offsets and writes out_starts / out_ends (device i32[cap]) and out_values (device, cap
+ *             elements of track_dtype, GVL_TRACK_*: the float32 values narrowed as by gvl_dev_realign_tracks_exec_dtype).
+ *             A row whose intervals would end past cap is not written. */
+int gvl_dev_track_intervals(gvl_ctx *ctx, const gvl_intervals *tracks, int64_t n_tracks, const int64_t *row_slot,
+                            const int32_t *row_track, const int32_t *row_w0, const int32_t *row_w1, int64_t n_rows,
+                            int64_t *out_offsets, int64_t cap, int32_t *out_starts, int32_t *out_ends, void *out_values,
+                            int32_t track_dtype, gvl_stream stream);
+
 /* ---- device layer: the small entries either side of reconstruction ------------------ */
 /* choose_exonic_variants, src/ffi/mod.rs:229-238 -> src/genotypes/mod.rs:132-176: for every (query, hap) row,
  * keep_offsets[k+1] - keep_offsets[k] = size of its genotype slice and keep[keep_offsets[k] + i] = 1 iff variant i
