@@ -699,8 +699,9 @@ class Dataset:
         Tracks: the element batch E lists every (element region, sample) of the selected pairs in output order.  One track
         call covers all of E and all active tracks -- realigned to the element haplotypes (rows (e, ploid)) or painted over
         the element regions (rows e) -- and writes every row straight into its place in the concatenated output through a
-        per-row destination table (gvl_dev_realign_tracks_plan_rows / gvl_dev_paint_tracks_rows).  The values are those of
-        one unspliced call over E: the same fill seed (of E's dataset indices), FlankSample rows and track lengths.
+        per-row destination table (GVL_TRACK_LAYOUT_ROWS of gvl_dev_realign_tracks / gvl_dev_paint_tracks).  The values
+        are those of one unspliced call over E: the same fill seed (of E's dataset indices), FlankSample rows and track
+        lengths.
 
         Variants: the genotype rows of E are gathered in cell order -- (pair, ploid, element), or (pair, element, ploid)
         under `unphased_union` so that the p rows folded into one belong to one element -- with every element's own strand

@@ -13,7 +13,7 @@ import torch
 
 from . import _ffi
 from ._ffi import (MODE_ANNOTATED, MODE_ONEHOT, MODE_ONEHOT_CF, MODE_U8, TRACK_BF16, TRACK_F16, TRACK_F32, DatasetView, Intervals,
-                   SparseTables, Svar2Channels, c_i32, c_i64, c_u8, c_u64, c_vp, check, lib, ptr)
+                   SparseTables, Svar2Channels, c_i32, c_i64, c_u8, c_vp, check, lib, ptr)
 
 _SVAR2_VARIANTS = ("`variants` output is built for the SVAR1 genotype CSR; the svar2 source decodes variants through its "
                    "store (decode_variants_from_svar2_readbound, src/ffi/mod.rs:1692)")
@@ -21,6 +21,8 @@ MODES = {"haplotypes": MODE_U8, "u8": MODE_U8, "onehot": MODE_ONEHOT, "onehot_cf
          "annotated": MODE_ANNOTATED}
 # element types of track outputs (GVL_TRACK_*): values are computed in float32 and narrowed at the kernel's store
 TRACK_DTYPES = {torch.float32: TRACK_F32, torch.bfloat16: TRACK_BF16, torch.float16: TRACK_F16}
+# where the rows of a track output land (GVL_TRACK_LAYOUT_*)
+TRACK_LAYOUTS = {"tbp": 0, "btp": 1, "rows": 2}
 
 
 def track_dtype_code(dtype) -> int:
@@ -29,6 +31,13 @@ def track_dtype_code(dtype) -> int:
     if code is None:
         raise ValueError(f"track dtype must be torch.float32, torch.bfloat16 or torch.float16, got {dtype!r}")
     return code
+
+
+def _layout_code(layout: str) -> int:
+    """GVL_TRACK_LAYOUT_* code of a track layout name ("tbp", "btp" or "rows")."""
+    if layout not in TRACK_LAYOUTS:
+        raise ValueError(f'track layout must be "tbp", "btp" or "rows", got {layout!r}')
+    return TRACK_LAYOUTS[layout]
 
 
 _raw_stream = getattr(torch._C, "_cuda_getCurrentRawStream", None)  # ~1 us; torch.cuda.current_stream() costs ~15 us
@@ -574,107 +583,43 @@ class Engine:
             return itv, None, None
         return itv, (c_i32 * n)(*[int(s) for s in strategy_ids]), (C.c_double * n)(*[float(p) for p in params])
 
-    def _realign_args(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets, total_per_track,
-                      strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc, query_seed, base_seed_dev, batch,
-                      sub_batch):
-        """The arguments every gvl_dev_realign_tracks* entry takes after its variant source and before its layout."""
-        b_cap, ploidy = geno_offset_idx.shape
-        batch = b_cap if batch is None else int(batch)  # (a prefix of preallocated buffers)
-        itv, sid, par = self.track_descs(names, strategy_ids, params)
-        return (ptr(regions), ptr(shifts), ptr(geno_offset_idx), c_i64(batch), c_i64(ploidy), ptr(keep), ptr(keep_offsets),
-                ptr(to_rc), c_i64(len(names)), itv, ptr(offset_idxs), ptr(track_lengths), ptr(out_offsets),
-                c_i64(int(total_per_track)), sid, par, c_u64(int(base_seed)), ptr(base_seed_dev), c_i64(int(sub_batch)),
-                ptr(query_seed), c_i64(int(max_records)))
-
     def realign_tracks(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                        total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
                        keep_offsets=None, to_rc=None, query_seed=None, out=None, layout="tbp", base_seed_dev=None,
                        batch=None, sub_batch: int = 0, row_dst=None, row_tstride=None, dtype=torch.float32):
         """gvl_dev_realign_tracks: all `names` in one plan + one execute launch.
         offset_idxs: int64 (n_tracks, batch) device; out: `dtype` (n_tracks * total_per_track,), track-major
-        (layout="tbp", the reference's flat buffer), with every query's tracks adjacent (layout="btp",
-        gvl_dev_realign_tracks_btp: the order the reference's (b, t, p, ~l) offsets describe) or wherever the
-        per-row table puts each row (layout="rows": row k of track t starts at row_dst[k] + t * row_tstride[k],
-        device int64 (batch * ploidy,) each; gvl_dev_realign_tracks_plan_rows).  `dtype` (of `out` when given): float32,
-        or bfloat16 / float16 -- the float32 values rounded to nearest even by the execute kernel's stores."""
+        (layout="tbp", the reference's flat buffer), with every query's tracks adjacent (layout="btp": the order the
+        reference's (b, t, p, ~l) offsets describe) or wherever the per-row table puts each row (layout="rows": row k of
+        track t starts at row_dst[k] + t * row_tstride[k], device int64 (batch * ploidy,) each).  `dtype` (of `out` when
+        given): float32, or bfloat16 / float16 -- the float32 values rounded to nearest even by the execute kernel's stores."""
+        code = track_dtype_code(dtype if out is None else out.dtype)
         if out is None:
-            track_dtype_code(dtype)
             out = torch.empty(len(names) * total_per_track, dtype=dtype, device=self.device)
-        if self.svar2 is not None or layout == "rows" or out.dtype != torch.float32:
-            self.realign_tracks_plan(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
-                                     total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
-                                     query_seed, layout, base_seed_dev, batch, sub_batch, row_dst, row_tstride)
-            return self.realign_tracks_exec(out)
-        args = self._realign_args(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
-                                  total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
-                                  query_seed, base_seed_dev, batch, sub_batch)
-        fn = lib.gvl_dev_realign_tracks_btp if layout == "btp" else lib.gvl_dev_realign_tracks
-        check(fn(self.ctx.handle, C.byref(self.tab), *args, ptr(out), _stream()))
-        return out
-
-    def realign_tracks_plan(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
-                            total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
-                            keep_offsets=None, to_rc=None, query_seed=None, layout="tbp", base_seed_dev=None, batch=None,
-                            sub_batch: int = 0, row_dst=None, row_tstride=None):
-        """gvl_dev_realign_tracks_plan (layout="rows": gvl_dev_realign_tracks_plan_rows): everything of `realign_tracks`
-        but the execute launch (variant plan, tile map, per-tile searches); `realign_tracks_exec(out)` writes the values,
-        possibly on another stream."""
-        if layout == "rows" and (row_dst is None or row_tstride is None):
-            raise ValueError('layout="rows" needs row_dst and row_tstride')
-        args = self._realign_args(names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
-                                  total_per_track, strategy_ids, params, base_seed, max_records, keep, keep_offsets, to_rc,
-                                  query_seed, base_seed_dev, batch, sub_batch)
+        b_cap, ploidy = geno_offset_idx.shape
+        batch = b_cap if batch is None else int(batch)  # (a prefix of preallocated buffers)
+        itv, sid, par = self.track_descs(names, strategy_ids, params)
         ch = self.svar2_channels(geno_offset_idx) if self.svar2 is not None else None
-        src = C.byref(ch) if ch is not None else c_vp(0)
-        if layout == "rows":
-            check(lib.gvl_dev_realign_tracks_plan_rows(self.ctx.handle, C.byref(self.tab), src, *args, ptr(row_dst),
-                                                       ptr(row_tstride), _stream()))
-        else:
-            check(lib.gvl_dev_realign_tracks_plan(self.ctx.handle, C.byref(self.tab), src, *args,
-                                                  C.c_int(1 if layout == "btp" else 0), _stream()))
-
-    def realign_tracks_exec(self, out):
-        """gvl_dev_realign_tracks_exec_dtype: the planned call's values into `out`, in out's dtype (float32, bfloat16,
-        float16)."""
-        check(lib.gvl_dev_realign_tracks_exec_dtype(self.ctx.handle, ptr(out), track_dtype_code(out.dtype), _stream()))
-        return out
-
-    def intervals_to_tracks(self, name, offset_idxs, starts, out_offsets, total: int, out=None):
-        """gvl_dev_intervals_to_tracks: paint one track's stored intervals into dense windows."""
-        n_q = int(starts.numel())
-        if out is None:
-            out = torch.empty(total, dtype=torch.float32, device=self.device)
-        check(lib.gvl_dev_intervals_to_tracks(self.ctx.handle, C.byref(self.tracks[name][4]), ptr(offset_idxs), ptr(starts),
-                                              c_i64(n_q), ptr(out_offsets), c_i64(int(total)), ptr(out), _stream()))
+        check(lib.gvl_dev_realign_tracks(self.ctx.handle, C.byref(self.tab), None if ch is None else C.byref(ch), ptr(regions),
+                                         ptr(shifts), ptr(geno_offset_idx), batch, ploidy, ptr(keep), ptr(keep_offsets),
+                                         ptr(to_rc), len(names), itv, ptr(offset_idxs), ptr(track_lengths), ptr(out_offsets),
+                                         int(total_per_track), sid, par, int(base_seed), ptr(base_seed_dev), int(sub_batch),
+                                         ptr(query_seed), int(max_records), _layout_code(layout), ptr(row_dst),
+                                         ptr(row_tstride), ptr(out), code, _stream()))
         return out
 
     def paint_tracks(self, names, offset_idxs, starts, out_offsets, total_per_track: int, to_rc=None, out=None,
                      n_queries=None, layout="btp", row_dst=None, row_tstride=None, dtype=torch.float32):
-        """gvl_dev_paint_tracks: stored intervals of all `names` painted in one launch, (b, t, ~l) order,
-        masked rows reversed.  offset_idxs: int64 (n_tracks, batch) device.  layout="rows"
-        (gvl_dev_paint_tracks_rows): query q of track t starts at row_dst[q] + t * row_tstride[q] instead.
-        `dtype` (of `out` when given): float32, bfloat16 or float16 (gvl_dev_paint_tracks_dtype)."""
+        """gvl_dev_paint_tracks: stored intervals of all `names` painted in one launch, masked rows reversed, one row per
+        query.  offset_idxs: int64 (n_tracks, batch) device.  `layout` as in `realign_tracks` (default "btp": (b, t, ~l)
+        order) and `dtype` (of `out` when given): float32, bfloat16 or float16."""
+        code = track_dtype_code(dtype if out is None else out.dtype)
         n_tracks, n_q = len(names), int(starts.numel() if n_queries is None else n_queries)
-        itv = self.track_descs(names)[0]
         if out is None:
-            track_dtype_code(dtype)
             out = torch.empty(n_tracks * int(total_per_track), dtype=dtype, device=self.device)
-        if layout == "rows" and (row_dst is None or row_tstride is None):
-            raise ValueError('layout="rows" needs row_dst and row_tstride')
-        if out.dtype != torch.float32:
-            rows = layout == "rows"
-            check(lib.gvl_dev_paint_tracks_dtype(self.ctx.handle, n_tracks, itv, ptr(offset_idxs), ptr(starts), n_q,
-                                                 ptr(out_offsets), int(total_per_track), ptr(to_rc), ptr(row_dst if rows else None),
-                                                 ptr(row_tstride if rows else None), ptr(out), track_dtype_code(out.dtype),
-                                                 _stream()))
-            return out
-        if layout == "rows":
-            check(lib.gvl_dev_paint_tracks_rows(self.ctx.handle, n_tracks, itv, ptr(offset_idxs), ptr(starts), n_q,
-                                                ptr(out_offsets), int(total_per_track), ptr(to_rc), ptr(row_dst),
-                                                ptr(row_tstride), ptr(out), _stream()))
-            return out
-        check(lib.gvl_dev_paint_tracks(self.ctx.handle, c_i64(n_tracks), itv, ptr(offset_idxs), ptr(starts), c_i64(n_q),
-                                       ptr(out_offsets), c_i64(int(total_per_track)), ptr(to_rc), ptr(out), _stream()))
+        check(lib.gvl_dev_paint_tracks(self.ctx.handle, n_tracks, self.track_descs(names)[0], ptr(offset_idxs), ptr(starts),
+                                       n_q, ptr(out_offsets), int(total_per_track), ptr(to_rc), _layout_code(layout),
+                                       ptr(row_dst), ptr(row_tstride), ptr(out), code, _stream()))
         return out
 
     def track_intervals(self, names, row_slot, row_track, row_w0, row_w1, dtype=torch.float32):

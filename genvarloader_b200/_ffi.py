@@ -97,15 +97,15 @@ def _load() -> C.CDLL:
     lib.gvl_dev_fixed_exec.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
     lib.gvl_dev_fixed_stage.argtypes = [c_vp, c_vp, C.c_int, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
     lib.gvl_dev_fixed_run.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
-    # track entries with an explicit destination per row (spliced output)
-    lib.gvl_dev_realign_tracks_plan_rows.argtypes = [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_i64,
-                                                     c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_u64, c_vp, c_i64, c_vp, c_i64,
-                                                     c_vp, c_vp, c_vp]
-    lib.gvl_dev_paint_tracks_rows.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
-    # track outputs of a chosen element type (GVL_TRACK_*)
-    lib.gvl_dev_realign_tracks_exec_dtype.argtypes = [c_vp, c_vp, c_i32, c_vp]
-    lib.gvl_dev_paint_tracks_dtype.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i32,
-                                               c_vp]
+    # the track entries (up to 30 arguments: a wrong count must fail here, not reach the device)
+    lib.gvl_dev_realign_tracks.argtypes = [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp,
+                                           c_vp, c_vp, c_i64, c_vp, c_vp, c_u64, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp,
+                                           c_i32, c_vp]
+    lib.gvl_dev_realign_tracks_exec.argtypes = [c_vp, c_vp, c_i32, c_vp]
+    lib.gvl_dev_shift_and_realign_tracks.argtypes = [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp,
+                                                     c_vp, c_vp, c_vp, c_i64, c_i32, C.c_double, c_u64, c_vp, c_i64, c_vp, c_vp]
+    lib.gvl_dev_paint_tracks.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp, c_i32,
+                                         c_vp]
     lib.gvl_dev_track_intervals.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32,
                                             c_vp]
     return lib

@@ -215,10 +215,10 @@ static int fixed_plan_prepared(gvl_ctx *ctx, const gvl_fixed_job *J, int64_t n, 
     if ((what & 2) && J->realign) {
         rc = gvl_dev_track_lengths(ctx, A.regions, J->diffs, n, J->ploidy, J->track_lengths, stream);
         if (rc) return rc;
-        rc = gvl_dev_realign_tracks_plan(ctx, J->tab, sv ? &ch : NULL, A.regions, A.shifts, A.goi, n, J->ploidy, NULL, NULL, to_rc,
-                                         J->n_tracks, J->itv, A.offset_idxs, J->track_lengths, J->out_offsets,
-                                         n * J->ploidy * J->output_length, J->strategy_ids, J->params, 0, A.base_seed, sub_batch,
-                                         NULL, cap, 1, stream);
+        rc = gvl_dev_realign_tracks(ctx, J->tab, sv ? &ch : NULL, A.regions, A.shifts, A.goi, n, J->ploidy, NULL, NULL, to_rc,
+                                    J->n_tracks, J->itv, A.offset_idxs, J->track_lengths, J->out_offsets,
+                                    n * J->ploidy * J->output_length, J->strategy_ids, J->params, 0, A.base_seed, sub_batch, NULL,
+                                    cap, GVL_TRACK_LAYOUT_BTP, NULL, NULL, NULL, J->track_dtype, stream);  // (plan only)
         if (rc) return rc;
     }
     return GVL_OK;
@@ -261,10 +261,10 @@ int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *J, int stage, const i
         case GVL_STAGE_TRK_EXEC:
             if (J->n_tracks <= 0) return GVL_OK;
             if (!trk) return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: track output missing");
-            if (J->realign) return gvl_dev_realign_tracks_exec_dtype(ctx, trk, J->track_dtype, stream);
-            return gvl_dev_paint_tracks_dtype(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
-                                              n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, NULL, NULL, trk,
-                                              J->track_dtype, stream);
+            if (J->realign) return gvl_dev_realign_tracks_exec(ctx, trk, J->track_dtype, stream);
+            return gvl_dev_paint_tracks(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
+                                        n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, GVL_TRACK_LAYOUT_BTP, NULL, NULL,
+                                        trk, J->track_dtype, stream);
         default: return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: unknown stage %d", stage);
     }
 }

@@ -819,11 +819,12 @@ int gvl_intervals_and_realign_track_fused(
     if ((rc = scratch(ctx, 2, total * 4, &d_out))) return rc;
     const int32_t strat = (int32_t)strategy_id;
     const int64_t max_rec = sum_variants(geno_offsets, n_geno, geno_offset_idx, n_work);
-    if ((rc = gvl_dev_realign_tracks(ctx, &t, pk.ptr<int32_t>(i_reg), pk.ptr<int32_t>(i_sh), pk.ptr<int64_t>(i_goi), batch,
-                                     ploidy, keep && keep_offsets ? pk.ptr<uint8_t>(i_kp) : nullptr,
+    if ((rc = gvl_dev_realign_tracks(ctx, &t, nullptr, pk.ptr<int32_t>(i_reg), pk.ptr<int32_t>(i_sh), pk.ptr<int64_t>(i_goi),
+                                     batch, ploidy, keep && keep_offsets ? pk.ptr<uint8_t>(i_kp) : nullptr,
                                      keep && keep_offsets ? pk.ptr<int64_t>(i_ko) : nullptr, pk.ptr<uint8_t>(i_rc), 1, &iv,
                                      pk.ptr<int64_t>(i_oi), pk.ptr<int32_t>(i_tl), pk.ptr<int64_t>(i_oo), total, &strat,
-                                     params, base_seed, nullptr, 0, nullptr, max_rec, (float *)d_out, ctx->own_stream)))
+                                     params, base_seed, nullptr, 0, nullptr, max_rec, GVL_TRACK_LAYOUT_TBP, nullptr, nullptr,
+                                     d_out, GVL_TRACK_F32, ctx->own_stream)))
         return rc;
     GVL_CUDA(cudaMemcpyAsync(out, d_out, (size_t)total * 4, cudaMemcpyDeviceToHost, ctx->own_stream));
     return gvl_ctx_check(ctx, ctx->own_stream);
@@ -866,7 +867,7 @@ int gvl_shift_and_realign_tracks_sparse(
     if ((rc = scratch(ctx, 2, total * 4, &d_out))) return rc;
     const int64_t max_rec = sum_variants(geno_offsets, n_geno, geno_offset_idx, n_work);
     if ((rc = gvl_dev_shift_and_realign_tracks(
-             ctx, &t, pk.ptr<int32_t>(i_reg), pk.ptr<int32_t>(i_sh), pk.ptr<int64_t>(i_goi), batch, ploidy,
+             ctx, &t, nullptr, pk.ptr<int32_t>(i_reg), pk.ptr<int32_t>(i_sh), pk.ptr<int64_t>(i_goi), batch, ploidy,
              keep && keep_offsets ? pk.ptr<uint8_t>(i_kp) : nullptr, keep && keep_offsets ? pk.ptr<int64_t>(i_ko) : nullptr,
              nullptr, (const float *)d_tracks, pk.ptr<int64_t>(i_to), pk.ptr<int32_t>(i_tl), pk.ptr<int64_t>(i_oo), total,
              (int32_t)strategy_id, params[0], base_seed, nullptr, max_rec, (float *)d_out, ctx->own_stream)))
@@ -918,10 +919,10 @@ int gvl_shift_and_realign_tracks_from_svar2(
     svar2_resolve(pk, ss, &ch);
     void *d_out;
     if ((rc = scratch(ctx, 2, total * 4, &d_out))) return rc;
-    if ((rc = gvl_dev_shift_and_realign_tracks_svar2(
-             ctx, &t, &ch, pk.ptr<int32_t>(i_reg), pk.ptr<int32_t>(i_sh), batch, ploidy, nullptr, (const float *)d_tracks,
-             pk.ptr<int64_t>(i_to), pk.ptr<int32_t>(i_tl), pk.ptr<int64_t>(i_oo), total, (int32_t)strategy_id, params[0],
-             base_seed, query_seed ? pk.ptr<int64_t>(i_qs) : nullptr, max_merged, (float *)d_out, ctx->own_stream)))
+    if ((rc = gvl_dev_shift_and_realign_tracks(
+             ctx, &t, &ch, pk.ptr<int32_t>(i_reg), pk.ptr<int32_t>(i_sh), nullptr, batch, ploidy, nullptr, nullptr, nullptr,
+             (const float *)d_tracks, pk.ptr<int64_t>(i_to), pk.ptr<int32_t>(i_tl), pk.ptr<int64_t>(i_oo), total,
+             (int32_t)strategy_id, params[0], base_seed, query_seed ? pk.ptr<int64_t>(i_qs) : nullptr, max_merged, (float *)d_out, ctx->own_stream)))
         return rc;
     GVL_CUDA(cudaMemcpyAsync(out, d_out, (size_t)total * 4, cudaMemcpyDeviceToHost, ctx->own_stream));
     return gvl_ctx_check(ctx, ctx->own_stream);
@@ -951,8 +952,8 @@ int gvl_intervals_to_tracks(gvl_ctx *ctx, const int64_t *offset_idxs, const int3
     if ((rc = pk.upload(ctx, 0))) return rc;
     void *d_out;
     if ((rc = scratch(ctx, 2, total * 4, &d_out))) return rc;
-    if ((rc = gvl_dev_intervals_to_tracks(ctx, &iv, pk.ptr<int64_t>(i_oi), pk.ptr<int32_t>(i_st), n_queries,
-                                          pk.ptr<int64_t>(i_oo), total, (float *)d_out, ctx->own_stream)))
+    if ((rc = gvl_dev_paint_tracks(ctx, 1, &iv, pk.ptr<int64_t>(i_oi), pk.ptr<int32_t>(i_st), n_queries, pk.ptr<int64_t>(i_oo),
+                                   total, nullptr, GVL_TRACK_LAYOUT_TBP, nullptr, nullptr, d_out, GVL_TRACK_F32, ctx->own_stream)))
         return rc;
     GVL_CUDA(cudaMemcpyAsync(out, d_out, (size_t)total * 4, cudaMemcpyDeviceToHost, ctx->own_stream));
     GVL_CUDA(cudaStreamSynchronize(ctx->own_stream));

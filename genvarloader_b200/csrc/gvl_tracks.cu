@@ -1,5 +1,5 @@
 // gvl_tracks.cu -- indel-aware track realignment on sm_100a (include/gvl_b200.h:
-// gvl_dev_realign_tracks, gvl_dev_intervals_to_tracks).
+// gvl_dev_realign_tracks, gvl_dev_shift_and_realign_tracks, gvl_dev_paint_tracks).
 //
 // Reference path replaced: intervals_and_realign_track_fused (src/ffi/mod.rs:2553-2672) =
 // intervals_to_tracks (src/intervals.rs:19-126) into a dense scratch -> shift_and_realign_tracks_sparse
@@ -12,8 +12,8 @@
 // coordinates (no dense scratch in HBM), then every thread writes chunks of 16 consecutive output values with 32-byte
 // stores (source span copies, deletion/insertion fills, trailing zeros, reversal for negative strands).  Unsorted
 // variant lists and dense sources resolve every value on its own.  gvl_tracks_exec.cuh has the details.
-// The output is float32, bfloat16 or float16 (GVL_TRACK_*): one execute instantiation per type, values narrowed at the
-// store.
+// The output is float32, bfloat16 or float16 (GVL_TRACK_*: one execute instantiation per type, values narrowed at the
+// store), each row placed by the tile preparation as the call's GVL_TRACK_LAYOUT_* says.
 //
 // gvl_dev_track_intervals returns the stored intervals themselves instead of painting them: a count kernel (one warp per
 // row, two 32-ary searches), the offset scan of the variants tail, and an emit kernel that copies each row's run.
@@ -34,7 +34,7 @@ constexpr int TRK_TILE = 8192;  // output values per execute CTA (one tile of on
 // plan: the scan-based plan kernel of the haplotype path in track mode (gvl_plan_par.cuh, hap_plan_par_kernel<NT, true>;
 // launched through gvl_trk_plan_launch, gvl_hap.cu) -- the same offset scan serves both paths
 // =====================================================================================
-// identity plan for intervals_to_tracks: one row per query, no records, source window = row
+// identity plan for painting (gvl_dev_paint_tracks): one row per query, no records, source window = row
 __global__ void paint_plan_kernel(int64_t n, const int32_t *__restrict__ starts, const int64_t *__restrict__ out_offsets,
                                   const uint8_t *__restrict__ to_rc, RowPlan *rows, int32_t *row_len) {
     int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -206,9 +206,21 @@ using namespace gvl;
 
 static bool track_dtype_ok(int32_t dtype) { return dtype == GVL_TRACK_F32 || dtype == GVL_TRACK_BF16 || dtype == GVL_TRACK_F16; }
 
+// layout, destination table and element type of gvl_dev_realign_tracks / gvl_dev_paint_tracks
+static int check_track_output(const char *who, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride,
+                              int32_t dtype) {
+    if (layout != GVL_TRACK_LAYOUT_TBP && layout != GVL_TRACK_LAYOUT_BTP && layout != GVL_TRACK_LAYOUT_ROWS)
+        return fail(GVL_ERR_ARG, "%s: unknown track layout %d", who, (int)layout);
+    const bool rows = layout == GVL_TRACK_LAYOUT_ROWS;
+    if (rows != (row_dst != nullptr) || rows != (row_tstride != nullptr))
+        return fail(GVL_ERR_ARG, "%s: row_dst and row_tstride go with GVL_TRACK_LAYOUT_ROWS, and only with it", who);
+    if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "%s: unknown track dtype %d", who, (int)dtype);
+    return GVL_OK;
+}
+
 static int trk_execute(gvl_ctx *ctx, void *out, int32_t dtype, cudaStream_t st) {
     if (!ctx->trk_plan_valid || !ctx->trk_params) return fail(GVL_ERR_STATE, "track execute without a track plan");
-    if (!out || ((uintptr_t)out & 3)) return fail(GVL_ERR_ARG, "track output must be an aligned buffer");
+    if (!out || ((uintptr_t)out & 15)) return fail(GVL_ERR_ARG, "track output must be a 16-byte aligned buffer");
     TrkExecParams P;
     memcpy(&P, ctx->trk_params, sizeof(P));
     P.out = out;
@@ -224,12 +236,12 @@ static int trk_execute(gvl_ctx *ctx, void *out, int32_t dtype, cudaStream_t st) 
     return GVL_OK;
 }
 
-static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t n_queries, int64_t n_tracks,
-                           const TrkDesc *host_desc, const int64_t *offset_idxs, int64_t total_per_track,
-                           const int64_t *query_seed, uint64_t base_seed, void *out, int layout_btp, cudaStream_t st,
-                           const uint64_t *base_seed_dev = nullptr, int64_t sub_batch = 0, const int64_t *row_dst = nullptr,
-                           const int64_t *row_tstride = nullptr, int32_t dtype = GVL_TRACK_F32) {
-    if (n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "at most %d tracks per call", MAX_TRACKS);
+// Everything of a planned call (rows and records in ctx->trk) up to the execute launch: descriptor copy, tile map, per-tile
+// descriptors, and the execute launch's parameters, kept in ctx so that trk_execute may follow later, on another stream.
+static int trk_prepare(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t n_queries, int64_t n_tracks,
+                       const TrkDesc *host_desc, const int64_t *offset_idxs, int64_t total_per_track, const int64_t *query_seed,
+                       uint64_t base_seed, const uint64_t *base_seed_dev, int64_t sub_batch, int32_t layout,
+                       const int64_t *row_dst, const int64_t *row_tstride, cudaStream_t st) {
     static_assert(sizeof(TrkDesc) * MAX_TRACKS <= GVL_TRK_DESC_BYTES, "descriptor buffer too small");
     TrkDesc *d_desc = nullptr;
     if (n_tracks > 8) {  // (not CUDA-graph safe: the copy reads the caller's host array at replay time)
@@ -247,14 +259,14 @@ static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t
     P.grid_per_track = total_per_track / TRK_TILE + n_work;
     P.total_per_track = total_per_track;
     P.n_tracks = n_tracks;
-    P.layout_btp = layout_btp;
+    P.layout_btp = layout == GVL_TRACK_LAYOUT_BTP;
     P.offset_idxs = offset_idxs;
     P.n_queries = n_queries;
     P.query_seed = query_seed;
     P.base_seed = base_seed;
     P.base_seed_dev = base_seed_dev;
     P.sub_batch = sub_batch;
-    P.out = out;
+    P.out = nullptr;
     P.tracks = d_desc;
     if (!d_desc)
         for (int64_t t = 0; t < n_tracks; t++) P.inl[t] = host_desc[t];
@@ -268,13 +280,11 @@ static int launch_trk_exec(gvl_ctx *ctx, int64_t n_work, int64_t ploidy, int64_t
     TileDesc *tdesc = (TileDesc *)ctx->trk.tdesc;
     trk_tile_prep_kernel<<<(unsigned)((grid + 3) / 4), 128, 0, st>>>(P, row_dst, row_tstride, tdesc);  // one warp per tile
     GVL_LAUNCH_CHECK();
-    // the execute launch may follow later, on another stream (gvl_dev_realign_tracks_exec): keep its parameters
     if (!ctx->trk_params) ctx->trk_params = malloc(sizeof(TrkExecParams));
     if (!ctx->trk_params) return fail(GVL_ERR_ARG, "out of host memory");
     memcpy(ctx->trk_params, &P, sizeof(P));
     ctx->trk_plan_valid = true;
-    if (!out) return GVL_OK;  // plan only
-    return trk_execute(ctx, out, dtype, st);
+    return GVL_OK;
 }
 
 // the scan-based plan kernel in track mode (gvl_hap.cu)
@@ -289,27 +299,31 @@ int gvl_svar2_merge_launch(gvl_ctx *ctx, gvl_workspace *ws, int64_t *words, cons
 
 extern "C" {
 
-static int realign_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2, const int32_t *regions,
-                        const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy,
-                        const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
+// gvl_dev_realign_tracks (interval sources `itv`) and gvl_dev_shift_and_realign_tracks (one track, `dense` source)
+static int realign_impl(const char *who, gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                        const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
+                        int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
                         int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
                         const float *dense, const int64_t *dense_offsets,
                         const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
                         const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                        const int64_t *query_seed, int64_t max_records, float *out, gvl_stream stream,
-                        int layout_btp = 0, const uint64_t *base_seed_dev = nullptr, int64_t sub_batch = 0,
-                        bool plan_only = false, const int64_t *row_dst = nullptr, const int64_t *row_tstride = nullptr) {
-    if (!ctx || !tab || !regions || !shifts || !(geno_offset_idx || svar2) || !(itv || dense) || !(offset_idxs || dense) ||
+                        const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed, int64_t max_records,
+                        int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
+                        gvl_stream stream) {
+    if (!ctx) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
+    // every argument is checked before the first launch: a rejected call leaves no plan behind, not even the previous one
+    ctx->trk_plan_valid = false;
+    if (!tab || !regions || !shifts || !(geno_offset_idx || svar2) || (itv ? !offset_idxs : !(dense && dense_offsets)) ||
         !track_lengths || !out_offsets || !strategy_ids || !params)
-        return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks: NULL argument");
+        return fail(GVL_ERR_ARG, "%s: NULL argument", who);
+    if (svar2 && (!svar2->vk_off || !svar2->dense_range || !svar2->dense_present_off))
+        return fail(GVL_ERR_ARG, "%s: NULL channel", who);
+    int rc;
+    if ((rc = check_track_output(who, layout, row_dst, row_tstride, dtype))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     GVL_CUDA(cudaSetDevice(ctx->device));
     const int64_t n_work = batch * ploidy;
-    ctx->trk_plan_valid = false;
     if (n_work == 0 || n_tracks == 0 || total_per_track == 0) return GVL_OK;
-    if (!plan_only && (!out || ((uintptr_t)out & 15))) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks: out must be 16-byte aligned");
-    if (plan_only) out = nullptr;
-    // every argument is checked before the first launch: a rejected call leaves no half-planned state behind
     if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "at most %d tracks per call", MAX_TRACKS);
     for (int64_t t = 0; t < n_tracks; t++) {
         if (strategy_ids[t] < 0 || strategy_ids[t] > GVL_FILL_INTERPOLATE)
@@ -317,7 +331,6 @@ static int realign_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_sv
         if (strategy_ids[t] == GVL_FILL_INTERPOLATE && !(params[t] >= 1 && params[t] <= 3))
             return fail(GVL_ERR_ARG, "Interpolate order must be 1, 2 or 3");
     }
-    int rc;
     if ((rc = ensure_rows(ctx, ctx->trk, n_work))) return rc;
     if ((rc = ensure_trecs(ctx, ctx->trk, max_records + n_work))) return rc;
     int64_t *words = ctx->dev_words + W_COUNT;  // (left at zero by the previous plan, see plan_row_done)
@@ -341,150 +354,62 @@ static int realign_impl(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_sv
         desc[t].strategy = strategy_ids[t];
         desc[t].param = params[t];
     }
-    return launch_trk_exec(ctx, n_work, ploidy, batch, n_tracks, desc, offset_idxs, total_per_track, query_seed,
-                           base_seed, out, layout_btp, st, base_seed_dev, sub_batch, row_dst, row_tstride);
+    if ((rc = trk_prepare(ctx, n_work, ploidy, batch, n_tracks, desc, offset_idxs, total_per_track, query_seed, base_seed,
+                          base_seed_dev, sub_batch, layout, row_dst, row_tstride, st)))
+        return rc;
+    return out ? trk_execute(ctx, out, dtype, st) : GVL_OK;  // (out == NULL: plan only)
 }
 
-int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
-                           const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy,
-                           const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
+int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                           const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
+                           int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
                            int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
                            const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
                            const int32_t *strategy_ids, const double *params, uint64_t base_seed,
                            const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed, int64_t max_records,
-                           float *out, gvl_stream stream) {
-    if (!itv || !offset_idxs) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks: NULL argument");
-    return realign_impl(ctx, tab, nullptr, regions, shifts, geno_offset_idx, batch, ploidy, keep, keep_offsets, to_rc, n_tracks,
-                        itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets, total_per_track, strategy_ids,
-                        params, base_seed, query_seed, max_records, out, stream, 0, base_seed_dev, sub_batch);
+                           int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
+                           gvl_stream stream) {
+    return realign_impl("gvl_dev_realign_tracks", ctx, tab, svar2, regions, shifts, geno_offset_idx, batch, ploidy, keep,
+                        keep_offsets, to_rc, n_tracks, itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets,
+                        total_per_track, strategy_ids, params, base_seed, base_seed_dev, sub_batch, query_seed, max_records,
+                        layout, row_dst, row_tstride, out, dtype, stream);
 }
 
-int gvl_dev_realign_tracks_btp(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
-                               const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy,
-                               const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
-                               int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                               const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
-                               const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                               const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
-                               int64_t max_records, float *out, gvl_stream stream) {
-    if (!itv || !offset_idxs) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_btp: NULL argument");
-    return realign_impl(ctx, tab, nullptr, regions, shifts, geno_offset_idx, batch, ploidy, keep, keep_offsets, to_rc, n_tracks,
-                        itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets, total_per_track, strategy_ids,
-                        params, base_seed, query_seed, max_records, out, stream, 1, base_seed_dev, sub_batch);
-}
-
-int gvl_dev_realign_tracks_plan(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
-                                const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy, const uint8_t *keep,
-                                const int64_t *keep_offsets, const uint8_t *to_rc, int64_t n_tracks, const gvl_intervals *itv,
-                                const int64_t *offset_idxs, const int32_t *track_lengths, const int64_t *out_offsets,
-                                int64_t total_per_track, const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                                const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
-                                int64_t max_records, int layout_btp, gvl_stream stream) {
-    if (!itv || !offset_idxs) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_plan: NULL argument");
-    if (svar2 && (!svar2->vk_off || !svar2->dense_range || !svar2->dense_present_off))
-        return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_plan: NULL channel");
-    return realign_impl(ctx, tab, svar2, regions, shifts, geno_offset_idx, batch, ploidy, keep, keep_offsets, to_rc, n_tracks,
-                        itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets, total_per_track, strategy_ids,
-                        params, base_seed, query_seed, max_records, nullptr, stream, layout_btp ? 1 : 0, base_seed_dev, sub_batch,
-                        true);
-}
-
-int gvl_dev_realign_tracks_plan_rows(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
-                                     const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
-                                     int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
-                                     int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                                     const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
-                                     const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                                     const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
-                                     int64_t max_records, const int64_t *row_dst, const int64_t *row_tstride, gvl_stream stream) {
-    if (!itv || !offset_idxs || !row_dst || !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_plan_rows: NULL argument");
-    if (svar2 && (!svar2->vk_off || !svar2->dense_range || !svar2->dense_present_off))
-        return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_plan_rows: NULL channel");
-    return realign_impl(ctx, tab, svar2, regions, shifts, geno_offset_idx, batch, ploidy, keep, keep_offsets, to_rc, n_tracks,
-                        itv, offset_idxs, nullptr, nullptr, track_lengths, out_offsets, total_per_track, strategy_ids,
-                        params, base_seed, query_seed, max_records, nullptr, stream, 0, base_seed_dev, sub_batch, true, row_dst,
-                        row_tstride);
-}
-
-int gvl_dev_realign_tracks_exec_dtype(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream) {
+int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream) {
     if (!ctx) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: ctx is NULL");
     if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: unknown track dtype %d", (int)dtype);
     GVL_CUDA(cudaSetDevice(ctx->device));
-    if (!ctx->trk_plan_valid) return GVL_OK;  // (the plan was empty: nothing to write)
-    if ((uintptr_t)out & 15) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: out must be 16-byte aligned");
+    if (!ctx->trk_plan_valid) return GVL_OK;  // (an empty or rejected plan: nothing to write)
     return trk_execute(ctx, out, dtype, (cudaStream_t)stream);
 }
 
-int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream) {
-    return gvl_dev_realign_tracks_exec_dtype(ctx, out, GVL_TRACK_F32, stream);
-}
-
-int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
-                                     const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
-                                     int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets,
+int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                                     const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx,
+                                     int64_t batch, int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets,
                                      const uint8_t *to_rc, const float *tracks, const int64_t *track_offsets,
                                      const int32_t *track_lengths, const int64_t *out_offsets, int64_t total,
                                      int32_t strategy_id, double param, uint64_t base_seed,
                                      const int64_t *query_seed, int64_t max_records, float *out, gvl_stream stream) {
-    if (!tracks || !track_offsets) return fail(GVL_ERR_ARG, "gvl_dev_shift_and_realign_tracks: NULL argument");
-    return realign_impl(ctx, tab, nullptr, regions, shifts, geno_offset_idx, batch, ploidy, keep, keep_offsets, to_rc, 1, nullptr,
-                        nullptr, tracks, track_offsets, track_lengths, out_offsets, total, &strategy_id, &param,
-                        base_seed, query_seed, max_records, out, stream);
+    return realign_impl("gvl_dev_shift_and_realign_tracks", ctx, tab, svar2, regions, shifts, geno_offset_idx, batch, ploidy,
+                        keep, keep_offsets, to_rc, 1, nullptr, nullptr, tracks, track_offsets, track_lengths, out_offsets,
+                        total, &strategy_id, &param, base_seed, nullptr, 0, query_seed, max_records, GVL_TRACK_LAYOUT_TBP,
+                        nullptr, nullptr, out, GVL_TRACK_F32, stream);
 }
 
-
-int gvl_dev_shift_and_realign_tracks_svar2(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *ch,
-                                           const int32_t *regions, const int32_t *shifts, int64_t batch, int64_t ploidy,
-                                           const uint8_t *to_rc, const float *tracks, const int64_t *track_offsets,
-                                           const int32_t *track_lengths, const int64_t *out_offsets, int64_t total,
-                                           int32_t strategy_id, double param, uint64_t base_seed,
-                                           const int64_t *query_seed, int64_t max_merged, float *out, gvl_stream stream) {
-    if (!ch || !ch->vk_off || !ch->dense_range || !ch->dense_present_off || !tracks || !track_offsets)
-        return fail(GVL_ERR_ARG, "gvl_dev_shift_and_realign_tracks_svar2: NULL argument");
-    return realign_impl(ctx, tab, ch, regions, shifts, nullptr, batch, ploidy, nullptr, nullptr, to_rc, 1, nullptr, nullptr,
-                        tracks, track_offsets, track_lengths, out_offsets, total, &strategy_id, &param, base_seed,
-                        query_seed, max_merged, out, stream);
-}
-
-int gvl_dev_intervals_to_tracks(gvl_ctx *ctx, const gvl_intervals *itv, const int64_t *offset_idxs,
-                                const int32_t *starts, int64_t n_queries, const int64_t *out_offsets,
-                                int64_t total, float *out, gvl_stream stream) {
-    if (!ctx || !itv || !offset_idxs || !starts || !out_offsets)
-        return fail(GVL_ERR_ARG, "gvl_dev_intervals_to_tracks: NULL argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    GVL_CUDA(cudaSetDevice(ctx->device));
-    if (n_queries == 0 || total == 0) return GVL_OK;
-    if (!out || ((uintptr_t)out & 15)) return fail(GVL_ERR_ARG, "gvl_dev_intervals_to_tracks: out must be 16-byte aligned");
-    int rc;
-    if ((rc = ensure_rows(ctx, ctx->trk, n_queries))) return rc;
-    if ((rc = ensure_trecs(ctx, ctx->trk, 1))) return rc;
-    paint_plan_kernel<<<(unsigned)((n_queries + 255) / 256), 256, 0, st>>>(n_queries, starts, out_offsets, nullptr,
-                                                                            ctx->trk.rows, ctx->trk.row_len);
-    GVL_LAUNCH_CHECK();
-    TrkDesc desc;
-    desc.itv_starts = itv->itv_starts;
-    desc.itv_ends = itv->itv_ends;
-    desc.itv_values = itv->itv_values;
-    desc.itv_offsets = itv->itv_offsets;
-    desc.dense = nullptr;
-    desc.dense_offsets = nullptr;
-    desc.strategy = GVL_FILL_REPEAT_5P;
-    desc.param = 0.0;
-    return launch_trk_exec(ctx, n_queries, 1, n_queries, 1, &desc, offset_idxs, total, nullptr, 0, out, 0, st);
-}
-
-static int paint_impl(const char *who, gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                      const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                      const uint8_t *to_rc, void *out, gvl_stream stream, const int64_t *row_dst = nullptr,
-                      const int64_t *row_tstride = nullptr, int32_t dtype = GVL_TRACK_F32) {
-    if (!ctx || !itv || !offset_idxs || !starts || !out_offsets) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
+int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                         const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                         const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out,
+                         int32_t dtype, gvl_stream stream) {
+    const char *who = "gvl_dev_paint_tracks";
+    if (!ctx) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
+    ctx->trk_plan_valid = false;  // (as in realign_impl)
+    if (!itv || !offset_idxs || !starts || !out_offsets) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
     if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "%s: 0..%d tracks per call", who, MAX_TRACKS);
-    if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "%s: unknown track dtype %d", who, (int)dtype);
+    int rc;
+    if ((rc = check_track_output(who, layout, row_dst, row_tstride, dtype))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     GVL_CUDA(cudaSetDevice(ctx->device));
     if (n_queries == 0 || n_tracks == 0 || total_per_track == 0) return GVL_OK;
-    if (!out || ((uintptr_t)out & 15)) return fail(GVL_ERR_ARG, "%s: out must be 16-byte aligned", who);
-    int rc;
     if ((rc = ensure_rows(ctx, ctx->trk, n_queries))) return rc;
     if ((rc = ensure_trecs(ctx, ctx->trk, 1))) return rc;
     paint_plan_kernel<<<(unsigned)((n_queries + 255) / 256), 256, 0, st>>>(n_queries, starts, out_offsets, to_rc,
@@ -501,33 +426,10 @@ static int paint_impl(const char *who, gvl_ctx *ctx, int64_t n_tracks, const gvl
         desc[t].strategy = GVL_FILL_REPEAT_5P;
         desc[t].param = 0.0;
     }
-    return launch_trk_exec(ctx, n_queries, 1, n_queries, n_tracks, desc, offset_idxs, total_per_track, nullptr, 0, out, 1, st,
-                           nullptr, 0, row_dst, row_tstride, dtype);
-}
-
-int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                         const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                         const uint8_t *to_rc, float *out, gvl_stream stream) {
-    return paint_impl("gvl_dev_paint_tracks", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets, total_per_track,
-                      to_rc, out, stream);
-}
-
-int gvl_dev_paint_tracks_rows(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                              const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                              const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, float *out,
-                              gvl_stream stream) {
-    if (!row_dst || !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks_rows: NULL argument");
-    return paint_impl("gvl_dev_paint_tracks_rows", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
-                      total_per_track, to_rc, out, stream, row_dst, row_tstride);
-}
-
-int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                               const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                               const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
-                               gvl_stream stream) {
-    if (!row_dst != !row_tstride) return fail(GVL_ERR_ARG, "gvl_dev_paint_tracks_dtype: row_dst and row_tstride go together");
-    return paint_impl("gvl_dev_paint_tracks_dtype", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
-                      total_per_track, to_rc, out, stream, row_dst, row_tstride, dtype);
+    if ((rc = trk_prepare(ctx, n_queries, 1, n_queries, n_tracks, desc, offset_idxs, total_per_track, nullptr, 0, nullptr, 0,
+                          layout, row_dst, row_tstride, st)))
+        return rc;
+    return trk_execute(ctx, out, dtype, st);
 }
 
 static int ensure_itv_counts(gvl_ctx *ctx, int64_t n) {

@@ -276,7 +276,7 @@ __device__ __forceinline__ void t2_set_bit(uint32_t *mk, uint32_t *mk2, int u) {
 // =====================================================================================
 // tile preparation: one warp per (track, tile)
 // =====================================================================================
-// row_dst / row_tstride (gvl_dev_*_rows): explicit destination of every row, out_base = row_dst[row] + track *
+// row_dst / row_tstride (GVL_TRACK_LAYOUT_ROWS): explicit destination of every row, out_base = row_dst[row] + track *
 // row_tstride[row]; NULL row_dst = the fixed layout of P.layout_btp.  (Kernel arguments of their own, not members of
 // TrkExecParams: the execute kernel takes the same struct, and a larger struct would move its tdesc argument.)
 __global__ void __launch_bounds__(128) trk_tile_prep_kernel(TrkExecParams P, const int64_t *__restrict__ row_dst,

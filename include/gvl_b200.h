@@ -189,10 +189,39 @@ int gvl_dev_get_diffs_sparse(gvl_ctx *ctx, const gvl_sparse_tables *tab, const i
                              gvl_stream stream);
 
 /* ---- device layer: tracks ---------------------------------------------------------- */
+/* Element type of a track output.  Values are computed in float32 as for GVL_TRACK_F32 and narrowed at the store with
+ * round-to-nearest-even (cvt.rn, no flush to zero: subnormals are kept, values beyond the float16 range become +-inf, NaN
+ * becomes the device's canonical NaN): bit for bit the float32 output cast to the type on the device.  Only the output
+ * changes: stored intervals stay float32. */
+#define GVL_TRACK_F32 0
+#define GVL_TRACK_BF16 1
+#define GVL_TRACK_F16 2
+
+/* Where the rows of a track call land in `out` (n_tracks * total_per_track elements).  Row k (= q*p + h; p = 1 when
+ * painting) has out_offsets[k+1] - out_offsets[k] values, written reversed on masked rows in every layout. */
+#define GVL_TRACK_LAYOUT_TBP 0  /* track-major (t, b, p, ~l): the reference's flat buffer (_reconstruct.py:238); row k of
+                                   track t starts at t * total_per_track + out_offsets[k] */
+#define GVL_TRACK_LAYOUT_BTP 1  /* (b, t, p, ~l): every query's tracks adjacent, the order the reference's offsets describe
+                                   (_reconstruct.py:292-300) and what Dataset returns; row (q, t, h) starts at n_tracks *
+                                   out_offsets[q*p] + t * (out_offsets[(q+1)*p] - out_offsets[q*p]) + out_offsets[q*p + h] -
+                                   out_offsets[q*p].  out_offsets must be gap-free. */
+#define GVL_TRACK_LAYOUT_ROWS 2 /* row k of track t starts at row_dst[k] + t * row_tstride[k] (device i64[b*p] each).  The
+                                   caller guarantees that the ranges of all (row, track) pairs are disjoint and lie inside
+                                   [0, n_tracks*total_per_track): every value is then written exactly once when they cover
+                                   the buffer.  out_offsets still gives each row's length and must be gap-free.  Used for
+                                   spliced output: the elements of a splice row are separate rows written straight into
+                                   their place in the concatenation. */
+/* row_dst and row_tstride are both given with GVL_TRACK_LAYOUT_ROWS and both NULL with the other layouts; an unknown layout
+ * or dtype (GVL_TRACK_*) is GVL_ERR_ARG.  These checks run before the first launch: a rejected call plans nothing and
+ * drops the plan of the call before it.  `out` is device memory, 16-byte aligned. */
+
 /*
  * intervals_and_realign_track_fused (src/ffi/mod.rs:2553-2672) for ALL tracks of a batch in one
  * plan launch + one execute launch: paints stored intervals (src/intervals.rs:19-126) and
  * realigns them to haplotype coordinates (src/tracks/mod.rs:224-406) without the dense scratch.
+ *   svar2                NULL: the variants come from the SVAR1 tables of `tab`; non-NULL: from the svar2 two-channel
+ *                        source (merged on the device like gvl_dev_hap_plan_svar2; geno_offset_idx and the keep mask are
+ *                        then ignored, max_records = max_merged)
  *   n_tracks             tracks realigned in this call (<= 64)
  *   itv[t]               HOST array of n_tracks descriptors holding DEVICE pointers
  *   offset_idxs          device i64[n_tracks*b]: interval slot per (track, query) (dataset idx for
@@ -209,126 +238,50 @@ int gvl_dev_get_diffs_sparse(gvl_ctx *ctx, const gvl_sparse_tables *tab, const i
  *   query_seed           optional device i64[b]: global batch row used as the FlankSample seed
  *                        component when one logical batch is split over several calls / GPUs
  *                        (src/tracks/mod.rs:696-702); NULL = local row index
- *   out                  device f32[n_tracks * total_per_track], track-major (_reconstruct.py:238)
+ *   layout, row_dst, row_tstride   GVL_TRACK_LAYOUT_*
+ *   out, dtype           `dtype` elements (GVL_TRACK_*) written in `layout`.  out == NULL plans the call without executing
+ *                        it: gvl_dev_realign_tracks_exec writes the values later, on the same stream or another (a
+ *                        pipeline runs the latency-bound part -- variant plan, tile map, per-tile searches -- on one stream
+ *                        and the bandwidth-bound execute launch on another; the caller orders the two).
  */
-int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
-                           const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy,
-                           const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
+int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                           const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
+                           int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
                            int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
                            const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
                            const int32_t *strategy_ids, const double *params, uint64_t base_seed,
                            const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed, int64_t max_records,
-                           float *out, gvl_stream stream);
+                           int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
+                           gvl_stream stream);
 
-/* gvl_dev_realign_tracks writing the layout the reference's offsets describe, (b, t, p, ~l) (_reconstruct.py:292-300):
- * all tracks of a query adjacent, so the flat buffer and lengths_to_offsets(repeat(out_lengths, "b p -> b t p")) agree
- * for any number of tracks.  Row (q, t, h) starts at n_tracks * out_offsets[q*p] + t * (out_offsets[(q+1)*p] -
- * out_offsets[q*p]) + out_offsets[q*p + h] - out_offsets[q*p].  Same arguments; out_offsets must be gap-free. */
-int gvl_dev_realign_tracks_btp(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
-                               const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy,
-                               const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
-                               int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                               const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
-                               const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                               const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
-                               int64_t max_records, float *out, gvl_stream stream);
+/* The execute launch of the last call planned on this context: writes elements of `dtype` (GVL_TRACK_*; any other value:
+ * GVL_ERR_ARG) into `out` (device, n_tracks * total_per_track elements, 16-byte aligned).  Writes nothing after an empty or
+ * rejected plan. */
+int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream);
 
-/* gvl_dev_realign_tracks in two steps, so that a pipeline can run the latency-bound part (variant plan, tile map, per-tile
- * searches) on one stream and the bandwidth-bound execute launch on another: _plan takes the arguments of
- * gvl_dev_realign_tracks (layout_btp selects the (b, t, p, ~l) order) except `out`, plus `svar2`: non-NULL = the variants
- * come from the svar2 two-channel source (merged on the device like gvl_dev_hap_plan_svar2; geno_offset_idx and the keep
- * mask are then ignored, max_records = max_merged); _exec writes the planned call into
- * `out` (device f32[n_tracks * total_per_track], 16-byte aligned).  The caller orders the two (stream / event). */
-int gvl_dev_realign_tracks_plan(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
-                                const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch, int64_t ploidy, const uint8_t *keep,
-                                const int64_t *keep_offsets, const uint8_t *to_rc, int64_t n_tracks, const gvl_intervals *itv,
-                                const int64_t *offset_idxs, const int32_t *track_lengths, const int64_t *out_offsets,
-                                int64_t total_per_track, const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                                const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
-                                int64_t max_records, int layout_btp, gvl_stream stream);
-int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, float *out, gvl_stream stream);
-
-/* Element type of a track output.  Values are computed in float32 as for GVL_TRACK_F32 and narrowed at the store with
- * round-to-nearest-even (cvt.rn, no flush to zero: subnormals are kept, values beyond the float16 range become +-inf, NaN
- * becomes the device's canonical NaN): bit for bit the float32 output cast to the type on the device.  Only the output
- * changes: stored intervals stay float32. */
-#define GVL_TRACK_F32 0
-#define GVL_TRACK_BF16 1
-#define GVL_TRACK_F16 2
-/* gvl_dev_realign_tracks_exec writing elements of `dtype` (GVL_TRACK_*; any other value: GVL_ERR_ARG) into `out`
- * (device, n_tracks * total_per_track elements, 16-byte aligned).  gvl_dev_realign_tracks_exec is its GVL_TRACK_F32 case.
- * Serves every plan entry above (fixed layouts, per-row destinations, svar2 sources). */
-int gvl_dev_realign_tracks_exec_dtype(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream);
-
-/* gvl_dev_realign_tracks_plan with an explicit destination for every row in place of a fixed layout (`layout_btp` is
- * replaced by the table); followed by gvl_dev_realign_tracks_exec like the plan it extends.
- *   row_dst      device i64[b*p]: flat index in `out` of value 0 of row k = q*p + h for track 0
- *   row_tstride  device i64[b*p]: distance from track t to track t+1 of row k
- * Row k of track t goes to out[row_dst[k] + t*row_tstride[k] ...], out_offsets[k+1]-out_offsets[k] values, reversed on
- * masked rows as in the other layouts.  The caller guarantees that the ranges of all (row, track) pairs are disjoint and
- * lie inside [0, n_tracks*total_per_track): every value is then written exactly once when they cover the buffer.
- * out_offsets still gives each row's length and must be gap-free.  Used for spliced output: the elements of a splice row
- * are separate rows written straight into their place in the concatenation. */
-int gvl_dev_realign_tracks_plan_rows(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
-                                     const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
-                                     int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets, const uint8_t *to_rc,
-                                     int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                                     const int32_t *track_lengths, const int64_t *out_offsets, int64_t total_per_track,
-                                     const int32_t *strategy_ids, const double *params, uint64_t base_seed,
-                                     const uint64_t *base_seed_dev, int64_t sub_batch, const int64_t *query_seed,
-                                     int64_t max_records, const int64_t *row_dst, const int64_t *row_tstride, gvl_stream stream);
-
-/* shift_and_realign_tracks_sparse on device (src/ffi/mod.rs:2439-2458): ONE track whose source is
- * a dense f32 window per query (`tracks` ragged by `track_offsets` i64[b+1]) instead of intervals.
- * track_lengths[q] = track_offsets[q+1]-track_offsets[q] as device i32[b]. */
-int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const int32_t *regions,
-                                     const int32_t *shifts, const int64_t *geno_offset_idx, int64_t batch,
-                                     int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets,
+/* shift_and_realign_tracks_sparse (src/ffi/mod.rs:2439-2458) and shift_and_realign_tracks_from_svar2
+ * (src/tracks/mod.rs:705-856) on device: ONE track whose source is a dense f32 window per query (`tracks` ragged by
+ * `track_offsets` i64[b+1]) instead of intervals, written track-major as float32.  svar2 as in gvl_dev_realign_tracks
+ * (`tab` then carries the decoded key table in ilens / n_variants; max_records = max_merged = sum over rows of (var_key
+ * entries + dense window size)).  track_lengths[q] = track_offsets[q+1]-track_offsets[q] as device i32[b]. */
+int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
+                                     const int32_t *regions, const int32_t *shifts, const int64_t *geno_offset_idx,
+                                     int64_t batch, int64_t ploidy, const uint8_t *keep, const int64_t *keep_offsets,
                                      const uint8_t *to_rc, const float *tracks, const int64_t *track_offsets,
                                      const int32_t *track_lengths, const int64_t *out_offsets, int64_t total,
                                      int32_t strategy_id, double param, uint64_t base_seed,
                                      const int64_t *query_seed, int64_t max_records, float *out, gvl_stream stream);
 
-/* shift_and_realign_tracks_from_svar2 on device (src/tracks/mod.rs:705-856, src/ffi/mod.rs `shift_and_realign_tracks_from_svar2`):
- * gvl_dev_shift_and_realign_tracks with the svar2 two-channel variant source (merged on the device like
- * gvl_dev_hap_plan_svar2; `tab` carries the decoded key table in ilens / n_variants).
- *   max_merged = sum over rows of (var_key entries + dense window size) */
-int gvl_dev_shift_and_realign_tracks_svar2(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *ch,
-                                           const int32_t *regions, const int32_t *shifts, int64_t batch, int64_t ploidy,
-                                           const uint8_t *to_rc, const float *tracks, const int64_t *track_offsets,
-                                           const int32_t *track_lengths, const int64_t *out_offsets, int64_t total,
-                                           int32_t strategy_id, double param, uint64_t base_seed,
-                                           const int64_t *query_seed, int64_t max_merged, float *out, gvl_stream stream);
-
-/* intervals_to_tracks on device (src/ffi/mod.rs:190-201): out f32[total = out_offsets[n]] fully written. */
-int gvl_dev_intervals_to_tracks(gvl_ctx *ctx, const gvl_intervals *itv, const int64_t *offset_idxs,
-                                const int32_t *starts, int64_t n_queries, const int64_t *out_offsets,
-                                int64_t total, float *out, gvl_stream stream);
-
 /* intervals_to_tracks for ALL tracks of a batch in one launch (the un-realigned track read, Tracks._call_float32
- * python/genvarloader/_dataset/_tracks.py:370-420): itv is a HOST array of n_tracks descriptors, offset_idxs device
- * i64[n_tracks*n_queries], out_offsets device i64[n_queries+1] (per track, gap-free), to_rc optional device u8[n_queries]
- * (masked rows are written reversed, src/reverse.rs:25-38).  out: device f32[n_tracks*total_per_track] in (b, t, ~l)
- * order: row (q, t) starts at n_tracks*out_offsets[q] + t*(out_offsets[q+1]-out_offsets[q]). */
+ * python/genvarloader/_dataset/_tracks.py:370-420; src/ffi/mod.rs:190-201 is the one-track GVL_TRACK_LAYOUT_TBP case):
+ * itv is a HOST array of n_tracks descriptors, offset_idxs device i64[n_tracks*n_queries], out_offsets device
+ * i64[n_queries+1] (per track, gap-free), to_rc optional device u8[n_queries] (masked rows are written reversed,
+ * src/reverse.rs:25-38).  One row per query; layout, row_dst, row_tstride, out and dtype as in gvl_dev_realign_tracks
+ * (`out` is required). */
 int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
                          const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                         const uint8_t *to_rc, float *out, gvl_stream stream);
-
-/* gvl_dev_paint_tracks with an explicit destination for every query (row_dst / row_tstride: device i64[n_queries], the
- * same table and the same caller guarantee as gvl_dev_realign_tracks_plan_rows): row (q, t) starts at
- * out[row_dst[q] + t*row_tstride[q]]. */
-int gvl_dev_paint_tracks_rows(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                              const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                              const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, float *out,
-                              gvl_stream stream);
-
-/* gvl_dev_paint_tracks_rows writing elements of `dtype` (GVL_TRACK_*, see gvl_dev_realign_tracks_exec_dtype) into `out`.
- * row_dst and row_tstride both NULL: the (b, t, ~l) layout of gvl_dev_paint_tracks.  gvl_dev_paint_tracks and
- * gvl_dev_paint_tracks_rows are its GVL_TRACK_F32 cases. */
-int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                               const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                               const uint8_t *to_rc, const int64_t *row_dst, const int64_t *row_tstride, void *out, int32_t dtype,
-                               gvl_stream stream);
+                         const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out,
+                         int32_t dtype, gvl_stream stream);
 
 /* The stored intervals of one slot over one window per row (the "intervals" kind of Dataset.with_tracks).  tracks is a
  * HOST array of n_tracks (<= 64) descriptors; row k (device arrays of n_rows entries) reads slot row_slot[k] of track
@@ -338,7 +291,7 @@ int gvl_dev_paint_tracks_dtype(gvl_ctx *ctx, int64_t n_tracks, const gvl_interva
  *   cap == 0: writes out_offsets (device i64[n_rows + 1], row k's intervals at [out_offsets[k], out_offsets[k + 1])) and
  *             nothing else; the caller reads out_offsets[n_rows] to size the outputs;
  *   cap > 0:  reads those out_offsets and writes out_starts / out_ends (device i32[cap]) and out_values (device, cap
- *             elements of track_dtype, GVL_TRACK_*: the float32 values narrowed as by gvl_dev_realign_tracks_exec_dtype).
+ *             elements of track_dtype, GVL_TRACK_*: the float32 values narrowed as by gvl_dev_realign_tracks_exec).
  *             A row whose intervals would end past cap is not written. */
 int gvl_dev_track_intervals(gvl_ctx *ctx, const gvl_intervals *tracks, int64_t n_tracks, const int64_t *row_slot,
                             const int32_t *row_track, const int32_t *row_w0, const int32_t *row_w1, int64_t n_rows,

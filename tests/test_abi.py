@@ -7,10 +7,22 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent.parent
 
 
+TRACK_ENTRIES = ("gvl_dev_realign_tracks", "gvl_dev_realign_tracks_exec", "gvl_dev_shift_and_realign_tracks",
+                 "gvl_dev_paint_tracks")
+
+
+def _header():
+    return re.sub(r"/\*.*?\*/", "", (ROOT / "include" / "gvl_b200.h").read_text(), flags=re.S)
+
+
 def _declared():
-    text = (ROOT / "include" / "gvl_b200.h").read_text()
-    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
-    return sorted(set(re.findall(r"\b(gvl_[a-z0-9_]+)\s*\(", text)))
+    return sorted(set(re.findall(r"\b(gvl_[a-z0-9_]+)\s*\(", _header())))
+
+
+def _n_params(name):
+    m = re.search(rf"\b{name}\s*\(([^)]*)\)\s*;", _header())
+    assert m, f"{name} is not declared in gvl_b200.h"
+    return len(m.group(1).split(","))
 
 
 def test_library_exports_every_declared_symbol():
@@ -33,6 +45,25 @@ def test_error_reporting_without_gpu():
     assert b"NULL" in _ffi.lib.gvl_last_error()
     rc = _ffi.lib.gvl_pin_static(None, None, ctypes.c_int64(0))
     assert rc == 2
+
+
+def test_track_entries_declare_every_argument():
+    """ctypes checks the argument count of the track entries against their prototypes (30-odd arguments: a wrong count
+    must fail in Python, not reach the device)."""
+    from genvarloader_b200 import _ffi
+
+    for name in TRACK_ENTRIES:
+        assert len(getattr(_ffi.lib, name).argtypes) == _n_params(name), name
+
+
+def test_track_entries_reject_a_null_context():
+    from genvarloader_b200 import _ffi
+
+    for name in TRACK_ENTRIES:
+        fn = getattr(_ffi.lib, name)
+        args = [0 if t in (ctypes.c_int64, ctypes.c_int32, ctypes.c_uint64, ctypes.c_double) else None for t in fn.argtypes]
+        assert fn(*args) == 2, name
+        assert b"NULL" in _ffi.lib.gvl_last_error(), name
 
 
 def test_only_tests_and_harness_touch_the_oracle():

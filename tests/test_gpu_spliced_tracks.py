@@ -1,7 +1,7 @@
 """Tracks of spliced datasets: a spliced cell is the concatenation, in splice-row order, of its elements' unspliced outputs
 (jitter 0, ragged length).  The element batch E lists the selected (splice row, sample) pairs in output order and, inside a
 pair, the row's elements; the expected values are one oracle call over E, regrouped -- bit-exact.  Also: the per-row
-destination entries (gvl_dev_realign_tracks_plan_rows, gvl_dev_paint_tracks_rows) against the fixed layouts they restate."""
+destination layout of the track entries (GVL_TRACK_LAYOUT_ROWS) against the fixed layouts it restates."""
 import numpy as np
 import pytest
 
@@ -109,8 +109,9 @@ def _seed(e_reg, e_s, n_samples):
 
 # ---------------------------------------------------------------------------------------------------- the ABI
 def test_rows_entries_restate_the_fixed_layouts(env):
-    """A destination table restating the (b, t, p, ~l) / (b, t, ~l) layout gives the bytes of gvl_dev_realign_tracks_btp /
-    gvl_dev_paint_tracks; a permutation of the query blocks permutes the output; every value is written (NaN sentinel)."""
+    """A destination table restating the (b, t, p, ~l) / (b, t, ~l) layout gives the bytes of GVL_TRACK_LAYOUT_BTP in
+    gvl_dev_realign_tracks / gvl_dev_paint_tracks; a permutation of the query blocks permutes the output; every value is
+    written (NaN sentinel)."""
     import torch
 
     from genvarloader_b200 import Constant, FlankSample, Interpolate, Repeat5p, Repeat5pNormalized
@@ -179,6 +180,76 @@ def test_rows_entries_restate_the_fixed_layouts(env):
         eng.paint_tracks(names, t_oi, starts, d_off, int(offs[-1]), q_rc, out=out, layout="rows",
                          row_dst=torch.from_numpy(base.astype(np.int64)).to(dev), row_tstride=torch.from_numpy(lens).to(dev))
         assert (out.cpu().numpy().view(np.uint32) == want).all()
+
+
+def test_rejected_layouts_leave_no_plan(env):
+    """An unknown layout, GVL_TRACK_LAYOUT_ROWS without both tables and a fixed layout with them are argument errors of
+    gvl_dev_realign_tracks and gvl_dev_paint_tracks, found before any launch.  A rejected call also drops the plan of the
+    call before it: the execute that follows writes nothing."""
+    import ctypes as C
+
+    import torch
+
+    from genvarloader_b200._engine import _stream
+    from genvarloader_b200._ffi import lib, ptr
+
+    d, ds, _, _ = env
+    eng, dev, p = ds.engine, ds.engine.device, int(d.ploidy)
+    names, b = ["track0", "track1"], 6
+    T = len(names)
+    r_idx, s_idx = np.arange(b), np.arange(b) % d.n_samples
+    ds_idx = r_idx * d.n_samples + s_idx
+    regions = np.ascontiguousarray(d.regions[r_idx, :3])
+    goi = ds_idx[:, None] * p + np.arange(p)[None, :]
+    t_reg, t_goi = torch.from_numpy(regions).to(dev), torch.from_numpy(goi).to(dev)
+    t_sh = torch.zeros(goi.shape, dtype=torch.int32, device=dev)
+    t_oi = torch.from_numpy(np.stack([ds_idx] * T)).to(dev)
+    diffs = eng.get_diffs(t_goi, t_reg[:, 1].contiguous(), t_reg[:, 2].contiguous())
+    lengths = torch.from_numpy((regions[:, 2] - regions[:, 1]).astype(np.int64)).to(dev)
+    track_lengths = (lengths - diffs.clamp(max=0).min(1).values.to(torch.int64)).to(torch.int32)
+    oo = torch.zeros(b * p + 1, dtype=torch.int64, device=dev)
+    torch.cumsum((lengths[:, None] + diffs).clamp(min=0).reshape(-1), 0, out=oo[1:])
+    total, mr = int(oo[-1]), int(eng.max_records(goi))
+    starts = t_reg[:, 1].contiguous()
+    p_off = torch.from_numpy(np.concatenate([[0], np.cumsum(regions[:, 2] - regions[:, 1])]).astype(np.int64)).to(dev)
+    itv, sid, par = eng.track_descs(names, [0] * T, [0.0] * T)
+    h, table = eng.ctx.handle, torch.zeros(b * p, dtype=torch.int64, device=dev)
+
+    def realign(layout, dst=None, ts=None, out=None):  # out = None: plan only
+        return lib.gvl_dev_realign_tracks(h, C.byref(eng.tab), None, ptr(t_reg), ptr(t_sh), ptr(t_goi), b, p, None, None, None,
+                                          T, itv, ptr(t_oi), ptr(track_lengths), ptr(oo), total, sid, par, 1, None, 0, None, mr,
+                                          layout, ptr(dst), ptr(ts), ptr(out), 0, _stream())
+
+    def paint(layout, dst=None, ts=None, out=None):
+        return lib.gvl_dev_paint_tracks(h, T, itv, ptr(t_oi), ptr(starts), b, ptr(p_off), int(p_off[-1]), None, layout, ptr(dst),
+                                        ptr(ts), ptr(out), 0, _stream())
+
+    def sentinel_buffer():
+        buf = torch.empty(T * total, dtype=torch.float32, device=dev)
+        buf.view(torch.int32).fill_(int(np.array(SENTINEL).view(np.int32)))
+        return buf
+
+    def untouched(buf):
+        return bool((buf.view(torch.int32) == int(np.array(SENTINEL).view(np.int32))).all())
+
+    out = sentinel_buffer()
+    for call in (realign, paint):
+        for args in ((2,), (2, table), (2, None, table), (1, table, table), (0, table, table), (3,), (-1,)):
+            assert call(*args, out=out) == 2, (call.__name__, args)
+            assert b"layout" in lib.gvl_last_error().lower(), (call.__name__, args)
+    assert untouched(out)
+    # a valid plan executes into the whole buffer ...
+    assert realign(1) == 0
+    assert lib.gvl_dev_realign_tracks_exec(h, ptr(out), 0, _stream()) == 0
+    torch.cuda.synchronize()
+    assert not (out.view(torch.int32) == int(np.array(SENTINEL).view(np.int32))).any()
+    # ... and into nothing once a rejected call of either entry followed it
+    for reject in (lambda: realign(3), lambda: paint(2), lambda: realign(1, table, table)):
+        assert realign(1) == 0 and reject() == 2
+        buf = sentinel_buffer()
+        assert lib.gvl_dev_realign_tracks_exec(h, ptr(buf), 0, _stream()) == 0
+        torch.cuda.synchronize()
+        assert untouched(buf)
 
 
 # ---------------------------------------------------------------------------------------------------- Dataset vs the oracle

@@ -420,18 +420,6 @@ def test_api(env, cuda_device):
     for dsx, idx in ((ds.with_len(900), IDX), (ds, IDX), (ds.with_settings(splice_info={"a": [1, 2]}), (0, 1))):
         x, y = dsx.with_settings(rng=3)[idx], dsx.with_track_dtype(torch.float32).with_settings(rng=3)[idx]
         assert all(_same(p, q) for p, q in zip(x, y))
-    # unknown dtype codes at the C ABI
-    h = ds.engine.ctx.handle
-    buf = torch.empty(64, dtype=torch.float32, device=cuda_device)
-    for code in (3, -1):
-        assert _ffi.lib.gvl_dev_realign_tracks_exec_dtype(h, _ffi.ptr(buf), code, _stream()) == 2
-        assert b"unknown track dtype" in _ffi.lib.gvl_last_error()
-    itv = ds.engine.track_descs(["track0"])[0]
-    z64 = torch.zeros(2, dtype=torch.int64, device=cuda_device)
-    z32 = torch.zeros(1, dtype=torch.int32, device=cuda_device)
-    rc = _ffi.lib.gvl_dev_paint_tracks_dtype(h, 1, itv, _ffi.ptr(z64), _ffi.ptr(z32), 1, _ffi.ptr(z64), 1, None, None, None,
-                                             _ffi.ptr(buf), 7, _stream())
-    assert rc == 2 and b"unknown track dtype" in _ffi.lib.gvl_last_error()
     pipe = FixedPipeline(ds.with_len(800).with_track_dtype(torch.float16), 4)
     job = pipe._scr0.job
     assert job.track_dtype == _ffi.TRACK_F16
@@ -441,3 +429,22 @@ def test_api(env, cuda_device):
         assert rc == 2 and b"unknown track dtype" in _ffi.lib.gvl_last_error()
     finally:
         job.track_dtype = _ffi.TRACK_F16
+
+
+def test_unknown_dtype_codes_at_the_track_entries(env, cuda_device):
+    """gvl_dev_realign_tracks_exec and gvl_dev_paint_tracks reject a dtype code outside GVL_TRACK_*."""
+    from genvarloader_b200 import _ffi
+    from genvarloader_b200._engine import TRACK_LAYOUTS, _stream
+
+    _, ds = env
+    h = ds.engine.ctx.handle
+    buf = torch.empty(64, dtype=torch.float32, device=cuda_device)
+    for code in (3, -1):
+        assert _ffi.lib.gvl_dev_realign_tracks_exec(h, _ffi.ptr(buf), code, _stream()) == 2
+        assert b"unknown track dtype" in _ffi.lib.gvl_last_error()
+    itv = ds.engine.track_descs(["track0"])[0]
+    z64 = torch.zeros(2, dtype=torch.int64, device=cuda_device)
+    z32 = torch.zeros(1, dtype=torch.int32, device=cuda_device)
+    rc = _ffi.lib.gvl_dev_paint_tracks(h, 1, itv, _ffi.ptr(z64), _ffi.ptr(z32), 1, _ffi.ptr(z64), 1, None, TRACK_LAYOUTS["btp"],
+                                       None, None, _ffi.ptr(buf), 7, _stream())
+    assert rc == 2 and b"unknown track dtype" in _ffi.lib.gvl_last_error()

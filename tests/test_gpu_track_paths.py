@@ -569,7 +569,7 @@ def _same_tiles_every_track(t, n_tracks):
 @pytest.mark.parametrize("n_tracks", [8, 9])
 def test_dataset_layouts_many_tracks(cuda_device, O, G, n_tracks):
     """(b, t, p, ~l) rows of different lengths through Dataset.__getitem__ (descriptors inline for <= 8 tracks, a device
-    array above), then the same slots as spliced rows (per-row destinations, gvl_dev_realign_tracks_plan_rows); every
+    array above), then the same slots as spliced rows (per-row destinations, GVL_TRACK_LAYOUT_ROWS); every
     track with intervals and a fill of its own, so a mix-up of track indices shows."""
     import genvarloader_b200 as m
     from genvarloader_b200._dataset import Dataset
