@@ -59,7 +59,7 @@ class Dataset:
     output_length: object = "ragged"                  # "ragged" | "variable" | int
     sequence_type: object = "haplotypes"              # "reference" | "haplotypes" | "annotated" | None
     active_tracks: tuple = ()
-    track_output: str = "tracks"                      # with_tracks(kind=...): "tracks" (values) | "intervals"
+    track_output: str = "tracks"                      # with_tracks(kind=...): "tracks" (values) | "intervals" | "realigned-intervals"
     insertion_fill: dict = field(default_factory=dict)
     jitter: int = 0
     deterministic: bool = True
@@ -367,6 +367,9 @@ class Dataset:
         if self.track_output == "intervals" and self._realigns:
             raise ValueError("kind='intervals' returns the stored intervals, which are not realigned to haplotypes: set "
                              "with_settings(realign_tracks=False), or use with_seqs('reference') or with_seqs(None).")
+        if self.track_output == "realigned-intervals" and self.active_tracks and not self._realigns:
+            raise ValueError("kind='realigned-intervals' cuts tracks realigned to haplotypes: it needs with_seqs('haplotypes') or "
+                             "with_seqs('annotated') and realign_tracks=True; use kind='intervals' for the stored intervals.")
         if self.encoding != "bytes" and self.sequence_type not in ("haplotypes", "reference"):
             raise ValueError("one-hot encoding applies to 'haplotypes' / 'reference' sequences only")
         if self.encoding == "onehot_cf":
@@ -487,9 +490,12 @@ class Dataset:
         """Reference: `Dataset.with_tracks`, _impl.py:785-839.  `False`/`[]` disables tracks.  `kind`: None keeps the
         current output kind; "tracks" returns base-pair values (painted or realigned), "intervals" the stored intervals
         that overlap each read's window, clipped to it (`RaggedIntervals`, one cell per (..., track); DESIGN.md §7).
-        Intervals are not realigned: with haplotypes, set `with_settings(realign_tracks=False)` first."""
-        if kind not in (None, "tracks", "intervals"):
-            raise ValueError(f"Unknown track kind {kind!r}: 'tracks' or 'intervals'")
+        Intervals are not realigned: with haplotypes, set `with_settings(realign_tracks=False)` first.
+        "realigned-intervals" returns the realigned tracks of haplotype reads (realign_tracks=True) as intervals in
+        haplotype coordinates from the read's start: the maximal runs of positions that take their value from one stored
+        interval (or one insertion fill), `RaggedIntervals` with one cell per (..., track, ploid)."""
+        if kind not in (None, "tracks", "intervals", "realigned-intervals"):
+            raise ValueError(f"Unknown track kind {kind!r}: 'tracks', 'intervals' or 'realigned-intervals'")
         if tracks is None:
             names = tuple(self.track_kinds)
         elif tracks is False:
@@ -768,6 +774,9 @@ class Dataset:
                 i_q = pk.add(q, np.int64)
                 i_pf = pk.add(rows_p * e_first[e_pair], np.int64)       # first sequence row of the element's pair
                 i_pn = pk.add(rows_p * e_first[e_pair + 1], np.int64)   # ... and of the next pair
+                if self.track_output == "realigned-intervals":
+                    # output rows (pair, track, ploid, element): cell (pair, track, ploid) is a run of its elements' rows
+                    i_rout, i_rcells = (pk.add(a, np.int64) for a in _realigned_interval_rows(e_first, n_el, e_pair, e_k, t, p))
             elif self.track_output == "intervals":
                 # rows (pair, track, element), each element over its own region: cell (pair, track) is a run of rows
                 tt = np.arange(t, dtype=np.int64)
@@ -809,16 +818,22 @@ class Dataset:
             row_len = (oo[1:] - oo[:-1])[t_q].reshape(-1)
             out_offsets = torch.zeros(n_e * p + 1, dtype=torch.int64, device=dev)
             torch.cumsum(row_len, 0, out=out_offsets[1:])
-            base = oo[pk.get(i_pf)][:, None]  # B_c of the element's pair: cell (c, track, h) starts at t * B_c + ...
-            row_dst = (t * base + oo[t_q] - base).reshape(-1)
-            row_tstride = (oo[pk.get(i_pn)] - base[:, 0]).repeat_interleave(p)  # (a materialised copy: the kernel reads it by index)
             keep = keep_off = None
             if self.var_filter == "exonic":
                 keep, keep_off = self._exonic_keep(pk.get(i_goi_e), pk.get(i_reg), goi_e)
-            results.append(self._realigned_tracks(
-                ds_idx_e, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), pk.get(i_len), diffs.view(-1)[t_q],
-                out_offsets, total, max_rec, keep, keep_off, pk.get(i_rc_e) if i_rc_e is not None else None, group_offsets,
-                (*outer, t, p, None), row_dst=row_dst, row_tstride=row_tstride))
+            if self.track_output == "realigned-intervals":
+                results.append(self._realigned_intervals(
+                    ds_idx_e, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), pk.get(i_len), diffs.view(-1)[t_q],
+                    out_offsets, total, max_rec, keep, keep_off, (*outer, t, p, None), row_out=pk.get(i_rout),
+                    cells=pk.get(i_rcells)))
+            else:
+                base = oo[pk.get(i_pf)][:, None]  # B_c of the element's pair: cell (c, track, h) starts at t * B_c + ...
+                row_dst = (t * base + oo[t_q] - base).reshape(-1)
+                row_tstride = (oo[pk.get(i_pn)] - base[:, 0]).repeat_interleave(p)  # (a materialised copy: the kernel reads it by index)
+                results.append(self._realigned_tracks(
+                    ds_idx_e, pk.get(i_reg), pk.get(i_sh_e), pk.get(i_goi_e), pk.get(i_oi), pk.get(i_len), diffs.view(-1)[t_q],
+                    out_offsets, total, max_rec, keep, keep_off, pk.get(i_rc_e) if i_rc_e is not None else None, group_offsets,
+                    (*outer, t, p, None), row_dst=row_dst, row_tstride=row_tstride))
         elif t and self.track_output == "intervals":
             results.append(self._track_intervals(pk.get(i_islot), pk.get(i_itw), (*outer, t, None), cells=pk.get(i_icells)))
         elif t:
@@ -990,7 +1005,10 @@ class Dataset:
             results.append(self._execute_seqs(oo, (b, None) if is_ref else (b, p, None), total))
         if want_tracks:
             t = len(self.active_tracks)
-            if self._realigns:
+            if self.track_output == "realigned-intervals":
+                results.append(self._realigned_intervals(ds_idx, t_reg, t_shifts, t_goi, pk.get(i_tr), torch.from_numpy(lengths).to(dev),
+                                                         diffs, oo, total, max_rec, keep, keep_off, (b, t, p, None)))
+            elif self._realigns:
                 results.append(self._realigned_tracks(ds_idx, t_reg, t_shifts, t_goi, pk.get(i_tr), torch.from_numpy(lengths).to(dev),
                                                       diffs, oo, total, max_rec, keep, keep_off, t_rc, oo, (b, t, p, None)))
             elif i_islot is not None:
@@ -1057,6 +1075,23 @@ class Dataset:
                                          self._fill_seed(ds_idx), max_rec, keep, keep_off, t_rc,
                                          layout="rows" if rows else "btp", dtype=self.track_dtype, **rows)
         return Ragged(out, _cell_offsets(seq_offsets, len(names), self.ploidy), shape)
+
+    def _realigned_intervals(self, ds_idx, t_reg, t_shifts, t_goi, t_oi, lengths, diffs, row_offsets, total: int, max_rec: int,
+                             keep, keep_off, shape, row_out=None, cells=None) -> RaggedIntervals:
+        """All active tracks realigned to planned haplotype rows as `_realigned_tracks` plans them, cut into intervals
+        instead of executed (gvl_dev_realigned_track_intervals): one cell per (query, track, ploid), or given `row_out`
+        (device int64: output row of (track, plan row)) and `cells` (device indices into the row offsets at which the
+        cells start, the last one = the end), wherever that table puts each row.  Draws the fill seed as the tracks read
+        does, so both reads of one generator state agree."""
+        names = list(self.active_tracks)
+        ids, params = self._fills(names)
+        track_lengths = (lengths - diffs.clamp(max=0).min(1).values.to(torch.int64)).to(torch.int32)
+        off, starts, ends, values = self.engine.realigned_track_intervals(
+            names, t_reg, t_shifts, t_goi, t_oi, track_lengths, row_offsets, total, ids, params, self._fill_seed(ds_idx),
+            max_rec, keep, keep_off, row_out=row_out, dtype=self.track_dtype)
+        if cells is not None:
+            off = off[cells]
+        return RaggedIntervals(Ragged(starts, off, shape), Ragged(ends, off, shape), Ragged(values, off, shape))
 
     def _painted_tracks(self, t_oi, starts, row_offsets, total: int, t_rc, offsets, shape, **rows) -> Ragged:
         """The stored intervals of all active tracks painted in one launch (Tracks._call_float32, _tracks.py:370-420),
@@ -1174,6 +1209,18 @@ def _interval_rows(oi: np.ndarray, w0: np.ndarray, w1: np.ndarray, row_of: np.nd
     tw[1, row_of] = np.asarray(w0)[:, None]
     tw[2, row_of] = np.asarray(w1)[:, None]
     return slot, tw
+
+
+def _realigned_interval_rows(e_first: np.ndarray, n_el: np.ndarray, e_pair: np.ndarray, e_k: np.ndarray, t: int, p: int):
+    """Output rows of a spliced `_realigned_intervals` read over the element batch E: plan row (e, h) of track tt goes to
+    row (pair, tt, h, element) -> (row_out int64 (t * n_e * p,) at tt * n_e * p + e * p + h, the cells' first rows + the
+    end, int64 (n_pairs * t * p + 1,))."""
+    tt = np.arange(t, dtype=np.int64)[:, None, None]
+    hh = np.arange(p, dtype=np.int64)[None, None, :]
+    c0 = (t * p * e_first[e_pair])[None, :, None]
+    row_out = (c0 + (tt * p + hh) * n_el[e_pair][None, :, None] + e_k[None, :, None]).reshape(-1)
+    cells = (t * p * e_first[:-1, None] + np.arange(t * p, dtype=np.int64)[None, :] * n_el[:, None]).reshape(-1)
+    return row_out, np.append(cells, t * p * e_first[-1])
 
 
 def _cell_offsets(row_offsets: torch.Tensor, t: int, p: int = 1) -> torch.Tensor:

@@ -643,6 +643,42 @@ class Engine:
                                               code, _stream()))
         return offsets, starts, ends, values
 
+    def realigned_track_intervals(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
+                                  total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
+                                  keep_offsets=None, row_out=None, dtype=torch.float32):
+        """gvl_dev_realign_tracks with no output (the plan only), then gvl_dev_realigned_track_intervals: every planned row
+        (query, ploid) of every track in `names` cut into the intervals of its realigned values, in haplotype coordinates
+        from the query start.  Arguments as in `realign_tracks`; `row_out` (device int64 (n_tracks * rows,)): output row of
+        (track t, plan row k) at t * rows + k, None = (query, track, ploid) order.  A sizing call, ONE wait for the total,
+        then the emit call.  Returns (offsets i64 (n_tracks * rows + 1,), starts i32, ends i32, values of `dtype`)."""
+        code = track_dtype_code(dtype)
+        n_q, ploidy = geno_offset_idx.shape
+        n_rows = len(names) * n_q * ploidy
+        dev = self.device
+        offsets = torch.zeros(n_rows + 1, dtype=torch.int64, device=dev)
+        empty = (offsets, torch.empty(0, dtype=torch.int32, device=dev), torch.empty(0, dtype=torch.int32, device=dev),
+                 torch.empty(0, dtype=dtype, device=dev))
+        if n_rows == 0 or int(total_per_track) == 0:
+            return empty  # (no rows, or only empty ones: the plan is empty too)
+        itv, sid, par = self.track_descs(names, strategy_ids, params)
+        ch = self.svar2_channels(geno_offset_idx) if self.svar2 is not None else None
+        check(lib.gvl_dev_realign_tracks(self.ctx.handle, C.byref(self.tab), None if ch is None else C.byref(ch), ptr(regions),
+                                         ptr(shifts), ptr(geno_offset_idx), n_q, ploidy, ptr(keep), ptr(keep_offsets), None,
+                                         len(names), itv, ptr(offset_idxs), ptr(track_lengths), ptr(out_offsets),
+                                         int(total_per_track), sid, par, int(base_seed), None, 0, None, int(max_records),
+                                         _layout_code("tbp"), None, None, None, code, _stream()))
+        check(lib.gvl_dev_realigned_track_intervals(self.ctx.handle, ptr(row_out), ptr(offsets), 0, None, None, None, code,
+                                                    _stream()))
+        total = int(offsets[-1])  # the read's one wait
+        if total == 0:
+            return empty
+        starts = torch.empty(total, dtype=torch.int32, device=dev)
+        ends = torch.empty(total, dtype=torch.int32, device=dev)
+        values = torch.empty(total, dtype=dtype, device=dev)
+        check(lib.gvl_dev_realigned_track_intervals(self.ctx.handle, ptr(row_out), ptr(offsets), total, ptr(starts), ptr(ends),
+                                                    ptr(values), code, _stream()))
+        return offsets, starts, ends, values
+
     def check(self) -> None:
         """Synchronise and surface device-side status flags (workspace overflow)."""
         self.ctx.check(torch.cuda.current_stream().cuda_stream)

@@ -108,6 +108,7 @@ def _load() -> C.CDLL:
                                          c_vp]
     lib.gvl_dev_track_intervals.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32,
                                             c_vp]
+    lib.gvl_dev_realigned_track_intervals.argtypes = [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32, c_vp]
     return lib
 
 

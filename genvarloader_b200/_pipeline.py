@@ -103,6 +103,8 @@ def supports(ds) -> str | None:
         return "nothing to read"
     if ds.track_output == "intervals" and ds.active_tracks:
         return "track intervals are ragged by nature"
+    if ds.track_output == "realigned-intervals" and ds.active_tracks:
+        return "realigned track intervals are ragged by nature"
     if len(ds.active_tracks) > 8:
         return "more than 8 tracks"
     return None

@@ -145,6 +145,10 @@ struct gvl_ctx {
     int64_t var_scratch_bytes = 0;
     int64_t *itv_counts = nullptr;  // per-row interval counts of gvl_dev_track_intervals (gvl_tracks.cu)
     int64_t itv_counts_cap = 0;
+    void *ritv_ws = nullptr;        // item table, counts and offsets of gvl_dev_realigned_track_intervals (gvl_tracks.cu)
+    int64_t ritv_ws_bytes = 0;
+    int64_t ritv_pairs = -1;        // (track, row) pairs and item slots of its last sizing call (-1: none yet)
+    int64_t ritv_item_cap = 0;
     std::vector<std::pair<void *, int64_t>> var_results;  // device results of the last host-layer variants entry (gvl_variants_fetch)
     // host layer
     std::map<const void *, gvl_static_entry> statics;

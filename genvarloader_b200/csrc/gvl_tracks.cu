@@ -17,6 +17,8 @@
 //
 // gvl_dev_track_intervals returns the stored intervals themselves instead of painting them: a count kernel (one warp per
 // row, two 32-ary searches), the offset scan of the variants tail, and an emit kernel that copies each row's run.
+// gvl_dev_realigned_track_intervals cuts the rows of a track plan into intervals instead of executing them: a count kernel
+// over the rows' items (one warp each), offset scans, and an emit kernel with one thread per output interval.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -197,6 +199,349 @@ __global__ void __launch_bounds__(ITV_THREADS) itv_emit_kernel(const __grid_cons
             o_ends[o + i] = e;
             o_values[o + i] = to_out<T>(__ldg(I->itv_values + lo + i));
         }
+    }
+}
+
+// =====================================================================================
+// realigned intervals: the rows of a track plan cut into intervals (gvl_dev_realigned_track_intervals)
+// =====================================================================================
+// Every output position p of a planned row has a source, resolved as t2_generic_value resolves it, and the source has an
+// IDENTITY: the index of the stored interval that holds it (none outside every interval and outside the window); one per
+// record for Repeat5pNormalized / Constant fills; one per position for Interpolate fills; FlankSample positions take the
+// identity of the position they sample.  The row's intervals are the maximal runs of one identity other than none.
+//
+// Row k of track t ("pair" t * n_work + k) is split into ITEMS in output order: the copy span before the first record, then
+// for every record its own span and the copy span after it -- 1 + 2 n_rec items, contiguous and covering [0, L).  A copy
+// span reads consecutive source positions, so its runs are the stored intervals that overlap its source range (two 32-ary
+// searches); a record span is one run or none, except FlankSample and Interpolate spans (a step per position).  A run that
+// crosses items belongs to the item where it starts: an item whose first identity equals that of the position before it
+// is MERGED and does not count that run.
+//   ritv_count_kernel  one warp per item: its geometry, pieces and merge flag into an RItem, its count into `counts`;
+//   (offset scans)     items -> per-pair totals -> the caller's out_offsets;
+//   ritv_emit_kernel   one thread per output interval (seg_emit_kernel of gvl_variants.cu): finds its item and pair with
+//                      two binary searches over the offsets, writes (start, end, value); the end of a run that reaches the
+//                      end of its item is read from the RItems of the items it crosses.
+constexpr int RI_COPY = 0, RI_SPAN = 1, RI_ONE = 2, RI_INTERP = 3, RI_FLANK = 4;  // RItem.flags & 7
+constexpr int RI_MERGED = 8;  // the run at p0 continues a run of an earlier item (not counted here)
+constexpr int RI_OPEN = 16;   // the run at p0 has an interval identity and covers [p0, p1)
+
+struct __align__(16) RItem {
+    int64_t lo;        // COPY: first stored interval that reaches the span; SPAN: the source's interval (-1: none);
+                       // fills: the record (index in the row)
+    int32_t p0, p1;    // output positions of the item
+    int32_t s0;        // COPY: relative source position feeding p0; SPAN: the variant's source position
+    int32_t flags;     // kind | RI_MERGED | RI_OPEN
+    int32_t head_end;  // end of the run that starts at p0 (meaningful with an interval identity at p0)
+    int32_t pad;
+};
+static_assert(sizeof(RItem) == 32, "RItem is 32 bytes");
+
+struct RItvParams {
+    TrkExecParams P;           // the plan's saved execute parameters: rows, records, track descriptors, seeds
+    const int64_t *item_base;  // [n_pairs + 1] first item of each pair
+    const int64_t *item_off;   // [item_cap + 1] first output interval of each item (emit)
+    const int64_t *row_out;    // optional [n_pairs]: output row of each pair
+    int64_t n_pairs, item_cap;
+    RItem *items;              // [item_cap]
+};
+
+// what a pair needs to resolve its positions (the execute kernel's TileCtx, for one row of one track)
+struct RRow {
+    const TRec *recs;
+    int32_t n_rec, L, ref0, q_start, track_n, strategy;
+    double param;
+    SrcGlobal src;
+    uint64_t base_seed, qseed, hap;
+};
+
+__device__ __forceinline__ RRow ritv_row(const RItvParams &R, int64_t pair) {
+    const TrkExecParams &P = R.P;
+    const int64_t t = pair / P.n_work, k = pair - t * P.n_work, query = k / P.ploidy;
+    const RowPlan rp = P.rows[k];
+    const TrkDesc &T = P.tracks ? P.tracks[t] : P.inl[t];
+    RRow w;
+    w.recs = P.trecs + rp.rec_off;
+    w.n_rec = rp.n_rec, w.L = rp.length, w.ref0 = rp.ref0, w.q_start = rp.q_start, w.track_n = rp.contig_len;
+    w.strategy = T.strategy, w.param = T.param;
+    const int64_t slot = P.offset_idxs[t * P.n_queries + query];
+    w.src.its = T.itv_starts, w.src.ite = T.itv_ends, w.src.itv = T.itv_values, w.src.dense = nullptr;
+    w.src.itv_lo = T.itv_offsets[slot], w.src.itv_hi = T.itv_offsets[slot + 1], w.src.q_start = rp.q_start;
+    w.src.track_n = rp.contig_len;
+    // seeds of the fills exactly as trk_exec3_kernel takes them
+    const uint32_t sub = P.sub_batch > 0 ? (uint32_t)P.sub_batch : 0u;
+    const uint32_t q_blk = sub ? (uint32_t)query / sub : 0u;
+    w.hap = (uint64_t)(k - query * P.ploidy);
+    w.qseed = P.query_seed ? (uint64_t)P.query_seed[query] : (uint64_t)(sub ? (uint32_t)query - q_blk * sub : (uint32_t)query);
+    w.base_seed = P.base_seed_dev ? P.base_seed_dev[q_blk] : P.base_seed;
+    return w;
+}
+
+__device__ __forceinline__ int64_t ritv_out_row(const RItvParams &R, int64_t pair) {
+    if (R.row_out) return __ldg(R.row_out + pair);
+    const int64_t t = pair / R.P.n_work, k = pair - t * R.P.n_work, q = k / R.P.ploidy;
+    return (q * R.P.n_tracks + t) * R.P.ploidy + (k - q * R.P.ploidy);  // (query, track, ploid)
+}
+
+// warp_upper_le over any non-decreasing sequence at(lo .. hi - 1): last index with at(i) <= key, or lo - 1
+template <class F>
+__device__ __forceinline__ int64_t warp_last_le(F at, int64_t lo, int64_t hi, int64_t key) {
+    const int lane = lane_id();
+    while (hi - lo > 32) {
+        const int64_t step = (hi - lo + 31) / 32;
+        const int64_t idx = lo + (int64_t)(lane + 1) * step - 1;
+        const int cnt = __popc(__ballot_sync(0xffffffffu, idx < hi && at(idx) <= key));
+        const int64_t nlo = lo + (int64_t)cnt * step;
+        hi = imin64(hi, lo + (int64_t)(cnt + 1) * step - 1);
+        lo = nlo;
+        if (lo > hi) hi = lo;
+    }
+    const int64_t idx = lo + lane;
+    return lo + __popc(__ballot_sync(0xffffffffu, idx < hi && at(idx) <= key)) - 1;
+}
+
+// last i in [0, n) with off[i] <= e (off non-decreasing, off[0] <= e): one thread
+__device__ __forceinline__ int64_t last_le_i64(const int64_t *__restrict__ off, int64_t n, int64_t e) {
+    int64_t lo = 0, hi = n;
+    while (hi - lo > 1) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(off + mid) <= e) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// identity of relative source position s: the stored interval that holds it, -1 = none (also outside [0, track_n))
+__device__ __forceinline__ int64_t ritv_src_id_warp(const RRow &w, int64_t s) {
+    if (s < 0 || s >= w.track_n) return -1;
+    const int64_t g = (int64_t)w.q_start + s;
+    const int64_t i = warp_upper_le(w.src.its, w.src.itv_lo, w.src.itv_hi, (int32_t)g);
+    return (i >= w.src.itv_lo && (int64_t)__ldg(w.src.ite + i) > g) ? i : -1;
+}
+__device__ __forceinline__ int64_t ritv_src_id(const RRow &w, int64_t s) {  // (one thread)
+    if (s < 0 || s >= w.track_n) return -1;
+    const int64_t g = (int64_t)w.q_start + s;
+    int64_t a = w.src.itv_lo, b = w.src.itv_hi;
+    while (a < b) {
+        const int64_t mid = (a + b) >> 1;
+        if ((int64_t)__ldg(w.src.its + mid) <= g) a = mid + 1; else b = mid;
+    }
+    return (a > w.src.itv_lo && (int64_t)__ldg(w.src.ite + a - 1) > g) ? a - 1 : -1;
+}
+
+// source position that FlankSample output position p of record r samples (insertion_fill_value)
+__device__ __forceinline__ int64_t ritv_flank_src(const RRow &w, const TRec &r, int32_t p) {
+    const int64_t width = (int64_t)w.param;
+    const int64_t pool_lo = imax64((int64_t)r.vrel - width, 0), pool_hi = imin64((int64_t)r.vrel + width, (int64_t)w.track_n - 1);
+    const uint64_t pool_size = (uint64_t)(pool_hi - pool_lo + 1);
+    return pool_lo + (int64_t)(hash4(w.base_seed, w.qseed, w.hap, (uint64_t)p) % pool_size);
+}
+
+__device__ __forceinline__ bool ritv_is_fill(const RRow &w, const TRec &r) { return r.vdiff > 0 && w.strategy != GVL_FILL_REPEAT_5P; }
+
+// identity of output position p (warp): >= 0 a stored interval, -1 none, -2 an identity of its own (fills)
+__device__ int64_t ritv_ident_warp(const RRow &w, int32_t p) {
+    const TRec *__restrict__ recs = w.recs;
+    const int64_t i = warp_last_le([&](int64_t j) { return (int64_t)recs[j].a; }, 0, w.n_rec, p);
+    int64_t s;
+    if (i < 0) {
+        s = (int64_t)w.ref0 + p;
+    } else {
+        const TRec r = recs[i];
+        if (p < r.e) {
+            if (ritv_is_fill(w, r)) {
+                if (w.strategy != GVL_FILL_FLANK_SAMPLE) return -2;
+                s = ritv_flank_src(w, r, p);
+            } else {
+                s = r.vrel;
+            }
+        } else {
+            s = (int64_t)r.resume + (p - r.e);
+        }
+    }
+    return ritv_src_id_warp(w, s);
+}
+
+// geometry of item u of a row: positions [p0, p1), kind, source of p0, record
+__device__ __forceinline__ RItem ritv_geom(const RRow &w, int64_t u) {
+    auto A = [&](int64_t i) { return i < w.n_rec ? min(max(w.recs[i].a, 0), w.L) : w.L; };  // where record i takes over
+    RItem o;
+    o.pad = 0;
+    if (u == 0) {
+        o.p0 = 0, o.p1 = A(0), o.s0 = w.ref0, o.flags = RI_COPY, o.lo = -1;
+    } else {
+        const int64_t i = (u - 1) >> 1;
+        const TRec r = w.recs[i];
+        const int32_t a0 = A(i), a1 = max(A(i + 1), a0);
+        const int32_t e = min(max(r.e, a0), a1);
+        o.lo = i;
+        if (u & 1) {  // the variant's own values
+            o.p0 = a0, o.p1 = e, o.s0 = r.vrel;
+            o.flags = !ritv_is_fill(w, r) ? RI_SPAN
+                      : w.strategy == GVL_FILL_FLANK_SAMPLE ? RI_FLANK
+                      : w.strategy == GVL_FILL_INTERPOLATE ? RI_INTERP : RI_ONE;
+        } else {      // the copy after it
+            o.p0 = e, o.p1 = a1, o.s0 = r.resume + (e - r.e), o.flags = RI_COPY;
+        }
+    }
+    o.head_end = o.p0;
+    return o;
+}
+
+__global__ void __launch_bounds__(ITV_THREADS) ritv_count_kernel(const __grid_constant__ RItvParams R, int64_t *__restrict__ counts) {
+    const int lane = lane_id();
+    const int64_t n_items = __ldg(R.item_base + R.n_pairs);
+    const int64_t n_warps = (int64_t)gridDim.x * (ITV_THREADS / 32);
+    for (int64_t it = ((int64_t)blockIdx.x * ITV_THREADS + threadIdx.x) / 32; it < R.item_cap; it += n_warps) {
+        if (it >= n_items) {  // (slots beyond the plan's items)
+            if (lane == 0) counts[it] = 0;
+            continue;
+        }
+        const int64_t pair = warp_last_le([&](int64_t j) { return __ldg(R.item_base + j); }, 0, R.n_pairs, it);
+        const RRow w = ritv_row(R, pair);
+        RItem o = ritv_geom(w, it - __ldg(R.item_base + pair));
+        const int kind = o.flags;
+        int64_t n = 0, id0 = -2;  // pieces of the item, identity at p0
+        if (o.p1 > o.p0) {
+            if (kind == RI_COPY) {  // the stored intervals that overlap the source range, clipped to the window
+                const int64_t c0 = imax64(o.s0, 0), c1 = imin64((int64_t)o.s0 + (o.p1 - o.p0), w.track_n);
+                id0 = -1;
+                if (c1 > c0) {
+                    const int64_t g0 = (int64_t)w.q_start + c0, g1 = (int64_t)w.q_start + c1;
+                    const int64_t a = warp_upper_le(w.src.ite, w.src.itv_lo, w.src.itv_hi, (int32_t)g0) + 1;
+                    const int64_t b = warp_upper_le(w.src.its, a, w.src.itv_hi, (int32_t)(g1 - 1)) + 1;
+                    n = b - a;
+                    o.lo = a;
+                    if (n > 0 && o.s0 >= 0 && (int64_t)__ldg(w.src.its + a) <= g0) {
+                        id0 = a;
+                        o.head_end = (int32_t)(o.p0 + (imin64(__ldg(w.src.ite + a), g1) - g0));
+                    }
+                }
+            } else if (kind == RI_SPAN) {  // one source position for the whole span
+                id0 = ritv_src_id_warp(w, o.s0);
+                n = id0 >= 0;
+                o.lo = id0;
+                o.head_end = o.p1;
+            } else if (kind == RI_ONE) {
+                n = 1;
+            } else if (kind == RI_INTERP) {
+                n = o.p1 - o.p0;
+            } else {  // FlankSample: the identity of every position, 32 at a time
+                const TRec r = w.recs[o.lo];
+                int64_t prev = -3;  // identity before the chunk (-3: the item starts there)
+                bool head = false;
+                for (int32_t p = o.p0; p < o.p1; p += 32) {
+                    const int32_t q = p + lane;
+                    const int64_t id = q < o.p1 ? ritv_src_id(w, ritv_flank_src(w, r, q)) : -1;
+                    int64_t before = __shfl_up_sync(0xffffffffu, id, 1);
+                    if (lane == 0) before = prev;
+                    n += __popc(__ballot_sync(0xffffffffu, q < o.p1 && id >= 0 && id != before));
+                    if (p == o.p0) id0 = __shfl_sync(0xffffffffu, id, 0);
+                    const unsigned brk = __ballot_sync(0xffffffffu, q < o.p1 && id != id0);
+                    if (!head && brk) {
+                        o.head_end = p + __ffs(brk) - 1;
+                        head = true;
+                    }
+                    prev = __shfl_sync(0xffffffffu, id, 31);
+                }
+                if (!head) o.head_end = o.p1;
+            }
+        }
+        if (id0 >= 0 && o.head_end == o.p1) o.flags |= RI_OPEN;
+        if (id0 >= 0 && o.p0 > 0 && ritv_ident_warp(w, o.p0 - 1) == id0) {  // the run began in an earlier item
+            o.flags |= RI_MERGED;
+            n--;
+        }
+        if (lane == 0) {
+            R.items[it] = o;
+            counts[it] = n;
+        }
+    }
+}
+
+// per output row: its intervals = those of its pair's items
+__global__ void ritv_rows_kernel(const __grid_constant__ RItvParams R, int64_t *__restrict__ row_cnt) {
+    const int64_t pair = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (pair >= R.n_pairs) return;
+    const int64_t row = ritv_out_row(R, pair);
+    if (row < 0 || row >= R.n_pairs) return;
+    row_cnt[row] = __ldg(R.item_off + __ldg(R.item_base + pair + 1)) - __ldg(R.item_off + __ldg(R.item_base + pair));
+}
+
+// end of a run that reaches the end p1 of item `slot`: it goes on through the merged items that follow
+__device__ __forceinline__ int32_t ritv_run_end(const RItvParams &R, int64_t slot, int32_t end, int64_t n_items) {
+    for (int64_t s = slot + 1; s < n_items; s++) {
+        const RItem x = R.items[s];
+        if (x.p1 == x.p0) continue;
+        if (!(x.flags & RI_MERGED)) break;
+        end = x.head_end;
+        if (!(x.flags & RI_OPEN)) break;
+    }
+    return end;
+}
+
+template <class T>
+__device__ __forceinline__ void ritv_store(int32_t *o_starts, int32_t *o_ends, T *o_values, int64_t o, int32_t w0, int32_t s,
+                                           int32_t e, float v) {
+    o_starts[o] = w0 + s;
+    o_ends[o] = w0 + e;
+    o_values[o] = to_out<T>(v);
+}
+
+template <class T>
+__global__ void __launch_bounds__(256) ritv_emit_kernel(const __grid_constant__ RItvParams R, const int64_t *__restrict__ out_off,
+                                                        int64_t cap, int32_t *__restrict__ o_starts, int32_t *__restrict__ o_ends,
+                                                        T *__restrict__ o_values) {
+    const int64_t total = imin64(__ldg(R.item_off + R.item_cap), cap);
+    const int64_t n_items = __ldg(R.item_base + R.n_pairs);
+    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < total; g += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t slot = last_le_i64(R.item_off, R.item_cap, g);
+        const int64_t pair = last_le_i64(R.item_base, R.n_pairs, slot);
+        const int64_t row = ritv_out_row(R, pair);
+        if (row < 0 || row >= R.n_pairs) continue;
+        const int64_t o = __ldg(out_off + row) + (g - __ldg(R.item_off + __ldg(R.item_base + pair)));
+        const int64_t j = g - __ldg(R.item_off + slot);  // the item's j-th interval
+        const RRow w = ritv_row(R, pair);
+        const RItem it = R.items[slot];
+        const int kind = it.flags & 7;
+        const int64_t raw = j + ((it.flags & RI_MERGED) ? 1 : 0);  // its j-th piece that is not a continued run
+        int32_t s, e;
+        float v;
+        if (kind == RI_COPY) {
+            const int64_t i = it.lo + raw;
+            const int64_t g0 = (int64_t)w.q_start + imax64(it.s0, 0);
+            const int64_t g1 = (int64_t)w.q_start + imin64((int64_t)it.s0 + (it.p1 - it.p0), w.track_n);
+            const int64_t base = (int64_t)w.q_start + it.s0 - it.p0;  // position p reads source q_start + p + (s0 - p0)
+            s = (int32_t)(imax64(__ldg(w.src.its + i), g0) - base);
+            e = (int32_t)(imin64(__ldg(w.src.ite + i), g1) - base);
+            v = __ldg(w.src.itv + i);
+        } else if (kind == RI_SPAN) {
+            s = it.p0, e = it.p1, v = __ldg(w.src.itv + it.lo);
+        } else if (kind == RI_ONE || kind == RI_INTERP) {
+            const TRec r = w.recs[it.lo];
+            s = kind == RI_ONE ? it.p0 : it.p0 + (int32_t)raw;
+            e = kind == RI_ONE ? it.p1 : s + 1;
+            v = insertion_fill_value(w.src, w.strategy, w.param, r.vlen, r.vrel, s - r.a, s, w.base_seed, w.qseed, w.hap);
+        } else {  // FlankSample: the thread of the item's first interval writes all of them (fills are short)
+            if (j != 0) continue;
+            const int64_t n = __ldg(R.item_off + slot + 1) - __ldg(R.item_off + slot);
+            if (o + n > cap) continue;
+            const TRec r = w.recs[it.lo];
+            int64_t prev = -3, k = 0;
+            int32_t run0 = it.p0;
+            for (int32_t p = it.p0; p <= it.p1; p++) {
+                const int64_t id = p < it.p1 ? ritv_src_id(w, ritv_flank_src(w, r, p)) : -3;
+                if (id == prev) continue;
+                if (prev >= 0 && !(run0 == it.p0 && (it.flags & RI_MERGED))) {
+                    const int32_t end = p == it.p1 ? ritv_run_end(R, slot, p, n_items) : p;
+                    ritv_store(o_starts, o_ends, o_values, o + k++, w.q_start, run0, end, __ldg(w.src.itv + prev));
+                }
+                run0 = p;
+                prev = id;
+            }
+            continue;
+        }
+        if (o < 0 || o >= cap) continue;
+        if (e == it.p1) e = ritv_run_end(R, slot, e, n_items);
+        ritv_store(o_starts, o_ends, o_values, o, w.q_start, s, e, v);
     }
 }
 
@@ -495,6 +840,41 @@ int gvl_dev_track_intervals(gvl_ctx *ctx, const gvl_intervals *tracks, int64_t n
     return GVL_OK;
 }
 
+// ---- gvl_dev_realigned_track_intervals ----
+__global__ void ritv_pair_items_kernel(const RowPlan *__restrict__ rows, int64_t n_work, int64_t n_pairs, int64_t *__restrict__ items) {
+    const int64_t pair = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (pair < n_pairs) items[pair] = 1 + 2 * (int64_t)rows[pair % n_work].n_rec;
+}
+
+// the workspace of one sizing call, kept in ctx->ritv_ws for its emit call: per-pair item counts (later per-row interval
+// counts), item_base, per-item interval counts, item_off, the RItems
+struct RitvWs {
+    int64_t *pair_cnt, *item_base, *item_cnt, *item_off;
+    RItem *items;
+};
+
+static RitvWs ritv_ws_layout(void *base, int64_t n_pairs, int64_t item_cap) {
+    RitvWs w;
+    w.items = (RItem *)base;  // (32-byte aligned first)
+    w.pair_cnt = (int64_t *)(w.items + item_cap);
+    w.item_base = w.pair_cnt + n_pairs;
+    w.item_cnt = w.item_base + n_pairs + 1;
+    w.item_off = w.item_cnt + item_cap;
+    return w;
+}
+
+static int ensure_ritv_ws(gvl_ctx *ctx, int64_t bytes) {
+    if (bytes <= ctx->ritv_ws_bytes) return GVL_OK;
+    GVL_CUDA(cudaDeviceSynchronize());
+    if (ctx->ritv_ws) GVL_CUDA(cudaFree(ctx->ritv_ws));
+    ctx->ritv_ws = nullptr;
+    ctx->ritv_ws_bytes = 0;
+    const int64_t cap = imax64(bytes + bytes / 2, 1 << 16);
+    GVL_CUDA(cudaMalloc(&ctx->ritv_ws, (size_t)cap));
+    ctx->ritv_ws_bytes = cap;
+    return GVL_OK;
+}
+
 static int run_prng(gvl_ctx *ctx, uint64_t a, uint64_t b, uint64_t c, uint64_t d, int which, uint64_t *out) {
     if (!ctx || !out) return fail(GVL_ERR_ARG, "gvl_debug prng: NULL argument");
     GVL_CUDA(cudaSetDevice(ctx->device));
@@ -503,6 +883,67 @@ static int run_prng(gvl_ctx *ctx, uint64_t a, uint64_t b, uint64_t c, uint64_t d
     GVL_LAUNCH_CHECK();
     GVL_CUDA(cudaMemcpyAsync(out, dv, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->own_stream));
     GVL_CUDA(cudaStreamSynchronize(ctx->own_stream));
+    return GVL_OK;
+}
+
+int gvl_dev_realigned_track_intervals(gvl_ctx *ctx, const int64_t *row_out, int64_t *out_offsets, int64_t cap, int32_t *out_starts,
+                                      int32_t *out_ends, void *out_values, int32_t track_dtype, gvl_stream stream) {
+    const char *who = "gvl_dev_realigned_track_intervals";
+    if (!ctx || !out_offsets || cap < 0) return fail(GVL_ERR_ARG, "%s: NULL argument or negative size", who);
+    if (!track_dtype_ok(track_dtype)) return fail(GVL_ERR_ARG, "%s: unknown track dtype %d", who, (int)track_dtype);
+    if (cap && (!out_starts || !out_ends || !out_values)) return fail(GVL_ERR_ARG, "%s: NULL output with cap > 0", who);
+    if (!ctx->trk_plan_valid || !ctx->trk_params) return fail(GVL_ERR_STATE, "%s: no track plan", who);
+    RItvParams R;
+    memset(&R, 0, sizeof(R));
+    memcpy(&R.P, ctx->trk_params, sizeof(R.P));
+    if (!R.P.tracks && R.P.inl[0].dense) return fail(GVL_ERR_STATE, "%s: the plan reads a dense source, not intervals", who);
+    R.n_pairs = R.P.n_tracks * R.P.n_work;
+    R.row_out = row_out;
+    cudaStream_t st = (cudaStream_t)stream;
+    GVL_CUDA(cudaSetDevice(ctx->device));
+    int rc;
+    if (cap == 0) {  // sizing call: items, their counts, per-row totals, out_offsets
+        // item slots: 1 + 2 n_rec per pair, and the plan's records lie in the record buffer
+        R.item_cap = R.P.n_tracks * (R.P.n_work + 2 * ctx->trk.trec_cap);
+        const int64_t bytes = (int64_t)sizeof(RItem) * R.item_cap + 8 * (2 * R.n_pairs + 1 + 2 * R.item_cap + 1);
+        if ((rc = ensure_ritv_ws(ctx, bytes))) return rc;
+        const RitvWs W = ritv_ws_layout(ctx->ritv_ws, R.n_pairs, R.item_cap);
+        ctx->ritv_pairs = -1;
+        const unsigned pb = (unsigned)((R.n_pairs + 255) / 256);
+        ritv_pair_items_kernel<<<pb, 256, 0, st>>>(R.P.rows, R.P.n_work, R.n_pairs, W.pair_cnt);
+        GVL_LAUNCH_CHECK();
+        if ((rc = scan_lengths(ctx, W.pair_cnt, R.n_pairs, W.item_base, st))) return rc;
+        R.item_base = W.item_base;
+        R.items = W.items;
+        const unsigned blocks = (unsigned)imin64((R.item_cap + ITV_THREADS / 32 - 1) / (ITV_THREADS / 32), 148 * 32);
+        ritv_count_kernel<<<blocks, ITV_THREADS, 0, st>>>(R, W.item_cnt);
+        GVL_LAUNCH_CHECK();
+        if ((rc = scan_lengths(ctx, W.item_cnt, R.item_cap, W.item_off, st))) return rc;
+        R.item_off = W.item_off;
+        GVL_CUDA(cudaMemsetAsync(W.pair_cnt, 0, sizeof(int64_t) * (size_t)R.n_pairs, st));
+        ritv_rows_kernel<<<pb, 256, 0, st>>>(R, W.pair_cnt);
+        GVL_LAUNCH_CHECK();
+        if ((rc = scan_lengths(ctx, W.pair_cnt, R.n_pairs, out_offsets, st))) return rc;
+        ctx->ritv_pairs = R.n_pairs;
+        ctx->ritv_item_cap = R.item_cap;
+        return GVL_OK;
+    }
+    if (ctx->ritv_pairs != R.n_pairs) return fail(GVL_ERR_STATE, "%s: no sizing call (cap = 0) over this plan", who);
+    R.item_cap = ctx->ritv_item_cap;
+    const RitvWs W = ritv_ws_layout(ctx->ritv_ws, R.n_pairs, R.item_cap);
+    R.item_base = W.item_base, R.item_off = W.item_off, R.items = W.items;
+    const unsigned blocks = (unsigned)imin64((cap + 255) / 256, 148 * 16);
+    switch (track_dtype) {
+        case GVL_TRACK_F32:
+            ritv_emit_kernel<float><<<blocks, 256, 0, st>>>(R, out_offsets, cap, out_starts, out_ends, (float *)out_values);
+            break;
+        case GVL_TRACK_BF16:
+            ritv_emit_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(R, out_offsets, cap, out_starts, out_ends, (__nv_bfloat16 *)out_values);
+            break;
+        default:
+            ritv_emit_kernel<__half><<<blocks, 256, 0, st>>>(R, out_offsets, cap, out_starts, out_ends, (__half *)out_values);
+    }
+    GVL_LAUNCH_CHECK();
     return GVL_OK;
 }
 

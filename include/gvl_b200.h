@@ -298,6 +298,23 @@ int gvl_dev_track_intervals(gvl_ctx *ctx, const gvl_intervals *tracks, int64_t n
                             int64_t *out_offsets, int64_t cap, int32_t *out_starts, int32_t *out_ends, void *out_values,
                             int32_t track_dtype, gvl_stream stream);
 
+/* The rows of the last track plan on this context (gvl_dev_realign_tracks with out == NULL) cut into intervals instead of
+ * executed (the "realigned-intervals" kind of Dataset.with_tracks).  Every output position p of a planned row has the
+ * source the execute resolves for it; the source's identity is the stored interval that holds it (none outside every
+ * interval and outside the track window), one per record for Repeat5pNormalized / Constant insertion fills, one per
+ * position for Interpolate fills, and that of the sampled position for FlankSample fills.  A row's intervals are the
+ * maximal runs of one identity other than none, in ascending order: (w0 + first, w0 + last + 1, value), w0 = the row's
+ * query start (regions[q, 1]), value = the float32 value the execute computes there narrowed to track_dtype.  Strand
+ * reverses nothing.  row_out (device i64[n_tracks * n_work], or NULL) gives the output row of (track t, plan row k) at
+ * t * n_work + k, a permutation; NULL = (query, track, ploid) order.  Two calls over the same plan:
+ *   cap == 0: writes out_offsets (device i64[n_tracks * n_work + 1]) and nothing else; keeps its item table on the context;
+ *   cap > 0:  writes out_starts / out_ends (device i32[cap]) and out_values (cap elements of track_dtype), reading the
+ *             out_offsets of the sizing call, which must be the last one on this context.
+ * GVL_ERR_STATE without a valid plan (or for a plan of gvl_dev_shift_and_realign_tracks), or for cap > 0 without its
+ * sizing call.  A record overflow of the plan is reported by gvl_ctx_check, as for the execute. */
+int gvl_dev_realigned_track_intervals(gvl_ctx *ctx, const int64_t *row_out, int64_t *out_offsets, int64_t cap, int32_t *out_starts,
+                                      int32_t *out_ends, void *out_values, int32_t track_dtype, gvl_stream stream);
+
 /* ---- device layer: the small entries either side of reconstruction ------------------ */
 /* choose_exonic_variants, src/ffi/mod.rs:229-238 -> src/genotypes/mod.rs:132-176: for every (query, hap) row,
  * keep_offsets[k+1] - keep_offsets[k] = size of its genotype slice and keep[keep_offsets[k] + i] = 1 iff variant i
