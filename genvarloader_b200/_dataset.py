@@ -20,7 +20,7 @@ from typing import Literal
 import numpy as np
 import torch
 
-from ._engine import Engine, track_dtype_code
+from ._engine import Engine, track_bin_codes, track_dtype_code
 from ._insertion_fill import InsertionFill, Repeat5p, lower
 from ._variant_sizes import variant_buffer_sizes
 from ._types import (AnnotatedHaps, DummyVariant, Ragged, RaggedAlleles, RaggedAnnotatedHaps, RaggedIntervals, RaggedVariants,
@@ -69,6 +69,8 @@ class Dataset:
     output_format: str = "ragged"                     # "ragged" | "flat"  (with_output_format)
     encoding: str = "bytes"                           # "bytes" | "onehot" | "onehot_cf"  (this build's fused one-hot)
     track_dtype: torch.dtype = torch.float32          # element type of track outputs (with_track_dtype, this build's extension)
+    track_bin: int = 1                                # with_track_bins: output positions per stored track value (1 = unbinned)
+    track_reduce: str = "mean"                        # with_track_bins: "mean" | "sum" | "max"
     var_fields: tuple = ("alt", "ilen", "start")      # fields of the "variants" output (_haps.py:268)
     dummy_variant: object = None                      # DummyVariant for empty (region, sample, ploid) groups, or None
     unphased_union: bool = False                      # fold the ploidy rows of a (region, sample) into one (_flat_variants.py:925-938)
@@ -229,7 +231,8 @@ class Dataset:
     def __repr__(self) -> str:
         return (f"GVL dataset (B200-resident) with shape {self.shape}: sequences={self.sequence_type!r}, tracks={list(self.active_tracks)}, "
                 f"output_length={self.output_length!r}, jitter={self.jitter} (max {self.max_jitter}), deterministic={self.deterministic}, "
-                f"rc_neg={self.rc_neg}, is_subset={self.is_subset}, is_spliced={self.is_spliced}, track_dtype={self.track_dtype}")
+                f"rc_neg={self.rc_neg}, is_subset={self.is_subset}, is_spliced={self.is_spliced}, track_dtype={self.track_dtype}"
+                + (f", track_bins={self.track_bin} ({self.track_reduce})" if self.track_bin > 1 else ""))
 
     def _shape_counts(self, x: np.ndarray, squeeze: bool, out_reshape):
         if squeeze:
@@ -377,6 +380,26 @@ class Dataset:
                 raise ValueError("channels-first one-hot needs a fixed output length")
             if int(self.output_length) % 4:
                 raise ValueError("channels-first one-hot needs an output length that is a multiple of 4")
+        if self.track_bin > 1:
+            self._check_track_bins()
+
+    def _check_track_bins(self) -> None:
+        """The states in which binned tracks are defined (with_track_bins)."""
+        b = self.track_bin
+        if not self.track_kinds:
+            raise ValueError("Dataset has no tracks; cannot bin tracks.")
+        if self.splice_rows is not None:
+            raise ValueError("binned tracks need fixed-length rows and spliced output is ragged: clear the splicing with "
+                             "with_settings(splice_info=False), or with_track_bins(1) first.")
+        if not isinstance(self.output_length, (int, np.integer)):
+            raise ValueError(f"binned tracks need a fixed output length: call with_len(<multiple of {b}>) before "
+                             f"with_track_bins({b}), or with_track_bins(1) first.")
+        if int(self.output_length) % b:
+            raise ValueError(f"the output length ({self.output_length}) must be a multiple of the track bin size ({b}): "
+                             f"use with_len({-(-int(self.output_length) // b) * b}) or a bin size that divides it.")
+        if self.track_output != "tracks":
+            raise ValueError(f"binned tracks apply to kind='tracks' only, not {self.track_output!r}: use "
+                             "with_tracks(kind='tracks'), or with_track_bins(1) first.")
 
     def _evolve(self, **kw) -> "Dataset":
         ds = replace(self, **kw, _cache={})
@@ -485,6 +508,22 @@ class Dataset:
             raise ValueError("Dataset has no tracks; cannot set a track dtype.")
         track_dtype_code(dtype)
         return self._evolve(track_dtype=dtype)
+
+    def with_track_bins(self, bin_size: int, reduce: str = "mean") -> "Dataset":
+        """Binned track outputs (this build's extension, like `with_track_dtype`): every track row is cut into bins of
+        `bin_size` output positions (a power of two from 2 to 4096; 1 restores the unbinned default) and the track kernels
+        store one value per bin, so a read returns (b, t, p, L // bin_size) realigned or (b, t, L // bin_size) painted
+        tracks and the base-pair values are never written.  Bin j covers output positions [j * bin_size, (j + 1) *
+        bin_size) of its row, so a reverse-complemented row is its forward bins reversed.  `reduce`:
+        "sum" -- the bin's float32 values summed in float64 and rounded to float32; "mean" -- that sum divided by
+        `bin_size` in float64, rounded to float32; "max" -- the largest value.  A NaN in a bin makes it NaN (a `Constant`
+        fill's default NaN included).  The result is then narrowed to the track dtype as `with_track_dtype` describes, and
+        a row's bins have the same bits in every read.  Needs tracks, a fixed output length that is a multiple of
+        `bin_size` (call `with_len` first), kind="tracks" and an unspliced dataset."""
+        b, _ = track_bin_codes(bin_size, reduce)
+        if not self.track_kinds:
+            raise ValueError("Dataset has no tracks; cannot bin tracks.")
+        return self._evolve(track_bin=b, track_reduce=reduce)
 
     def with_tracks(self, tracks=None, kind=None) -> "Dataset":
         """Reference: `Dataset.with_tracks`, _impl.py:785-839.  `False`/`[]` disables tracks.  `kind`: None keeps the
@@ -1073,8 +1112,8 @@ class Dataset:
         # (:292-300); the kernel writes the latter directly so data and offsets agree for t > 1
         out = self.engine.realign_tracks(names, t_reg, t_shifts, t_goi, t_oi, track_lengths, row_offsets, total, ids, params,
                                          self._fill_seed(ds_idx), max_rec, keep, keep_off, t_rc,
-                                         layout="rows" if rows else "btp", dtype=self.track_dtype, **rows)
-        return Ragged(out, _cell_offsets(seq_offsets, len(names), self.ploidy), shape)
+                                         layout="rows" if rows else "btp", dtype=self.track_dtype, **self._bins(), **rows)
+        return Ragged(out, _cell_offsets(seq_offsets, len(names), self.ploidy) // self.track_bin, shape)
 
     def _realigned_intervals(self, ds_idx, t_reg, t_shifts, t_goi, t_oi, lengths, diffs, row_offsets, total: int, max_rec: int,
                              keep, keep_off, shape, row_out=None, cells=None) -> RaggedIntervals:
@@ -1098,8 +1137,12 @@ class Dataset:
         negative-strand rows reversed, in (query, track) order or, given `row_dst` / `row_tstride`, where that table puts
         each row.  `offsets`: of the output cells."""
         out = self.engine.paint_tracks(list(self.active_tracks), t_oi, starts, row_offsets, total, t_rc,
-                                       layout="rows" if rows else "btp", dtype=self.track_dtype, **rows)
-        return Ragged(out, offsets, shape)
+                                       layout="rows" if rows else "btp", dtype=self.track_dtype, **self._bins(), **rows)
+        return Ragged(out, offsets // self.track_bin, shape)
+
+    def _bins(self) -> dict:
+        """The binning arguments of a track read (Engine.realign_tracks / paint_tracks)."""
+        return dict(bin=self.track_bin, reduce=self.track_reduce)
 
     def _track_intervals(self, row_slot, row_tw, shape, cells=None) -> RaggedIntervals:
         """The stored intervals of the active tracks over one window per row (gvl_dev_track_intervals): row k reads slot
@@ -1184,8 +1227,9 @@ class Dataset:
                 res = o.to_padded(0.0)                               # tracks (any track dtype) pad with 0 (_query.py:545-548)
             else:
                 res = o.to_padded(0 if o.data.dim() > 1 else N_CHAR)  # bytes pad with N; one-hot with zeros
-        else:
-            res = o.to_fixed(int(self.output_length))
+        else:  # (binned tracks: L // bin per row; tracks are the floating-point outputs)
+            binned = isinstance(o, Ragged) and o.data.is_floating_point()
+            res = o.to_fixed(int(self.output_length) // (self.track_bin if binned else 1))
         if out_reshape is not None:
             if isinstance(res, torch.Tensor):
                 res = res.reshape(*out_reshape, *res.shape[1:])

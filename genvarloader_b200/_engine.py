@@ -12,7 +12,8 @@ import numpy as np
 import torch
 
 from . import _ffi
-from ._ffi import (MODE_ANNOTATED, MODE_ONEHOT, MODE_ONEHOT_CF, MODE_U8, TRACK_BF16, TRACK_F16, TRACK_F32, DatasetView, Intervals,
+from ._ffi import (MODE_ANNOTATED, MODE_ONEHOT, MODE_ONEHOT_CF, MODE_U8, TRACK_BF16, TRACK_BIN_MAX, TRACK_F16, TRACK_F32,
+                   TRACK_REDUCE_MAX, TRACK_REDUCE_MEAN, TRACK_REDUCE_SUM, DatasetView, Intervals,
                    SparseTables, Svar2Channels, c_i32, c_i64, c_u8, c_vp, check, lib, ptr)
 
 _SVAR2_VARIANTS = ("`variants` output is built for the SVAR1 genotype CSR; the svar2 source decodes variants through its "
@@ -31,6 +32,21 @@ def track_dtype_code(dtype) -> int:
     if code is None:
         raise ValueError(f"track dtype must be torch.float32, torch.bfloat16 or torch.float16, got {dtype!r}")
     return code
+
+
+# reductions of binned track outputs (GVL_TRACK_REDUCE_*)
+TRACK_REDUCES = {"mean": TRACK_REDUCE_MEAN, "sum": TRACK_REDUCE_SUM, "max": TRACK_REDUCE_MAX}
+
+
+def track_bin_codes(bin_size: int, reduce: str) -> tuple:
+    """(bin, GVL_TRACK_REDUCE_*) of a binned track output; bin 1 = unbinned.  ValueError for a bin that is not 1 or a power
+    of two in [2, 4096], or a reduction other than "mean", "sum" and "max"."""
+    if reduce not in TRACK_REDUCES:
+        raise ValueError(f'track reduction must be "mean", "sum" or "max", got {reduce!r}')
+    if (isinstance(bin_size, bool) or not isinstance(bin_size, (int, np.integer)) or not 1 <= bin_size <= TRACK_BIN_MAX
+            or bin_size & (bin_size - 1)):
+        raise ValueError(f"track bin size must be 1 (unbinned) or a power of two from 2 to {TRACK_BIN_MAX}, got {bin_size!r}")
+    return int(bin_size), TRACK_REDUCES[reduce]
 
 
 def _layout_code(layout: str) -> int:
@@ -586,16 +602,21 @@ class Engine:
     def realign_tracks(self, names, regions, shifts, geno_offset_idx, offset_idxs, track_lengths, out_offsets,
                        total_per_track: int, strategy_ids, params, base_seed: int, max_records: int, keep=None,
                        keep_offsets=None, to_rc=None, query_seed=None, out=None, layout="tbp", base_seed_dev=None,
-                       batch=None, sub_batch: int = 0, row_dst=None, row_tstride=None, dtype=torch.float32):
+                       batch=None, sub_batch: int = 0, row_dst=None, row_tstride=None, dtype=torch.float32, bin: int = 1,
+                       reduce: str = "mean"):
         """gvl_dev_realign_tracks: all `names` in one plan + one execute launch.
         offset_idxs: int64 (n_tracks, batch) device; out: `dtype` (n_tracks * total_per_track,), track-major
         (layout="tbp", the reference's flat buffer), with every query's tracks adjacent (layout="btp": the order the
         reference's (b, t, p, ~l) offsets describe) or wherever the per-row table puts each row (layout="rows": row k of
         track t starts at row_dst[k] + t * row_tstride[k], device int64 (batch * ploidy,) each).  `dtype` (of `out` when
-        given): float32, or bfloat16 / float16 -- the float32 values rounded to nearest even by the execute kernel's stores."""
+        given): float32, or bfloat16 / float16 -- the float32 values rounded to nearest even by the execute kernel's stores.
+        `bin` > 1: every row reduced per `bin` output positions by `reduce` ("mean", "sum", "max") before the store
+        (gvl_dev_realign_tracks_exec_binned); `out` then holds n_tracks * total_per_track / bin values, and row lengths and
+        offsets must be multiples of `bin`."""
         code = track_dtype_code(dtype if out is None else out.dtype)
+        bin, red = track_bin_codes(bin, reduce)
         if out is None:
-            out = torch.empty(len(names) * total_per_track, dtype=dtype, device=self.device)
+            out = torch.empty(len(names) * total_per_track // bin, dtype=dtype, device=self.device)
         b_cap, ploidy = geno_offset_idx.shape
         batch = b_cap if batch is None else int(batch)  # (a prefix of preallocated buffers)
         itv, sid, par = self.track_descs(names, strategy_ids, params)
@@ -605,21 +626,29 @@ class Engine:
                                          ptr(to_rc), len(names), itv, ptr(offset_idxs), ptr(track_lengths), ptr(out_offsets),
                                          int(total_per_track), sid, par, int(base_seed), ptr(base_seed_dev), int(sub_batch),
                                          ptr(query_seed), int(max_records), _layout_code(layout), ptr(row_dst),
-                                         ptr(row_tstride), ptr(out), code, _stream()))
+                                         ptr(row_tstride), ptr(out) if bin == 1 else None, code, _stream()))
+        if bin > 1:  # the plan above, then the binned execute
+            check(lib.gvl_dev_realign_tracks_exec_binned(self.ctx.handle, ptr(out), code, bin, red, _stream()))
         return out
 
     def paint_tracks(self, names, offset_idxs, starts, out_offsets, total_per_track: int, to_rc=None, out=None,
-                     n_queries=None, layout="btp", row_dst=None, row_tstride=None, dtype=torch.float32):
+                     n_queries=None, layout="btp", row_dst=None, row_tstride=None, dtype=torch.float32, bin: int = 1,
+                     reduce: str = "mean"):
         """gvl_dev_paint_tracks: stored intervals of all `names` painted in one launch, masked rows reversed, one row per
         query.  offset_idxs: int64 (n_tracks, batch) device.  `layout` as in `realign_tracks` (default "btp": (b, t, ~l)
-        order) and `dtype` (of `out` when given): float32, bfloat16 or float16."""
+        order), `dtype` (of `out` when given): float32, bfloat16 or float16, and `bin` / `reduce` as in `realign_tracks`
+        (gvl_dev_paint_tracks_binned)."""
         code = track_dtype_code(dtype if out is None else out.dtype)
+        bin, red = track_bin_codes(bin, reduce)
         n_tracks, n_q = len(names), int(starts.numel() if n_queries is None else n_queries)
         if out is None:
-            out = torch.empty(n_tracks * int(total_per_track), dtype=dtype, device=self.device)
-        check(lib.gvl_dev_paint_tracks(self.ctx.handle, n_tracks, self.track_descs(names)[0], ptr(offset_idxs), ptr(starts),
-                                       n_q, ptr(out_offsets), int(total_per_track), ptr(to_rc), _layout_code(layout),
-                                       ptr(row_dst), ptr(row_tstride), ptr(out), code, _stream()))
+            out = torch.empty(n_tracks * int(total_per_track) // bin, dtype=dtype, device=self.device)
+        args = (self.ctx.handle, n_tracks, self.track_descs(names)[0], ptr(offset_idxs), ptr(starts), n_q, ptr(out_offsets),
+                int(total_per_track), ptr(to_rc), _layout_code(layout), ptr(row_dst), ptr(row_tstride), ptr(out), code)
+        if bin == 1:
+            check(lib.gvl_dev_paint_tracks(*args, _stream()))
+        else:
+            check(lib.gvl_dev_paint_tracks_binned(*args, bin, red, _stream()))
         return out
 
     def track_intervals(self, names, row_slot, row_track, row_w0, row_w1, dtype=torch.float32):

@@ -16,6 +16,8 @@ LIB_PATH = _PKG / "_lib" / os.environ.get("GVL_LIB_NAME", "libgvl_b200.so")  # (
 GVL_OK = 0
 MODE_U8, MODE_ONEHOT, MODE_ANNOTATED, MODE_ONEHOT_CF = 0, 1, 2, 3
 TRACK_F32, TRACK_BF16, TRACK_F16 = 0, 1, 2  # GVL_TRACK_*: element type of a track output
+TRACK_REDUCE_MEAN, TRACK_REDUCE_SUM, TRACK_REDUCE_MAX = 0, 1, 2  # GVL_TRACK_REDUCE_*: reduction of a binned track output
+TRACK_BIN_MAX = 4096  # GVL_TRACK_BIN_MAX
 
 c_i64, c_i32, c_u8, c_u64, c_vp = C.c_int64, C.c_int32, C.c_uint8, C.c_uint64, C.c_void_p
 
@@ -75,7 +77,7 @@ class FixedJob(C.Structure):
                 ("track_lengths", c_vp), ("paint_offsets", c_vp), ("itv", c_vp), ("strategy_ids", c_vp), ("params", c_vp),
                 ("ploidy", c_i64), ("rows_p", c_i64), ("output_length", c_i64), ("ref_slot", c_i64), ("n_tracks", c_i64),
                 ("max_slot_len", c_i64), ("typ_slot_len", c_i64), ("annot_mask", C.c_uint32), ("mode", c_i32), ("realign", c_i32), ("rc_neg", c_i32),
-                ("pad_char", c_u8), ("track_dtype", c_i32)]
+                ("pad_char", c_u8), ("track_dtype", c_i32), ("track_bin", c_i32), ("track_reduce", c_i32)]
 
 
 def _load() -> C.CDLL:
@@ -102,10 +104,13 @@ def _load() -> C.CDLL:
                                            c_vp, c_vp, c_i64, c_vp, c_vp, c_u64, c_vp, c_i64, c_vp, c_i64, c_i32, c_vp, c_vp, c_vp,
                                            c_i32, c_vp]
     lib.gvl_dev_realign_tracks_exec.argtypes = [c_vp, c_vp, c_i32, c_vp]
+    lib.gvl_dev_realign_tracks_exec_binned.argtypes = [c_vp, c_vp, c_i32, c_i32, c_i32, c_vp]
     lib.gvl_dev_shift_and_realign_tracks.argtypes = [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp,
                                                      c_vp, c_vp, c_vp, c_i64, c_i32, C.c_double, c_u64, c_vp, c_i64, c_vp, c_vp]
     lib.gvl_dev_paint_tracks.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp, c_i32,
                                          c_vp]
+    lib.gvl_dev_paint_tracks_binned.argtypes = [c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_i32, c_vp, c_vp, c_vp,
+                                                c_i32, c_i32, c_i32, c_vp]
     lib.gvl_dev_track_intervals.argtypes = [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32,
                                             c_vp]
     lib.gvl_dev_realigned_track_intervals.argtypes = [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_i32, c_vp]

@@ -30,7 +30,7 @@ import torch
 
 from . import _ffi
 from ._dataset import _as_rng, _batch_tail, epoch_order
-from ._engine import MODES, Engine, _raw_stream, _stream, track_dtype_code
+from ._engine import MODES, Engine, _raw_stream, _stream, track_bin_codes, track_dtype_code
 from ._ffi import BatchArgs, DatasetView, FixedJob, c_i64, c_u8, c_u64, c_vp, check, lib, ptr
 from ._types import AnnotatedHaps
 
@@ -85,6 +85,9 @@ class _Spec:
                 self.annot_mask |= 1 << i
         self.fill_ids, self.fill_params = ds._fills(self.names)
         self.track_dtype = ds.track_dtype
+        self.bin = int(ds.track_bin)      # binned tracks: Lt = L // bin values per track row
+        self.Lt = self.L // self.bin
+        self.reduce_code = track_bin_codes(self.bin, ds.track_reduce)[1]
 
 
 def supports(ds) -> str | None:
@@ -144,7 +147,7 @@ class _Out:
                 self.av = torch.empty(b * rp * L, dtype=torch.int32, device=dev)
                 self.ap = torch.empty(b * rp * L, dtype=torch.int32, device=dev)
         if t:
-            self.trk = torch.empty(b * t * (p if spec.realign else 1) * L, dtype=spec.track_dtype, device=dev)
+            self.trk = torch.empty(b * t * (p if spec.realign else 1) * spec.Lt, dtype=spec.track_dtype, device=dev)
         self.spec, self.b = spec, b
 
     def result(self, lo: int = 0, n: int | None = None, clone: bool = False):
@@ -170,7 +173,7 @@ class _Out:
                 s = AnnotatedHaps(s, f(self.av.view(*lead, L)), f(self.ap.view(*lead, L)))
             res.append(s)
         if t:
-            res.append(f(self.trk.view(b, t, p, L) if sp.realign else self.trk.view(b, t, L)))
+            res.append(f(self.trk.view(b, t, p, sp.Lt) if sp.realign else self.trk.view(b, t, sp.Lt)))
         return res[0] if len(res) == 1 else tuple(res)
 
 
@@ -234,7 +237,8 @@ class FixedPipeline:
         return FixedJob(adr(self.view), adr(eng.tab), adr(sv), scr.args, ptr(scr.out_offsets), ptr(scr.diffs), ptr(scr.track_lengths),
                         ptr(self._paint_off) if (sp.t and not sp.realign) else c_vp(0), adr(itv), adr(sid), adr(par),
                         sp.p, sp.rows_p, sp.L, self.ref_slot, sp.t, max(eng.max_slot_len, 1), int(getattr(eng, "typ_slot_len", 0)), sp.annot_mask, mode,
-                        1 if sp.realign else 0, 1 if sp.rc_neg else 0, eng.pad_char, track_dtype_code(sp.track_dtype))
+                        1 if sp.realign else 0, 1 if sp.rc_neg else 0, eng.pad_char, track_dtype_code(sp.track_dtype),
+                        sp.bin if sp.bin > 1 else 0, sp.reduce_code)
 
     # ------------------------------------------------------------------ one device call over n queries
     # Stage P ("plan"): batch prep + variant plan (+ track plan / tile prep).  Stage E ("execute"): the bandwidth-bound
@@ -433,7 +437,7 @@ class PipelinedLoader:
         self._rng = _as_rng(generator)
         n_batches = len(self)
         if not ring:  # ~256 MiB of output per half, at least one batch, no more than half an epoch
-            per_batch = self.batch_size * max(ds.ploidy, 1) * int(ds.output_length) * (4 + 4 * len(ds.active_tracks))
+            per_batch = self.batch_size * max(ds.ploidy, 1) * int(ds.output_length) * (4 + 4 * len(ds.active_tracks) // ds.track_bin)
             ring = max(1, min((256 << 20) // max(per_batch, 1), 64))
         ring = max(1, min(int(ring), -(-n_batches // 2)))
         self.pipe = FixedPipeline(ds, self.batch_size, ring=ring)

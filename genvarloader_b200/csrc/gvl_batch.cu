@@ -232,6 +232,9 @@ static int fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *J, const int64_t *ds_id
         return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: realigned tracks need haplotypes, diffs and track_lengths scratch");
     if (J->track_dtype != GVL_TRACK_F32 && J->track_dtype != GVL_TRACK_BF16 && J->track_dtype != GVL_TRACK_F16)
         return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: unknown track dtype %d", (int)J->track_dtype);
+    if (J->track_bin < 0 || J->track_bin > GVL_TRACK_BIN_MAX || (J->track_bin & (J->track_bin - 1)) ||
+        (J->track_reduce != GVL_TRACK_REDUCE_MEAN && J->track_reduce != GVL_TRACK_REDUCE_SUM && J->track_reduce != GVL_TRACK_REDUCE_MAX))
+        return fail(GVL_ERR_ARG, "gvl_dev_fixed_plan: bad track bin %d / reduction %d", (int)J->track_bin, (int)J->track_reduce);
     int rc = launch_batch_prep(ctx, J->view, ds_idx, jitter, inline_host, n, sub_batch, J->ref_slot, J->n_tracks, J->annot_mask,
                                &J->args, stream);
     if (rc) return rc;
@@ -261,10 +264,10 @@ int gvl_dev_fixed_stage(gvl_ctx *ctx, const gvl_fixed_job *J, int stage, const i
         case GVL_STAGE_TRK_EXEC:
             if (J->n_tracks <= 0) return GVL_OK;
             if (!trk) return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: track output missing");
-            if (J->realign) return gvl_dev_realign_tracks_exec(ctx, trk, J->track_dtype, stream);
-            return gvl_dev_paint_tracks(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
-                                        n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, GVL_TRACK_LAYOUT_BTP, NULL, NULL,
-                                        trk, J->track_dtype, stream);
+            if (J->realign) return gvl_dev_realign_tracks_exec_binned(ctx, trk, J->track_dtype, J->track_bin, J->track_reduce, stream);
+            return gvl_dev_paint_tracks_binned(ctx, J->n_tracks, J->itv, J->args.offset_idxs, J->args.starts, n, J->paint_offsets,
+                                               n * J->output_length, J->rc_neg ? J->args.to_rc_q : NULL, GVL_TRACK_LAYOUT_BTP, NULL,
+                                               NULL, trk, J->track_dtype, J->track_bin, J->track_reduce, stream);
         default: return fail(GVL_ERR_ARG, "gvl_dev_fixed_stage: unknown stage %d", stage);
     }
 }

@@ -563,7 +563,16 @@ static int check_track_output(const char *who, int32_t layout, const int64_t *ro
     return GVL_OK;
 }
 
-static int trk_execute(gvl_ctx *ctx, void *out, int32_t dtype, cudaStream_t st) {
+// bin 0 or 1: unbinned; else a power of two in [2, GVL_TRACK_BIN_MAX]
+static int check_track_bin(const char *who, int32_t bin, int32_t reduce) {
+    if (bin < 0 || bin > GVL_TRACK_BIN_MAX || (bin & (bin - 1)))
+        return fail(GVL_ERR_ARG, "%s: track bin %d is not 0, 1 or a power of two up to %d", who, (int)bin, GVL_TRACK_BIN_MAX);
+    if (reduce != GVL_TRACK_REDUCE_MEAN && reduce != GVL_TRACK_REDUCE_SUM && reduce != GVL_TRACK_REDUCE_MAX)
+        return fail(GVL_ERR_ARG, "%s: unknown track reduction %d", who, (int)reduce);
+    return GVL_OK;
+}
+
+static int trk_execute(gvl_ctx *ctx, void *out, int32_t dtype, int32_t bin, int32_t reduce, cudaStream_t st) {
     if (!ctx->trk_plan_valid || !ctx->trk_params) return fail(GVL_ERR_STATE, "track execute without a track plan");
     if (!out || ((uintptr_t)out & 15)) return fail(GVL_ERR_ARG, "track output must be a 16-byte aligned buffer");
     TrkExecParams P;
@@ -571,11 +580,21 @@ static int trk_execute(gvl_ctx *ctx, void *out, int32_t dtype, cudaStream_t st) 
     P.out = out;
     const dim3 grid((unsigned)P.grid_per_track, (unsigned)P.n_tracks);
     const TileDesc *tdesc = (const TileDesc *)ctx->trk.tdesc;
-    switch (dtype) {
-        case GVL_TRACK_F32: trk_exec3_kernel<float><<<grid, T2_THREADS, 0, st>>>(P, tdesc); break;
-        case GVL_TRACK_BF16: trk_exec3_kernel<__nv_bfloat16><<<grid, T2_THREADS, 0, st>>>(P, tdesc); break;
-        case GVL_TRACK_F16: trk_exec3_kernel<__half><<<grid, T2_THREADS, 0, st>>>(P, tdesc); break;
-        default: return fail(GVL_ERR_ARG, "unknown track dtype %d", (int)dtype);
+    const TrkBin bn{bin > 1 ? __builtin_ctz((unsigned)bin) : 0, reduce};
+    if (bin > 1) {
+        switch (dtype) {
+            case GVL_TRACK_F32: trk_exec3_kernel<float, true><<<grid, T2_THREADS, 0, st>>>(P, tdesc, bn); break;
+            case GVL_TRACK_BF16: trk_exec3_kernel<__nv_bfloat16, true><<<grid, T2_THREADS, 0, st>>>(P, tdesc, bn); break;
+            case GVL_TRACK_F16: trk_exec3_kernel<__half, true><<<grid, T2_THREADS, 0, st>>>(P, tdesc, bn); break;
+            default: return fail(GVL_ERR_ARG, "unknown track dtype %d", (int)dtype);
+        }
+    } else {
+        switch (dtype) {
+            case GVL_TRACK_F32: trk_exec3_kernel<float, false><<<grid, T2_THREADS, 0, st>>>(P, tdesc, bn); break;
+            case GVL_TRACK_BF16: trk_exec3_kernel<__nv_bfloat16, false><<<grid, T2_THREADS, 0, st>>>(P, tdesc, bn); break;
+            case GVL_TRACK_F16: trk_exec3_kernel<__half, false><<<grid, T2_THREADS, 0, st>>>(P, tdesc, bn); break;
+            default: return fail(GVL_ERR_ARG, "unknown track dtype %d", (int)dtype);
+        }
     }
     GVL_LAUNCH_CHECK();
     return GVL_OK;
@@ -702,7 +721,7 @@ static int realign_impl(const char *who, gvl_ctx *ctx, const gvl_sparse_tables *
     if ((rc = trk_prepare(ctx, n_work, ploidy, batch, n_tracks, desc, offset_idxs, total_per_track, query_seed, base_seed,
                           base_seed_dev, sub_batch, layout, row_dst, row_tstride, st)))
         return rc;
-    return out ? trk_execute(ctx, out, dtype, st) : GVL_OK;  // (out == NULL: plan only)
+    return out ? trk_execute(ctx, out, dtype, 0, GVL_TRACK_REDUCE_MEAN, st) : GVL_OK;  // (out == NULL: plan only)
 }
 
 int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
@@ -725,7 +744,18 @@ int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stre
     if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "gvl_dev_realign_tracks_exec: unknown track dtype %d", (int)dtype);
     GVL_CUDA(cudaSetDevice(ctx->device));
     if (!ctx->trk_plan_valid) return GVL_OK;  // (an empty or rejected plan: nothing to write)
-    return trk_execute(ctx, out, dtype, (cudaStream_t)stream);
+    return trk_execute(ctx, out, dtype, 0, GVL_TRACK_REDUCE_MEAN, (cudaStream_t)stream);
+}
+
+int gvl_dev_realign_tracks_exec_binned(gvl_ctx *ctx, void *out, int32_t dtype, int32_t bin, int32_t reduce, gvl_stream stream) {
+    const char *who = "gvl_dev_realign_tracks_exec_binned";
+    if (!ctx) return fail(GVL_ERR_ARG, "%s: ctx is NULL", who);
+    if (!track_dtype_ok(dtype)) return fail(GVL_ERR_ARG, "%s: unknown track dtype %d", who, (int)dtype);
+    int rc;
+    if ((rc = check_track_bin(who, bin, reduce))) return rc;
+    GVL_CUDA(cudaSetDevice(ctx->device));
+    if (!ctx->trk_plan_valid) return GVL_OK;
+    return trk_execute(ctx, out, dtype, bin, reduce, (cudaStream_t)stream);
 }
 
 int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl_svar2_channels *svar2,
@@ -741,17 +771,17 @@ int gvl_dev_shift_and_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab,
                         nullptr, nullptr, out, GVL_TRACK_F32, stream);
 }
 
-int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
-                         const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
-                         const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out,
-                         int32_t dtype, gvl_stream stream) {
-    const char *who = "gvl_dev_paint_tracks";
+static int paint_impl(const char *who, gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                      const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                      const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out,
+                      int32_t dtype, int32_t bin, int32_t reduce, gvl_stream stream) {
     if (!ctx) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
     ctx->trk_plan_valid = false;  // (as in realign_impl)
     if (!itv || !offset_idxs || !starts || !out_offsets) return fail(GVL_ERR_ARG, "%s: NULL argument", who);
     if (n_tracks < 0 || n_tracks > MAX_TRACKS) return fail(GVL_ERR_ARG, "%s: 0..%d tracks per call", who, MAX_TRACKS);
     int rc;
     if ((rc = check_track_output(who, layout, row_dst, row_tstride, dtype))) return rc;
+    if ((rc = check_track_bin(who, bin, reduce))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     GVL_CUDA(cudaSetDevice(ctx->device));
     if (n_queries == 0 || n_tracks == 0 || total_per_track == 0) return GVL_OK;
@@ -774,7 +804,23 @@ int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *it
     if ((rc = trk_prepare(ctx, n_queries, 1, n_queries, n_tracks, desc, offset_idxs, total_per_track, nullptr, 0, nullptr, 0,
                           layout, row_dst, row_tstride, st)))
         return rc;
-    return trk_execute(ctx, out, dtype, st);
+    return trk_execute(ctx, out, dtype, bin, reduce, st);
+}
+
+int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                         const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                         const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out,
+                         int32_t dtype, gvl_stream stream) {
+    return paint_impl("gvl_dev_paint_tracks", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets, total_per_track,
+                      to_rc, layout, row_dst, row_tstride, out, dtype, 0, GVL_TRACK_REDUCE_MEAN, stream);
+}
+
+int gvl_dev_paint_tracks_binned(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                                const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                                const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride,
+                                void *out, int32_t dtype, int32_t bin, int32_t reduce, gvl_stream stream) {
+    return paint_impl("gvl_dev_paint_tracks_binned", ctx, n_tracks, itv, offset_idxs, starts, n_queries, out_offsets,
+                      total_per_track, to_rc, layout, row_dst, row_tstride, out, dtype, bin, reduce, stream);
 }
 
 static int ensure_itv_counts(gvl_ctx *ctx, int64_t n) {

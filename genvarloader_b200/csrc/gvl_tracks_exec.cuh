@@ -31,6 +31,10 @@
 // Rows that need the reference's sequential semantics literally (variant lists that are not position-sorted leave
 // "jump" records) and dense f32 sources (shift_and_realign_tracks_sparse) take `t2_generic_segment`: every value
 // resolved on its own against the row's records and the source -- slow, exact for any input.
+// Binned output (trk_exec3_kernel<T, true>, `t3_bin_pass`): the same values are reduced per bin of 2..4096 output
+// positions before the store, so only one value per bin is written.  A bin never straddles a tile (tiles start at
+// multiples of T3_TILE in the row), but may straddle the sub-passes of a TD_BIG tile: the open bin's partial result
+// carries to the next sub-pass in shared memory.
 #pragma once
 
 constexpr int T3_TILE = TRK_TILE;           // output values per execute CTA
@@ -67,8 +71,8 @@ struct T3Smem {
     uint32_t mk2[T3_WORDS / 32];    // second level: bit w = word w of mk is non-zero
     int32_t fill_list[T3_REC];      // staged records whose insertion fill has to be computed
     int32_t n_fill;
-    int32_t bc_i32[4];              // broadcast slots of the (rare) sub-pass hand-over
-    int64_t bc_i64[2];
+    int32_t bc_i32[4];              // broadcast slots of the (rare) sub-pass hand-over; binned: [0, 1] = the TrkBin
+    int64_t bc_i64[2];              // binned: [1] = the open bin's partial result (a double) carried to the next sub-pass
     float bc_f32;
     alignas(16) unsigned char big_ctx[128];  // TileCtx handed to the out-of-line sub-pass variant
 };
@@ -271,6 +275,105 @@ __device__ __forceinline__ int32_t t2_map(const TRec *R, int m, int32_t x, bool 
 __device__ __forceinline__ void t2_set_bit(uint32_t *mk, uint32_t *mk2, int u) {
     const uint32_t old = atomicOr(&mk[u >> 5], 1u << (u & 31));
     if (old == 0) atomicOr(&mk2[u >> 10], 1u << ((u >> 5) & 31));
+}
+
+// ---- binned store ------------------------------------------------------------------------------------------
+// Bins of B = 1 << shift output positions; bin k of a row covers its positions [k B, (k + 1) B) and is stored at
+// out_bins[k].  Values are combined in float64 (sum, mean) or as float32 values held in float64 (max, NaN first), in an
+// order fixed by the row alone: sequentially over each 16-position chunk of the row (haplotype order), then a fixed
+// tree over the chunks of a bin (xor shuffles, then warps in order), and across the sub-passes of a TD_BIG tile in
+// haplotype order.  The tile geometry is a function of the row, so a row's bins have the same bits in every call.
+struct TrkBin {
+    int32_t shift, reduce;  // log2 of the bin size; GVL_TRACK_REDUCE_*
+};
+
+__device__ __forceinline__ double bin_op(int32_t reduce, double a, double b) {
+    if (reduce != GVL_TRACK_REDUCE_MAX) return __dadd_rn(a, b);
+    if (a != a) return a;  // NaN propagates
+    if (b != b) return b;
+    return b > a ? b : a;
+}
+
+// One (sub-)pass [cur, pass_end) (haplotype positions) of a tile, binned.  The CTA walks the pass in row-aligned chunks
+// of 16 output positions, T2_THREADS chunks per round (whole bins: B divides 16 * T2_THREADS), every thread calling
+// begin(j) for its chunk at output position j and then next(i, valid) for i = 0..15: the value at haplotype position
+// (RC ? L - 16 - j : j) + i.  Every thread runs the same rounds (the barriers of bins that span warps).
+template <class T, class Begin, class Next>
+__device__ __forceinline__ void t3_bin_pass(T3Smem &S, T *__restrict__ out_bins, bool rc, int32_t L, int32_t cur, int32_t pass_end,
+                                            TrkBin bn, Begin &&begin, Next &&next) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int32_t B = 1 << bn.shift;
+    const int32_t jo_lo = rc ? L - pass_end : cur, jo_hi = rc ? L - cur : pass_end;  // the pass in output positions
+    const int32_t jb = jo_lo & ~(max(B, 16) - 1);
+    const int32_t n_chunks = (jo_hi - jb + 15) >> 4;
+    const double id = bn.reduce == GVL_TRACK_REDUCE_MAX ? __longlong_as_double((long long)0xfff0000000000000ull) : 0.0;  // -inf
+    // a sub-pass that starts inside a bin continues the previous one's partial result; one that ends inside a bin leaves it
+    const bool contd = (cur & (B - 1)) != 0, open = (pass_end & (B - 1)) != 0;
+    const int32_t k_in = (rc ? L - 1 - cur : cur) >> bn.shift, k_out = (rc ? L - pass_end : pass_end - 1) >> bn.shift;
+    double *carry = reinterpret_cast<double *>(&S.bc_i64[1]);
+    const double carry_in = contd ? *carry : id;
+    if (contd && open) __syncthreads();  // (read before it is rewritten)
+    auto finish = [&](int32_t bs, double v) {  // the bin at output position bs, reduced over the pass's positions in it
+        if (bs >= jo_hi || bs + B <= jo_lo || bs + B > L) return;
+        const int32_t k = bs >> bn.shift;
+        if (contd && k == k_in) v = bin_op(bn.reduce, carry_in, v);
+        if (open && k == k_out) {
+            *carry = v;
+            return;
+        }
+        if (bn.reduce == GVL_TRACK_REDUCE_MEAN) v = __ddiv_rn(v, (double)B);
+        out_bins[k] = to_out<T>((float)v);
+    };
+    double *wpart = reinterpret_cast<double *>(S.itv);  // per-warp results (the staged intervals are no longer read)
+    const int n_rounds = (n_chunks + T2_THREADS - 1) / T2_THREADS;
+    for (int it = 0; it < n_rounds; it++) {
+        const int32_t j = jb + 16 * (it * T2_THREADS + tid);
+        const int32_t vlo = max(jo_lo - j, 0), vhi = min(jo_hi - j, 16);  // chunk values inside the pass
+        double acc = id;
+        if (vlo < vhi) {
+            begin(j);
+#pragma unroll
+            for (int i = 0; i < 16; i++) {
+                const int32_t o = rc ? 15 - i : i;  // output position j + o
+                const bool valid = o >= vlo && o < vhi;
+                const float x = next(i, valid);
+                if (valid) acc = bin_op(bn.reduce, acc, (double)x);
+                if (B < 16 && ((i + 1) & (B - 1)) == 0) {
+                    finish(rc ? j + 15 - i : j + i + 1 - B, acc);
+                    acc = id;
+                }
+            }
+        }
+        if (B >= 16) {
+            const int G = min(B >> 4, 32);  // chunks of a bin within a warp
+            for (int o = 1; o < G; o <<= 1) acc = bin_op(bn.reduce, acc, __shfl_xor_sync(0xffffffffu, acc, o));
+            if (B <= 512) {
+                if ((lane & (G - 1)) == 0) finish(j, acc);
+            } else {
+                if (lane == 0) wpart[tid >> 5] = acc;
+                __syncthreads();
+                const int W = B >> 9;  // warps of a bin
+                if (tid < (T2_THREADS / 32) / W) {
+                    double v = wpart[tid * W];
+                    for (int w = 1; w < W; w++) v = bin_op(bn.reduce, v, wpart[tid * W + w]);
+                    finish(jb + 16 * (it * T2_THREADS + tid * W * 32), v);
+                }
+                __syncthreads();
+            }
+        }
+    }
+}
+
+// t2_generic_segment, binned: the tile [h0, h1) (haplotype positions) in one pass
+template <class T>
+__device__ __noinline__ void t2_generic_bins(const TRec *__restrict__ recs, int32_t n_rec, int32_t ref0, SrcGlobal src, int strategy,
+                                             double param, T3Smem *S, T *__restrict__ out_bins, int32_t L, bool rc, int32_t h0,
+                                             int32_t h1, uint64_t base_seed, uint64_t qseed, uint64_t hap, TrkBin bn) {
+    int32_t hint = -2, hb = 0;
+    t3_bin_pass<T>(*S, out_bins, rc, L, h0, h1, bn, [&](int32_t j) { hb = rc ? L - 16 - j : j; },
+                   [&](int i, bool valid) {
+                       return valid ? t2_generic_value(recs, n_rec, ref0, src, strategy, param, hb + i, base_seed, qseed, hap, hint) : 0.0f;
+                   });
 }
 
 // =====================================================================================
@@ -492,8 +595,8 @@ struct TileCtx {
 
 // One tile.  BIG = false: everything the tile needs fits the staging (the descriptor says how much of it): one pass,
 // extents known.  BIG = true: sub-passes, each as long as the staged records / intervals reach.
-template <bool BIG, class T>
-__device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, T3Smem &S) {
+template <bool BIG, class T, bool BIN = false>
+__device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, T3Smem &S, TrkBin bn = TrkBin{0, 0}) {
     const int tid = threadIdx.x;
     const int32_t L = D.L;
     const bool rc = (D.flags & TD_RC) != 0;
@@ -632,6 +735,41 @@ __device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, 
             __syncthreads();
         }
 
+        if constexpr (BIN) {
+            // ---- binned output: chunks of 16 values on 16-position aligned ROW positions, the walk of t3_write_chunks ----
+            int32_t u_lo = 0;
+            uint32_t bits = 0u;
+            float cv = 0.0f;
+            t3_bin_pass<T>(S, out_row, rc, L, cur, pass_end, bn,
+                           [&](int32_t j) {
+                               u_lo = (rc ? (L - 16 - j) : j) - cur;
+                               const uint32_t *mk = S.mk, *mk2 = S.mk2;
+                               if (u_lo >= 0) {
+                                   const int w = u_lo >> 5;
+                                   bits = __funnelshift_r(mk[w], mk[w + 1], u_lo & 31) & 0xffffu;
+                               } else {
+                                   bits = (mk[0] << (-u_lo)) & 0xffffu;
+                               }
+                               cv = 0.0f;
+                               const int q = max(u_lo, 0) - 1;
+                               if (q >= 0) {
+                                   int w = q >> 5;
+                                   uint32_t mm = mk[w] & (0xffffffffu >> (31 - (q & 31)));
+                                   if (mm == 0u) {
+                                       int w2 = w >> 5;
+                                       uint32_t m2 = mk2[w2] & ((1u << (w & 31)) - 1u);
+                                       while (m2 == 0u) m2 = mk2[--w2];
+                                       w = 32 * w2 + 31 - __clz(m2);
+                                       mm = mk[w];
+                                   }
+                                   cv = S.val[32 * w + 31 - __clz(mm)];
+                               }
+                           },
+                           [&](int i, bool) {
+                               if ((bits >> i) & 1u) cv = S.val[u_lo + i];
+                               return cv;
+                           });
+        } else {
         // ---- output: chunks of 16 values on 16-element (float: 64-byte, 16-bit: 32-byte) aligned addresses ----
         const int32_t jo_lo = rc ? L - pass_end : cur;
         const int32_t jo_hi = rc ? L - cur : pass_end;
@@ -640,6 +778,7 @@ __device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, 
         // (the two directions are separate instantiations: the walk then writes its registers in output order)
         if (rc) t3_write_chunks<true, T>(S, out_row, j0, n_chunks, jo_lo, jo_hi, L, cur);
         else t3_write_chunks<false, T>(S, out_row, j0, n_chunks, jo_lo, jo_hi, L, cur);
+        }
         if (!BIG || pass_end >= h1) break;
 
         // ---- (rare) the tile goes on: cursors of the next sub-pass ----
@@ -687,20 +826,27 @@ __device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, 
 // (the rare sub-pass variant is kept out of line: its register needs must not weigh on the common path)
 // (it takes its context from shared memory and re-reads the descriptor: structs passed by value or reference would
 //  make every thread of EVERY tile spill them to local memory before the branch)
-template <class T>
+template <class T, bool BIN>
 __device__ __noinline__ void t3_tile_big(T3Smem *S, const TileDesc *__restrict__ dp) {
     const TileCtx<T> X = *reinterpret_cast<const TileCtx<T> *>(S->big_ctx);
     const TileDesc D = *dp;
-    __syncthreads();  // everyone holds its copy before shared memory is reused
-    t3_tile<true, T>(X, D, *S);
+    if constexpr (BIN) {
+        const TrkBin bn{S->bc_i32[0], S->bc_i32[1]};
+        __syncthreads();  // everyone holds its copy before shared memory is reused
+        t3_tile<true, T, true>(X, D, *S, bn);
+    } else {
+        __syncthreads();  // everyone holds its copy before shared memory is reused
+        t3_tile<true, T>(X, D, *S);
+    }
 }
 static_assert(sizeof(TileCtx<float>) <= 128, "TileCtx must fit T3Smem::big_ctx");
 
 // 5 CTAs per SM (48 registers, 80 bytes of spills; shared memory allows no more): the kernel is bound by the latency chain of a
 // tile, so the fifth tile in flight pays (tracks step of a 20-batch ring 63.7 -> 60.3 us) although a single 134 MB call gains little
 constexpr int T3_MIN_CTAS = 5;
-template <class T>
-__global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkExecParams P, const TileDesc *__restrict__ tdesc) {
+// BIN: the binned store (bn); the row's bins start at out + out_base / B (row offsets are multiples of B)
+template <class T, bool BIN>
+__global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkExecParams P, const TileDesc *__restrict__ tdesc, TrkBin bn) {
     __shared__ __align__(16) T3Smem S;
     const unsigned track = blockIdx.y;
     const TileDesc *dp = tdesc + ((size_t)track * (size_t)P.grid_per_track + blockIdx.x);
@@ -717,7 +863,7 @@ __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkE
         X.qseed = P.query_seed ? (uint64_t)P.query_seed[query] : (uint64_t)(sub ? (uint32_t)D.query - q_blk * sub : (uint32_t)D.query);
         X.base_seed = P.base_seed_dev ? P.base_seed_dev[q_blk] : P.base_seed;
         X.recs = P.trecs + D.rec_base;
-        X.out_row = static_cast<T *>(P.out) + D.out_base;
+        X.out_row = static_cast<T *>(P.out) + (BIN ? D.out_base >> bn.shift : D.out_base);
         X.base_elems = (int64_t)(reinterpret_cast<uintptr_t>(P.out) / sizeof(T)) + D.out_base;
         // (kernel parameters are indexed with a compile-time subscript: a run-time one would copy them to local memory)
         const TrkDesc *Td = Tp;
@@ -738,14 +884,21 @@ __global__ void __launch_bounds__(T2_THREADS, T3_MIN_CTAS) trk_exec3_kernel(TrkE
         const int32_t L = D.L;
         const bool rc = (D.flags & TD_RC) != 0;
         const int32_t t0 = rc ? L - D.h1 : D.h0, t1 = rc ? L - D.h0 : D.h1;
-        t2_generic_segment(X.recs, D.n_rec, D.ref0, X.srcg, X.strategy, X.param, X.out_row, L, rc, t0, t1, X.base_seed, X.qseed, X.hap);
+        if constexpr (BIN)
+            t2_generic_bins(X.recs, D.n_rec, D.ref0, X.srcg, X.strategy, X.param, &S, X.out_row, L, rc, D.h0, D.h1, X.base_seed, X.qseed,
+                            X.hap, bn);
+        else
+            t2_generic_segment(X.recs, D.n_rec, D.ref0, X.srcg, X.strategy, X.param, X.out_row, L, rc, t0, t1, X.base_seed, X.qseed, X.hap);
         return;
     }
     if (D.flags & TD_BIG) {
-        if (threadIdx.x == 0) *reinterpret_cast<TileCtx<T> *>(S.big_ctx) = X;
+        if (threadIdx.x == 0) {
+            *reinterpret_cast<TileCtx<T> *>(S.big_ctx) = X;
+            if constexpr (BIN) S.bc_i32[0] = bn.shift, S.bc_i32[1] = bn.reduce;
+        }
         __syncthreads();
-        t3_tile_big<T>(&S, dp);
+        t3_tile_big<T, BIN>(&S, dp);
     } else {
-        t3_tile<false, T>(X, D, S);
+        t3_tile<false, T, BIN>(X, D, S, bn);
     }
 }

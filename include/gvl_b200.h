@@ -197,6 +197,22 @@ int gvl_dev_get_diffs_sparse(gvl_ctx *ctx, const gvl_sparse_tables *tab, const i
 #define GVL_TRACK_BF16 1
 #define GVL_TRACK_F16 2
 
+/* Binned track output (gvl_dev_realign_tracks_exec_binned, gvl_dev_paint_tracks_binned, gvl_fixed_job.track_bin): every
+ * row is cut into bins of `bin` output positions (a power of two, 2..GVL_TRACK_BIN_MAX; 0 or 1 = unbinned) and one value
+ * per bin is stored: bin k of a row covers its output positions [k*bin, (k+1)*bin), so a reversed row's bins are its
+ * forward bins reversed.  Row lengths and row offsets (out_offsets, row_dst, row_tstride) stay in unbinned positions and
+ * must be multiples of `bin`: a row whose values start at element o of the unbinned layout has its bins at o / bin, and
+ * `out` holds n_tracks * total_per_track / bin elements.  The reduction runs on the float32 values:
+ *   SUM   the bin's values summed in float64, rounded to float32, then narrowed to the dtype like every value;
+ *   MEAN  that float64 sum divided by bin in float64, with the same roundings;
+ *   MAX   the largest value, narrowed.
+ * A NaN in the bin makes it NaN for all three.  The float64 order is fixed by the row alone, so a row's bins have the same
+ * bits in every call.  An unknown bin or reduction is GVL_ERR_ARG before any launch. */
+#define GVL_TRACK_REDUCE_MEAN 0
+#define GVL_TRACK_REDUCE_SUM 1
+#define GVL_TRACK_REDUCE_MAX 2
+#define GVL_TRACK_BIN_MAX 4096
+
 /* Where the rows of a track call land in `out` (n_tracks * total_per_track elements).  Row k (= q*p + h; p = 1 when
  * painting) has out_offsets[k+1] - out_offsets[k] values, written reversed on masked rows in every layout. */
 #define GVL_TRACK_LAYOUT_TBP 0  /* track-major (t, b, p, ~l): the reference's flat buffer (_reconstruct.py:238); row k of
@@ -258,6 +274,8 @@ int gvl_dev_realign_tracks(gvl_ctx *ctx, const gvl_sparse_tables *tab, const gvl
  * GVL_ERR_ARG) into `out` (device, n_tracks * total_per_track elements, 16-byte aligned).  Writes nothing after an empty or
  * rejected plan. */
 int gvl_dev_realign_tracks_exec(gvl_ctx *ctx, void *out, int32_t dtype, gvl_stream stream);
+/* The same launch with a binned store (GVL_TRACK_REDUCE_*): `out` holds n_tracks * total_per_track / bin elements. */
+int gvl_dev_realign_tracks_exec_binned(gvl_ctx *ctx, void *out, int32_t dtype, int32_t bin, int32_t reduce, gvl_stream stream);
 
 /* shift_and_realign_tracks_sparse (src/ffi/mod.rs:2439-2458) and shift_and_realign_tracks_from_svar2
  * (src/tracks/mod.rs:705-856) on device: ONE track whose source is a dense f32 window per query (`tracks` ragged by
@@ -282,6 +300,11 @@ int gvl_dev_paint_tracks(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *it
                          const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
                          const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride, void *out,
                          int32_t dtype, gvl_stream stream);
+/* gvl_dev_paint_tracks with a binned store (GVL_TRACK_REDUCE_*): `out` holds n_tracks * total_per_track / bin elements. */
+int gvl_dev_paint_tracks_binned(gvl_ctx *ctx, int64_t n_tracks, const gvl_intervals *itv, const int64_t *offset_idxs,
+                                const int32_t *starts, int64_t n_queries, const int64_t *out_offsets, int64_t total_per_track,
+                                const uint8_t *to_rc, int32_t layout, const int64_t *row_dst, const int64_t *row_tstride,
+                                void *out, int32_t dtype, int32_t bin, int32_t reduce, gvl_stream stream);
 
 /* The stored intervals of one slot over one window per row (the "intervals" kind of Dataset.with_tracks).  tracks is a
  * HOST array of n_tracks (<= 64) descriptors; row k (device arrays of n_rows entries) reads slot row_slot[k] of track
@@ -422,12 +445,14 @@ typedef struct gvl_fixed_job {
     int32_t rc_neg;                   /* reverse(-complement) rows of negative-strand regions */
     uint8_t pad_char;
     int32_t track_dtype;              /* GVL_TRACK_* element type of `trk` (0 = float32) */
+    int32_t track_bin, track_reduce;  /* binned tracks (0 = unbinned; output_length must be a multiple of track_bin) */
 } gvl_fixed_job;
 /* batch prep + variant plan (+ track plan and tile prep) of `n` queries; sub_batch as in gvl_dev_batch_prep. */
 int gvl_dev_fixed_plan(gvl_ctx *ctx, const gvl_fixed_job *job, const int64_t *ds_idx, const int32_t *jitter, int64_t n,
                        int64_t sub_batch, gvl_stream stream);
 /* the bandwidth-bound launches of the batch planned last on `ctx`: seq u8[n*rows_p*L (*4 one-hot)], annot_* i32[n*rows_p*L]
- * (GVL_MODE_ANNOTATED), trk [n*n_tracks*(ploidy|1)*L] elements of job->track_dtype in (b, t, p, L) / (b, t, L) order.
+ * (GVL_MODE_ANNOTATED), trk [n*n_tracks*(ploidy|1)*L] elements of job->track_dtype in (b, t, p, L) / (b, t, L) order
+ * (binned: L / track_bin per row).
  * Unused outputs NULL. */
 int gvl_dev_fixed_exec(gvl_ctx *ctx, const gvl_fixed_job *job, int64_t n, uint8_t *seq, int32_t *annot_v, int32_t *annot_pos,
                        void *trk, gvl_stream stream);
