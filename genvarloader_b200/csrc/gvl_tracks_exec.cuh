@@ -696,7 +696,9 @@ __device__ __forceinline__ void t3_tile(const TileCtx<T> &X, const TileDesc &D, 
             const int32_t e = (int32_t)imax64(imin64((int64_t)ie[q] - q_start, track_n), 0);
             if (e <= s || e <= src_lo || s >= src_hi) continue;  // empty after clipping, behind the sub-pass, beyond it
             if (s > src_lo) place(s, iv[q]);  // (an interval that covers the first position is the start marker's)
-            const bool adjacent = (k + 1 < cnt) && ((int64_t)S.its[k + 1] - q_start == (int64_t)e);  // the next interval starts right there
+            // the next interval starts right there -- unless there is the window's end: the next one is clipped away and
+            // the positions past the window read 0 (src/tracks/mod.rs:381-404)
+            const bool adjacent = e < track_n && (k + 1 < cnt) && ((int64_t)S.its[k + 1] - q_start == (int64_t)e);
             if (!adjacent && e < src_hi) place(e, 0.0f);
         }
         // ---- markers: records (threads from the top of the CTA) + the first position ----

@@ -654,15 +654,20 @@ GVL_API uint64_t gvl_oracle_hash4(uint64_t a, uint64_t b, uint64_t c, uint64_t d
 
 enum { REPEAT_5P = 0, REPEAT_5P_NORM = 1, CONSTANT = 2, FLANK_SAMPLE = 3, INTERPOLATE = 4 }; /* :15-19 */
 
+/* A track value at relative source position i of a window of n values.  Positions outside the window are out of
+ * the reference's contract (a slice index past the track panics, src/tracks/mod.rs:102-188, :317-404); they read 0
+ * here, as past the end of a row (:400-404) and as the track kernels do. */
+static inline float trk_at(const float *track, int64_t n, int64_t i) { return (i >= 0 && i < n) ? track[i] : 0.0f; }
+
 /* `double` arithmetic below must not be contracted into FMAs: build with -ffp-contract=off. */
 static void apply_insertion_fill(float *out, int64_t out_idx, int64_t writable_length, int64_t v_len,
                                  const float *track, int64_t track_len, int64_t v_rel_pos, int64_t strategy_id,
                                  const double *params, uint64_t base_seed, uint64_t query, uint64_t hap) {
     if (strategy_id == REPEAT_5P) { /* :102-108 */
-        float val = track[v_rel_pos];
+        float val = trk_at(track, track_len, v_rel_pos);
         for (int64_t i = 0; i < writable_length; i++) out[out_idx + i] = val;
     } else if (strategy_id == REPEAT_5P_NORM) { /* :109-118 f32 / f32 */
-        float val = track[v_rel_pos] / (float)v_len;
+        float val = trk_at(track, track_len, v_rel_pos) / (float)v_len;
         for (int64_t i = 0; i < writable_length; i++) out[out_idx + i] = val;
     } else if (strategy_id == CONSTANT) { /* :119-124 */
         float val = (float)params[0];
@@ -675,7 +680,7 @@ static void apply_insertion_fill(float *out, int64_t out_idx, int64_t writable_l
         for (int64_t i = 0; i < writable_length; i++) {
             uint64_t seed = gvl_oracle_hash4(base_seed, query, hap, (uint64_t)(out_idx + i));
             int64_t offset = (int64_t)(seed % pool_size);
-            out[out_idx + i] = track[pool_lo + offset];
+            out[out_idx + i] = trk_at(track, track_len, pool_lo + offset);
         }
     } else if (strategy_id == INTERPOLATE) { /* :138-188 */
         int64_t order = (int64_t)params[0];
@@ -685,12 +690,12 @@ static void apply_insertion_fill(float *out, int64_t out_idx, int64_t writable_l
         for (int64_t j = 0; j < k; j++) { /* 5' side :153-157 */
             int64_t ri = i64max(v_rel_pos - j, 0);
             xs[j] = -(double)j;
-            ys[j] = (double)track[ri];
+            ys[j] = (double)trk_at(track, track_len, ri);
         }
         for (int64_t j = 0; j < k; j++) { /* 3' side :160-164 */
             int64_t ri = i64min(v_rel_pos + 1 + j, track_len - 1);
             xs[k + j] = (double)v_len + (double)j;
-            ys[k + j] = (double)track[ri];
+            ys[k + j] = (double)trk_at(track, track_len, ri);
         }
         for (int64_t i = 0; i < writable_length; i++) { /* :168-188 */
             double x = (double)i;
@@ -718,7 +723,7 @@ static void shift_and_realign_track_core(int64_t n_variants, gvl_provide_track_f
                                          float *out, int64_t length, const double *params, const uint8_t *keep,
                                          int64_t strategy_id, uint64_t base_seed, uint64_t query, uint64_t hap) {
     if (n_variants == 0) { /* :240-246 */
-        for (int64_t i = 0; i < length; i++) out[i] = track[i];
+        for (int64_t i = 0; i < length; i++) out[i] = trk_at(track, track_n, i);
         return;
     }
     int64_t track_idx = 0, out_idx = 0, shifted = 0; /* :249-251 */
@@ -755,14 +760,14 @@ static void shift_and_realign_track_core(int64_t n_variants, gvl_provide_track_f
         if (v_diff == 0) continue; /* :312-314 SNPs match the reference track */
         int64_t track_len = v_rel_pos - track_idx;   /* :317 */
         if (out_idx + track_len >= length) break;    /* :319-321 */
-        for (int64_t i = 0; i < track_len; i++) out[out_idx + i] = track[track_idx + i];
+        for (int64_t i = 0; i < track_len; i++) out[out_idx + i] = trk_at(track, track_n, track_idx + i);
         out_idx += track_len;
         int64_t writable_length = i64min(v_len, length - out_idx); /* :329 */
         if (v_diff > 0 && strategy_id != REPEAT_5P) {              /* :333-346 */
             apply_insertion_fill(out, out_idx, writable_length, v_len, track, track_n, v_rel_pos, strategy_id,
                                  params, base_seed, query, hap);
         } else { /* :347-354 */
-            float val = track[v_rel_pos];
+            float val = trk_at(track, track_n, v_rel_pos);
             for (int64_t i = 0; i < writable_length; i++) out[out_idx + i] = val;
         }
         out_idx += writable_length;
