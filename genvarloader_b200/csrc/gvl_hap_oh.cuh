@@ -8,7 +8,8 @@
 //     whatever the indel shift of the row is;
 //   * reverse-complement of the 8 positions (src/reverse.rs:45-69) is ONE bit reversal (brev): reversing the nibble
 //     order reverses the positions, reversing the bits inside a nibble swaps A<->T and C<->G;
-//   * a 256-entry shared-memory table maps a byte (2 codes) to its 8 one-hot bytes: 4 lookups per lane;
+//   * a 256-entry shared-memory table maps a byte (2 codes) to its 8 one-hot bytes: 4 lookups per lane, at swizzled
+//     indices so that the bytes of A/C/G/T fall into distinct banks (oh_swizzle);
 //   * the lane's 32 output bytes leave with one 256-bit store (STG.256): a warp writes 1 KiB per instruction.
 // Groups of 256 positions that are plain reference (the common case) take exactly that path; groups that contain
 // a variant, a pad or a tile edge classify every lane on its own, and only the lanes that straddle a record edge
@@ -27,7 +28,12 @@ constexpr int OH_GROUP = 256;                                  // positions per 
 constexpr int OH_MAX_TILE_WANTED = 32768;                      // haplotype positions per CTA, at most
 
 constexpr int OH_THREADS = 128;                                // threads per CTA of the packed kernel
+// 4-warp CTAs per SM the register budget is sized for (64 registers at 8, 72 at 6).  The unroll-4 kernel of long sparse rows
+// runs faster at 6 (cfg3: 384 -> 380 us per 32-batch launch; 5 CTAs: 414 us, 10 CTAs at 48 registers: 425 us), the unroll-2
+// kernel of dense rows needs the 8 to hide its record lookups (cfg2d at 6: 994 us per launch against 877 us for the kernel
+// before the swizzle, in one call) -- profiles/r3_oh_swizzle.md
 constexpr int OH_MIN_CTAS = 8;
+constexpr int OH_MIN_CTAS_LONG = 6;
 // one thread per group builds the group table: a pass may not touch more groups than the CTA has threads
 constexpr int OH_MAX_TILE = OH_MAX_TILE_WANTED < (OH_THREADS - 2) * OH_GROUP ? OH_MAX_TILE_WANTED : (OH_THREADS - 2) * OH_GROUP / 1024 * 1024;
 constexpr int OH_MAX_GROUPS = OH_MAX_TILE / OH_GROUP + 2;      // groups a pass can touch (+ misaligned edges)
@@ -65,6 +71,16 @@ __global__ void __launch_bounds__(256) pack_ref_kernel(const uint8_t *__restrict
         }
         out[w] = v;
     }
+}
+
+// Index of the one-hot table entry of each byte of x (two codes per byte; bytes are independent).  The 8-byte entries sit
+// in 16 bank pairs, entry i in pair i mod 16, and the low code of an ACGT byte takes only 4 values (1, 2, 4, 8): with the
+// byte as index, the 16 ACGT x ACGT bytes share 4 bank pairs and a warp's lookup of random sequence replays to ~7
+// shared-memory wavefronts.  XOR-ing bits of the high code into the low nibble puts those 16 bytes into 16 distinct bank
+// pairs (2 wavefronts, the minimum for 32 lanes x 8 bytes).  A bijection on 0..255: the high nibble is kept, and for a
+// fixed high nibble the low one maps by a triangular XOR (bit 0 ^= bit 3; bits 1..3 ^= bits of the high nibble).
+__host__ __device__ __forceinline__ uint32_t oh_swizzle(uint32_t x) {
+    return x ^ ((x >> 3) & 0x0F0F0F0Fu) ^ ((x >> 4) & 0x0E0E0E0Eu);
 }
 
 __device__ __forceinline__ uint2 lds_u64(uint32_t addr) {
@@ -182,7 +198,7 @@ __device__ __forceinline__ int oh_classify(const OhRecs &S, int il, int32_t p_lo
 // NT = threads per CTA: 128, or 64 for rows of at most 8,192 positions (one tile per row: twelve 2-warp CTAs per SM keep more
 // rows in flight against the ~3.3 us of fixed latency per CTA than eight 4-warp ones -- cfg4: 551 -> 479 us per 20 batches).
 template <int OH_UNROLL, int NT>
-__global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_kernel(HapExecParams P) {
+__global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_UNROLL == OH_UNROLL_LONG ? OH_MIN_CTAS_LONG : OH_MIN_CTAS) hap_exec_oh_kernel(HapExecParams P) {
     constexpr int EDGE_ROUNDS = (2 * REC_CAP + 2 + NT - 1) / NT;  // edge slots per thread and pass
     __shared__ OhRecs S;
     __shared__ __align__(16) uint2 s_lut[256];         // byte (2 codes) -> 8 one-hot bytes
@@ -238,9 +254,10 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
             if (b_hi > b_lo) asm volatile("prefetch.global.L2 [%0];" ::"l"(base + (line << 7)));
     }
 
-    // spread(n): byte c = bit c of the 4-bit code n   (n * 0x204081 puts bit c at bit 8c, no carries)
+    // spread(n): byte c = bit c of the 4-bit code n   (n * 0x204081 puts bit c at bit 8c, no carries); entry of byte i at
+    // oh_swizzle(i) (a bijection on bytes)
     for (int i = tid; i < 256; i += NT)
-        s_lut[i] = make_uint2(((i & 15) * 0x204081u) & 0x01010101u, ((i >> 4) * 0x204081u) & 0x01010101u);
+        s_lut[oh_swizzle(i)] = make_uint2(((i & 15) * 0x204081u) & 0x01010101u, ((i >> 4) * 0x204081u) & 0x01010101u);
 
     const int32_t *__restrict__ ra = P.rec.a + rp.rec_off;
     if (!P.dir && warp == 0) {
@@ -288,6 +305,7 @@ __global__ void __launch_bounds__(NT, NT == 64 ? 12 : OH_MIN_CTAS) hap_exec_oh_k
 
     // common epilogue of a full unit: 8 codes (output order) -> 32 one-hot bytes, one 256-bit store
     auto emit8 = [&](uint8_t *dst, uint32_t v) {
+        v = oh_swizzle(v);  // each byte to its table index
         const char *lut = reinterpret_cast<const char *>(s_lut);  // (a link-time constant: folds into the LDS offset)
         const uint2 o0 = *reinterpret_cast<const uint2 *>(lut + ((v << 3) & 0x7f8u));
         const uint2 o1 = *reinterpret_cast<const uint2 *>(lut + ((v >> 5) & 0x7f8u));
